@@ -9,6 +9,7 @@ F = 128 fp32).  With --gpus N the same step is sharded over N ranks (strong scal
 the row<->slab exchange inside our kernels over NVLink peer memory by default (--partition, DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload mag_regcn]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout from rank 0.  `--impl reference` times the CPU restatement of the reference
 (oracle/regnn_oracle.py; DGL itself cannot be installed) on the box's host cores.
@@ -46,7 +47,16 @@ def parse():
     ap.add_argument('--no-others', action='store_true', help='skip the secondary HGB-shaped workloads')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='multi-GPU: run the step eagerly instead of replaying a CUDA graph')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed to DIR/<name>.npy (float32): y and d_x '
+                         '(the output and the feature gradient, on a fixed seeded sample of rows) and d_theta (the '
+                         'relation-embedding gradient, whole); single GPU, --workload mag_regcn, --impl ours')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload != 'mag_regcn'):
+        ap.error('--dump-outputs covers the default workload only (--workload mag_regcn --impl ours)')
+    return args
 
 
 def peaks():
@@ -102,6 +112,17 @@ class ClockSampler(threading.Thread):
         self.join(timeout=2)
         med = float(np.median(self.samples)) if self.samples else None
         return {'sm_mhz': med, 'sm_max_mhz': self.max_mhz, 'reasons': sorted(self.reasons)}
+
+
+def dump_outputs(path, y, dx, d_theta):
+    """Writes one step's results for output-for-output comparison of two builds: ``y`` and ``d_x`` on the same seeded
+    sample of rows (at most 16 MB each), ``d_theta`` whole, all float32."""
+    n, f = y.shape
+    rows = np.sort(np.random.RandomState(0).choice(n, min(n, (16 << 20) // (4 * f)), replace=False))
+    idx = torch.as_tensor(rows, device=y.device)
+    os.makedirs(path, exist_ok=True)
+    for name, t in (('y', y[idx]), ('d_x', dx[idx]), ('d_theta', d_theta)):
+        np.save(os.path.join(path, name + '.npy'), t.detach().float().cpu().numpy())
 
 
 def theta_init(r, w, seed=0):
@@ -441,6 +462,8 @@ def run_ours(args, d):
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
+    if args.dump_outputs and world > 1:
+        raise SystemExit('bench.py: --dump-outputs runs on one GPU')
     assert torch.cuda.is_available(), 'bench.py needs a CUDA device (no CPU fallback)'
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)
@@ -469,11 +492,15 @@ def run_ours(args, d):
         args.partition = 'none'
         x = x_full.clone().requires_grad_(True)
         gout = g_full
+        last = {}     # --dump-outputs: the output of the latest step; x.grad and theta.grad hold its gradients
 
         def step():
             x.grad = theta.grad = None
             nrm = RF.weighted_degree_norm(g, etv, theta, ALPHA, -0.5)
-            RF.propagate(g, etv, x, theta, ALPHA, nrm).backward(gout)
+            y = RF.propagate(g, etv, x, theta, ALPHA, nrm)
+            y.backward(gout)
+            if args.dump_outputs:   # kept only then: otherwise Y is freed before the next step, as a caller would
+                last['y'] = y
     else:
         bounds = partition.row_blocks(csr['indptr'], world, balance='edges' if args.partition == 'edges' else 'rows')
         rb, re = bounds[rank], bounds[rank + 1]
@@ -569,6 +596,8 @@ def run_ours(args, d):
     total = timed(timed_step, args.steps, args.warmup, sync, barrier)
     launches = launches_per_step * args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last['y'], x.grad, theta.grad)
     # ---- per-phase device timeline of a few extra (eager) steps: CUDA events around every ABI call, barrier and
     # collective (re_gnn_b200._lib.Trace); max over ranks per phase
     with _lib.Trace() as tr:

@@ -2,7 +2,7 @@
 parity checked) where the reference checkout is absent.  Same constructor arguments, sub-module /
 parameter names and forward conventions as model/REGCN.py:6-46, model/REGAT.py:6-66,
 model/REMixHop.py:19-101 and model/REGIN.py:35-84; the reference's own files also run unmodified on
-``re_gnn_b200.layer`` (tests/test_layers_host.py)."""
+``re_gnn_b200.layer`` (tests/test_layers_host.py, run with REGNN_REFERENCE set to a reference checkout)."""
 import torch
 from torch import nn
 

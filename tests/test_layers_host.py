@@ -15,7 +15,7 @@ from re_gnn_b200 import Graph
 
 LAYER_CASES = [c for c in helpers.golden_cases() if not c.startswith('model_')]
 MODEL_CASES = helpers.golden_cases('model_')
-REF = os.environ.get('REGNN_REFERENCE', '/root/reference')
+REF = os.environ.get('REGNN_REFERENCE', '')   # a checkout of the reference RE-GNN repository, if one is at hand
 
 
 def run_layer_case(case, device='cpu', dtype=torch.float64):
@@ -97,7 +97,8 @@ def test_product_path_has_no_cpu_fallback():
         conv(g, torch.randn(2, 4), torch.tensor([1, 2]))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'model')), reason='reference checkout not present')
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, 'model')),
+                    reason='needs REGNN_REFERENCE set to a checkout of the reference RE-GNN repository')
 @pytest.mark.parametrize('name', MODEL_CASES)
 def test_reference_models_run_unmodified_on_our_layers(name, cpu_ops, monkeypatch):
     """model/REGCN.py, REGAT.py, REMixHop.py, REGIN.py imported from the reference, with OUR package registered
