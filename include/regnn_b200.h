@@ -207,6 +207,17 @@ typedef struct regnn_peer_rows {
 int regnn_rows_to_slabs(const float* X, int64_t ldx, int64_t num_rows, int feat, int num_ranks, int64_t row_offset,
                         float* const* peer_slabs /* device array [num_ranks] */, void* stream);
 
+/* Halo exchange of destination-row blocks (partition.halo_propagate; it replaces the all-gather of the whole [N, F]
+ * matrix that partition.partitioned_propagate does per direction): for every peer q, the rows
+ * X[send_rows[send_ptr[q] .. send_ptr[q+1])] of this rank's row block are stored to
+ * peer_bufs[q] + (recv_offset[q] + i) * ldb, i = 0, 1, ...  send_ptr [num_ranks+1] and recv_offset [num_ranks] are HOST
+ * arrays (set up once per partition); send_rows (int32, local row ids) and peer_bufs [num_ranks] are device arrays; lists
+ * may be empty.  The pointers need not be peer-mapped: P local buffers work the same.  feat % 4 == 0, 16-byte aligned
+ * rows, num_ranks <= REGNN_HALO_MAX_RANKS. */
+#define REGNN_HALO_MAX_RANKS 64
+int regnn_halo_push(const float* X, int64_t ldx, int feat, const int32_t* send_rows, const int64_t* send_ptr,
+                    const int64_t* recv_offset, float* const* peer_bufs, int64_t ldb, int num_ranks, int rank, void* stream);
+
 /* The reverse re-partition for kernels without a scatter epilogue (the fused attention kernels, one head slice per
  * rank): S [num_rows, feat] is this rank's column slab (ld lds); row v is stored to
  * peers->base[v / rows_per_rank][(v % rows_per_rank) * ld + col_offset .. + feat). */

@@ -160,6 +160,33 @@ __global__ void rows_to_slabs_kernel(const float* __restrict__ X, int64_t ldx, i
   }
 }
 
+// Indexed row push of the halo exchange (destination-row blocks that exchange only the rows a peer's edges reference):
+// the rows send_rows[ptr[q] .. ptr[q+1]) of this rank's block go to consecutive rows of peer q's halo buffer, from row
+// recv_offset[q] on.  One group of G lanes per row (G = the row's 128-bit chunks rounded up to a power of two, at most
+// 32): the row index is loaded once, then the group streams the row with 128-bit reads and one contiguous store burst.
+// Peers in rank-rotated order as in rows_to_slabs_kernel.  The small per-peer tables travel as a kernel parameter.
+struct HaloPeers {
+  int64_t ptr[REGNN_HALO_MAX_RANKS + 1];
+  int64_t recv_offset[REGNN_HALO_MAX_RANKS];
+};
+
+__global__ void halo_push_kernel(const float* __restrict__ X, int64_t ldx, int L, int G,
+                                 const int32_t* __restrict__ send_rows, const __grid_constant__ HaloPeers hp,
+                                 float* const* __restrict__ peer_bufs, int64_t ldb, int first_peer) {
+  const int q = (int)((blockIdx.y + (unsigned)first_peer) % gridDim.y);
+  const int64_t begin = hp.ptr[q];
+  const int64_t cnt = hp.ptr[q + 1] - begin;
+  if (cnt == 0) return;
+  float* dst = peer_bufs[q] + hp.recv_offset[q] * ldb;
+  const int lane = threadIdx.x % G;
+  const int64_t groups = (int64_t)gridDim.x * (blockDim.x / G);
+  for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G; i < cnt; i += groups) {
+    const float* src = X + (int64_t)__ldg(send_rows + begin + i) * ldx;
+    float* out = dst + i * ldb;
+    for (int c = lane; c < L; c += G) st4(out + 4 * c, ldg4_stream(src + 4 * c));
+  }
+}
+
 // Column slab -> row blocks over peer memory, for the kernels that have no scatter epilogue of their own (the fused
 // attention kernels: one head slice per rank): rows [q*per, (q+1)*per) of this rank's slab S [N, Fc] go to rank q's row
 // block at column col_offset.  The local read is contiguous, every destination row gets one Fc*4-byte store burst
@@ -1484,6 +1511,40 @@ extern "C" int regnn_rows_to_slabs(const float* X, int64_t ldx, int64_t num_rows
   rows_to_slabs_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(X, ldx, num_rows, Fc, row_offset,
                                                                                      peer_slabs, first_peer);
   return check_launch("regnn_rows_to_slabs");
+}
+
+extern "C" int regnn_halo_push(const float* X, int64_t ldx, int feat, const int32_t* send_rows, const int64_t* send_ptr,
+                               const int64_t* recv_offset, float* const* peer_bufs, int64_t ldb, int num_ranks, int rank,
+                               void* stream) {
+  REGNN_REQUIRE(X && send_ptr && recv_offset && peer_bufs && num_ranks >= 1 && rank >= 0 && rank < num_ranks,
+                REGNN_ERR_INVALID_ARG, "halo_push: bad argument");
+  REGNN_REQUIRE(num_ranks <= REGNN_HALO_MAX_RANKS, REGNN_ERR_UNSUPPORTED_SHAPE, "halo_push: %d ranks (max %d)", num_ranks,
+                REGNN_HALO_MAX_RANKS);
+  REGNN_REQUIRE(feat >= 4 && feat % 4 == 0 && ldx >= feat && ldb >= feat && ldx % 4 == 0 && ldb % 4 == 0 &&
+                    aligned_to(X, 16),
+                REGNN_ERR_UNSUPPORTED_SHAPE, "halo_push: F=%d must be whole 128-bit chunks in 16-byte aligned rows", feat);
+  HaloPeers hp;
+  int64_t most = 0;
+  hp.ptr[0] = send_ptr[0];
+  REGNN_REQUIRE(send_ptr[0] >= 0, REGNN_ERR_INVALID_ARG, "halo_push: negative send offset");
+  for (int q = 0; q < num_ranks; ++q) {
+    const int64_t cnt = send_ptr[q + 1] - send_ptr[q];
+    REGNN_REQUIRE(cnt >= 0 && recv_offset[q] >= 0, REGNN_ERR_INVALID_ARG,
+                  "halo_push: peer %d has a negative row count or receive offset", q);
+    hp.ptr[q + 1] = send_ptr[q + 1];
+    hp.recv_offset[q] = recv_offset[q];
+    most = cnt > most ? cnt : most;
+  }
+  if (most == 0) return REGNN_OK;
+  REGNN_REQUIRE(send_rows != nullptr, REGNN_ERR_INVALID_ARG, "halo_push: null send list");
+  const int L = feat / 4;
+  int G = 1;
+  while (G < L && G < 32) G <<= 1;
+  const int64_t want = (most * G + 255) / 256;
+  const unsigned bx = (unsigned)(want < 148 * 8 ? want : 148 * 8);
+  halo_push_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(X, ldx, L, G, send_rows, hp,
+                                                                                  peer_bufs, ldb, rank);
+  return check_launch("regnn_halo_push");
 }
 
 extern "C" int regnn_slabs_to_rows(const float* S, int64_t lds, int64_t num_rows, int feat,

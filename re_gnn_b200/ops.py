@@ -34,15 +34,17 @@ def _rows(rows, n):
 
 def wdeg_norm_fwd(csr, et_csr, theta, alpha, exponent, rows=None, counts=None, clamp_min=1.0):
     """deg[v] = sum_in w[etype], norm = max(deg,1)^exponent -> (deg[N], norm[N]).
-    ``counts``: the per-(row, relation) in-edge counts of this e_feat (Graph.etype_views()[2])."""
+    ``counts``: the per-(row, relation) in-edge counts of this e_feat (Graph.etype_views()[2]); with counts, ``csr``
+    may be None (the table's rows are the rows)."""
     theta = _f32(theta).view(-1)
-    n = csr['indptr'].numel() - 1
+    n = csr['indptr'].numel() - 1 if csr is not None else counts.numel() // theta.numel()
     rb, re = _rows(rows, n)
     deg = torch.empty(n, dtype=torch.float32, device=theta.device)
     norm = torch.empty(n, dtype=torch.float32, device=theta.device)
     with torch.cuda.device(theta.device):
-        _lib.call('regnn_wdeg_norm_fwd', _ptr(csr['indptr']), _ptr(et_csr), _ptr(counts), _ptr(theta), float(alpha),
-                  theta.numel(), float(exponent), float(clamp_min), rb, re, _ptr(deg), _ptr(norm), _stream())
+        _lib.call('regnn_wdeg_norm_fwd', _ptr(csr['indptr'] if csr is not None else None), _ptr(et_csr), _ptr(counts),
+                  _ptr(theta), float(alpha), theta.numel(), float(exponent), float(clamp_min), rb, re, _ptr(deg),
+                  _ptr(norm), _stream())
         _lib.count_launches(1)
     return deg, norm
 
@@ -50,15 +52,15 @@ def wdeg_norm_fwd(csr, et_csr, theta, alpha, exponent, rows=None, counts=None, c
 def wdeg_norm_bwd(csr, et_csr, theta, alpha, exponent, deg, d_norm, rows=None, counts=None, clamp_min=1.0):
     theta = _f32(theta).view(-1)
     d_norm = _f32(d_norm)
-    n = csr['indptr'].numel() - 1
-    rb, re = _rows(rows, n)
     r = theta.numel()
+    n = csr['indptr'].numel() - 1 if csr is not None else counts.numel() // r
+    rb, re = _rows(rows, n)
     partials = torch.empty(_lib.partial_blocks(re - rb) * r, dtype=torch.float64, device=theta.device)
     d_theta = torch.empty(r, dtype=torch.float32, device=theta.device)
     with torch.cuda.device(theta.device):
-        _lib.call('regnn_wdeg_norm_bwd', _ptr(csr['indptr']), _ptr(et_csr), _ptr(counts), _ptr(theta), float(alpha), r,
-                  float(exponent), float(clamp_min), rb, re, _ptr(deg), _ptr(d_norm), _ptr(partials), _ptr(d_theta),
-                  _stream())
+        _lib.call('regnn_wdeg_norm_bwd', _ptr(csr['indptr'] if csr is not None else None), _ptr(et_csr), _ptr(counts),
+                  _ptr(theta), float(alpha), r, float(exponent), float(clamp_min), rb, re, _ptr(deg), _ptr(d_norm),
+                  _ptr(partials), _ptr(d_theta), _stream())
         _lib.count_launches(2)
     return d_theta
 
@@ -207,6 +209,20 @@ def rows_to_slabs(x_own, num_ranks, row_offset, peer_slab_ptrs):
         _lib.call('regnn_rows_to_slabs', _ptr(x_own), x_own.stride(0), x_own.shape[0], x_own.shape[1], int(num_ranks),
                   int(row_offset), _ptr(peer_slab_ptrs), _stream())
         _lib.count_launches(1)
+
+
+def halo_push(x_own, send_rows, send_ptr, recv_offset, peer_buf_ptrs, ldb, rank):
+    """Stores rows ``x_own[send_rows[send_ptr[q]:send_ptr[q+1]]]`` to rows ``recv_offset[q], ...`` of peer q's halo buffer
+    (regnn_halo_push).  ``send_rows``: int32 device tensor of local row ids; ``send_ptr`` [P+1] / ``recv_offset`` [P]:
+    host sequences of ints; ``peer_buf_ptrs``: int64 device tensor [P] of buffer base addresses (leading dimension
+    ``ldb`` floats)."""
+    x_own = _f32(x_own)
+    p = len(recv_offset)
+    with torch.cuda.device(x_own.device):
+        _lib.call('regnn_halo_push', _ptr(x_own), x_own.stride(0), x_own.shape[1], _ptr(send_rows),
+                  (ctypes.c_int64 * (p + 1))(*send_ptr), (ctypes.c_int64 * p)(*recv_offset), _ptr(peer_buf_ptrs),
+                  int(ldb), p, int(rank), _stream())
+        _lib.count_launches(1 if send_ptr[-1] > send_ptr[0] else 0)
 
 
 def slabs_to_rows(slab, num_rows, peers):

@@ -17,6 +17,11 @@ relation-degree norm for all rows; the caller sums the R-float relation gradient
      blocks into the peers' slabs, the ``regnn_spmm_*_scatter`` epilogues store finished rows into their owners'
      row blocks; torch symmetric memory supplies the mapped buffers and the device-side barrier.
    The norm gradient's row dots span all columns, but the row owner has complete rows: ``d_norm`` is a local pass.
+3. ``halo_propagate`` -- destination-row blocks that exchange only their **halo** (the remote rows their edges
+   reference) and hold only local views (``HaloPartition``): every rank gathers E/P edges at the full row width.  The
+   degree norm is computed inside from a local relation-count table (halo rows get their owner's bits); the exchange is
+   one uneven all-to-all (``exchange=None``) or ``regnn_halo_push`` over peer memory (``exchange=HaloExchange(...)``).
+   It pays off on graphs with locality (``synth.hetero_graph_local``, or a real graph after partitioning).
 """
 import torch
 import torch.distributed as dist
@@ -197,43 +202,20 @@ class _ColumnSlabPropagate(torch.autograd.Function):
         return None, None, dx_own, d_theta, None, d_norm, None, None, None
 
 
-class SlabExchange:
-    """Peer-mapped (torch symmetric memory over NVLink) buffers of ONE feature-sliced aggregation call site: the
-    two column slabs (X and dL/dY, [P*per, F/P]) that peers push their row blocks into, the two row blocks
-    (Y and dX, [per, F]) that the SpMM kernels of all ranks store finished rows into, and a [P, 256]-float table
-    every rank writes its share of the relation gradient into (``allreduce_relation_grads``).  ``y_cols`` is a plain
-    local slab: this rank's columns of Y, kept for the folded norm gradient of the backward kernel.  Create it once
-    per layer; a forward must be followed by its backward before the next forward (the buffers are reused)."""
+class _PeerBuffers:
+    """Peer-mapped buffers (torch symmetric memory over NVLink) of one call site, the device-side barrier across the
+    ranks, and a [P, 256]-float table every rank writes its share of the relation gradient into
+    (``allreduce_relation_grads``)."""
 
     GRAD_SLOTS = 256
 
-    def __init__(self, feat, bounds, rank, device, group=None):
+    def _alloc(self, rows, cols, device, group):
+        """-> (local buffer, int64 device tensor [P] of every rank's mapped base address)."""
         import torch.distributed._symmetric_memory as symm
-        group = group if group is not None else dist.group.WORLD
-        self.parts, self.per, self.rank, self.feat = len(bounds) - 1, _uniform_rows(bounds), rank, feat
-        if not self.per or feat % (4 * self.parts):
-            raise ValueError('SlabExchange needs equal row blocks and F divisible by 4 * ranks')
-        self.fc = feat // self.parts
-        self._handles = []
-
-        def alloc(rows, cols):
-            t = symm.empty((rows, cols), dtype=torch.float32, device=device)
-            h = symm.rendezvous(t, group)
-            self._handles.append(h)
-            return t, torch.tensor([int(p) for p in h.buffer_ptrs], dtype=torch.int64, device=device)
-
-        self.x_cols, self.x_ptrs = alloc(self.parts * self.per, self.fc)
-        self.g_cols, self.g_ptrs = alloc(self.parts * self.per, self.fc)
-        self.y_rows, self.y_ptrs = alloc(self.per, feat)
-        self.dx_rows, self.dx_ptrs = alloc(self.per, feat)
-        self.grad_tab, self.grad_ptrs = alloc(self.parts, self.GRAD_SLOTS)
-        self.y_cols = torch.zeros((self.parts * self.per, self.fc), dtype=torch.float32, device=device)
-        self.x_cols.zero_()
-        self.g_cols.zero_()
-        self.grad_tab.zero_()
-        self.peer_y = _lib.PeerRows(self.y_ptrs.data_ptr(), self.parts, self.per, feat, rank * self.fc)
-        self.peer_dx = _lib.PeerRows(self.dx_ptrs.data_ptr(), self.parts, self.per, feat, rank * self.fc)
-        self.barrier()
+        t = symm.empty((rows, cols), dtype=torch.float32, device=device)
+        h = symm.rendezvous(t, group)
+        self._handles.append(h)
+        return t, torch.tensor([int(p) for p in h.buffer_ptrs], dtype=torch.int64, device=device)
 
     def barrier(self):
         """Device-side barrier across the ranks on the current stream: everything the ranks wrote into each
@@ -255,6 +237,35 @@ class SlabExchange:
         ops.rows_to_slabs(self._grad_row, self.parts, self.rank, self.grad_ptrs)
         self.barrier()
         return self.grad_tab[:, :n].sum(dim=0)
+
+
+class SlabExchange(_PeerBuffers):
+    """Peer-mapped buffers of ONE feature-sliced aggregation call site: the
+    two column slabs (X and dL/dY, [P*per, F/P]) that peers push their row blocks into, the two row blocks
+    (Y and dX, [per, F]) that the SpMM kernels of all ranks store finished rows into, and a [P, 256]-float table
+    every rank writes its share of the relation gradient into (``allreduce_relation_grads``).  ``y_cols`` is a plain
+    local slab: this rank's columns of Y, kept for the folded norm gradient of the backward kernel.  Create it once
+    per layer; a forward must be followed by its backward before the next forward (the buffers are reused)."""
+
+    def __init__(self, feat, bounds, rank, device, group=None):
+        group = group if group is not None else dist.group.WORLD
+        self.parts, self.per, self.rank, self.feat = len(bounds) - 1, _uniform_rows(bounds), rank, feat
+        if not self.per or feat % (4 * self.parts):
+            raise ValueError('SlabExchange needs equal row blocks and F divisible by 4 * ranks')
+        self.fc = feat // self.parts
+        self._handles = []
+        self.x_cols, self.x_ptrs = self._alloc(self.parts * self.per, self.fc, device, group)
+        self.g_cols, self.g_ptrs = self._alloc(self.parts * self.per, self.fc, device, group)
+        self.y_rows, self.y_ptrs = self._alloc(self.per, feat, device, group)
+        self.dx_rows, self.dx_ptrs = self._alloc(self.per, feat, device, group)
+        self.grad_tab, self.grad_ptrs = self._alloc(self.parts, self.GRAD_SLOTS, device, group)
+        self.y_cols = torch.zeros((self.parts * self.per, self.fc), dtype=torch.float32, device=device)
+        self.x_cols.zero_()
+        self.g_cols.zero_()
+        self.grad_tab.zero_()
+        self.peer_y = _lib.PeerRows(self.y_ptrs.data_ptr(), self.parts, self.per, feat, rank * self.fc)
+        self.peer_dx = _lib.PeerRows(self.dx_ptrs.data_ptr(), self.parts, self.per, feat, rank * self.fc)
+        self.barrier()
 
 
 class _PeerSlabPropagate(torch.autograd.Function):
@@ -444,9 +455,9 @@ def head_sliced_gat(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, boun
 
 def allreduce_relation_grads(params, group=None, exchange=None):
     """Sums the per-rank relation-embedding gradients (R x H floats each) -- the only cross-rank floating-point
-    reduction of the partitioned layer.  ``exchange`` (a ``SlabExchange``): all-gather over peer memory and a sum in
-    rank order (bit-identical on every rank and topology); otherwise all-gather with the collective library (NCCL /
-    gloo) followed by the same fixed-order sum."""
+    reduction of the partitioned layer.  ``exchange`` (a ``SlabExchange`` or ``HaloExchange``): all-gather over peer
+    memory and a sum in rank order (bit-identical on every rank and topology); otherwise all-gather with the collective
+    library (NCCL / gloo) followed by the same fixed-order sum."""
     grads = [p.grad for p in params if p.grad is not None]
     if not grads:
         return
@@ -465,3 +476,254 @@ def allreduce_relation_grads(params, group=None, exchange=None):
     for g in grads:
         g.copy_(total[off:off + g.numel()].view_as(g))
         off += g.numel()
+
+
+# ---- destination-row blocks with a halo exchange -------------------------------------------------------------------
+def _owner(ids, bounds_t):
+    """Rank owning each global row id (empty blocks own nothing)."""
+    return torch.bucketize(ids, bounds_t[1:-1], right=True)
+
+
+def _send_lists(own_local, remote_global, bounds_t, rank, parts, n_own):
+    """Unique (peer, own row) pairs of one view, peer-major and row-ascending -> (local row ids int32, counts [P] int64).
+    ``own_local``: this rank's row of every entry; ``remote_global``: the other end of the entry."""
+    peer = _owner(remote_global, bounds_t)
+    keep = peer != rank
+    key = torch.unique(peer[keep] * max(n_own, 1) + own_local[keep])
+    peer_of = key // max(n_own, 1)
+    return (key - peer_of * max(n_own, 1)).to(torch.int32), torch.bincount(peer_of, minlength=parts)
+
+
+class HaloPartition:
+    """Local views of one destination-row block [rb, re) for ``halo_propagate``, built once per
+    (graph, e_feat, bounds, rank) from the global ``Graph`` and its ``etype_views``; afterwards only local structures
+    are kept.
+
+    * in-view: rows [rb, re) of the destination-sorted CSR (slots ``indptr[rb]:indptr[re]``, global slot order).  An own
+      source u is column ``u - rb``; a remote one is ``n_own + k``, k its position in the **in-halo** (remote sources
+      sorted by global id, hence grouped by owner).
+    * out-view: rows [rb, re) of the transposed view, destinations renumbered the same way into own rows plus an
+      **out-halo**.
+    * ``csr``: both views in the layout of ``Graph.csr()`` (with their own long-row splits and row orders): row lengths
+      are the global ones, so fragments and kernel choice -- and hence every row's bits -- match the single-device run.
+    * ``counts``: the [n_own + halo rows, R] relation-count table (own rows, in-halo, then the out-halo unless it is the
+      same set): the degree norm of every row this rank touches, computed locally with the owner's bits.
+    * send lists: for every peer q, the own rows (local ids) in q's in-halo / out-halo; ``recv_offset_*[q]``: the row of
+      q's extended buffer at which this rank's segment lands (one all-gather of the halo counts at setup).
+
+    Index bookkeeping with device-agnostic torch ops."""
+
+    def __init__(self, graph, etv, bounds, rank, group=None):
+        self._build(graph, etv, bounds, rank)
+        table = self.halo_counts.view(1, -1)
+        if self.parts > 1:
+            gathered = [torch.empty_like(table) for _ in range(self.parts)]
+            dist.all_gather(gathered, table, group=group)
+            table = torch.cat(gathered)
+        self._set_offsets(table.cpu())
+
+    @classmethod
+    def virtual_ranks(cls, graph, etv, bounds):
+        """All P partitions of ``bounds`` in one process (one device, no process group)."""
+        parts = []
+        for p in range(len(bounds) - 1):     # the counts exchange is this list: no process group, no collective
+            part = cls.__new__(cls)
+            part._build(graph, etv, bounds, p)
+            parts.append(part)
+        table = torch.stack([p.halo_counts for p in parts]).cpu()
+        for p in parts:
+            p._set_offsets(table)
+        return parts
+
+    def _build(self, graph, etv, bounds, rank):
+        from .graph import SPLIT_THRESHOLD, _row_split
+        if etv[2] is None:
+            raise ValueError('HaloPartition needs the [N, R] relation-count table of etype_views(), which is not built for '
+                             'this graph (N * R * 4 bytes > graph.COUNTS_MAX_BYTES): the halo rows\' norms come from it')
+        csr = graph.csr()
+        n, parts = graph.number_of_nodes(), len(bounds) - 1
+        r = etv[2].numel() // max(n, 1)
+        dev = csr['indptr'].device
+        rb, re = int(bounds[rank]), int(bounds[rank + 1])
+        n_own = re - rb
+        self.parts, self.rank, self.bounds, self.n_own, self.num_relations = parts, rank, list(bounds), n_own, r
+        bounds_t = torch.tensor(bounds, dtype=torch.int64, device=dev)
+        own_rows = torch.arange(n_own, dtype=torch.int64, device=dev)
+
+        def view(indptr, indices, et):
+            s0, s1 = int(indptr[rb]), int(indptr[re])
+            ip = (indptr[rb:re + 1] - s0).to(torch.int32).contiguous()
+            other = indices[s0:s1].to(torch.int64)
+            remote = (other < rb) | (other >= re)
+            halo = torch.unique(other[remote])
+            local = torch.where(remote, n_own + torch.searchsorted(halo, other), other - rb)
+            row_of = torch.repeat_interleave(own_rows, (ip[1:] - ip[:-1]).to(torch.int64))
+            return ip, local.to(torch.int32).contiguous(), et[s0:s1].clone(), halo, row_of, other
+
+        ip_in, idx_in, self.et_in, self.in_halo, dst_of, src_of = view(csr['indptr'], csr['indices'], etv[0])
+        ip_out, idx_out, self.et_out, self.out_halo, src_of_t, dst_of_t = view(csr['indptr_t'], csr['indices_t'], etv[1])
+        self.csr = {'indptr': ip_in, 'indices': idx_in, 'indptr_t': ip_out, 'indices_t': idx_out,
+                    'split': _row_split(ip_in, SPLIT_THRESHOLD), 'split_t': _row_split(ip_out, SPLIT_THRESHOLD)}
+        # q's in-halo from this rank = own sources of an edge into q's block (seen from the out-view), and the other way
+        self.send_in, self.send_in_counts = _send_lists(src_of_t, dst_of_t, bounds_t, rank, parts, n_own)
+        self.send_out, self.send_out_counts = _send_lists(dst_of, src_of, bounds_t, rank, parts, n_own)
+        self.n_in, self.n_out = self.in_halo.numel(), self.out_halo.numel()
+        self.same_halo = bool(torch.equal(self.in_halo, self.out_halo))
+        own_global = torch.arange(rb, re, dtype=torch.int64, device=dev)
+        # global row of every row of the two extended buffers (own rows, then the halo)
+        self.rows_in, self.rows_out = torch.cat([own_global, self.in_halo]), torch.cat([own_global, self.out_halo])
+        rows = [own_global, self.in_halo]
+        if not self.same_halo:
+            rows.append(self.out_halo)
+        self.counts = etv[2].view(n, r)[torch.cat(rows)].contiguous().view(-1)
+        self.n_ext = self.counts.numel() // r
+        # [2, P]: rows of my in-halo / out-halo that each rank owns
+        self.halo_counts = torch.stack([torch.bincount(_owner(self.in_halo, bounds_t), minlength=parts),
+                                        torch.bincount(_owner(self.out_halo, bounds_t), minlength=parts)]).view(-1)
+
+    def _set_offsets(self, table):
+        """``table`` [P, 2, P] (host): every rank's ``halo_counts``."""
+        table = table.view(self.parts, 2, self.parts).to(torch.int64)
+        per = [self.bounds[q + 1] - self.bounds[q] for q in range(self.parts)]
+        before = torch.cumsum(table, dim=2) - table           # rows of q's halo owned by ranks < p
+        p = self.rank
+        self.recv_offset_in = [0 if q == p else per[q] + int(before[q, 0, p]) for q in range(self.parts)]
+        self.recv_offset_out = [0 if q == p else per[q] + int(before[q, 1, p]) for q in range(self.parts)]
+        self.recv_counts_in = table[p, 0].tolist()
+        self.recv_counts_out = table[p, 1].tolist()
+        self.max_rows_in = max(per[q] + int(table[q, 0].sum()) for q in range(self.parts))
+        self.max_rows_out = max(per[q] + int(table[q, 1].sum()) for q in range(self.parts))
+        # push lists of regnn_halo_push: the send lists with this rank's own rows as the self entry (into the head)
+        self.push_in = self._push_list(self.send_in, self.send_in_counts, self.recv_offset_in)
+        self.push_out = self._push_list(self.send_out, self.send_out_counts, self.recv_offset_out)
+
+    def _push_list(self, rows, counts, offsets):
+        counts = counts.tolist()
+        counts[self.rank] = self.n_own
+        cut = sum(counts[:self.rank])
+        own = torch.arange(self.n_own, dtype=torch.int32, device=rows.device)
+        ptr = [0]
+        for c in counts:
+            ptr.append(ptr[-1] + c)
+        return torch.cat([rows[:cut], own, rows[cut:]]).contiguous(), ptr, offsets
+
+
+class HaloExchange(_PeerBuffers):
+    """Peer-mapped halo buffers of ONE ``halo_propagate`` call site: X [n_own + in-halo, F] and dL/dY
+    [n_own + out-halo, F], own rows in the head, halos in the tail, written by every rank's ``regnn_halo_push``.
+    Symmetric allocation needs one size on every rank: the maximum over ranks.  Also carries the [P, 256] table of
+    ``allreduce_relation_grads``.  A forward must be followed by its backward before the next forward (the buffers
+    are reused)."""
+
+    def __init__(self, part, feat, device, group=None):
+        group = group if group is not None else dist.group.WORLD
+        self.parts, self.rank, self.feat = part.parts, part.rank, feat
+        self._handles = []
+        self.x_ext, self.x_ptrs = self._alloc(max(part.max_rows_in, 1), feat, device, group)
+        self.g_ext, self.g_ptrs = self._alloc(max(part.max_rows_out, 1), feat, device, group)
+        self.grad_tab, self.grad_ptrs = self._alloc(self.parts, self.GRAD_SLOTS, device, group)
+        self.grad_tab.zero_()
+        self.barrier()
+
+
+def _fill_halo(part, own, direction, group, xch):
+    """[n_own + halo, F] buffer of one direction ('in': X for the forward, 'out': dL/dY for the backward): own rows in
+    the head, the halo -- rows pushed by their owners -- in the tail."""
+    n_halo = part.n_in if direction == 'in' else part.n_out
+    if xch is not None:
+        rows, ptr, offsets = part.push_in if direction == 'in' else part.push_out
+        buf, ptrs = (xch.x_ext, xch.x_ptrs) if direction == 'in' else (xch.g_ext, xch.g_ptrs)
+        if ptr[-1]:              # an empty row block has nothing to send (and no edges)
+            ops.halo_push(own, rows, ptr, offsets, ptrs, buf.stride(0), part.rank)
+        xch.barrier()            # every owner's rows of my halo have landed
+        return buf[:part.n_own + n_halo]
+    send = part.send_in if direction == 'in' else part.send_out
+    send_counts = part.send_in_counts if direction == 'in' else part.send_out_counts
+    recv_counts = part.recv_counts_in if direction == 'in' else part.recv_counts_out
+    buf = torch.empty((part.n_own + n_halo, own.shape[1]), dtype=own.dtype, device=own.device)
+    buf[:part.n_own] = own
+    if part.parts > 1:
+        with _lib.phase('halo_all_to_all'):
+            dist.all_to_all_single(buf[part.n_own:], own.index_select(0, send.to(torch.int64)),
+                                   output_split_sizes=recv_counts, input_split_sizes=send_counts.tolist(), group=group)
+    return buf
+
+
+def _halo_norm(part, theta, alpha):
+    """(deg, norm) of every row of the count table: own rows, in-halo, out-halo."""
+    if part.n_ext == 0:
+        z = theta.new_zeros(0)
+        return z, z
+    return ops.wdeg_norm_fwd(None, None, theta, alpha, -0.5, counts=part.counts)
+
+
+def _halo_forward(part, x_ext, theta, alpha, weighted):
+    """-> (y_own, deg, norm) from the filled [n_own + in-halo, F] buffer: the degree norm of every count-table row, then
+    the SpMM over the in-view."""
+    if weighted and not ops.fused_bwd_fits(x_ext.shape[1], theta.numel()):
+        raise ValueError('halo_propagate: the weighted backward runs the fused kernel only, which does not cover F=%d '
+                         'with %d relations (ops.fused_bwd_fits: F <= 1024 and its shared-memory tile must fit)'
+                         % (x_ext.shape[1], theta.numel()))
+    deg, norm = _halo_norm(part, theta, alpha)
+    if not part.n_own:
+        return x_ext.new_zeros((0, x_ext.shape[1])), deg, norm
+    csr = part.csr
+    norm_in = norm[:part.n_own + part.n_in]
+    y_own = ops.spmm(csr['indptr'], csr['indices'], part.et_in if weighted else None, theta if weighted else None,
+                     alpha, norm_in, norm_in, x_ext, split=csr['split'],
+                     order=ops.row_order(csr) if x_ext.shape[1] <= ops.NARROW_FEAT else None)
+    return y_own, deg, norm
+
+
+def _halo_backward(part, x_own, y_own, g_ext, theta, alpha, weighted, deg, norm):
+    """-> (dX own rows, this rank's share of d_theta) from the filled [n_own + out-halo, F] dL/dY buffer."""
+    n_own, f = part.n_own, x_own.shape[1]
+    if not n_own:
+        return x_own.new_zeros(x_own.shape), torch.zeros_like(theta)
+    csr = part.csr
+    g_own = g_ext[:n_own]
+    # norms of the out-view: own rows, then the out-halo (the same rows as the in-halo on a symmetric graph)
+    norm_out = norm if part.same_halo else torch.cat([norm[:n_own], norm[n_own + part.n_in:]])
+    norm_own = norm[:n_own]
+    d_theta = None
+    if weighted:
+        fold = ops.fused_dnorm_fits(f)
+        dx_own, d_theta, extra = ops.spmm_bwd_fused(csr, part.et_out, theta, alpha, norm_out, x_own, g_ext,
+                                                    want_xdx=not fold, y=y_own if fold else None, want_dnorm=fold)
+        d_norm = extra if fold else ops.rowdot_norm_bwd(norm_own, x_own, y_own, g_own, dx_own, xdx=extra)
+    else:   # REMixHop: the transposed SpMM alone, then the owner's row dots
+        dx_own = ops.spmm(csr['indptr_t'], csr['indices_t'], None, None, alpha, norm_out, norm_out, g_ext,
+                          split=csr['split_t'], order=ops.row_order(csr, True) if f <= ops.NARROW_FEAT else None)
+        d_norm = ops.rowdot_norm_bwd(norm_own, x_own, y_own, g_own, dx_own)
+    # the norm's share of the relation gradient: own rows only (a halo row's norm gradient is its owner's)
+    d_theta_norm = ops.wdeg_norm_bwd(None, None, theta, alpha, -0.5, deg, d_norm, rows=(0, n_own), counts=part.counts)
+    return dx_own, (d_theta_norm if d_theta is None else d_theta + d_theta_norm).view_as(theta)
+
+
+class _HaloPropagate(torch.autograd.Function):
+    """Rows [rb, re) of  Y = n (.) A_w (n (.) X)  (``weighted=False``: A instead of A_w, REMixHop) with the degree norm
+    n computed inside from the relation weights; X and dL/dY row-partitioned, only halo rows exchanged."""
+
+    @staticmethod
+    def forward(ctx, part, x_own, theta, alpha, weighted, group, xch):
+        x_own = x_own.contiguous()
+        y_own, deg, norm = _halo_forward(part, _fill_halo(part, x_own, 'in', group, xch), theta, alpha, weighted)
+        ctx.part, ctx.alpha, ctx.weighted, ctx.group, ctx.xch = part, alpha, weighted, group, xch
+        ctx.save_for_backward(x_own, y_own, theta, deg, norm)
+        return y_own
+
+    @staticmethod
+    def backward(ctx, g_own):
+        x_own, y_own, theta, deg, norm = ctx.saved_tensors
+        g_ext = _fill_halo(ctx.part, g_own.contiguous(), 'out', ctx.group, ctx.xch)
+        dx_own, d_theta = _halo_backward(ctx.part, x_own, y_own, g_ext, theta, ctx.alpha, ctx.weighted, deg, norm)
+        return None, dx_own, d_theta, None, None, None, None
+
+
+def halo_propagate(part, x_own, theta, alpha, weighted=True, group=None, exchange=None):
+    """Row block in, row block out (``part``: this rank's ``HaloPartition``): the REGCN aggregation
+    Y = n (.) A_w (n (.) X) with n = max(sum_in w, 1)^-1/2 from ``theta`` (``weighted=False``: REMixHop's
+    Y = n (.) A (n (.) X)).  Only halo rows are exchanged: ``exchange`` (a ``HaloExchange``) pushes them over peer
+    memory with regnn_halo_push; None: one uneven all-to-all (NCCL / gloo).  Y and dX are bit-identical to
+    ``functional.propagate``; ``theta.grad`` holds this rank's share (``allreduce_relation_grads``)."""
+    return _HaloPropagate.apply(part, x_own, theta, alpha, weighted, group, exchange)

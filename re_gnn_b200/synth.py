@@ -75,6 +75,76 @@ def hetero_graph(name, seed=123, skew=2.5, scale=1.0):
                 num_etype=et, num_relations=et + len(sizes), name=name)
 
 
+def _draw_relation_local(rng, n_src, n_dst, n_edges, skew, locality, src_cuts, dst_comm):
+    """``_draw_relation`` with locality: with probability ``locality`` the source is drawn uniformly from the
+    destination's community (``src_cuts``: community boundaries of the source type's local ids; ``dst_comm``: the
+    community of every destination), otherwise from the whole source type."""
+    got = np.zeros(0, dtype=np.int64)
+    perm = rng.permutation(n_dst)
+    while got.size < n_edges:
+        m = int((n_edges - got.size) * 1.25) + 64
+        v = perm[np.minimum((n_dst * rng.random_sample(m) ** skew).astype(np.int64), n_dst - 1)]
+        lo, hi = src_cuts[dst_comm[v]], src_cuts[dst_comm[v] + 1]
+        near = (rng.random_sample(m) < locality) & (hi > lo)
+        u_near = lo + np.minimum((rng.random_sample(m) * (hi - lo)).astype(np.int64), np.maximum(hi - lo - 1, 0))
+        u = np.where(near, u_near, rng.randint(0, n_src, size=m).astype(np.int64))
+        got = np.unique(np.concatenate([got, u * n_dst + v]))
+    if got.size > n_edges:
+        got = np.sort(rng.choice(got, size=n_edges, replace=False))
+    return got // n_dst, got % n_dst
+
+
+def hetero_graph_local(name, parts, locality, seed=123, skew=2.5, scale=1.0):
+    """``hetero_graph`` with community structure, for row-block partitioning with halos.  The node-type sizes, relation
+    counts, edge-type numbering, de-duplication and the self loops appended last are those of ``hetero_graph``; the
+    layout differs: nodes are community-major -- community c holds about 1/``parts`` of every node type in one contiguous
+    id range -- so node types are NOT contiguous id blocks any more (``ntype`` is per node, as always).  Destinations
+    keep the power-law popularity; with probability ``locality`` a source is drawn from the destination's community
+    (same source type), otherwise from all nodes of its type.  Returns ``hetero_graph``'s dict plus
+    ``community_bounds`` ([parts + 1] row boundaries, usable as ``bounds`` of ``partition``)."""
+    sizes, relations = SHAPES[name]
+    sizes = [max(2, int(round(s * scale))) for s in sizes]
+    rng = np.random.RandomState(seed)
+    # cuts[t][c]: first local id of type t in community c; community c = type blocks in type order
+    cuts = [np.array([s * c // parts for c in range(parts + 1)], dtype=np.int64) for s in sizes]
+    per_comm = np.array([[cuts[t][c + 1] - cuts[t][c] for t in range(len(sizes))] for c in range(parts)], dtype=np.int64)
+    comm_start = np.concatenate([[0], np.cumsum(per_comm.sum(1))]).astype(np.int64)
+    gid, comm_of = [], []     # per type: global id / community of every local id
+    for t, s in enumerate(sizes):
+        c = np.repeat(np.arange(parts, dtype=np.int64), np.diff(cuts[t]))
+        within = np.arange(s, dtype=np.int64) - cuts[t][c]
+        gid.append(comm_start[c] + per_comm[c, :t].sum(1) + within)
+        comm_of.append(c)
+    srcs, dsts, ets = [], [], []
+    et = 0
+    for (ts, td, ne, symmetric) in relations:
+        ne = max(1, int(round(ne * scale)))
+        ne = min(ne, sizes[ts] * sizes[td] // 2)
+        u, v = _draw_relation_local(rng, sizes[ts], sizes[td], ne, skew, locality, cuts[ts], comm_of[td])
+        if ts == td:
+            keep = u != v
+            u, v = u[keep], v[keep]
+        u, v = gid[ts][u], gid[td][v]
+        if symmetric:
+            srcs += [u, v]; dsts += [v, u]; ets += [np.full(2 * u.size, et + 1, dtype=np.int64)]
+            et += 1
+        else:
+            srcs += [u, v]; dsts += [v, u]
+            ets += [np.full(u.size, et + 1, dtype=np.int64), np.full(u.size, et + 2, dtype=np.int64)]
+            et += 2
+    n = int(comm_start[-1])
+    ntype = np.empty(n, dtype=np.int64)
+    for t in range(len(sizes)):
+        ntype[gid[t]] = t
+    loop = np.arange(n, dtype=np.int64)
+    src = np.concatenate(srcs + [loop])
+    dst = np.concatenate(dsts + [loop])
+    etype = np.concatenate(ets + [et + 1 + ntype])
+    return dict(src=src, dst=dst, etype=etype, num_nodes=n, ntype=ntype, type_sizes=sizes,
+                num_etype=et, num_relations=et + len(sizes), name=name,
+                community_bounds=[int(b) for b in comm_start])
+
+
 def random_multigraph(n, e, r, seed=0, hubs=4, self_loops=True):
     """Small adversarial test graph: duplicate edges, a few hub destinations, zero-in-degree nodes
     (when ``self_loops`` is False), 1-based edge types in [1, r]."""
