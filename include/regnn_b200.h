@@ -218,6 +218,15 @@ int regnn_rows_to_slabs(const float* X, int64_t ldx, int64_t num_rows, int feat,
 int regnn_halo_push(const float* X, int64_t ldx, int feat, const int32_t* send_rows, const int64_t* send_ptr,
                     const int64_t* recv_offset, float* const* peer_bufs, int64_t ldb, int num_ranks, int rank, void* stream);
 
+/* The reverse exchange of the REGAT halo backward (partition.halo_gat: the logit gradient of an edge whose destination
+ * is remote goes to the destination's owner, into its CSR slot): for every peer q, the rows X[k], k in
+ * send_ptr[q] .. send_ptr[q+1], of this rank's [rows, width] buffer are stored to peer_bufs[q] + dst_rows[k] * ldb.
+ * Any width >= 1 (stores are 4-byte words); send_ptr [num_ranks+1] is a HOST array, dst_rows (int32) and peer_bufs
+ * [num_ranks] are device arrays; lists may be empty.  Local buffers work the same as peer-mapped ones.
+ * num_ranks <= REGNN_HALO_MAX_RANKS. */
+int regnn_halo_scatter(const float* X, int64_t ldx, int width, const int64_t* send_ptr, const int32_t* dst_rows,
+                       float* const* peer_bufs, int64_t ldb, int num_ranks, int rank, void* stream);
+
 /* The reverse re-partition for kernels without a scatter epilogue (the fused attention kernels, one head slice per
  * rank): S [num_rows, feat] is this rank's column slab (ld lds); row v is stored to
  * peers->base[v / rows_per_rank][(v % rows_per_rank) * ld + col_offset .. + feat). */

@@ -187,6 +187,26 @@ __global__ void halo_push_kernel(const float* __restrict__ X, int64_t ldx, int L
   }
 }
 
+// Indexed row scatter, the reverse direction of halo_push_kernel (the per-slot logit gradients of the REGAT backward go
+// back to the owners of their destination rows): the rows ptr[q] .. ptr[q+1] of this rank's buffer go to rows
+// dst_rows[k] of peer q's buffer.  The rows are W = num_heads floats (1..8), not whole 128-bit chunks: one lane per
+// float, so consecutive lanes read consecutive floats of the contiguous source range and store 4-byte words.  Peers in
+// rank-rotated order; the per-peer offsets travel as a kernel parameter.
+__global__ void halo_scatter_kernel(const float* __restrict__ X, int64_t ldx, int W,
+                                    const int32_t* __restrict__ dst_rows, const __grid_constant__ HaloPeers hp,
+                                    float* const* __restrict__ peer_bufs, int64_t ldb, int first_peer) {
+  const int q = (int)((blockIdx.y + (unsigned)first_peer) % gridDim.y);
+  const int64_t begin = hp.ptr[q];
+  const int64_t total = (hp.ptr[q + 1] - begin) * W;
+  if (total == 0) return;
+  float* dst = peer_bufs[q];
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = e / W;
+    const int c = (int)(e - i * W);
+    dst[(int64_t)__ldg(dst_rows + begin + i) * ldb + c] = __ldg(X + (begin + i) * ldx + c);
+  }
+}
+
 // Column slab -> row blocks over peer memory, for the kernels that have no scatter epilogue of their own (the fused
 // attention kernels: one head slice per rank): rows [q*per, (q+1)*per) of this rank's slab S [N, Fc] go to rank q's row
 // block at column col_offset.  The local read is contiguous, every destination row gets one Fc*4-byte store burst
@@ -1545,6 +1565,34 @@ extern "C" int regnn_halo_push(const float* X, int64_t ldx, int feat, const int3
   halo_push_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(X, ldx, L, G, send_rows, hp,
                                                                                   peer_bufs, ldb, rank);
   return check_launch("regnn_halo_push");
+}
+
+extern "C" int regnn_halo_scatter(const float* X, int64_t ldx, int width, const int64_t* send_ptr, const int32_t* dst_rows,
+                                  float* const* peer_bufs, int64_t ldb, int num_ranks, int rank, void* stream) {
+  REGNN_REQUIRE(X && send_ptr && peer_bufs && num_ranks >= 1 && rank >= 0 && rank < num_ranks, REGNN_ERR_INVALID_ARG,
+                "halo_scatter: bad argument");
+  REGNN_REQUIRE(num_ranks <= REGNN_HALO_MAX_RANKS, REGNN_ERR_UNSUPPORTED_SHAPE, "halo_scatter: %d ranks (max %d)",
+                num_ranks, REGNN_HALO_MAX_RANKS);
+  REGNN_REQUIRE(width >= 1 && ldx >= width && ldb >= width, REGNN_ERR_INVALID_ARG,
+                "halo_scatter: W=%d with leading dimensions %lld / %lld", width, (long long)ldx, (long long)ldb);
+  REGNN_REQUIRE(send_ptr[0] >= 0, REGNN_ERR_INVALID_ARG, "halo_scatter: negative send offset");
+  HaloPeers hp;
+  int64_t most = 0;
+  hp.ptr[0] = send_ptr[0];
+  for (int q = 0; q < num_ranks; ++q) {
+    const int64_t cnt = send_ptr[q + 1] - send_ptr[q];
+    REGNN_REQUIRE(cnt >= 0, REGNN_ERR_INVALID_ARG, "halo_scatter: peer %d has a negative row count", q);
+    hp.ptr[q + 1] = send_ptr[q + 1];
+    hp.recv_offset[q] = 0;
+    most = cnt > most ? cnt : most;
+  }
+  if (most == 0) return REGNN_OK;
+  REGNN_REQUIRE(dst_rows != nullptr, REGNN_ERR_INVALID_ARG, "halo_scatter: null destination rows");
+  const int64_t want = (most * width + 255) / 256;
+  const unsigned bx = (unsigned)(want < 148 * 8 ? want : 148 * 8);
+  halo_scatter_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(X, ldx, width, dst_rows, hp,
+                                                                                     peer_bufs, ldb, rank);
+  return check_launch("regnn_halo_scatter");
 }
 
 extern "C" int regnn_slabs_to_rows(const float* S, int64_t lds, int64_t num_rows, int feat,

@@ -225,6 +225,19 @@ def halo_push(x_own, send_rows, send_ptr, recv_offset, peer_buf_ptrs, ldb, rank)
         _lib.count_launches(1 if send_ptr[-1] > send_ptr[0] else 0)
 
 
+def halo_scatter(x, send_ptr, dst_rows, peer_buf_ptrs, ldb, rank):
+    """Stores rows ``x[send_ptr[q]:send_ptr[q+1]]`` to rows ``dst_rows[send_ptr[q]:send_ptr[q+1]]`` of peer q's buffer
+    (regnn_halo_scatter; any row width).  ``send_ptr`` [P+1]: host sequence of ints; ``dst_rows``: int32 device tensor
+    indexed like the rows of ``x``; ``peer_buf_ptrs``: int64 device tensor [P] of buffer base addresses (leading
+    dimension ``ldb`` floats)."""
+    x = _f32(x)
+    p = len(send_ptr) - 1
+    with torch.cuda.device(x.device):
+        _lib.call('regnn_halo_scatter', _ptr(x), x.stride(0), x.shape[1], (ctypes.c_int64 * (p + 1))(*send_ptr),
+                  _ptr(dst_rows), _ptr(peer_buf_ptrs), int(ldb), p, int(rank), _stream())
+        _lib.count_launches(1 if send_ptr[-1] > send_ptr[0] else 0)
+
+
 def slabs_to_rows(slab, num_rows, peers):
     """Pushes rows [0, num_rows) of this rank's column slab ``slab`` [>= num_rows, F/P] to their owner ranks' row blocks
     (regnn_slabs_to_rows; ``peers``: a ``_lib.PeerRows``)."""
@@ -295,12 +308,17 @@ def _full(rb, re, n):
 
 
 def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn=False, rows=None):
+    """-> (out, rowmax, rowsum, attention | None) for the rows of ``csr``.  ``feat`` / ``el`` are indexed by the column
+    ids of ``csr`` and may have more rows than the CSR (a halo of remote sources after the own rows)."""
     feat, el, er, keep = _f32(feat), _f32(el), _f32(er), _f32(keep)
-    n, h, d = feat.shape
+    _, h, d = feat.shape
+    n = csr['indptr'].numel() - 1
     rb, re = _rows(rows, n)
     theta, et_csr, r = _rel(theta, et_csr)
     dev = feat.device
-    out = torch.empty_like(feat) if _full(rb, re, n) else torch.zeros_like(feat)
+    out = torch.empty((n, h, d), dtype=torch.float32, device=dev)
+    if not _full(rb, re, n):
+        out.zero_()
     rowmax = torch.zeros((n, h), dtype=torch.float32, device=dev)
     rowsum = torch.zeros((n, h), dtype=torch.float32, device=dev)
     e = csr['indices'].numel()
@@ -308,7 +326,7 @@ def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn
     sp, ws = _attn_split(csr.get('split'), h, d, dev)
     order = row_order(csr) if _full(rb, re, n) else None
     with torch.cuda.device(dev):
-        _lib.call('regnn_gat_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr['eid']), _ptr(et_csr),
+        _lib.call('regnn_gat_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr.get('eid')), _ptr(et_csr),
                   _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el), _ptr(er), float(slope), _ptr(keep), h, d,
                   rb, re, _ptr(out), _ptr(rowmax), _ptr(rowsum), _ptr(attn), sp, _ptr(ws), _ptr(order), _stream())
         _lib.count_launches(1 + (sp is not None))
@@ -360,6 +378,80 @@ def gat_bwd(csr, et_csr, et_t, theta, alpha, feat, el, er, slope, keep, out, row
                       _ptr(d_ar), _ptr(d_feat), _ptr(attn_r), _stream())
             _lib.count_launches(3)
     return d_feat, d_el, d_er, d_theta, d_al, d_ar
+
+
+# The stages of ``gat_bwd`` one by one, for callers that move data between them (partition.halo_gat exchanges the
+# statistics before the edge pass and the per-slot logit gradients between the edge pass and the reduction).  Full row
+# ranges, no attention dropout.
+
+def gat_bwd_stats(out, g, er, rowmax, rowsum):
+    """-> stats [N, H, 4] = (er, rowmax, 1/rowsum, <out, G>) per (row, head) (regnn_gat_bwd_stats)."""
+    out, g, er = _f32(out), _f32(g), _f32(er)
+    n, h, d = out.shape
+    stats = torch.empty((n, h, 4), dtype=torch.float32, device=out.device)
+    with torch.cuda.device(out.device):
+        _lib.call('regnn_gat_bwd_stats', _ptr(out), _ptr(g), _ptr(er), _ptr(rowmax), _ptr(rowsum), n, h, d, _ptr(stats),
+                  _stream())
+        _lib.count_launches(1)
+    return stats
+
+
+def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=None):
+    """Source-major pass over the rows of the transposed view ``csr['indptr_t']`` -> (d_feat, d_el) of those rows; the
+    logit gradient of every entry j is written to ``dpre[csr['slot_t'][j]]`` ([slots, H]).  ``feat`` / ``el``: the rows'
+    own values; ``g`` / ``stats``: indexed by the column ids of the view.  ``attn_l`` folds the gradient through el into
+    d_feat (regnn_gat_bwd_edges)."""
+    feat, el, g = _f32(feat), _f32(el), _f32(g)
+    theta, et_t, r = _rel(theta, et_t)
+    n = csr['indptr_t'].numel() - 1
+    _, h, d = feat.shape
+    dev = feat.device
+    d_feat = torch.empty((n, h, d), dtype=torch.float32, device=dev)
+    d_el = torch.zeros((n, h), dtype=torch.float32, device=dev)
+    attn_l = _f32(attn_l).view(-1) if attn_l is not None else None
+    sp_t, ws_t = _attn_split(csr.get('split_t'), h, d, dev)
+    with torch.cuda.device(dev):
+        _lib.call('regnn_gat_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
+                  _ptr(et_t) if r else None, None, _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el), _ptr(stats),
+                  float(slope), None, _ptr(g), h, d, 0, n, _ptr(d_feat), _ptr(d_el), _ptr(dpre), _ptr(attn_l), sp_t,
+                  _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
+        _lib.count_launches(1 + (3 if sp_t is not None else 0))
+    return d_feat, d_el
+
+
+def gat_bwd_reduce(csr, et_csr, theta, alpha, dpre):
+    """Destination-side reductions of ``dpre`` over the rows of ``csr['indptr']`` -> (d_er [N, H], d_theta [R, H] | None)
+    (regnn_gat_bwd_reduce)."""
+    theta, et_csr, r = _rel(theta, et_csr)
+    n = csr['indptr'].numel() - 1
+    h = dpre.shape[1]
+    dev = dpre.device
+    d_er = torch.zeros((n, h), dtype=torch.float32, device=dev)
+    partials = torch.empty(max(_lib.partial_blocks(n) * r * h, 1), dtype=torch.float64, device=dev)
+    d_theta = torch.zeros((r, h), dtype=torch.float32, device=dev) if r else None
+    sp, ws = _attn_split(csr.get('split'), h, 0, dev)
+    with torch.cuda.device(dev):
+        _lib.call('regnn_gat_bwd_reduce', _ptr(csr['indptr']), _ptr(et_csr) if r else None, _ptr(theta), float(alpha), r,
+                  _ptr(dpre), h, 0, n, _ptr(d_er), _ptr(partials), _ptr(d_theta), sp, _ptr(ws), _stream())
+        _lib.count_launches(((1 if n >= 65536 else 2) if r else 0) + 1 + (sp is not None))
+    return d_er, d_theta
+
+
+def attn_scores_bwd(feat, d_el, d_er, attn_r=None, d_feat=None):
+    """-> (d_attn_l [H*D], d_attn_r [H*D]) of the projection scores; with ``d_feat`` and ``attn_r`` also
+    d_feat += d_er * attn_r in place (regnn_attn_scores_bwd)."""
+    feat = _f32(feat)
+    n, h, d = feat.shape
+    dev = feat.device
+    attn_r = _f32(attn_r).view(-1) if attn_r is not None else None
+    partials = torch.empty(max(_lib.partial_blocks(n) * 2 * h * d, 1), dtype=torch.float64, device=dev)
+    d_al = torch.empty(h * d, dtype=torch.float32, device=dev)
+    d_ar = torch.empty(h * d, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.call('regnn_attn_scores_bwd', _ptr(feat), _ptr(d_el), _ptr(d_er), n, h, d, _ptr(partials), _ptr(d_al),
+                  _ptr(d_ar), _ptr(d_feat), _ptr(attn_r), _stream())
+        _lib.count_launches(3)
+    return d_al, d_ar
 
 
 def attn_scores_fwd(feat, attn_l, attn_r):

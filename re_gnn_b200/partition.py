@@ -22,6 +22,9 @@ relation-degree norm for all rows; the caller sums the R-float relation gradient
    degree norm is computed inside from a local relation-count table (halo rows get their owner's bits); the exchange is
    one uneven all-to-all (``exchange=None``) or ``regnn_halo_push`` over peer memory (``exchange=HaloExchange(...)``).
    It pays off on graphs with locality (``synth.hetero_graph_local``, or a real graph after partitioning).
+4. ``halo_gat`` -- the REGAT core on the same row blocks (``HaloPartition(..., attention=True)``): the features go
+   forward through the in-halo, dL/dY and the softmax statistics backward through the out-halo, and the logit gradient
+   of every cut edge goes back to its destination's owner (``regnn_halo_scatter`` or one more uneven all-to-all).
 """
 import torch
 import torch.distributed as dist
@@ -511,10 +514,25 @@ class HaloPartition:
     * send lists: for every peer q, the own rows (local ids) in q's in-halo / out-halo; ``recv_offset_*[q]``: the row of
       q's extended buffer at which this rank's segment lands (one all-gather of the halo counts at setup).
 
+    ``attention=True`` (``halo_gat``) also keeps what the REGAT backward needs to send the logit gradient of an edge back
+    to the owner of its destination (the slot belongs to the destination's in-view row):
+
+    * ``eid_in``: global edge ids of the in-view slots (the kernels read them only for attention dropout, which the
+      halo path does not take, so they stay out of ``csr``);
+    * ``csr['slot_t']``: for every out-view entry (own source u -> destination v), its position in the **extended dpre
+      buffer** [E_in_own + cut_out, H]: v's local in-view slot when v is own, else ``E_in_own + k`` with k its position
+      in the **tail** -- grouped by owner, and within an owner by that owner's local slot (global slot order is both);
+    * ``tail_ptr`` [P+1] (host, offsets into the tail) and ``tail_dst`` (int32): the owner's local slot of every tail
+      entry -- the send side of regnn_halo_scatter;
+    * ``dpre_recv`` (int64) and ``dpre_recv_counts`` [P]: per peer, the own in-view slots whose source that peer owns,
+      slot-ascending -- the receive side of the all-to-all variant, entry for entry the peer's tail segment;
+    * ``max_dpre_rows``: the largest extended dpre buffer over all ranks (the symmetric allocation size), computed from
+      the global CSR like the tails, so no collective is needed.
+
     Index bookkeeping with device-agnostic torch ops."""
 
-    def __init__(self, graph, etv, bounds, rank, group=None):
-        self._build(graph, etv, bounds, rank)
+    def __init__(self, graph, etv, bounds, rank, group=None, attention=False):
+        self._build(graph, etv, bounds, rank, attention)
         table = self.halo_counts.view(1, -1)
         if self.parts > 1:
             gathered = [torch.empty_like(table) for _ in range(self.parts)]
@@ -523,19 +541,19 @@ class HaloPartition:
         self._set_offsets(table.cpu())
 
     @classmethod
-    def virtual_ranks(cls, graph, etv, bounds):
+    def virtual_ranks(cls, graph, etv, bounds, attention=False):
         """All P partitions of ``bounds`` in one process (one device, no process group)."""
         parts = []
         for p in range(len(bounds) - 1):     # the counts exchange is this list: no process group, no collective
             part = cls.__new__(cls)
-            part._build(graph, etv, bounds, p)
+            part._build(graph, etv, bounds, p, attention)
             parts.append(part)
         table = torch.stack([p.halo_counts for p in parts]).cpu()
         for p in parts:
             p._set_offsets(table)
         return parts
 
-    def _build(self, graph, etv, bounds, rank):
+    def _build(self, graph, etv, bounds, rank, attention=False):
         from .graph import SPLIT_THRESHOLD, _row_split
         if etv[2] is None:
             raise ValueError('HaloPartition needs the [N, R] relation-count table of etype_views(), which is not built for '
@@ -580,6 +598,46 @@ class HaloPartition:
         # [2, P]: rows of my in-halo / out-halo that each rank owns
         self.halo_counts = torch.stack([torch.bincount(_owner(self.in_halo, bounds_t), minlength=parts),
                                         torch.bincount(_owner(self.out_halo, bounds_t), minlength=parts)]).view(-1)
+        self.attention = attention
+        if attention:
+            self._build_attention(csr, bounds_t, src_of, dst_of_t)
+
+    def _build_attention(self, csr, bounds_t, src_of, dst_of_t):
+        """The attention views of the class docstring.  ``src_of``: global source of every in-view slot;
+        ``dst_of_t``: global destination of every out-view entry."""
+        rank, parts, rb, re = self.rank, self.parts, self.bounds[self.rank], self.bounds[self.rank + 1]
+        slot_bounds = csr['indptr'].to(torch.int64)[bounds_t]      # global CSR slot range of every row block
+        s0, s1 = int(slot_bounds[rank]), int(slot_bounds[rank + 1])
+        t0, t1 = int(csr['indptr_t'][rb]), int(csr['indptr_t'][re])
+        self.e_in = s1 - s0
+        self.eid_in = csr['eid'][s0:s1].clone()
+        gslot = csr['slot_t'][t0:t1].to(torch.int64)
+        remote = (dst_of_t < rb) | (dst_of_t >= re)
+        tail_glob, perm = torch.sort(gslot[remote])                # global slot order = owner-major, owner-slot order
+        pos = torch.empty_like(perm)
+        pos[perm] = torch.arange(perm.numel(), dtype=torch.int64, device=perm.device)
+        slot_t = gslot - s0
+        slot_t[remote] = self.e_in + pos
+        self.csr['slot_t'] = slot_t.to(torch.int32).contiguous()
+        tail_owner = _owner(dst_of_t[remote][perm], bounds_t)
+        self.tail_dst = (tail_glob - slot_bounds[tail_owner]).to(torch.int32).contiguous()
+        self.tail_counts = torch.bincount(tail_owner, minlength=parts).tolist()
+        self.tail_ptr = [0]
+        for c in self.tail_counts:
+            self.tail_ptr.append(self.tail_ptr[-1] + c)
+        # receive side: own in-view slots by the owner of their source, slot-ascending within an owner
+        src_owner = _owner(src_of, bounds_t)
+        rem_in = src_owner != rank
+        slots = torch.arange(self.e_in, dtype=torch.int64, device=src_of.device)[rem_in]
+        key, _ = torch.sort(src_owner[rem_in] * max(self.e_in, 1) + slots)
+        self.dpre_recv = key % max(self.e_in, 1)
+        self.dpre_recv_counts = torch.bincount(src_owner[rem_in], minlength=parts).tolist()
+        # the extended buffer of every rank: its in-view slots plus its cut out-edges (source own, destination not)
+        all_src_owner = _owner(csr['indices'].to(torch.int64), bounds_t)
+        all_dst_owner = _owner(torch.arange(int(slot_bounds[-1]), dtype=torch.int64, device=src_of.device), slot_bounds)
+        cross = all_src_owner != all_dst_owner
+        cut = torch.bincount(all_src_owner[cross], minlength=parts)
+        self.max_dpre_rows = int((slot_bounds[1:] - slot_bounds[:-1] + cut).max())
 
     def _set_offsets(self, table):
         """``table`` [P, 2, P] (host): every rank's ``halo_counts``."""
@@ -613,14 +671,25 @@ class HaloExchange(_PeerBuffers):
     [n_own + out-halo, F], own rows in the head, halos in the tail, written by every rank's ``regnn_halo_push``.
     Symmetric allocation needs one size on every rank: the maximum over ranks.  Also carries the [P, 256] table of
     ``allreduce_relation_grads``.  A forward must be followed by its backward before the next forward (the buffers
-    are reused)."""
+    are reused).
 
-    def __init__(self, part, feat, device, group=None):
+    ``heads`` (a ``halo_gat`` call site, ``feat`` = heads * head_dim, ``part`` built with ``attention=True``): also the
+    softmax statistics of the out-halo [n_own + out-halo, 4 * heads], the extended dpre buffer
+    [E_in_own + cut_out, heads] that peers scatter the logit gradients of this rank's in-view slots into, and a gradient
+    table wide enough for d_attn_l, d_attn_r and d_theta together (2 * feat + R * heads floats)."""
+
+    def __init__(self, part, feat, device, group=None, heads=None):
         group = group if group is not None else dist.group.WORLD
-        self.parts, self.rank, self.feat = part.parts, part.rank, feat
+        self.parts, self.rank, self.feat, self.heads = part.parts, part.rank, feat, heads
         self._handles = []
         self.x_ext, self.x_ptrs = self._alloc(max(part.max_rows_in, 1), feat, device, group)
         self.g_ext, self.g_ptrs = self._alloc(max(part.max_rows_out, 1), feat, device, group)
+        if heads is not None:
+            if not getattr(part, 'attention', False):
+                raise ValueError('HaloExchange(heads=...) needs a HaloPartition built with attention=True')
+            self.s_ext, self.s_ptrs = self._alloc(max(part.max_rows_out, 1), 4 * heads, device, group)
+            self.dpre, self.dpre_ptrs = self._alloc(max(part.max_dpre_rows, 1), heads, device, group)
+            self.GRAD_SLOTS = max(self.GRAD_SLOTS, (2 * feat + part.num_relations * heads + 63) // 64 * 64)
         self.grad_tab, self.grad_ptrs = self._alloc(self.parts, self.GRAD_SLOTS, device, group)
         self.grad_tab.zero_()
         self.barrier()
@@ -727,3 +796,181 @@ def halo_propagate(part, x_own, theta, alpha, weighted=True, group=None, exchang
     memory with regnn_halo_push; None: one uneven all-to-all (NCCL / gloo).  Y and dX are bit-identical to
     ``functional.propagate``; ``theta.grad`` holds this rank's share (``allreduce_relation_grads``)."""
     return _HaloPropagate.apply(part, x_own, theta, alpha, weighted, group, exchange)
+
+
+def _check_gat_shape(heads, dim, num_relations, relational):
+    """The head widths the fused attention kernels take (check_shape of csrc/gat.cu), refused before any work."""
+    if not (1 <= heads <= 32 and 4 <= dim <= 128 and dim & (dim - 1) == 0 and heads * dim <= 1024):
+        raise ValueError('halo_gat: the fused attention kernels take 1 <= H <= 32 heads of a power-of-two width D in '
+                         '[4, 128] with H * D <= 1024, not H=%d D=%d' % (heads, dim))
+    if relational and not (1 <= num_relations <= 200 and num_relations * heads <= 4096):
+        raise ValueError('halo_gat: the fused attention kernels take 1..200 relations with R * H <= 4096, not R=%d H=%d'
+                         % (num_relations, heads))
+
+
+def _fill_out_halo_gat(part, g_own, stats_own, group, xch):
+    """dL/dY [n_own + out-halo, H*D] and the softmax statistics [n_own + out-halo, 4H] of the backward: the same rows,
+    pushed by their owners (one barrier for both over peer memory, two uneven all-to-alls otherwise)."""
+    if xch is None:
+        return _fill_halo(part, g_own, 'out', group, None), _fill_halo(part, stats_own, 'out', group, None)
+    rows, ptr, offsets = part.push_out
+    if ptr[-1]:
+        ops.halo_push(g_own, rows, ptr, offsets, xch.g_ptrs, xch.g_ext.stride(0), part.rank)
+        ops.halo_push(stats_own, rows, ptr, offsets, xch.s_ptrs, xch.s_ext.stride(0), part.rank)
+    xch.barrier()
+    n = part.n_own + part.n_out
+    return xch.g_ext[:n], xch.s_ext[:n]
+
+
+def _return_dpre(part, dpre, group, xch):
+    """Sends the tail of the extended dpre buffer (logit gradients of this rank's out-edges into remote rows) to the
+    owners of those rows; afterwards ``dpre[:e_in]`` holds every in-view slot of this rank."""
+    e_in = part.e_in
+    if xch is not None:
+        if part.tail_ptr[-1]:
+            ops.halo_scatter(dpre[e_in:], part.tail_ptr, part.tail_dst, xch.dpre_ptrs, xch.dpre.stride(0), part.rank)
+        xch.barrier()            # every peer's gradients of my in-view slots have landed
+        return
+    if part.parts > 1:
+        recv = dpre.new_empty((sum(part.dpre_recv_counts), dpre.shape[1]))
+        with _lib.phase('halo_all_to_all'):
+            dist.all_to_all_single(recv, dpre[e_in:], output_split_sizes=part.dpre_recv_counts,
+                                   input_split_sizes=part.tail_counts, group=group)
+        dpre.index_copy_(0, part.dpre_recv, recv)
+
+
+def _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope):
+    """-> (out, el, er, rowmax, rowsum) of the own rows from the filled [n_own + in-halo, H, D] feature buffer: el / er
+    of own AND halo rows computed here (row-wise, so a halo row carries its owner's bits and el is never exchanged),
+    then the fused kernel over the in-view."""
+    n_own, heads, dim = part.n_own, f_ext.shape[1], f_ext.shape[2]
+    if not n_own:                # an empty row block has no edges and no halo
+        z = f_ext.new_zeros((0, heads))
+        return f_ext.new_zeros((0, heads, dim)), z, z, z, z
+    el, er = ops.attn_scores_fwd(f_ext, attn_l, attn_r)
+    out, rowmax, rowsum, _ = ops.gat_fwd(part.csr, part.et_in if theta is not None else None, theta, alpha, f_ext, el,
+                                         er, slope)
+    return out, el[:n_own], er[:n_own], rowmax, rowsum
+
+
+def _gat_stats(out, g_own, er, rowmax, rowsum):
+    """[n_own, 4H] softmax statistics of the own rows (the rows peers' edge passes read through their out-halo)."""
+    n_own, heads, _ = out.shape
+    if not n_own:
+        return out.new_zeros((0, 4 * heads))
+    return ops.gat_bwd_stats(out, g_own, er, rowmax, rowsum).view(n_own, 4 * heads)
+
+
+def _gat_backward_edges(part, f_own, el, attn_l, theta, alpha, slope, g_ext, s_ext, dpre):
+    """-> (d_feat without the destination-side score term, d_el) of the own rows; writes the logit gradient of every
+    out-view entry into the extended ``dpre`` buffer [e_in + tail, H] through ``csr['slot_t']``."""
+    n_own, heads, dim = f_own.shape
+    if not n_own:
+        return torch.zeros_like(f_own), f_own.new_zeros((0, heads))
+    return ops.gat_bwd_edges(part.csr, part.et_out if theta is not None else None, theta, alpha, f_own, el,
+                             s_ext.view(-1, heads, 4), slope, g_ext.view(-1, heads, dim), dpre, attn_l=attn_l)
+
+
+def _gat_backward_reduce(part, f_own, d_feat, d_el, attn_r, theta, alpha, dpre):
+    """-> (d_feat, this rank's d_attn_l, d_attn_r [H*D] and d_theta | None) once ``dpre[:e_in]`` holds every in-view
+    slot: d_er and the relation bins over the in-view, then the projection-score gradients of the own rows (which add
+    d_er * attn_r to d_feat in place)."""
+    n_own, heads, dim = f_own.shape
+    if not n_own:
+        z = f_own.new_zeros(heads * dim)
+        return d_feat, z, z.clone(), (f_own.new_zeros(theta.shape) if theta is not None else None)
+    d_er, d_theta = ops.gat_bwd_reduce(part.csr, part.et_in if theta is not None else None, theta, alpha,
+                                       dpre[:part.e_in])
+    d_al, d_ar = ops.attn_scores_bwd(f_own, d_el, d_er, attn_r=attn_r, d_feat=d_feat)
+    return d_feat, d_al, d_ar, d_theta
+
+
+class _HaloGat(torch.autograd.Function):
+    """REGAT core (projection scores + fused logits / edge softmax / aggregation) on destination-row blocks with a halo
+    exchange.  Forward: the in-halo of the features, then ``_gat_forward``.  Backward: the statistics of own rows; the
+    out-halo of dL/dY and of the statistics; the source-major edge pass over the out-view, which writes the logit
+    gradient of every out-edge into the extended dpre buffer; the tail of that buffer goes back to the destinations'
+    owners (the third exchange); then d_er and the relation bins over the in-view and the projection-score gradients of
+    own rows."""
+
+    @staticmethod
+    def forward(ctx, part, f_own, attn_l, attn_r, theta, alpha, slope, group, xch):
+        n_own, heads, dim = f_own.shape
+        f_own = f_own.contiguous()
+        f_ext = _fill_halo(part, f_own.view(n_own, heads * dim), 'in', group, xch).view(-1, heads, dim)
+        out, el, er, rowmax, rowsum = _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope)
+        ctx.part, ctx.alpha, ctx.slope, ctx.group, ctx.xch = part, alpha, slope, group, xch
+        ctx.save_for_backward(f_own, el, er, attn_l, attn_r, theta, out, rowmax, rowsum)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_own):
+        f_own, el, er, attn_l, attn_r, theta, out, rowmax, rowsum = ctx.saved_tensors
+        part, xch = ctx.part, ctx.xch
+        n_own, heads, dim = f_own.shape
+        g_own = g_own.reshape(n_own, heads, dim).contiguous()
+        stats = _gat_stats(out, g_own, er, rowmax, rowsum)
+        g_ext, s_ext = _fill_out_halo_gat(part, g_own.view(n_own, heads * dim), stats, ctx.group, xch)
+        rows = part.e_in + part.tail_ptr[-1]
+        dpre = xch.dpre[:rows] if xch is not None else f_own.new_empty((rows, heads))
+        d_feat, d_el = _gat_backward_edges(part, f_own, el, attn_l, theta, ctx.alpha, ctx.slope, g_ext, s_ext, dpre)
+        _return_dpre(part, dpre, ctx.group, xch)
+        d_feat, d_al, d_ar, d_th = _gat_backward_reduce(part, f_own, d_feat, d_el, attn_r, theta, ctx.alpha, dpre)
+        return (None, d_feat, d_al.view_as(attn_l), d_ar.view_as(attn_r),
+                d_th.view_as(theta) if d_th is not None else None, None, None, None, None)
+
+
+def halo_gat(part, f_own, attn_l, attn_r, theta, alpha, slope, group=None, exchange=None, keep=None):
+    """f_own [n_own, H, D] -> out [n_own, H, D] (``part``: this rank's ``HaloPartition`` built with ``attention=True``):
+    the REGAT core of ``functional.gat_layer`` on destination-row blocks, exchanging only halo rows.  ``exchange`` (a
+    ``HaloExchange`` with ``heads=H`` and width H*D): the features, dL/dY and the statistics are pushed over peer memory
+    (regnn_halo_push) and the logit gradients of cut edges are scattered to their owners (regnn_halo_scatter); None:
+    uneven all-to-alls (NCCL / gloo).  ``theta=None`` drops the relation term.  out and d_feat are bit-identical to
+    ``functional.gat_layer``; ``attn_l.grad``, ``attn_r.grad`` and ``theta.grad`` hold this rank's shares
+    (``allreduce_relation_grads``)."""
+    _, heads, dim = f_own.shape
+    if keep is not None:
+        raise ValueError('halo_gat: attention dropout is not supported (its mask is in edge-id order over all edges)')
+    if not getattr(part, 'attention', False):
+        raise ValueError('halo_gat needs a HaloPartition built with attention=True')
+    _check_gat_shape(heads, dim, part.num_relations, theta is not None)
+    if theta is not None and tuple(theta.shape) != (part.num_relations, heads):
+        raise ValueError('halo_gat: theta must be [R=%d, H=%d], got %s' % (part.num_relations, heads, tuple(theta.shape)))
+    if exchange is not None and (exchange.heads != heads or exchange.feat != heads * dim):
+        raise ValueError('halo_gat: the HaloExchange must be built with heads=%d and width %d' % (heads, heads * dim))
+    return _HaloGat.apply(part, f_own, attn_l, attn_r, theta, alpha, slope, group, exchange)
+
+
+def _virtual_halo_gat(parts, f, gout, attn_l, attn_r, theta, alpha, slope, scatter=False):
+    """Every rank of ``HaloPartition.virtual_ranks(..., attention=True)`` one after another in one process (no process
+    group), each on its local views: halos filled by indexing the global [N, H, D] arrays, the dpre tails returned with
+    ``index_copy_`` at the owners' receive lists or -- ``scatter=True`` -- by regnn_halo_scatter into the P local buffers.
+    -> (out, d_feat, d_attn_l, d_attn_r, d_theta | None): rows in global order, parameter gradients summed in rank
+    order."""
+    n, heads, dim = f.shape
+    g2 = gout.reshape(n, heads * dim)
+    bounds = parts[0].bounds
+    own = [slice(bounds[p], bounds[p + 1]) for p in range(len(parts))]
+    fw = [_gat_forward(part, f[part.rows_in], attn_l, attn_r, theta, alpha, slope) for part in parts]
+    stats = torch.cat([_gat_stats(o, gout[s].contiguous(), er, mx, sm) for (o, _, er, mx, sm), s in zip(fw, own)])
+    dpres = [f.new_empty((part.e_in + part.tail_ptr[-1], heads)) for part in parts]
+    edges = [_gat_backward_edges(part, f[s].contiguous(), fw[p][1], attn_l, theta, alpha, slope, g2[part.rows_out],
+                                 stats[part.rows_out], dpres[p]) for p, (part, s) in enumerate(zip(parts, own))]
+    if scatter:
+        ptrs = torch.tensor([d.data_ptr() for d in dpres], dtype=torch.int64, device=f.device)
+        for p, part in enumerate(parts):
+            if part.tail_ptr[-1]:
+                ops.halo_scatter(dpres[p][part.e_in:], part.tail_ptr, part.tail_dst, ptrs, heads, p)
+    else:
+        for q, owner in enumerate(parts):
+            segs = [dpres[p][part.e_in + part.tail_ptr[q]:part.e_in + part.tail_ptr[q + 1]] for p, part in enumerate(parts)]
+            dpres[q].index_copy_(0, owner.dpre_recv, torch.cat(segs))
+    outs, d_feats, d_al, d_ar, d_th = [], [], 0, 0, 0
+    for p, part in enumerate(parts):
+        df, al, ar, th = _gat_backward_reduce(part, f[own[p]].contiguous(), edges[p][0], edges[p][1], attn_r, theta,
+                                              alpha, dpres[p])
+        outs.append(fw[p][0])
+        d_feats.append(df)
+        d_al, d_ar = d_al + al, d_ar + ar
+        d_th = d_th + th if th is not None else None
+    return torch.cat(outs), torch.cat(d_feats), d_al, d_ar, d_th
