@@ -587,6 +587,18 @@ spmm_stream_kernel(StreamArgs sa) {
 // F = 16 -- the extra loads ahead of every row's gathers cost more than the shorter per-row chain saves.
 // Cooperative slot loads pay off where the kernel is issue-bound (fused backward: 2.73 -> 2.44 ms at F = 128,
 // 1.37 -> 1.22 at 64, 0.53 -> 0.50 at 16); the forward kernel is HBM-bound and slightly faster without (2.05 vs 2.14).
+// Dropped (r5a, measured, profiles/r5a_check_l2_hot.jsonl, one B200 at 1000 W): an L2 eviction policy meant to keep the
+// most-gathered rows cached.  Per slot a uint8 gather count min(255, degree of the gathered row), loaded like the edge
+// type; gathers of rows below a threshold (the hot set filling a budget of 32..112 MB) loaded evict-first
+// (createpolicy.fractional.L2::evict_first + ld.global.nc.L2::cache_hint, predicated against a plain load because the
+// policy is a warp-uniform descriptor operand), the index / edge-type / count loads, X[u] and the result stores
+// evict-first too; no L2 set-aside.  Bit-identical, but every arm lost, MAG graph, forward / fused backward (DNORM):
+// F = 128 plain 1.91 / 2.69 ms, streams demoted with every gather hot 2.42 / 2.89, budgets 32..112 MB 2.31..2.36 /
+// 2.81..2.84; F = 64 plain 1.09 / 1.36, streams only 1.22 / 1.47, budgets 1.15..1.17 / 1.45.  The byte model put 22..38 %
+// of the gathers in the hot set at F = 128 (30..56 % at F = 64); demoting the cold gathers won back 0.05..0.1 ms against
+// the streams-only arm, far less than the hinted loads cost (the extra count load per slot, two predicated gathers, and
+// at <false,32> 36 bytes of spill under the 32-register cap).  Hit rates were not measured (no profiler): inferred from
+// time only.  Whole-step bench: 5.04..5.07 ms against 4.77..4.78 for the plain kernels.
 #ifndef REGNN_RG_COOP
 #define REGNN_RG_COOP BINS
 #endif
@@ -726,10 +738,12 @@ spmm_rowgroup_kernel(StreamArgs sa) {
         float ns[U];
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-          const bool ok = idx[u] >= 0;
-          x[u] = ok ? ldg4(reinterpret_cast<const float*>(xbytes + (uint64_t)(uint32_t)idx[u] * ldxb))
-                    : make_float4(0.f, 0.f, 0.f, 0.f);
-          ns[u] = ok ? (a.norm_src != nullptr ? __ldg(a.norm_src + idx[u]) : 1.f) : 0.f;
+          // The gather and the norm[src] load test the slot separately on purpose: with one shared flag the two loads
+          // become one branch, and at the 32-register cap of <false,32> (8 blocks/SM) ptxas spilled 28 bytes inside the
+          // gather loop (552 instructions; 512 and no spill this way).  MAG, F = 128: 2.05 -> 1.89 ms (profiles/r5a_*).
+          x[u] = idx[u] >= 0 ? ldg4(reinterpret_cast<const float*>(xbytes + (uint64_t)(uint32_t)idx[u] * ldxb))
+                             : make_float4(0.f, 0.f, 0.f, 0.f);
+          ns[u] = idx[u] >= 0 ? (a.norm_src != nullptr ? __ldg(a.norm_src + idx[u]) : 1.f) : 0.f;
         }
 #pragma unroll
         for (int u = 0; u < U; ++u) {  // indices of the next round: in flight behind this round's gathers
