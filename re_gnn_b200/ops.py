@@ -334,55 +334,26 @@ def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn
 
 
 def gat_bwd(csr, et_csr, et_t, theta, alpha, feat, el, er, slope, keep, out, rowmax, rowsum, g, attn_l=None,
-            attn_r=None, rows=None):
-    """Backward of ``gat_fwd`` as one gather pass (regnn_gat_bwd_stats -> regnn_gat_bwd_edges -> regnn_gat_bwd_reduce)
+            attn_r=None):
+    """Backward of ``gat_fwd`` as one gather pass (``gat_bwd_stats`` -> ``gat_bwd_edges`` -> ``gat_bwd_reduce``)
     -> (d_feat, d_el, d_er, d_theta | None, d_attn_l | None, d_attn_r | None).
     With ``attn_l`` / ``attn_r`` ([H*D], the projection-score vectors of layer/REGATConv.py:68-69, el = <feat, attn_l>,
     er = <feat, attn_r>) the gradients through the scores are folded in: ``d_feat`` is the total feature gradient and
-    the two parameter gradients are returned (regnn_attn_scores_bwd)."""
-    feat, el, er, keep, g, out = _f32(feat), _f32(el), _f32(er), _f32(keep), _f32(g), _f32(out)
-    n, h, d = feat.shape
-    rb, re = _rows(rows, n)
-    theta, et_csr, r = _rel(theta, et_csr)
-    dev = feat.device
+    the two parameter gradients are returned (``attn_scores_bwd``)."""
+    stats = gat_bwd_stats(out, g, er, rowmax, rowsum)
     e = csr['indices'].numel()
-    full = _full(rb, re, n)
-    fold = attn_l is not None
-    if fold:
-        attn_l, attn_r = _f32(attn_l).view(-1), _f32(attn_r).view(-1)
-    stats = torch.empty((n, h, 4), dtype=torch.float32, device=dev)
-    dpre_csr = torch.empty((max(e, 1), h), dtype=torch.float32, device=dev)[:e]
-    d_feat = torch.empty_like(g) if full else torch.zeros_like(g)
-    d_el = torch.zeros((n, h), dtype=torch.float32, device=dev)
-    d_er = torch.zeros((n, h), dtype=torch.float32, device=dev)
-    partials = torch.empty(max(_lib.partial_blocks(n) * max(r * h, 2 * h * d if fold else 0), 1), dtype=torch.float64,
-                           device=dev)
-    d_theta = torch.zeros((r, h), dtype=torch.float32, device=dev) if r else None   # stays 0 when the graph has no edges
-    sp_t, ws_t = _attn_split(csr.get('split_t'), h, d, dev)
-    sp, ws = _attn_split(csr.get('split'), h, 0, dev)
-    with torch.cuda.device(dev):
-        _lib.call('regnn_gat_bwd_stats', _ptr(out), _ptr(g), _ptr(er), _ptr(rowmax), _ptr(rowsum), n, h, d, _ptr(stats),
-                  _stream())
-        _lib.call('regnn_gat_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
-                  _ptr(et_t) if r else None, _ptr(csr['eid']), _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el),
-                  _ptr(stats), float(slope), _ptr(keep), _ptr(g), h, d, rb, re, _ptr(d_feat), _ptr(d_el), _ptr(dpre_csr),
-                  _ptr(attn_l) if fold else None, sp_t, _ptr(ws_t), _ptr(row_order(csr, True)) if full else None, _stream())
-        _lib.call('regnn_gat_bwd_reduce', _ptr(csr['indptr']), _ptr(et_csr) if r else None, _ptr(theta), float(alpha), r,
-                  _ptr(dpre_csr), h, rb, re, _ptr(d_er), _ptr(partials), _ptr(d_theta), sp, _ptr(ws), _stream())
-        _lib.count_launches(3 + ((1 if re - rb >= 65536 else 2) if r else 0) + (3 if sp_t is not None else 0) + (sp is not None))
-        d_al = d_ar = None
-        if fold:
-            d_al = torch.empty(h * d, dtype=torch.float32, device=dev)
-            d_ar = torch.empty(h * d, dtype=torch.float32, device=dev)
-            _lib.call('regnn_attn_scores_bwd', _ptr(feat), _ptr(d_el), _ptr(d_er), n, h, d, _ptr(partials), _ptr(d_al),
-                      _ptr(d_ar), _ptr(d_feat), _ptr(attn_r), _stream())
-            _lib.count_launches(3)
+    dpre = torch.empty((max(e, 1), stats.shape[1]), dtype=torch.float32, device=stats.device)[:e]   # never a NULL pointer
+    d_feat, d_el = gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=attn_l, keep=keep)
+    d_er, d_theta = gat_bwd_reduce(csr, et_csr, theta, alpha, dpre)
+    d_al = d_ar = None
+    if attn_l is not None:
+        d_al, d_ar = attn_scores_bwd(feat, d_el, d_er, attn_r=attn_r, d_feat=d_feat)
     return d_feat, d_el, d_er, d_theta, d_al, d_ar
 
 
-# The stages of ``gat_bwd`` one by one, for callers that move data between them (partition.halo_gat exchanges the
-# statistics before the edge pass and the per-slot logit gradients between the edge pass and the reduction).  Full row
-# ranges, no attention dropout.
+# The stages of ``gat_bwd``, which is built from them.  partition.halo_gat calls them one at a time, to exchange the
+# statistics before the edge pass and the per-slot logit gradients between the edge pass and the reduction.  Full row
+# ranges.
 
 def gat_bwd_stats(out, g, er, rowmax, rowsum):
     """-> stats [N, H, 4] = (er, rowmax, 1/rowsum, <out, G>) per (row, head) (regnn_gat_bwd_stats)."""
@@ -396,12 +367,13 @@ def gat_bwd_stats(out, g, er, rowmax, rowsum):
     return stats
 
 
-def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=None):
+def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=None, keep=None):
     """Source-major pass over the rows of the transposed view ``csr['indptr_t']`` -> (d_feat, d_el) of those rows; the
     logit gradient of every entry j is written to ``dpre[csr['slot_t'][j]]`` ([slots, H]).  ``feat`` / ``el``: the rows'
     own values; ``g`` / ``stats``: indexed by the column ids of the view.  ``attn_l`` folds the gradient through el into
-    d_feat (regnn_gat_bwd_edges)."""
-    feat, el, g = _f32(feat), _f32(el), _f32(g)
+    d_feat; ``keep``: the attention-dropout mask of ``gat_fwd``, in edge-id order through ``csr['eid']``
+    (regnn_gat_bwd_edges)."""
+    feat, el, g, keep = _f32(feat), _f32(el), _f32(g), _f32(keep)
     theta, et_t, r = _rel(theta, et_t)
     n = csr['indptr_t'].numel() - 1
     _, h, d = feat.shape
@@ -412,9 +384,9 @@ def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn
     sp_t, ws_t = _attn_split(csr.get('split_t'), h, d, dev)
     with torch.cuda.device(dev):
         _lib.call('regnn_gat_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
-                  _ptr(et_t) if r else None, None, _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el), _ptr(stats),
-                  float(slope), None, _ptr(g), h, d, 0, n, _ptr(d_feat), _ptr(d_el), _ptr(dpre), _ptr(attn_l), sp_t,
-                  _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
+                  _ptr(et_t) if r else None, _ptr(csr['eid']) if keep is not None else None, _ptr(theta), float(alpha),
+                  r, _ptr(feat), _ptr(el), _ptr(stats), float(slope), _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_feat),
+                  _ptr(d_el), _ptr(dpre), _ptr(attn_l), sp_t, _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
         _lib.count_launches(1 + (3 if sp_t is not None else 0))
     return d_feat, d_el
 
@@ -503,46 +475,41 @@ def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_at
 V2_STAGE_CHUNKS = 592   # REGNN_V2_STAGE_CHUNKS (csrc/gat.cu)
 
 
-def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax, rowsum, saved, g, rows=None):
-    """Backward of ``gatv2_fwd(..., save=True)``: regnn_gat_bwd_stats -> regnn_gatv2_bwd_edges (the one gather pass) ->
+def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax, rowsum, saved, g):
+    """Backward of ``gatv2_fwd(..., save=True)``: ``gat_bwd_stats`` -> regnn_gatv2_bwd_edges (the one gather pass) ->
     regnn_gatv2_bwd_dst (streaming) -> (d_fs, d_fd, d_attn [H*D], d_theta | None)."""
-    fs, fd, keep, g, out = _f32(fs), _f32(fd), _f32(keep), _f32(g), _f32(out)
+    fs, fd, keep, g = _f32(fs), _f32(fd), _f32(keep), _f32(g)
     attn = _f32(attn).view(-1)
     logit_csr, qmask = saved
     n, h, d = fd.shape
-    rb, re = _rows(rows, n)
     theta, et_csr, r = _rel(theta, et_csr)
     dev = fs.device
     e = csr['indices'].numel()
-    full = _full(rb, re, n)
-    stats = torch.empty((n, h, 4), dtype=torch.float32, device=dev)
+    stats = gat_bwd_stats(out, g, None, rowmax, rowsum)
     dl_csr = torch.empty((max(e, 1), h), dtype=torch.float32, device=dev)
-    d_fs = torch.empty_like(g) if full else torch.zeros_like(g)
-    d_fd = torch.empty_like(fd) if full else torch.zeros_like(fd)
+    d_fs = torch.empty_like(g)
+    d_fd = torch.empty_like(fd)
     d_attn_src = torch.empty(h * d, dtype=torch.float32, device=dev)
     d_attn_dst = torch.empty(h * d, dtype=torch.float32, device=dev)
     d_theta = torch.zeros((r, h), dtype=torch.float32, device=dev) if r else None   # stays 0 when the graph has no edges
     split_t, split = csr.get('split_t'), csr.get('split')
     sp_t, ws_t = _attn_split(split_t, h, d, dev)
     sp, ws = _attn_split(split, h, d, dev)
-    order_t = row_order(csr, True) if full else None
-    nblocks = _lib.load().regnn_gatv2_bwd_edges_blocks(re - rb, split_t['struct'].num_frags if split_t else 0,
-                                                       split_t['struct'].num_long if split_t else 0, h, d,
-                                                       int(order_t is not None))
+    order_t = row_order(csr, True)
+    nblocks = _lib.load().regnn_gatv2_bwd_edges_blocks(n, split_t['struct'].num_frags if split_t else 0,
+                                                       split_t['struct'].num_long if split_t else 0, h, d, 1)
     block_partials = torch.empty(max(nblocks, 1) * h * d, dtype=torch.float32, device=dev)
     partials = torch.empty(max(_lib.partial_blocks() * h * d, V2_STAGE_CHUNKS * max(r * h, h * d)), dtype=torch.float64,
                            device=dev)
     with torch.cuda.device(dev):
-        _lib.call('regnn_gat_bwd_stats', _ptr(out), _ptr(g), None, _ptr(rowmax), _ptr(rowsum), n, h, d, _ptr(stats),
-                  _stream())
         _lib.call('regnn_gatv2_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
                   _ptr(csr['eid']), _ptr(fs), _ptr(stats), _ptr(logit_csr), _ptr(qmask), _ptr(attn), float(slope),
-                  _ptr(keep), _ptr(g), h, d, rb, re, _ptr(d_fs), _ptr(dl_csr), _ptr(d_attn_src), _ptr(block_partials),
+                  _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_fs), _ptr(dl_csr), _ptr(d_attn_src), _ptr(block_partials),
                   _ptr(partials), sp_t, _ptr(ws_t), _ptr(order_t), _stream())
         _lib.call('regnn_gatv2_bwd_dst', _ptr(csr['indptr']), _ptr(et_csr) if r else None, _ptr(theta), float(alpha), r,
-                  _ptr(fd), _ptr(dl_csr), _ptr(qmask), _ptr(attn), float(slope), h, d, rb, re, _ptr(d_fd),
+                  _ptr(fd), _ptr(dl_csr), _ptr(qmask), _ptr(attn), float(slope), h, d, 0, n, _ptr(d_fd),
                   _ptr(d_attn_dst), _ptr(partials), _ptr(d_theta), sp, _ptr(ws), _stream())
-        _lib.count_launches(6 + (2 if r else 0) + (sp_t is not None) + (sp is not None))
+        _lib.count_launches(5 + (2 if r else 0) + (sp_t is not None) + (sp is not None))
     return d_fs, d_fd, d_attn_src + d_attn_dst, d_theta
 
 

@@ -333,127 +333,92 @@ def feature_sliced_propagate(graph, etv, x_own, theta, alpha, norm, bounds, rank
     return _ColumnSlabPropagate.apply(graph, etv, x_own, theta, alpha, norm, bounds, rank, group)
 
 
+def _rows_to_head_slab(own, n, bounds, rank, group, xch, grad=False):
+    """Row block [rows_own, H, D] -> this rank's head slab of all N rows [N, H*D/P]: one all-to-all, or (``xch``) pushed
+    into every rank's ``x_cols`` (``g_cols`` with ``grad``) over peer memory."""
+    own = own.flatten(1).contiguous()      # [0, H*D] for a rank that owns no rows
+    if xch is None:
+        return _rows_to_columns(own, _uniform_rows(bounds), len(bounds) - 1, group)[:n]
+    cols, ptrs = (xch.g_cols, xch.g_ptrs) if grad else (xch.x_cols, xch.x_ptrs)
+    ops.rows_to_slabs(own, xch.parts, rank * xch.per, ptrs)
+    xch.barrier()            # every rank's rows of my heads have landed in my slab
+    return cols[:n]
+
+
+def _head_slab_to_rows(slab, rows_own, bounds, group, xch, grad=False):
+    """Inverse of ``_rows_to_head_slab``: head slab [N, H/P, D] -> this rank's row block [rows_own, H*D], through
+    ``xch.y_rows`` (``dx_rows`` with ``grad``) over peer memory."""
+    n = slab.shape[0]
+    slab = slab.flatten(1)
+    if xch is None:
+        parts, per = len(bounds) - 1, _uniform_rows(bounds)
+        pad = torch.cat([slab, slab.new_zeros((parts * per - n, slab.shape[1]))]) if parts * per > n else slab
+        return _columns_to_rows(pad.contiguous(), per, parts, rows_own, group)
+    ops.slabs_to_rows(slab, n, xch.peer_dx if grad else xch.peer_y)
+    xch.barrier()            # every rank's heads of my rows have landed in my row block
+    return (xch.dx_rows if grad else xch.y_rows)[:rows_own].clone()
+
+
+def _head_slice_grad(param, grad, sl):
+    """The gradient of a [*, H, ...] parameter with this rank's head slice ``sl`` filled and zeros elsewhere."""
+    if grad is None:
+        return None
+    full = torch.zeros_like(param)
+    full[:, sl] = grad.view(full[:, sl].shape)
+    return full
+
+
 class _HeadSlicedGat(torch.autograd.Function):
     """REGAT core (projection scores + fused logits / edge softmax / aggregation) sharded over the HEADS: attention
     heads are independent (el / er, the softmax statistics and the aggregation never mix heads), so rank q runs all
-    rows for heads [q*H/P, (q+1)*H/P) -- the same column-slab scheme as the REGCN aggregation, with the row <-> slab
-    re-partition done by one all-to-all on each side (NCCL; gloo in the CPU tests).  Row block in, row block out;
-    parameter gradients (attn_l, attn_r, relation embedding) come back with this rank's head slice filled and zeros
-    elsewhere: the caller sums them across ranks (``allreduce_relation_grads``)."""
+    rows for heads [q*H/P, (q+1)*H/P) -- the same column-slab scheme as the REGCN aggregation.  The four row <-> slab
+    re-partitions (``_rows_to_head_slab``, ``_head_slab_to_rows``) are one all-to-all each (NCCL; gloo in the CPU tests)
+    or, with a ``SlabExchange`` ``xch`` of width H*D, our own kernels over peer memory (regnn_rows_to_slabs,
+    regnn_slabs_to_rows), where the head slab of the features stays in ``xch.x_cols`` for the backward.  Row block in,
+    row block out; parameter gradients (attn_l, attn_r, relation embedding) come back with this rank's head slice filled
+    and zeros elsewhere: the caller sums them across ranks (``allreduce_relation_grads``)."""
 
     @staticmethod
-    def forward(ctx, graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group):
+    def forward(ctx, graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, xch):
         csr = graph.csr()
         n = graph.number_of_nodes()
-        parts, per = len(bounds) - 1, _uniform_rows(bounds)
         rows_own, heads, dim = f_own.shape
-        if not per or heads % parts:
-            raise ValueError('head-sliced attention needs equal row blocks and num_heads divisible by the number of ranks')
-        hs = heads // parts
+        hs = heads // (len(bounds) - 1)
         sl = slice(rank * hs, (rank + 1) * hs)
-        f_cols = _rows_to_columns(f_own.reshape(rows_own, heads * dim), per, parts, group)[:n].view(n, hs, dim)
+        f_cols = _rows_to_head_slab(f_own, n, bounds, rank, group, xch).view(n, hs, dim)
         al, ar = attn_l[:, sl].contiguous(), attn_r[:, sl].contiguous()
         th = theta[:, sl].contiguous() if etv is not None else None
-        et = etv[0] if etv is not None else None
         el, er = ops.attn_scores_fwd(f_cols, al, ar)
-        out, rowmax, rowsum, _ = ops.gat_fwd(csr, et, th, alpha, f_cols, el, er, slope)
-        ctx.graph, ctx.etv, ctx.alpha, ctx.slope, ctx.bounds, ctx.rank, ctx.group = graph, etv, alpha, slope, bounds, rank, group
-        ctx.shape, ctx.sl = (rows_own, heads, dim), sl
+        out, rowmax, rowsum, _ = ops.gat_fwd(csr, etv[0] if etv is not None else None, th, alpha, f_cols, el, er, slope)
+        ctx.graph, ctx.etv, ctx.alpha, ctx.slope, ctx.bounds, ctx.rank, ctx.group, ctx.xch = \
+            graph, etv, alpha, slope, bounds, rank, group, xch
+        ctx.sl = sl
         ctx.save_for_backward(f_cols, el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta)
-        pad = torch.cat([out.view(n, hs * dim), out.new_zeros((parts * per - n, hs * dim))]) if parts * per > n else out.view(n, hs * dim)
-        return _columns_to_rows(pad.contiguous(), per, parts, rows_own, group).view(rows_own, heads, dim)
+        return _head_slab_to_rows(out, rows_own, bounds, group, xch).view(rows_own, heads, dim)
 
     @staticmethod
     def backward(ctx, g_own):
         f_cols, el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta = ctx.saved_tensors
-        csr = ctx.graph.csr()
-        rows_own, heads, dim = ctx.shape
-        n = ctx.graph.number_of_nodes()
-        parts, per = len(ctx.bounds) - 1, _uniform_rows(ctx.bounds)
-        hs = heads // parts
-        g_cols = _rows_to_columns(g_own.reshape(rows_own, heads * dim).contiguous(), per, parts, ctx.group)[:n].view(n, hs, dim)
+        n, hs, dim = f_cols.shape
+        rows_own, heads, _ = g_own.shape
+        g_cols = _rows_to_head_slab(g_own, n, ctx.bounds, ctx.rank, ctx.group, ctx.xch, grad=True).view(n, hs, dim)
         et, et_t = (ctx.etv[0], ctx.etv[1]) if ctx.etv is not None else (None, None)
-        d_f, _, _, d_th, d_al, d_ar = ops.gat_bwd(csr, et, et_t, th, ctx.alpha, f_cols, el, er, ctx.slope, None, out,
-                                                   rowmax, rowsum, g_cols.contiguous(), attn_l=al, attn_r=ar)
-        pad = torch.cat([d_f.view(n, hs * dim), d_f.new_zeros((parts * per - n, hs * dim))]) if parts * per > n else d_f.view(n, hs * dim)
-        d_f_own = _columns_to_rows(pad.contiguous(), per, parts, rows_own, ctx.group).view(rows_own, heads, dim)
-        g_al, g_ar = torch.zeros_like(attn_l), torch.zeros_like(attn_r)
-        g_al[:, ctx.sl] = d_al.view(1, hs, dim)
-        g_ar[:, ctx.sl] = d_ar.view(1, hs, dim)
-        g_th = None
-        if d_th is not None:
-            g_th = torch.zeros_like(theta)
-            g_th[:, ctx.sl] = d_th
-        return None, None, d_f_own, g_al, g_ar, g_th, None, None, None, None, None
-
-
-class _PeerHeadSlicedGat(torch.autograd.Function):
-    """``_HeadSlicedGat`` with the four re-partitions done by our own kernels over peer memory (a ``SlabExchange`` of
-    width H*D): row blocks are pushed into the peers' head slabs (regnn_rows_to_slabs), the finished head slab is pushed
-    back to the row owners (regnn_slabs_to_rows) -- no collective library call, no pack / unpack pass.  The head slab of
-    the features stays in the exchange buffer for the backward pass."""
-
-    @staticmethod
-    def forward(ctx, graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, xch):
-        csr = graph.csr()
-        n = graph.number_of_nodes()
-        parts = xch.parts
-        rows_own, heads, dim = f_own.shape
-        if heads % parts or xch.feat != heads * dim:
-            raise ValueError('peer head-sliced attention needs num_heads divisible by the number of ranks and a '
-                             'SlabExchange of width num_heads * head_dim')
-        hs = heads // parts
-        sl = slice(rank * hs, (rank + 1) * hs)
-        ops.rows_to_slabs(f_own.reshape(rows_own, heads * dim).contiguous(), parts, rank * xch.per, xch.x_ptrs)
-        xch.barrier()            # every rank's rows of my heads have landed in my slab
-        f_cols = xch.x_cols[:n].view(n, hs, dim)
-        al, ar = attn_l[:, sl].contiguous(), attn_r[:, sl].contiguous()
-        th = theta[:, sl].contiguous() if etv is not None else None
-        et = etv[0] if etv is not None else None
-        el, er = ops.attn_scores_fwd(f_cols, al, ar)
-        out, rowmax, rowsum, _ = ops.gat_fwd(csr, et, th, alpha, f_cols, el, er, slope)
-        ops.slabs_to_rows(out.view(n, hs * dim), n, xch.peer_y)
-        xch.barrier()            # every rank's heads of my rows have landed in my row block
-        ctx.graph, ctx.etv, ctx.alpha, ctx.slope, ctx.rank, ctx.xch = graph, etv, alpha, slope, rank, xch
-        ctx.shape, ctx.sl = (rows_own, heads, dim), sl
-        ctx.save_for_backward(el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta)
-        return xch.y_rows[:rows_own].clone().view(rows_own, heads, dim)
-
-    @staticmethod
-    def backward(ctx, g_own):
-        el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta = ctx.saved_tensors
-        xch, rank = ctx.xch, ctx.rank
-        csr = ctx.graph.csr()
-        rows_own, heads, dim = ctx.shape
-        n = ctx.graph.number_of_nodes()
-        parts = xch.parts
-        hs = heads // parts
-        ops.rows_to_slabs(g_own.reshape(rows_own, heads * dim).contiguous(), parts, rank * xch.per, xch.g_ptrs)
-        xch.barrier()
-        f_cols = xch.x_cols[:n].view(n, hs, dim)
-        g_cols = xch.g_cols[:n].view(n, hs, dim)
-        et, et_t = (ctx.etv[0], ctx.etv[1]) if ctx.etv is not None else (None, None)
-        d_f, _, _, d_th, d_al, d_ar = ops.gat_bwd(csr, et, et_t, th, ctx.alpha, f_cols, el, er, ctx.slope, None, out,
-                                                   rowmax, rowsum, g_cols, attn_l=al, attn_r=ar)
-        ops.slabs_to_rows(d_f.view(n, hs * dim), n, xch.peer_dx)
-        xch.barrier()
-        d_f_own = xch.dx_rows[:rows_own].clone().view(rows_own, heads, dim)
-        g_al, g_ar = torch.zeros_like(attn_l), torch.zeros_like(attn_r)
-        g_al[:, ctx.sl] = d_al.view(1, hs, dim)
-        g_ar[:, ctx.sl] = d_ar.view(1, hs, dim)
-        g_th = None
-        if d_th is not None:
-            g_th = torch.zeros_like(theta)
-            g_th[:, ctx.sl] = d_th
-        return None, None, d_f_own, g_al, g_ar, g_th, None, None, None, None, None
+        d_f, _, _, d_th, d_al, d_ar = ops.gat_bwd(ctx.graph.csr(), et, et_t, th, ctx.alpha, f_cols, el, er, ctx.slope,
+                                                   None, out, rowmax, rowsum, g_cols, attn_l=al, attn_r=ar)
+        d_f_own = _head_slab_to_rows(d_f, rows_own, ctx.bounds, ctx.group, ctx.xch, grad=True).view(rows_own, heads, dim)
+        return (None, None, d_f_own, _head_slice_grad(attn_l, d_al, ctx.sl), _head_slice_grad(attn_r, d_ar, ctx.sl),
+                _head_slice_grad(theta, d_th, ctx.sl), None, None, None, None, None, None)
 
 
 def head_sliced_gat(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group=None, exchange=None):
     """f_own [rows_own, H, D] -> out rows [rows_own, H, D]; see ``_HeadSlicedGat``.  ``exchange`` (a ``SlabExchange`` of
     width H*D): the re-partitions run over peer memory inside our own kernels instead of NCCL / gloo all-to-alls."""
-    if exchange is not None:
-        return _PeerHeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, exchange)
-    return _HeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group)
+    _, heads, dim = f_own.shape
+    if not _uniform_rows(bounds) or heads % (len(bounds) - 1):
+        raise ValueError('head-sliced attention needs equal row blocks and num_heads divisible by the number of ranks')
+    if exchange is not None and exchange.feat != heads * dim:
+        raise ValueError('head-sliced attention over peer memory needs a SlabExchange of width num_heads * head_dim')
+    return _HeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, exchange)
 
 
 def allreduce_relation_grads(params, group=None, exchange=None):

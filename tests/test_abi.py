@@ -110,6 +110,23 @@ def test_scatter_entry_points_validate_arguments(lib):
                                             None, None, 0, None, None, None, None, ctypes.byref(peers), None) == -1
 
 
+def test_every_entry_point_is_called_from_one_wrapper():
+    """ops.py's contract, one Python function per C-ABI entry point: each regnn_* name passed to ``_lib.call`` appears
+    in exactly one call of the package, so a change to an entry point's arguments, buffers or launch count has one
+    place to go."""
+    import collections
+    import glob
+    counts, calls = collections.Counter(), 0
+    for path in glob.glob(os.path.join(ROOT, 're_gnn_b200', '*.py')):
+        with open(path) as f:
+            text = f.read()
+        calls += text.count('_lib.call(')
+        counts.update(re.findall(r"_lib\.call\(\s*'(regnn_\w+)'", text))
+    assert counts and sum(counts.values()) == calls, 'every _lib.call names its entry point as a literal'
+    shared = {name: c for name, c in counts.items() if c > 1}
+    assert not shared, shared
+
+
 def test_integration_doc_lists_every_entry_point():
     """INTEGRATION.md maps every exported symbol to the reference call site it replaces."""
     text = open(os.path.join(ROOT, 'INTEGRATION.md')).read()

@@ -109,15 +109,19 @@ def _attn_worker(rank, world, port, ret, kind):
         def setattr(obj, name, val):
             setattr(obj, name, val)
     cpu_shim.install(MP)
-    d = synth.hetero_graph('imdb', seed=7, scale=0.02)
+    if kind == 'gat_empty_block':   # 4 rows over 3 ranks: bounds [0, 2, 4, 4], the last rank owns no rows
+        d = dict(src=np.array([0, 1, 2, 3, 0, 2]), dst=np.array([1, 2, 3, 0, 0, 1]),
+                 etype=np.array([1, 2, 1, 2, 2, 1]), num_nodes=4, num_relations=2)
+    else:
+        d = synth.hetero_graph('imdb', seed=7, scale=0.02)
     n, r = d['num_nodes'], d['num_relations']
     rng = np.random.RandomState(1)
     g = Graph(d['src'], d['dst'], n)
     etv = g.etype_views(torch.as_tensor(d['etype']), r)
     bounds = partition.row_blocks(g.csr()['indptr'], world, balance='rows')
     rb, re = bounds[rank], bounds[rank + 1]
-    if kind == 'gat':
-        heads, dim = 4, 8
+    if kind != 'mixhop':
+        heads, dim = (3, 8) if kind == 'gat_empty_block' else (4, 8)
         f = torch.as_tensor(rng.randn(n, heads, dim) * 0.5)
         gout = torch.as_tensor(rng.randn(n, heads, dim))
         al0, ar0 = torch.as_tensor(rng.randn(1, heads, dim) * 0.3), torch.as_tensor(rng.randn(1, heads, dim) * 0.3)
@@ -159,4 +163,15 @@ def test_sharded_attention_and_mixhop_match_single_process_world2(kind):
     port = 23500 + (os.getpid() % 2000) + (0 if kind == 'gat' else 2500)
     ret = mp.get_context('spawn').Manager().dict()
     mp.spawn(_attn_worker, args=(world, port, ret, kind), nprocs=world, join=True)
+    assert all(ret.get(r) for r in range(world)), dict(ret)
+
+
+@pytest.mark.timeout(300)
+def test_head_sliced_attention_with_an_empty_row_block_world3():
+    """A rank whose row block is empty (row_blocks(..., balance='rows') gives [0, 2, 4, 4] for 4 rows over 3 ranks)
+    still takes part in every all-to-all of the forward and the backward."""
+    world = 3
+    port = 19000 + (os.getpid() % 2000)
+    ret = mp.get_context('spawn').Manager().dict()
+    mp.spawn(_attn_worker, args=(world, port, ret, 'gat_empty_block'), nprocs=world, join=True)
     assert all(ret.get(r) for r in range(world)), dict(ret)
