@@ -227,6 +227,18 @@ int regnn_halo_push(const float* X, int64_t ldx, int feat, const int32_t* send_r
 int regnn_halo_scatter(const float* X, int64_t ldx, int width, const int64_t* send_ptr, const int32_t* dst_rows,
                        float* const* peer_bufs, int64_t ldb, int num_ranks, int rank, void* stream);
 
+/* The per-slot forward exchange of the REGATv2 halo backward (partition.halo_gatv2: regnn_gatv2_bwd_edges runs on the
+ * owner of an edge's source, but regnn_gatv2_fwd stored the edge's logit and sign mask in its destination's slot): for
+ * every peer q and k in send_ptr[q] .. send_ptr[q+1], slot s = send_slots[k] is stored to row
+ * r = recv_offset[q] + (k - send_ptr[q]) of peer q's buffers: logit[s*H .. +H) to peer_logit[q] + r*H and
+ * qmask[s*4C .. +4C) to peer_mask[q] + r*4C (C = num_chunks 128-bit words, the layout of regnn_gatv2_fwd's qmask).  Both
+ * arrays move in one launch.  send_ptr [num_ranks+1] and recv_offset [num_ranks] are HOST arrays; send_slots (int32) and
+ * peer_logit / peer_mask [num_ranks] are device arrays; lists may be empty.  Local buffers work the same as peer-mapped
+ * ones.  qmask 16-byte aligned, num_ranks <= REGNN_HALO_MAX_RANKS. */
+int regnn_halo_push_slots(const float* logit, int num_heads, const uint32_t* qmask, int num_chunks,
+                          const int32_t* send_slots, const int64_t* send_ptr, const int64_t* recv_offset,
+                          float* const* peer_logit, float* const* peer_mask, int num_ranks, int rank, void* stream);
+
 /* The reverse re-partition for kernels without a scatter epilogue (the fused attention kernels, one head slice per
  * rank): S [num_rows, feat] is this rank's column slab (ld lds); row v is stored to
  * peers->base[v / rows_per_rank][(v % rows_per_rank) * ld + col_offset .. + feat). */

@@ -37,6 +37,7 @@ SIGNATURES = {
     'regnn_slabs_to_rows': (_i32, [_p, _i64, _i64, _i32, _p, _p]),
     'regnn_halo_push': (_i32, [_p, _i64, _i32, _p, _p, _p, _p, _i64, _i32, _i32, _p]),
     'regnn_halo_scatter': (_i32, [_p, _i64, _i32, _p, _p, _p, _i64, _i32, _i32, _p]),
+    'regnn_halo_push_slots': (_i32, [_p, _i32, _p, _i32, _p, _p, _p, _p, _p, _i32, _i32, _p]),
     'regnn_spmm_fwd_scatter': (_i32, [_p, _p, _p, _p, _f32, _i32, _p, _p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _p, _i64,
                                       _p]),
     'regnn_spmm_bwd_fused_scatter': (_i32, [_p, _p, _p, _p, _f32, _i32, _p, _i32, _p, _i64, _p, _i64, _i64, _i32,

@@ -207,6 +207,33 @@ __global__ void halo_scatter_kernel(const float* __restrict__ X, int64_t ldx, in
   }
 }
 
+// Indexed per-slot push of the REGATv2 halo backward, the transpose of halo_scatter_kernel: the forward stored the logit
+// and the sign mask of an edge in its destination's in-view slot, but the source-major edge pass runs on the owner of
+// the source.  For k in ptr[q] .. ptr[q+1], slot s = send_slots[k] goes to row recv_offset[q] + (k - ptr[q]) of peer
+// q's two buffers: logit[s, 0:H] (4-byte words) and mask[s, 0:C] (C = ceil(H*D/128) 128-bit words).  One group of G
+// lanes per slot (G = H + C rounded up to a power of two, at most 32): the slot index is loaded once per group, lanes
+// [0, C) move the mask words and lanes [C, C+H) the logits.  Peers in rank-rotated order as in halo_push_kernel.
+__global__ void halo_push_slots_kernel(const float* __restrict__ logit, int H, const uint4* __restrict__ mask, int C,
+                                       int G, const int32_t* __restrict__ send_slots, const __grid_constant__ HaloPeers hp,
+                                       float* const* __restrict__ peer_logit, float* const* __restrict__ peer_mask,
+                                       int first_peer) {
+  const int q = (int)((blockIdx.y + (unsigned)first_peer) % gridDim.y);
+  const int64_t begin = hp.ptr[q];
+  const int64_t cnt = hp.ptr[q + 1] - begin;
+  if (cnt == 0) return;
+  float* dl = peer_logit[q] + hp.recv_offset[q] * H;
+  uint4* dm = reinterpret_cast<uint4*>(peer_mask[q]) + hp.recv_offset[q] * C;
+  const int lane = threadIdx.x % G, W = C + H;
+  const int64_t groups = (int64_t)gridDim.x * (blockDim.x / G);
+  for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G; i < cnt; i += groups) {
+    const int64_t s = __ldg(send_slots + begin + i);
+    for (int c = lane; c < W; c += G) {
+      if (c < C) dm[i * C + c] = __ldg(mask + s * C + c);
+      else dl[i * H + (c - C)] = __ldg(logit + s * H + (c - C));
+    }
+  }
+}
+
 // Column slab -> row blocks over peer memory, for the kernels that have no scatter epilogue of their own (the fused
 // attention kernels: one head slice per rank): rows [q*per, (q+1)*per) of this rank's slab S [N, Fc] go to rank q's row
 // block at column col_offset.  The local read is contiguous, every destination row gets one Fc*4-byte store burst
@@ -1607,6 +1634,40 @@ extern "C" int regnn_halo_scatter(const float* X, int64_t ldx, int width, const 
   halo_scatter_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(X, ldx, width, dst_rows, hp,
                                                                                      peer_bufs, ldb, rank);
   return check_launch("regnn_halo_scatter");
+}
+
+extern "C" int regnn_halo_push_slots(const float* logit, int num_heads, const uint32_t* qmask, int num_chunks,
+                                     const int32_t* send_slots, const int64_t* send_ptr, const int64_t* recv_offset,
+                                     float* const* peer_logit, float* const* peer_mask, int num_ranks, int rank,
+                                     void* stream) {
+  REGNN_REQUIRE(logit && qmask && send_ptr && recv_offset && peer_logit && peer_mask && num_heads >= 1 &&
+                    num_chunks >= 1 && num_ranks >= 1 && rank >= 0 && rank < num_ranks,
+                REGNN_ERR_INVALID_ARG, "halo_push_slots: bad argument");
+  REGNN_REQUIRE(num_ranks <= REGNN_HALO_MAX_RANKS, REGNN_ERR_UNSUPPORTED_SHAPE, "halo_push_slots: %d ranks (max %d)",
+                num_ranks, REGNN_HALO_MAX_RANKS);
+  REGNN_REQUIRE(aligned_to(qmask, 16), REGNN_ERR_UNSUPPORTED_SHAPE,
+                "halo_push_slots: the mask rows must be 16-byte aligned 128-bit words");
+  REGNN_REQUIRE(send_ptr[0] >= 0, REGNN_ERR_INVALID_ARG, "halo_push_slots: negative send offset");
+  HaloPeers hp;
+  int64_t most = 0;
+  hp.ptr[0] = send_ptr[0];
+  for (int q = 0; q < num_ranks; ++q) {
+    const int64_t cnt = send_ptr[q + 1] - send_ptr[q];
+    REGNN_REQUIRE(cnt >= 0 && recv_offset[q] >= 0, REGNN_ERR_INVALID_ARG,
+                  "halo_push_slots: peer %d has a negative slot count or receive offset", q);
+    hp.ptr[q + 1] = send_ptr[q + 1];
+    hp.recv_offset[q] = recv_offset[q];
+    most = cnt > most ? cnt : most;
+  }
+  if (most == 0) return REGNN_OK;
+  REGNN_REQUIRE(send_slots != nullptr, REGNN_ERR_INVALID_ARG, "halo_push_slots: null send list");
+  int G = 1;
+  while (G < num_heads + num_chunks && G < 32) G <<= 1;
+  const int64_t want = (most * G + 255) / 256;
+  const unsigned bx = (unsigned)(want < 148 * 8 ? want : 148 * 8);
+  halo_push_slots_kernel<<<dim3(bx, (unsigned)num_ranks), 256, 0, (cudaStream_t)stream>>>(
+      logit, num_heads, reinterpret_cast<const uint4*>(qmask), num_chunks, G, send_slots, hp, peer_logit, peer_mask, rank);
+  return check_launch("regnn_halo_push_slots");
 }
 
 extern "C" int regnn_slabs_to_rows(const float* S, int64_t lds, int64_t num_rows, int feat,

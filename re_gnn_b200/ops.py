@@ -238,6 +238,21 @@ def halo_scatter(x, send_ptr, dst_rows, peer_buf_ptrs, ldb, rank):
         _lib.count_launches(1 if send_ptr[-1] > send_ptr[0] else 0)
 
 
+def halo_push_slots(logit, qmask, send_slots, send_ptr, recv_offset, peer_logit_ptrs, peer_mask_ptrs, rank):
+    """Stores the per-slot records ``logit[s]`` ([E, H] fp32) and ``qmask[s]`` ([E, C, 4] int32, the sign masks of
+    ``gatv2_fwd(save=True)``) of the slots ``s = send_slots[send_ptr[q]:send_ptr[q+1]]`` to rows ``recv_offset[q], ...``
+    of peer q's logit and mask buffers (regnn_halo_push_slots).  ``send_slots``: int32 device tensor; ``send_ptr``
+    [P+1] / ``recv_offset`` [P]: host sequences of ints; ``peer_*_ptrs``: int64 device tensors [P] of buffer base
+    addresses (rows of H floats and of C 128-bit words)."""
+    logit = _f32(logit)
+    p = len(recv_offset)
+    with torch.cuda.device(logit.device):
+        _lib.call('regnn_halo_push_slots', _ptr(logit), logit.shape[1], _ptr(qmask), qmask.shape[1], _ptr(send_slots),
+                  (ctypes.c_int64 * (p + 1))(*send_ptr), (ctypes.c_int64 * p)(*recv_offset), _ptr(peer_logit_ptrs),
+                  _ptr(peer_mask_ptrs), p, int(rank), _stream())
+        _lib.count_launches(1 if send_ptr[-1] > send_ptr[0] else 0)
+
+
 def slabs_to_rows(slab, num_rows, peers):
     """Pushes rows [0, num_rows) of this rank's column slab ``slab`` [>= num_rows, F/P] to their owner ranks' row blocks
     (regnn_slabs_to_rows; ``peers``: a ``_lib.PeerRows``)."""
@@ -439,10 +454,15 @@ def attn_scores_fwd(feat, attn_l, attn_r):
     return el, er
 
 
-def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_attn=False, rows=None, save=False):
+def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_attn=False, rows=None, save=False,
+              saved=None):
     """-> (out, rowmax, rowsum, attention | None, saved | None).  ``save``: also store what the backward needs, the raw
     logit of every (CSR slot, head) and the 128-bit sign mask of fs[src]+fd[dst] per (slot, 128-float slice):
-    ``saved = (logit_csr [E,H], qmask [E, ceil(H*D/128), 4] int32)``."""
+    ``saved = (logit_csr [E,H], qmask [E, ceil(H*D/128), 4] int32)``.  ``saved`` given (implies ``save``): the caller's
+    buffers of that layout with at least E rows, written in place (partition.halo_gatv2 passes the head of its
+    per-slot exchange buffers).  ``fs`` is indexed by the column ids of ``csr`` and may have more rows than the CSR (a
+    halo of remote sources after the own rows); ``fd`` has one row per CSR row.  ``csr['eid']`` is only needed with
+    ``keep`` or ``want_attn``."""
     fs, fd, keep = _f32(fs), _f32(fd), _f32(keep)
     attn = _f32(attn).view(-1)
     n, h, d = fd.shape
@@ -454,17 +474,22 @@ def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_at
     rowsum = torch.zeros((n, h), dtype=torch.float32, device=dev)
     e = csr['indices'].numel()
     att = torch.zeros((max(e, 1), h), dtype=torch.float32, device=dev)[:e] if want_attn else None
-    saved = None
+    save = save or saved is not None
     if save and e * max(h, (h * d + 127) // 128) >= 2 ** 32:
         raise ValueError('gatv2_fwd(save=True): E * max(H, ceil(H*D/128)) = %d exceeds the 32-bit slot offsets of the kernel'
                          % (e * max(h, (h * d + 127) // 128)))
-    if save:
+    if saved is not None:
+        if not (saved[0].dtype == torch.float32 and saved[1].dtype == torch.int32 and saved[0].is_contiguous()
+                and saved[1].is_contiguous() and tuple(saved[0].shape[1:]) == (h,)
+                and tuple(saved[1].shape[1:]) == ((h * d + 127) // 128, 4) and min(saved[0].shape[0], saved[1].shape[0]) >= e):
+            raise ValueError('gatv2_fwd: saved must be contiguous fp32 [>=E, H] and int32 [>=E, ceil(H*D/128), 4] buffers')
+    elif save:
         saved = (torch.empty((max(e, 1), h), dtype=torch.float32, device=dev),    # max(E, 1): never a NULL pointer
                  torch.empty((max(e, 1), (h * d + 127) // 128, 4), dtype=torch.int32, device=dev))
     sp, ws = _attn_split(csr.get('split'), h, d, dev)
     order = row_order(csr) if _full(rb, re, n) else None
     with torch.cuda.device(dev):
-        _lib.call('regnn_gatv2_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr['eid']), _ptr(et_csr),
+        _lib.call('regnn_gatv2_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr.get('eid')), _ptr(et_csr),
                   _ptr(theta), float(alpha), r, _ptr(fs), _ptr(fd), _ptr(attn), float(slope), _ptr(keep), h, d,
                   rb, re, _ptr(out), _ptr(rowmax), _ptr(rowsum), _ptr(att), _ptr(saved[0]) if save else None,
                   _ptr(saved[1]) if save else None, sp, _ptr(ws), _ptr(order), _stream())
@@ -476,41 +501,70 @@ V2_STAGE_CHUNKS = 592   # REGNN_V2_STAGE_CHUNKS (csrc/gat.cu)
 
 
 def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax, rowsum, saved, g):
-    """Backward of ``gatv2_fwd(..., save=True)``: ``gat_bwd_stats`` -> regnn_gatv2_bwd_edges (the one gather pass) ->
-    regnn_gatv2_bwd_dst (streaming) -> (d_fs, d_fd, d_attn [H*D], d_theta | None)."""
-    fs, fd, keep, g = _f32(fs), _f32(fd), _f32(keep), _f32(g)
-    attn = _f32(attn).view(-1)
+    """Backward of ``gatv2_fwd(..., save=True)``: ``gat_bwd_stats`` -> ``gatv2_bwd_edges`` (the one gather pass) ->
+    ``gatv2_bwd_dst`` (streaming) -> (d_fs, d_fd, d_attn [H*D], d_theta | None)."""
     logit_csr, qmask = saved
-    n, h, d = fd.shape
-    theta, et_csr, r = _rel(theta, et_csr)
-    dev = fs.device
-    e = csr['indices'].numel()
     stats = gat_bwd_stats(out, g, None, rowmax, rowsum)
-    dl_csr = torch.empty((max(e, 1), h), dtype=torch.float32, device=dev)
-    d_fs = torch.empty_like(g)
-    d_fd = torch.empty_like(fd)
+    e = csr['indices'].numel()
+    dl_csr = stats.new_empty((max(e, 1), stats.shape[1]))   # never a NULL pointer
+    d_fs, d_attn_src = gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl_csr, keep=keep)
+    d_fd, d_attn_dst, d_theta = gatv2_bwd_dst(csr, et_csr, theta, alpha, fd, dl_csr, qmask, attn, slope)
+    return d_fs, d_fd, d_attn_src + d_attn_dst, d_theta
+
+
+# The stages of ``gatv2_bwd``.  partition.halo_gatv2 calls them one at a time, to bring the stored logits and sign masks
+# of cut edges to the source's owner before the edge pass and to return the per-slot dl between the two passes.  Full
+# row ranges.
+
+def gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl, keep=None):
+    """Source-major pass over the rows of the transposed view ``csr['indptr_t']`` -> (d_fs of those rows, their share
+    d_attn_src [H*D] of d_attn); the logit and the sign mask of every entry j are read from, and its dl is written to,
+    slot ``csr['slot_t'][j]`` of ``logit_csr`` / ``qmask`` / ``dl`` ([slots, H], [slots, C, 4], [slots, H]).  ``fs``: the
+    rows' own values; ``g`` / ``stats`` (``gat_bwd_stats`` with er=None): indexed by the column ids of the view.
+    ``keep``: the attention-dropout mask of ``gatv2_fwd``, in edge-id order through ``csr['eid']``
+    (regnn_gatv2_bwd_edges)."""
+    fs, keep, g = _f32(fs), _f32(keep), _f32(g)
+    attn = _f32(attn).view(-1)
+    n = csr['indptr_t'].numel() - 1
+    _, h, d = fs.shape
+    dev = fs.device
+    d_fs = torch.empty((n, h, d), dtype=torch.float32, device=dev)
     d_attn_src = torch.empty(h * d, dtype=torch.float32, device=dev)
-    d_attn_dst = torch.empty(h * d, dtype=torch.float32, device=dev)
-    d_theta = torch.zeros((r, h), dtype=torch.float32, device=dev) if r else None   # stays 0 when the graph has no edges
-    split_t, split = csr.get('split_t'), csr.get('split')
+    split_t = csr.get('split_t')
     sp_t, ws_t = _attn_split(split_t, h, d, dev)
-    sp, ws = _attn_split(split, h, d, dev)
-    order_t = row_order(csr, True)
     nblocks = _lib.load().regnn_gatv2_bwd_edges_blocks(n, split_t['struct'].num_frags if split_t else 0,
                                                        split_t['struct'].num_long if split_t else 0, h, d, 1)
     block_partials = torch.empty(max(nblocks, 1) * h * d, dtype=torch.float32, device=dev)
-    partials = torch.empty(max(_lib.partial_blocks() * h * d, V2_STAGE_CHUNKS * max(r * h, h * d)), dtype=torch.float64,
-                           device=dev)
+    partials = torch.empty(V2_STAGE_CHUNKS * h * d, dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
         _lib.call('regnn_gatv2_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
-                  _ptr(csr['eid']), _ptr(fs), _ptr(stats), _ptr(logit_csr), _ptr(qmask), _ptr(attn), float(slope),
-                  _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_fs), _ptr(dl_csr), _ptr(d_attn_src), _ptr(block_partials),
-                  _ptr(partials), sp_t, _ptr(ws_t), _ptr(order_t), _stream())
+                  _ptr(csr['eid']) if keep is not None else None, _ptr(fs), _ptr(stats), _ptr(logit_csr), _ptr(qmask),
+                  _ptr(attn), float(slope), _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_fs), _ptr(dl), _ptr(d_attn_src),
+                  _ptr(block_partials), _ptr(partials), sp_t, _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
+        _lib.count_launches(3 + (sp_t is not None))
+    return d_fs, d_attn_src
+
+
+def gatv2_bwd_dst(csr, et_csr, theta, alpha, fd, dl, qmask, attn, slope):
+    """Destination-side streaming pass over the rows of ``csr['indptr']``, reading ``dl`` and ``qmask`` in slot order
+    -> (d_fd of those rows, their share d_attn_dst [H*D] of d_attn, d_theta [R, H] | None) (regnn_gatv2_bwd_dst)."""
+    fd = _f32(fd)
+    attn = _f32(attn).view(-1)
+    theta, et_csr, r = _rel(theta, et_csr)
+    n = csr['indptr'].numel() - 1
+    _, h, d = fd.shape
+    dev = fd.device
+    d_fd = torch.empty((n, h, d), dtype=torch.float32, device=dev)
+    d_attn_dst = torch.empty(h * d, dtype=torch.float32, device=dev)
+    d_theta = torch.zeros((r, h), dtype=torch.float32, device=dev) if r else None   # stays 0 when the graph has no edges
+    sp, ws = _attn_split(csr.get('split'), h, d, dev)
+    partials = torch.empty(max(_lib.partial_blocks() * h * d, V2_STAGE_CHUNKS * r * h), dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
         _lib.call('regnn_gatv2_bwd_dst', _ptr(csr['indptr']), _ptr(et_csr) if r else None, _ptr(theta), float(alpha), r,
-                  _ptr(fd), _ptr(dl_csr), _ptr(qmask), _ptr(attn), float(slope), h, d, 0, n, _ptr(d_fd),
+                  _ptr(fd), _ptr(dl), _ptr(qmask), _ptr(attn), float(slope), h, d, 0, n, _ptr(d_fd),
                   _ptr(d_attn_dst), _ptr(partials), _ptr(d_theta), sp, _ptr(ws), _stream())
-        _lib.count_launches(5 + (2 if r else 0) + (sp_t is not None) + (sp is not None))
-    return d_fs, d_fd, d_attn_src + d_attn_dst, d_theta
+        _lib.count_launches(2 + (2 if r else 0) + (sp is not None))
+    return d_fd, d_attn_dst, d_theta
 
 
 # ---- grouped per-node-type input projection ---------------------------------------------------------------------

@@ -25,6 +25,9 @@ relation-degree norm for all rows; the caller sums the R-float relation gradient
 4. ``halo_gat`` -- the REGAT core on the same row blocks (``HaloPartition(..., attention=True)``): the features go
    forward through the in-halo, dL/dY and the softmax statistics backward through the out-halo, and the logit gradient
    of every cut edge goes back to its destination's owner (``regnn_halo_scatter`` or one more uneven all-to-all).
+5. ``halo_gatv2`` -- the REGATv2 core on the same row blocks: as ``halo_gat``, plus a per-slot exchange in the forward
+   direction -- the logit and sign mask the forward stored in the destination's slot go to the source's owner, whose
+   edge pass reads them (``regnn_halo_push_slots`` or one more pair of uneven all-to-alls).
 """
 import torch
 import torch.distributed as dist
@@ -492,7 +495,11 @@ class HaloPartition:
     * ``dpre_recv`` (int64) and ``dpre_recv_counts`` [P]: per peer, the own in-view slots whose source that peer owns,
       slot-ascending -- the receive side of the all-to-all variant, entry for entry the peer's tail segment;
     * ``max_dpre_rows``: the largest extended dpre buffer over all ranks (the symmetric allocation size), computed from
-      the global CSR like the tails, so no collective is needed.
+      the global CSR like the tails, so no collective is needed;
+    * ``push_slots`` = (send_slots int32, send_ptr [P+1], recv_offset [P]): the same exchange in the other direction, for
+      ``halo_gatv2``, whose edge pass reads the logit and the sign mask that the forward stored in the destination's
+      slot: ``send_slots`` is ``dpre_recv`` and lands on peer q from row ``e_in_q + tail_ptr_q[rank]`` of its extended
+      buffers, i.e. on q's tail segment of this rank (regnn_halo_push_slots); also from the global CSR.
 
     Index bookkeeping with device-agnostic torch ops."""
 
@@ -601,8 +608,17 @@ class HaloPartition:
         all_src_owner = _owner(csr['indices'].to(torch.int64), bounds_t)
         all_dst_owner = _owner(torch.arange(int(slot_bounds[-1]), dtype=torch.int64, device=src_of.device), slot_bounds)
         cross = all_src_owner != all_dst_owner
-        cut = torch.bincount(all_src_owner[cross], minlength=parts)
-        self.max_dpre_rows = int((slot_bounds[1:] - slot_bounds[:-1] + cut).max())
+        # [P, P] cut edges by (source owner, destination owner): row q is rank q's tail counts
+        cut_pairs = torch.bincount(all_src_owner[cross] * parts + all_dst_owner[cross], minlength=parts * parts)
+        cut_pairs = cut_pairs.view(parts, parts).cpu()
+        e_in_all = (slot_bounds[1:] - slot_bounds[:-1]).cpu()
+        self.max_dpre_rows = int((e_in_all + cut_pairs.sum(dim=1)).max())
+        # push list of regnn_halo_push_slots (REGATv2): the receive list read the other way -- the stored logit and sign
+        # mask of every own in-view slot whose source q owns go to q's tail segment of this rank
+        tail_before = torch.cumsum(cut_pairs, dim=1) - cut_pairs      # [q, p]: q's tail entries owned by ranks < p
+        self.push_slots = (self.dpre_recv.to(torch.int32).contiguous(),
+                           [0] + torch.tensor(self.dpre_recv_counts, dtype=torch.int64).cumsum(0).tolist(),
+                           [int(e_in_all[q] + tail_before[q, rank]) for q in range(parts)])
 
     def _set_offsets(self, table):
         """``table`` [P, 2, P] (host): every rank's ``halo_counts``."""
@@ -641,11 +657,18 @@ class HaloExchange(_PeerBuffers):
     ``heads`` (a ``halo_gat`` call site, ``feat`` = heads * head_dim, ``part`` built with ``attention=True``): also the
     softmax statistics of the out-halo [n_own + out-halo, 4 * heads], the extended dpre buffer
     [E_in_own + cut_out, heads] that peers scatter the logit gradients of this rank's in-view slots into, and a gradient
-    table wide enough for d_attn_l, d_attn_r and d_theta together (2 * feat + R * heads floats)."""
+    table wide enough for d_attn_l, d_attn_r and d_theta together (2 * feat + R * heads floats).
 
-    def __init__(self, part, feat, device, group=None, heads=None):
+    ``gatv2=True`` (a ``halo_gatv2`` call site, with ``heads``): also the extended per-slot buffers of the stored logits
+    [E_in_own + cut_out, heads] and sign masks [E_in_own + cut_out, 4 * C] (fp32 storage of int32 [., C, 4] words,
+    C = ceil(feat / 128)): the forward writes the head, peers fill the tail with regnn_halo_push_slots.  dl reuses the
+    dpre buffer."""
+
+    def __init__(self, part, feat, device, group=None, heads=None, gatv2=False):
         group = group if group is not None else dist.group.WORLD
-        self.parts, self.rank, self.feat, self.heads = part.parts, part.rank, feat, heads
+        self.parts, self.rank, self.feat, self.heads, self.gatv2 = part.parts, part.rank, feat, heads, gatv2
+        if gatv2 and heads is None:
+            raise ValueError('HaloExchange(gatv2=True) needs heads=H')
         self._handles = []
         self.x_ext, self.x_ptrs = self._alloc(max(part.max_rows_in, 1), feat, device, group)
         self.g_ext, self.g_ptrs = self._alloc(max(part.max_rows_out, 1), feat, device, group)
@@ -655,6 +678,12 @@ class HaloExchange(_PeerBuffers):
             self.s_ext, self.s_ptrs = self._alloc(max(part.max_rows_out, 1), 4 * heads, device, group)
             self.dpre, self.dpre_ptrs = self._alloc(max(part.max_dpre_rows, 1), heads, device, group)
             self.GRAD_SLOTS = max(self.GRAD_SLOTS, (2 * feat + part.num_relations * heads + 63) // 64 * 64)
+        if gatv2:
+            chunks = (feat + 127) // 128
+            _check_slot_offsets(part, heads, chunks)
+            self.logit_ext, self.logit_ptrs = self._alloc(max(part.max_dpre_rows, 1), heads, device, group)
+            mask, self.mask_ptrs = self._alloc(max(part.max_dpre_rows, 1), 4 * chunks, device, group)
+            self.mask_ext = mask.view(torch.int32).view(-1, chunks, 4)
         self.grad_tab, self.grad_ptrs = self._alloc(self.parts, self.GRAD_SLOTS, device, group)
         self.grad_tab.zero_()
         self.barrier()
@@ -763,25 +792,39 @@ def halo_propagate(part, x_own, theta, alpha, weighted=True, group=None, exchang
     return _HaloPropagate.apply(part, x_own, theta, alpha, weighted, group, exchange)
 
 
-def _check_gat_shape(heads, dim, num_relations, relational):
+def _check_gat_shape(heads, dim, num_relations, relational, name='halo_gat'):
     """The head widths the fused attention kernels take (check_shape of csrc/gat.cu), refused before any work."""
     if not (1 <= heads <= 32 and 4 <= dim <= 128 and dim & (dim - 1) == 0 and heads * dim <= 1024):
-        raise ValueError('halo_gat: the fused attention kernels take 1 <= H <= 32 heads of a power-of-two width D in '
-                         '[4, 128] with H * D <= 1024, not H=%d D=%d' % (heads, dim))
+        raise ValueError('%s: the fused attention kernels take 1 <= H <= 32 heads of a power-of-two width D in '
+                         '[4, 128] with H * D <= 1024, not H=%d D=%d' % (name, heads, dim))
     if relational and not (1 <= num_relations <= 200 and num_relations * heads <= 4096):
-        raise ValueError('halo_gat: the fused attention kernels take 1..200 relations with R * H <= 4096, not R=%d H=%d'
-                         % (num_relations, heads))
+        raise ValueError('%s: the fused attention kernels take 1..200 relations with R * H <= 4096, not R=%d H=%d'
+                         % (name, num_relations, heads))
 
 
-def _fill_out_halo_gat(part, g_own, stats_own, group, xch):
+def _check_slot_offsets(part, heads, chunks):
+    """The REGATv2 kernels address the per-slot buffers with 32-bit offsets (slot * H, slot * C)."""
+    if part.max_dpre_rows * max(heads, chunks) >= 2 ** 32:
+        raise ValueError('halo_gatv2: %d extended slots * max(H, ceil(H*D/128)) exceeds the 32-bit slot offsets of the '
+                         'REGATv2 kernels' % part.max_dpre_rows)
+
+
+def _fill_out_halo_gat(part, g_own, stats_own, group, xch, slots=None):
     """dL/dY [n_own + out-halo, H*D] and the softmax statistics [n_own + out-halo, 4H] of the backward: the same rows,
-    pushed by their owners (one barrier for both over peer memory, two uneven all-to-alls otherwise)."""
+    pushed by their owners (one barrier for both over peer memory, two uneven all-to-alls otherwise).  ``slots``
+    (REGATv2: the extended logit and mask buffers): their tails are filled in the same exchange
+    (``_push_slot_records``), behind the same barrier."""
     if xch is None:
-        return _fill_halo(part, g_own, 'out', group, None), _fill_halo(part, stats_own, 'out', group, None)
+        g_ext, s_ext = _fill_halo(part, g_own, 'out', group, None), _fill_halo(part, stats_own, 'out', group, None)
+        if slots is not None:
+            _push_slot_records(part, slots, group, None)
+        return g_ext, s_ext
     rows, ptr, offsets = part.push_out
     if ptr[-1]:
         ops.halo_push(g_own, rows, ptr, offsets, xch.g_ptrs, xch.g_ext.stride(0), part.rank)
         ops.halo_push(stats_own, rows, ptr, offsets, xch.s_ptrs, xch.s_ext.stride(0), part.rank)
+    if slots is not None:
+        _push_slot_records(part, slots, group, xch)
     xch.barrier()
     n = part.n_own + part.n_out
     return xch.g_ext[:n], xch.s_ext[:n]
@@ -939,3 +982,187 @@ def _virtual_halo_gat(parts, f, gout, attn_l, attn_r, theta, alpha, slope, scatt
         d_al, d_ar = d_al + al, d_ar + ar
         d_th = d_th + th if th is not None else None
     return torch.cat(outs), torch.cat(d_feats), d_al, d_ar, d_th
+
+
+# ---- REGATv2 on destination-row blocks with a halo exchange --------------------------------------------------------
+def _slot_buffers(part, heads, chunks, like, xch):
+    """The extended per-slot buffers of the stored logits [e_in + tail, H] and sign masks [e_in + tail, C, 4] (int32):
+    the own in-view slots in the head, the cut out-edges of own sources in the tail (``csr['slot_t']`` order).  Views
+    of the exchange's symmetric buffers over peer memory, local buffers otherwise."""
+    rows = part.e_in + part.tail_ptr[-1]
+    if xch is not None:
+        return xch.logit_ext[:rows], xch.mask_ext[:rows]
+    return (like.new_empty((max(rows, 1), heads))[:rows],        # max(rows, 1): never a NULL pointer
+            torch.empty((max(rows, 1), chunks, 4), dtype=torch.int32, device=like.device)[:rows])
+
+
+def _push_slot_records(part, slots, group, xch):
+    """Sends the stored logit and sign mask of every own in-view slot whose source a peer owns to that peer, into its
+    tail (the transpose of ``_return_dpre``); afterwards the tails of ``slots`` hold every cut out-edge of this rank's
+    sources.  Over peer memory this is the push only: the caller's barrier completes it."""
+    logit, mask = slots
+    if xch is not None:
+        send, ptr, offsets = part.push_slots
+        if ptr[-1]:
+            ops.halo_push_slots(logit, mask, send, ptr, offsets, xch.logit_ptrs, xch.mask_ptrs, part.rank)
+        return
+    if part.parts > 1:
+        e_in = part.e_in
+        with _lib.phase('halo_all_to_all'):
+            for buf in (logit, mask.flatten(1)):
+                dist.all_to_all_single(buf[e_in:], buf.index_select(0, part.dpre_recv),
+                                       output_split_sizes=part.tail_counts, input_split_sizes=part.dpre_recv_counts,
+                                       group=group)
+
+
+def _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots):
+    """-> (out, rowmax, rowsum) of the own rows from the filled [n_own + in-halo, H, D] source features and the own
+    rows' destination features; the logit and the sign mask of every in-view slot go to the head of ``slots``."""
+    n_own, heads, dim = fd_own.shape
+    if not n_own:                # an empty row block has no edges and no halo
+        z = fd_own.new_zeros((0, heads))
+        return fd_own.new_zeros((0, heads, dim)), z, z
+    out, rowmax, rowsum, _, _ = ops.gatv2_fwd(part.csr, part.et_in if theta is not None else None, theta, alpha, fs_ext,
+                                              fd_own, attn, slope, saved=slots)
+    return out, rowmax, rowsum
+
+
+def _gatv2_backward_edges(part, fs_own, attn, slope, g_ext, s_ext, slots, dl):
+    """-> (d_fs, this rank's d_attn_src [H*D]) of the own rows once the tails of ``slots`` are filled; writes the dl of
+    every out-view entry into the extended ``dl`` buffer [e_in + tail, H] through ``csr['slot_t']``."""
+    n_own, heads, dim = fs_own.shape
+    if not n_own:
+        return torch.zeros_like(fs_own), fs_own.new_zeros(heads * dim)
+    return ops.gatv2_bwd_edges(part.csr, fs_own, s_ext.view(-1, heads, 4), slots[0], slots[1], attn, slope,
+                               g_ext.view(-1, heads, dim), dl)
+
+
+def _gatv2_backward_dst(part, fd_own, attn, theta, alpha, slope, dl, mask):
+    """-> (d_fd, this rank's d_attn_dst [H*D], d_theta | None) once ``dl[:e_in]`` holds every in-view slot: the
+    streaming destination pass over the in-view."""
+    n_own, heads, dim = fd_own.shape
+    if not n_own:
+        return (torch.zeros_like(fd_own), fd_own.new_zeros(heads * dim),
+                fd_own.new_zeros(theta.shape) if theta is not None else None)
+    return ops.gatv2_bwd_dst(part.csr, part.et_in if theta is not None else None, theta, alpha, fd_own,
+                             dl[:part.e_in], mask[:part.e_in], attn, slope)
+
+
+class _HaloGatV2(torch.autograd.Function):
+    """REGATv2 core (fused logits / edge softmax / aggregation of ``functional.gatv2_aggregate``) on destination-row
+    blocks with a halo exchange.  Forward: the in-halo of the source features (the destination features are read for
+    own rows only), then the fused kernel over the in-view, which stores the logit and the sign mask of every in-view
+    slot in the head of the extended per-slot buffers.  Backward: the statistics of own rows; one exchange of the
+    dL/dY and statistics out-halo and of the slot records of cut edges (to the source's owner, into the buffers'
+    tails); the source-major edge pass over the out-view, which writes the dl of every out-edge into the extended dl
+    buffer; the tail of that buffer goes back to the destinations' owners; then the destination pass over the in-view.
+
+    Over peer memory the exchange's buffers are reused by every call: a forward must be followed by its backward
+    before the next forward, as for every ``HaloExchange``."""
+
+    @staticmethod
+    def forward(ctx, part, fs_own, fd_own, attn, theta, alpha, slope, group, xch):
+        n_own, heads, dim = fs_own.shape
+        fs_own, fd_own = fs_own.contiguous(), fd_own.contiguous()
+        fs_ext = _fill_halo(part, fs_own.view(n_own, heads * dim), 'in', group, xch).view(-1, heads, dim)
+        slots = _slot_buffers(part, heads, (heads * dim + 127) // 128, fs_own, xch)
+        out, rowmax, rowsum = _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots)
+        ctx.part, ctx.alpha, ctx.slope, ctx.group, ctx.xch, ctx.slots = part, alpha, slope, group, xch, slots
+        ctx.save_for_backward(fs_own, fd_own, attn, theta, out, rowmax, rowsum)
+        return out
+
+    @staticmethod
+    def backward(ctx, g_own):
+        fs_own, fd_own, attn, theta, out, rowmax, rowsum = ctx.saved_tensors
+        part, xch, slots = ctx.part, ctx.xch, ctx.slots
+        n_own, heads, dim = fs_own.shape
+        g_own = g_own.reshape(n_own, heads, dim).contiguous()
+        stats = _gat_stats(out, g_own, None, rowmax, rowsum)
+        g_ext, s_ext = _fill_out_halo_gat(part, g_own.view(n_own, heads * dim), stats, ctx.group, xch, slots=slots)
+        rows = part.e_in + part.tail_ptr[-1]
+        dl = xch.dpre[:rows] if xch is not None else fs_own.new_empty((max(rows, 1), heads))[:rows]
+        d_fs, d_attn_src = _gatv2_backward_edges(part, fs_own, attn, ctx.slope, g_ext, s_ext, slots, dl)
+        _return_dpre(part, dl, ctx.group, xch)
+        d_fd, d_attn_dst, d_th = _gatv2_backward_dst(part, fd_own, attn, theta, ctx.alpha, ctx.slope, dl, slots[1])
+        return (None, d_fs, d_fd, (d_attn_src + d_attn_dst).view_as(attn),
+                d_th.view_as(theta) if d_th is not None else None, None, None, None, None)
+
+
+def halo_gatv2(part, fs_own, fd_own, attn, theta, alpha, slope, group=None, exchange=None, keep=None):
+    """fs_own, fd_own [n_own, H, D] -> out [n_own, H, D] (``part``: this rank's ``HaloPartition`` built with
+    ``attention=True``): the REGATv2 core of ``functional.gatv2_aggregate`` on destination-row blocks, exchanging only
+    halo rows and the per-slot records of cut edges.  With shared weights pass the same tensor as ``fs_own`` and
+    ``fd_own``.  ``exchange`` (a ``HaloExchange`` with ``heads=H``, width H*D and ``gatv2=True``): the source features,
+    dL/dY and the statistics are pushed over peer memory (regnn_halo_push), the stored logits and sign masks of cut
+    edges go to the sources' owners (regnn_halo_push_slots) and their dl back to the destinations' owners
+    (regnn_halo_scatter); None: uneven all-to-alls (NCCL / gloo).  ``theta=None`` drops the relation term.  out, d_fs
+    and d_fd are bit-identical to ``functional.gatv2_aggregate``; ``attn.grad`` and ``theta.grad`` hold this rank's
+    shares (``allreduce_relation_grads``).  The MAG stack's ``softmax_eps`` (a global maximum over all logits) is not
+    taken."""
+    _, heads, dim = fs_own.shape
+    if keep is not None:
+        raise ValueError('halo_gatv2: attention dropout is not supported (its mask is in edge-id order over all edges)')
+    if not getattr(part, 'attention', False):
+        raise ValueError('halo_gatv2 needs a HaloPartition built with attention=True')
+    _check_gat_shape(heads, dim, part.num_relations, theta is not None, 'halo_gatv2')
+    if tuple(fd_own.shape) != tuple(fs_own.shape):
+        raise ValueError('halo_gatv2: fs_own and fd_own must both be [n_own, H, D], got %s and %s'
+                         % (tuple(fs_own.shape), tuple(fd_own.shape)))
+    if theta is not None and tuple(theta.shape) != (part.num_relations, heads):
+        raise ValueError('halo_gatv2: theta must be [R=%d, H=%d], got %s' % (part.num_relations, heads, tuple(theta.shape)))
+    _check_slot_offsets(part, heads, (heads * dim + 127) // 128)
+    if exchange is not None and (exchange.heads != heads or exchange.feat != heads * dim or not exchange.gatv2):
+        raise ValueError('halo_gatv2: the HaloExchange must be built with heads=%d, width %d and gatv2=True'
+                         % (heads, heads * dim))
+    return _HaloGatV2.apply(part, fs_own, fd_own, attn, theta, alpha, slope, group, exchange)
+
+
+def _virtual_halo_gatv2(parts, fs, fd, gout, attn, theta, alpha, slope, push=False):
+    """Every rank of ``HaloPartition.virtual_ranks(..., attention=True)`` one after another in one process (no process
+    group), each on its local views: halos filled by indexing the global [N, H, D] arrays; the slot records of cut
+    edges moved to the sources' owners by indexing and the dl tails returned with ``index_copy_`` at the owners'
+    receive lists, or -- ``push=True`` -- by regnn_halo_push_slots and regnn_halo_scatter into the P local buffers.
+    -> (out, d_fs, d_fd, d_attn, d_theta | None): rows in global order, parameter gradients summed in rank order."""
+    n, heads, dim = fs.shape
+    g2 = gout.reshape(n, heads * dim)
+    bounds = parts[0].bounds
+    own = [slice(bounds[p], bounds[p + 1]) for p in range(len(parts))]
+    slots = [_slot_buffers(part, heads, (heads * dim + 127) // 128, fs, None) for part in parts]
+    fw = [_gatv2_forward(part, fs[part.rows_in], fd[s].contiguous(), attn, theta, alpha, slope, sl)
+          for part, s, sl in zip(parts, own, slots)]
+    stats = torch.cat([_gat_stats(o, gout[s].contiguous(), None, mx, sm) for (o, mx, sm), s in zip(fw, own)])
+    if push:
+        ptrs = [torch.tensor([sl[i].data_ptr() for sl in slots], dtype=torch.int64, device=fs.device) for i in (0, 1)]
+        for p, part in enumerate(parts):
+            send, ptr, offsets = part.push_slots
+            if ptr[-1]:
+                ops.halo_push_slots(slots[p][0], slots[p][1], send, ptr, offsets, ptrs[0], ptrs[1], p)
+    else:
+        for q, owner in enumerate(parts):      # q's tail segment of rank p: p's slots at its receive list from q
+            for p, part in enumerate(parts):
+                seg = slice(owner.e_in + owner.tail_ptr[p], owner.e_in + owner.tail_ptr[p + 1])
+                idx = part.dpre_recv[part.push_slots[1][q]:part.push_slots[1][q + 1]]
+                for dst, src in zip(slots[q], slots[p]):
+                    dst[seg] = src.index_select(0, idx)
+    dls = [fs.new_empty((max(part.e_in + part.tail_ptr[-1], 1), heads))[:part.e_in + part.tail_ptr[-1]] for part in parts]
+    edges = [_gatv2_backward_edges(part, fs[s].contiguous(), attn, slope, g2[part.rows_out], stats[part.rows_out],
+                                   slots[p], dls[p]) for p, (part, s) in enumerate(zip(parts, own))]
+    if push:
+        ptrs = torch.tensor([d.data_ptr() for d in dls], dtype=torch.int64, device=fs.device)
+        for p, part in enumerate(parts):
+            if part.tail_ptr[-1]:
+                ops.halo_scatter(dls[p][part.e_in:], part.tail_ptr, part.tail_dst, ptrs, heads, p)
+    else:
+        for q, owner in enumerate(parts):
+            segs = [dls[p][part.e_in + part.tail_ptr[q]:part.e_in + part.tail_ptr[q + 1]] for p, part in enumerate(parts)]
+            dls[q].index_copy_(0, owner.dpre_recv, torch.cat(segs))
+    outs, d_fss, d_fds, d_attn, d_th = [], [], [], 0, 0
+    for p, part in enumerate(parts):
+        d_fd, d_at_dst, th = _gatv2_backward_dst(part, fd[own[p]].contiguous(), attn, theta, alpha, slope, dls[p],
+                                                 slots[p][1])
+        outs.append(fw[p][0])
+        d_fss.append(edges[p][0])
+        d_fds.append(d_fd)
+        d_attn = d_attn + (edges[p][1] + d_at_dst)
+        d_th = d_th + th if th is not None else None
+    return torch.cat(outs), torch.cat(d_fss), torch.cat(d_fds), d_attn, d_th
