@@ -63,6 +63,27 @@ typedef struct regnn_rowsplit {
   int32_t num_long, num_frags, threshold;
 } regnn_rowsplit_t;
 
+/* Counter-based attention dropout of the fused REGAT / REGATv2 kernels (the alternative to an explicit [E,H] `keep`
+ * tensor): the keep factor of edge id e and head h of the call is a pure function of (key, e, global head), computed in
+ * registers from the edge id the kernel already loads, so every kernel, rank and partition of the graph sees the same
+ * mask without storing or exchanging it:
+ *   c      = e * num_heads_total + head_offset + h                          (64-bit counter)
+ *   x      = mix32( lo32(c) ^ lo32(key) )
+ *   x      = mix32( x + hi32(c) * 0x9E3779B1 + hi32(key) )                  (uint32 arithmetic, wrapping)
+ *   keep   = x >= threshold ? scale : 0
+ *   mix32(z): z ^= z >> 16; z *= 0x7feb352d; z ^= z >> 15; z *= 0x846ca68b; z ^= z >> 16
+ * With drop probability p: threshold = floor(p * 2^32), scale = (float)(1 / (1 - p)); p = 0 is threshold 0, scale 1
+ * (every factor is exactly 1).  head_offset / num_heads_total let a call over a slice of the heads reproduce that
+ * slice of the full-H mask (num_heads_total >= head_offset + num_heads of the call).  Restated in
+ * oracle/attn_dropout_oracle.py. */
+typedef struct regnn_attn_dropout {
+  uint64_t key;
+  uint32_t threshold;
+  float scale;
+  int32_t head_offset;
+  int32_t num_heads_total;
+} regnn_attn_dropout_t;
+
 int regnn_version(void);
 const char* regnn_status_string(int status);
 const char* regnn_last_error_string(void);
@@ -284,13 +305,17 @@ int regnn_rowdot_norm_bwd(const float* norm, int norm_sides, const float* X, int
  * Replaces apply_edges(u_add_v) + index/add/LeakyReLU + edge_softmax (4 kernels) +
  * update_all(u_mul_e, sum).  etype == NULL drops the relation term (`edge_feats=None`).
  * keep: optional [E,H] attention-dropout scale (0 or 1/(1-p)) in EDGE-ID order, NULL = none.
+ * dropout: optional counter-based dropout (regnn_attn_dropout_t), keep_e computed from eid[slot]; NULL = none.  At
+ *   most one of keep and dropout; either needs eid.  The factor multiplies a at the same place in both modes, so a
+ *   keep tensor holding the hashed factors gives the same bits.
  * attn_out: optional [E,H] output of a*keep in EDGE-ID order (`get_attention`), NULL = skip.
  * Saves rowmax/rowsum [N,H] for the backward pass.  theta: [R,H].
  */
 int regnn_gat_fwd(const int32_t* indptr, const int32_t* indices, const int32_t* eid,
                   const uint8_t* etype_csr, const float* theta, float alpha, int num_relations,
                   const float* feat, const float* el, const float* er, float negative_slope,
-                  const float* keep, int num_heads, int head_dim, int64_t row_begin, int64_t row_end,
+                  const float* keep, const regnn_attn_dropout_t* dropout, int num_heads, int head_dim,
+                  int64_t row_begin, int64_t row_end,
                   float* out, float* rowmax, float* rowsum, float* attn_out, const regnn_rowsplit_t* split,
     float* split_workspace /* num_frags * (H*D + 2*H) floats, or NULL */,
     const int32_t* row_order /* as regnn_spmm_fwd's: degree-sorted rows that are not long, or NULL (natural order) */,
@@ -312,11 +337,13 @@ int regnn_gat_bwd_stats(const float* out, const float* G, const float* er, const
  *   d_feat[u,h,:] = sum_{e in Out(u)} a_e*keep_e * G[v,h,:]  (+ d_el[u,h]*attn_l[h,:] when attn_l != NULL: the gradient
  *                   through el = <feat, attn_l>, layer/REGATConv.py:68)
  *   d_el[u,h]     = sum_{e in Out(u)} dpre_e
- * etype_t: edge types per transposed entry; eid: CSR slot -> edge id (only read when keep != NULL). */
+ * etype_t: edge types per transposed entry; eid: slot -> edge id, read through slot_t (only with keep or dropout);
+ * keep / dropout: as in regnn_gat_fwd (at most one). */
 int regnn_gat_bwd_edges(const int32_t* indptr_t, const int32_t* indices_t, const int32_t* slot_t,
                         const uint8_t* etype_t, const int32_t* eid, const float* theta, float alpha, int num_relations,
                         const float* feat, const float* el, const float* stats, float negative_slope,
-                        const float* keep, const float* G, int num_heads, int head_dim, int64_t row_begin,
+                        const float* keep, const regnn_attn_dropout_t* dropout, const float* G, int num_heads,
+                        int head_dim, int64_t row_begin,
                         int64_t row_end, float* d_feat, float* d_el, float* dpre_csr, const float* attn_l,
                         const regnn_rowsplit_t* split_t /* of the transposed view */,
                         float* split_workspace /* num_frags * (H*D + 2*H) floats, or NULL */,
@@ -349,12 +376,13 @@ int regnn_attn_scores_bwd(const float* feat, const float* d_el, const float* d_e
  * Fused REGATv2 layer core (layer/REGATv2Conv.py:133-152):
  *   l[e,h] = sum_d attn[h,d] * LeakyReLU_slope( fs[src,h,d] + fd[v,h,d] ) + w[etype,h]
  *   a = edge_softmax(l);  out[v,h,:] = sum_e a*keep * fs[src,h,:]
- * The [E,H,D] intermediates of the reference are never materialised.
+ * The [E,H,D] intermediates of the reference are never materialised.  keep / dropout / attn_out as in regnn_gat_fwd.
  */
 int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, const int32_t* eid,
                     const uint8_t* etype_csr, const float* theta, float alpha, int num_relations,
                     const float* fs, const float* fd, const float* attn, float negative_slope,
-                    const float* keep, int num_heads, int head_dim, int64_t row_begin,
+                    const float* keep, const regnn_attn_dropout_t* dropout, int num_heads, int head_dim,
+                    int64_t row_begin,
                     int64_t row_end, float* out, float* rowmax, float* rowsum, float* attn_out,
                     float* logit_csr /* [E,H] CSR-slot order, or NULL (inference) */,
                     uint32_t* qmask /* [E, ceil(H*D/128), 4], or NULL; see below */,
@@ -382,9 +410,11 @@ int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, const int32_t
 int64_t regnn_gatv2_bwd_edges_blocks(int64_t num_rows, int num_frags /* of split_t */, int num_long /* of split_t */,
                                      int num_heads, int head_dim, int ordered /* row_order_t given and row_begin == 0 */);
 int regnn_gatv2_bwd_edges(const int32_t* indptr_t, const int32_t* indices_t, const int32_t* slot_t,
-                          const int32_t* eid /* CSR slot -> edge id; only read with keep */, const float* fs,
-                          const float* stats, const float* logit_csr, const uint32_t* qmask, const float* attn,
-                          float negative_slope, const float* keep, const float* G, int num_heads, int head_dim,
+                          const int32_t* eid /* slot -> edge id through slot_t; only read with keep or dropout */,
+                          const float* fs, const float* stats, const float* logit_csr, const uint32_t* qmask,
+                          const float* attn, float negative_slope, const float* keep,
+                          const regnn_attn_dropout_t* dropout /* as regnn_gat_fwd; at most one of keep and dropout */,
+                          const float* G, int num_heads, int head_dim,
                           int64_t row_begin, int64_t row_end, float* d_fs, float* dl_csr, float* d_attn_src,
                           float* block_partials, double* partials, const regnn_rowsplit_t* split_t /* transposed view */,
     float* split_workspace /* num_frags * (H*D + 2*H) floats, or NULL */, const int32_t* row_order_t, void* stream);

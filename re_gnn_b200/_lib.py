@@ -45,20 +45,20 @@ SIGNATURES = {
     'regnn_rowdot_norm_bwd': (_i32, [_p, _i32, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _i32, _p, _p]),
     'regnn_random_walk': (_i32, [_p, _p, _i64, _i64, _i32, ctypes.c_uint64, _p, _p]),
     'regnn_sample_neighbors': (_i32, [_p, _p, _i64, _i32, ctypes.c_uint64, _p, _p]),
-    'regnn_gat_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _i32, _i32, _i64, _i64,
+    'regnn_gat_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
                              _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gat_bwd_stats': (_i32, [_p, _p, _p, _p, _p, _i64, _i32, _i32, _p, _p]),
-    'regnn_gat_bwd_edges': (_i32, [_p, _p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
-                                   _p, _p, _p, _p, _p, _p, _p, _p]),
+    'regnn_gat_bwd_edges': (_i32, [_p, _p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _p, _i32, _i32, _i64,
+                                   _i64, _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gat_bwd_reduce': (_i32, [_p, _p, _p, _f32, _i32, _p, _i32, _i64, _i64, _p, _p, _p, _p, _p, _p]),
     'regnn_attn_scores_fwd': (_i32, [_p, _p, _p, _i64, _i32, _i32, _p, _p, _p]),
     'regnn_attn_scores_bwd': (_i32, [_p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _p, _p]),
     'regnn_grouped_linear_fwd': (_i32, [_i32, _p, _p, _p, _p, _p, _i32, _i64, _p, _p, _p, _p, _i64, _p]),
     'regnn_grouped_linear_bwd': (_i32, [_i32, _p, _p, _p, _i32, _i64, _p, _p, _p, _p, _i64, _i32, _p, _p, _p]),
-    'regnn_gatv2_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _i32, _i32, _i64, _i64,
+    'regnn_gatv2_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
                                _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gatv2_bwd_edges_blocks': (_i64, [_i64, _i32, _i32, _i32, _i32, _i32]),
-    'regnn_gatv2_bwd_edges': (_i32, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
+    'regnn_gatv2_bwd_edges': (_i32, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _f32, _p, _p, _p, _i32, _i32, _i64, _i64,
                                      _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gatv2_bwd_dst': (_i32, [_p, _p, _p, _f32, _i32, _p, _p, _p, _p, _f32, _i32, _i32, _i64, _i64,
                                    _p, _p, _p, _p, _p, _p, _p]),
@@ -70,6 +70,12 @@ class RowSplit(ctypes.Structure):
     """Mirror of ``regnn_rowsplit_t`` (include/regnn_b200.h)."""
     _fields_ = [('long_rows', _p), ('frag_ptr', _p), ('frag_row', _p), ('frag_begin', _p),
                 ('num_long', ctypes.c_int32), ('num_frags', ctypes.c_int32), ('threshold', ctypes.c_int32)]
+
+
+class AttnDropout(ctypes.Structure):
+    """Mirror of ``regnn_attn_dropout_t`` (include/regnn_b200.h)."""
+    _fields_ = [('key', ctypes.c_uint64), ('threshold', ctypes.c_uint32), ('scale', ctypes.c_float),
+                ('head_offset', ctypes.c_int32), ('num_heads_total', ctypes.c_int32)]
 
 
 class PeerRows(ctypes.Structure):

@@ -74,7 +74,8 @@ void launch_colsum_finalize(const double* partials, int num_blocks, int stride, 
 
 extern "C" {
 
-int regnn_version(void) { return 200; }  // 2xx: round-2 ABI (regnn_spmm_bwd_fused takes Y / d_norm)
+int regnn_version(void) { return 201; }  // 2xx: round-2 ABI (regnn_spmm_bwd_fused takes Y / d_norm); 201: the attention
+                                         // entry points take a regnn_attn_dropout_t next to keep
 
 const char* regnn_status_string(int status) {
   switch (status) {

@@ -23,6 +23,14 @@ int check_launch(const char* what);
     }                                         \
   } while (0)
 
+// 32-bit integer finaliser of the counter-based generators (neighbour sampling, attention dropout)
+__host__ __device__ __forceinline__ uint32_t mix32(uint32_t z) {
+  z ^= z >> 16; z *= 0x7feb352du;
+  z ^= z >> 15; z *= 0x846ca68bu;
+  z ^= z >> 16;
+  return z;
+}
+
 __device__ __forceinline__ float leaky(float x, float slope) { return x > 0.f ? x : x * slope; }
 // PyTorch's leaky_relu_backward convention: the negative slope applies at x == 0.
 __device__ __forceinline__ float leaky_grad(float x, float slope) { return x > 0.f ? 1.f : slope; }

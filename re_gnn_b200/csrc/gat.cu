@@ -56,7 +56,21 @@ struct AttnArgs {
   // gat_bwd_src epilogue (optional): d_feat[u,h,:] += d_el[u,h]*attn_l[h,:] + d_er[u,h]*attn_r[h,:]
   const float* attn_l;
   const int32_t* a_csr_eid;  // gat_bwd_edges with a dropout mask: CSR slot -> edge id
+  // counter-based attention dropout (regnn_attn_dropout_t), read by the HASH instantiations only
+  uint32_t drop_key_lo, drop_key_hi, drop_threshold;
+  float drop_scale;
+  int drop_head_offset, drop_heads_total;
 };
+
+// Keep factor of edge id e, head h of the call under regnn_attn_dropout_t (the counter hash stated in
+// include/regnn_b200.h): a few integer instructions from the edge id the kernel has already loaded, in place of a
+// 4-byte load from an [E,H] mask.
+__device__ __forceinline__ float hashed_keep(const AttnArgs& a, int e, int h) {
+  const uint64_t c = (uint64_t)(uint32_t)e * (uint32_t)a.drop_heads_total + (uint32_t)(a.drop_head_offset + h);
+  uint32_t x = mix32((uint32_t)c ^ a.drop_key_lo);
+  x = mix32(x + (uint32_t)(c >> 32) * 0x9E3779B1u + a.drop_key_hi);
+  return x >= a.drop_threshold ? a.drop_scale : 0.f;
+}
 
 __device__ __forceinline__ void load_rel_table(float* w_s, const AttnArgs& a) {
   if (a.etype != nullptr) {
@@ -175,9 +189,14 @@ __device__ __forceinline__ int64_t rg_num_work(const AttnArgs& a, int G) {
 #endif
 constexpr int kUG = 4;  // edges per online-softmax batch (= gathers in flight per lane)
 
-template <int G, bool EXTRA>   // EXTRA: attention dropout mask and / or attention output (both need edge ids)
+// EXTRA: attention dropout mask and / or attention output (both need edge ids); HASH (implies EXTRA): the dropout
+// factor comes from hashed_keep instead of a.keep
+// The HASH instantiations keep their explicit-mask siblings' blocks per SM: one block less removes most of their spills
+// but was slower on the MAG graph (B200, forward + backward of the core: REGAT H8 D16 11.8 ms instead of 10.5)
+template <int G, bool EXTRA, bool HASH = false>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, (EXTRA || G < 32) ? 4 : 5)   // 48 registers spill for G < 32
 gat_fwd_rg_kernel(AttnArgs a) {
+  static_assert(EXTRA || !HASH, "the hashed dropout factor needs the edge ids");
   constexpr int U = kUG;
   static_assert(G % U == 0, "a batch must not straddle a cooperative slot load");
   extern __shared__ __align__(16) float smem[];
@@ -259,7 +278,8 @@ gat_fwd_rg_kernel(AttnArgs a) {
           if (EXTRA && si[u] >= 0 && act) {
             const size_t o = (size_t)seid[u] * H + h;
             if (a.o3 != nullptr && leader) a.o3[o] = l[u];  // raw logit; normalised after the row
-            if (a.keep != nullptr) p *= __ldg(a.keep + o);
+            if (HASH) p *= hashed_keep(a, seid[u], h);
+            else if (a.keep != nullptr) p *= __ldg(a.keep + o);
           }
           fma4(acc, p, x[u]);
         }
@@ -292,7 +312,8 @@ gat_fwd_rg_kernel(AttnArgs a) {
       for (int t = lg & (lph - 1); t < len; t += lph) {
         const size_t o = (size_t)eidp[t] * H + h;
         float av = __expf(a.o3[o] - mm) * inv;
-        if (a.keep != nullptr) av *= a.keep[o];
+        if (HASH) av *= hashed_keep(a, eidp[t], h);
+        else if (a.keep != nullptr) av *= a.keep[o];
         a.o3[o] = av;
       }
   }
@@ -355,9 +376,12 @@ gat_bwd_stats_kernel(const float* __restrict__ out, const float* __restrict__ Gd
 #ifndef REGNN_GATB_U
 #define REGNN_GATB_U 2
 #endif
-template <int G, int LPH, bool KEEP>   // LPH = min(G, D/4): lanes per head (compile-time butterfly)
+// LPH = min(G, D/4): lanes per head (compile-time butterfly); KEEP: attention dropout, its factor from a.keep or -- HASH --
+// from hashed_keep
+template <int G, int LPH, bool KEEP, bool HASH = false>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_GATB_BLOCKS)
 gat_bwd_edges_kernel(AttnArgs a) {
+  static_assert(KEEP || !HASH, "HASH is a dropout mode");
   constexpr int U = REGNN_GATB_U;  // rows of G (and statistics vectors) in flight per lane
   static_assert(G % U == 0, "a round must not straddle a slot batch");
   extern __shared__ __align__(16) float smem[];
@@ -441,7 +465,10 @@ gat_bwd_edges_kernel(AttnArgs a) {
         const float aa = __expf(leaky(pre, a.slope) - st[u].y) * st[u].z;
         float at = aa;
         if (KEEP) {
-          if (sd[u] >= 0 && act) at *= __ldg(a.keep + (size_t)__ldg(a.a_csr_eid + ss) * H + h);
+          if (sd[u] >= 0 && act) {
+            const int e = __ldg(a.a_csr_eid + ss);
+            at *= HASH ? hashed_keep(a, e, h) : __ldg(a.keep + (size_t)e * H + h);
+          }
         }
         const float dp = (at * da[u] - aa * st[u].w) * leaky_grad(pre, a.slope);
         fma4(acc, at, x[u]);
@@ -717,9 +744,10 @@ attn_scores_bwd_kernel(const float* __restrict__ feat, const float* __restrict__
 #ifndef REGNN_V2F_BLOCKS
 #define REGNN_V2F_BLOCKS 4
 #endif
-template <int G, int LPH, bool EXTRA>
+template <int G, int LPH, bool EXTRA, bool HASH = false>   // EXTRA / HASH as gat_fwd_rg_kernel
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_V2F_BLOCKS)
 gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__ qmask) {
+  static_assert(EXTRA || !HASH, "the hashed dropout factor needs the edge ids");
   constexpr int U = kUG;
   static_assert(G % U == 0, "a batch must not straddle a cooperative slot load");
   extern __shared__ __align__(16) float smem[];
@@ -817,7 +845,8 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
           if (EXTRA && si[u] >= 0 && act) {
             const size_t o = (size_t)seid[u] * H + h;
             if (a.o3 != nullptr && leader) a.o3[o] = l[u];
-            if (a.keep != nullptr) p *= __ldg(a.keep + o);
+            if (HASH) p *= hashed_keep(a, seid[u], h);
+            else if (a.keep != nullptr) p *= __ldg(a.keep + o);
           }
           fma4(acc, p, x[u]);
         }
@@ -849,7 +878,8 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
       for (int t = lg & (LPH - 1); t < len; t += LPH) {
         const size_t o = (size_t)eidp[t] * H + h;
         float av = __expf(a.o3[o] - mm) * inv;
-        if (a.keep != nullptr) av *= a.keep[o];
+        if (HASH) av *= hashed_keep(a, eidp[t], h);
+        else if (a.keep != nullptr) av *= a.keep[o];
         a.o3[o] = av;
       }
   }
@@ -901,10 +931,11 @@ __device__ __forceinline__ float4 phi_total(const PhiAcc& t, float slope) {
 __device__ __forceinline__ float4 mul4(float4 a, float4 b) { return make_float4(a.x * b.x, a.y * b.y, a.z * b.z, a.w * b.w); }
 
 // AttnArgs: indptr/indices/eid = indptr_t/indices_t/slot_t, feat = fs, fd = stats (float4[N*H]), el = attn, a_csr = the
-// stored logits, a_csr_eid = slot -> edge id (keep only), o0 = d_fs, o2 = dl per slot.  dat_part: [gridDim.x][H*D].
-template <int G, int LPH, bool KEEP>
+// stored logits, a_csr_eid = slot -> edge id (keep / dropout only), o0 = d_fs, o2 = dl per slot.  dat_part: [gridDim.x][H*D].
+template <int G, int LPH, bool KEEP, bool HASH = false>   // KEEP / HASH as gat_bwd_edges_kernel
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_V2E_BLOCKS)
 gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __restrict__ dat_part) {
+  static_assert(KEEP || !HASH, "HASH is a dropout mode");
   constexpr int U = 2;
   static_assert(G % U == 0, "a round must not straddle a slot batch");
   __shared__ __align__(16) float dat_s[kWarpsPerBlock * 128];
@@ -970,7 +1001,10 @@ gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __
         const float aa = __expf(lv[u] - st[u].y) * st[u].z;
         float at = aa;
         if (KEEP) {
-          if (sd[u] >= 0 && act) at *= __ldg(a.keep + (size_t)__ldg(a.a_csr_eid + ss[u]) * H + h);
+          if (sd[u] >= 0 && act) {
+            const int e = __ldg(a.a_csr_eid + ss[u]);
+            at *= HASH ? hashed_keep(a, e, h) : __ldg(a.keep + (size_t)e * H + h);
+          }
         }
         const float dl = at * da[u] - aa * st[u].w;
         fma4(acc, at, x[u]);
@@ -1157,7 +1191,9 @@ gatv2_bwd_dst_stream_kernel(AttnArgs a, const uint32_t* __restrict__ qmask) {
 // =================================================================================================
 // Merges the fragments of every long row of a forward pass (online-softmax combine in fragment order):
 //   M = max_f m_f;  S = sum_f s_f*exp(m_f-M);  out = sum_f acc_f*exp(m_f-M) / S
-// and, for get_attention, normalises the row's stored logits.  One warp per (long row, head group).
+// and, for get_attention, normalises the row's stored logits.  One warp per (long row, head group).  HASH: the dropout
+// factor of get_attention from hashed_keep.
+template <bool HASH>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 attn_frag_finalize_kernel(AttnArgs a, const int32_t* __restrict__ long_rows,
                           const int32_t* __restrict__ frag_ptr, int num_long) {
@@ -1195,10 +1231,12 @@ attn_frag_finalize_kernel(AttnArgs a, const int32_t* __restrict__ long_rows,
     const int s0 = a.indptr[v], len = a.indptr[v + 1] - s0;
     for (int i = lane; i < len * g.nh; i += 32) {
       const int h = g.h_lo + i % g.nh;
-      const size_t o = (size_t)a.eid[s0 + i / g.nh] * H + h;
+      const int e = a.eid[s0 + i / g.nh];
+      const size_t o = (size_t)e * H + h;
       const float s = a.o2[(size_t)v * H + h];
       float av = expf(a.o3[o] - a.o1[(size_t)v * H + h]) * (s > 0.f ? 1.f / s : 0.f);
-      if (a.keep != nullptr) av *= a.keep[o];
+      if (HASH) av *= hashed_keep(a, e, h);
+      else if (a.keep != nullptr) av *= a.keep[o];
       a.o3[o] = av;
     }
   }
@@ -1281,8 +1319,9 @@ static int check_shape(const char* who, int H, int D, int R, bool has_rel, bool 
     KERNEL<<<GRID, kWarpsPerBlock * 32, SMEM, stream>>>(a);                   \
   } while (0)
 
-#define REGNN_DISPATCH_FINALIZE(GRID) \
-  attn_frag_finalize_kernel<<<GRID, kWarpsPerBlock * 32, 0, stream>>>(a, split->long_rows, split->frag_ptr, split->num_long)
+#define REGNN_DISPATCH_FINALIZE(GRID, HASH_)                                                                           \
+  attn_frag_finalize_kernel<HASH_><<<GRID, kWarpsPerBlock * 32, 0, stream>>>(a, split->long_rows, split->frag_ptr,      \
+                                                                             split->num_long)
 
 static int head_groups(int H, int D) { return (H * D + 127) / 128; }
 
@@ -1304,6 +1343,20 @@ static void apply_order(AttnArgs& a, const int32_t* row_order, const regnn_rowsp
   }
 }
 
+// Fills the dropout fields of `a` (dropout != NULL); returns false if the struct is inconsistent with the call's heads.
+static bool apply_dropout(AttnArgs& a, const regnn_attn_dropout_t* dropout) {
+  if (dropout == nullptr) return true;
+  if (dropout->head_offset < 0 || dropout->num_heads_total < dropout->head_offset + a.H) return false;
+  if (!(dropout->scale >= 0.f) || dropout->scale == INFINITY) return false;
+  a.drop_key_lo = (uint32_t)dropout->key;
+  a.drop_key_hi = (uint32_t)(dropout->key >> 32);
+  a.drop_threshold = dropout->threshold;
+  a.drop_scale = dropout->scale;
+  a.drop_head_offset = dropout->head_offset;
+  a.drop_heads_total = dropout->num_heads_total;
+  return true;
+}
+
 }  // namespace regnn
 
 using namespace regnn;
@@ -1311,13 +1364,15 @@ using namespace regnn;
 extern "C" int regnn_gat_fwd(const int32_t* indptr, const int32_t* indices, const int32_t* eid,
                              const uint8_t* etype_csr, const float* theta, float alpha,
                              int num_relations, const float* feat, const float* el, const float* er,
-                             float negative_slope, const float* keep, int num_heads, int head_dim,
-                             int64_t row_begin, int64_t row_end, float* out, float* rowmax,
+                             float negative_slope, const float* keep, const regnn_attn_dropout_t* dropout,
+                             int num_heads, int head_dim, int64_t row_begin, int64_t row_end, float* out, float* rowmax,
                              float* rowsum, float* attn_out, const regnn_rowsplit_t* split, float* split_workspace,
                              const int32_t* row_order, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   REGNN_REQUIRE(indptr && feat && el && er && out && rowmax && rowsum, REGNN_ERR_INVALID_ARG, "gat_fwd: null pointer");
-  REGNN_REQUIRE((keep == nullptr && attn_out == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG, "gat_fwd: keep/attn_out need eid");
+  REGNN_REQUIRE(keep == nullptr || dropout == nullptr, REGNN_ERR_INVALID_ARG, "gat_fwd: keep and dropout are exclusive");
+  REGNN_REQUIRE((keep == nullptr && dropout == nullptr && attn_out == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG,
+                "gat_fwd: keep/dropout/attn_out need eid");
   REGNN_REQUIRE(etype_csr == nullptr || theta != nullptr, REGNN_ERR_INVALID_ARG, "gat_fwd: etype without theta");
   int rc = check_shape("gat_fwd", num_heads, head_dim, num_relations, etype_csr != nullptr, true);  // as the backward: fail early
   if (rc != REGNN_OK) return rc;
@@ -1331,10 +1386,18 @@ extern "C" int regnn_gat_fwd(const int32_t* indptr, const int32_t* indices, cons
   a.H = num_heads; a.D = head_dim; a.row_begin = row_begin; a.row_end = row_end;
   a.o0 = out; a.o1 = rowmax; a.o2 = rowsum; a.o3 = attn_out;
   REGNN_REQUIRE(apply_split(a, split, split_workspace), REGNN_ERR_INVALID_ARG, "gat_fwd: incomplete row split");
+  REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gat_fwd: dropout heads / scale inconsistent");
   apply_order(a, row_order, split, rows);
   const size_t smem = sizeof(float) * ((size_t)a.R * num_heads) + 16;
   const unsigned grid = (unsigned)((rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock);
-  if (keep != nullptr || attn_out != nullptr) {
+  if (dropout != nullptr) {
+    switch (rg_lanes(a.H * a.D)) {
+      case 4: REGNN_DISPATCH_C((gat_fwd_rg_kernel<4, true, true>), grid, smem); break;
+      case 8: REGNN_DISPATCH_C((gat_fwd_rg_kernel<8, true, true>), grid, smem); break;
+      case 16: REGNN_DISPATCH_C((gat_fwd_rg_kernel<16, true, true>), grid, smem); break;
+      default: REGNN_DISPATCH_C((gat_fwd_rg_kernel<32, true, true>), grid, smem); break;
+    }
+  } else if (keep != nullptr || attn_out != nullptr) {
     switch (rg_lanes(a.H * a.D)) {
       case 4: REGNN_DISPATCH_C((gat_fwd_rg_kernel<4, true>), grid, smem); break;
       case 8: REGNN_DISPATCH_C((gat_fwd_rg_kernel<8, true>), grid, smem); break;
@@ -1351,7 +1414,8 @@ extern "C" int regnn_gat_fwd(const int32_t* indptr, const int32_t* indices, cons
   }
   if (a.nfrag > 0) {
     const unsigned fgrid = (unsigned)(((int64_t)split->num_long * head_groups(a.H, a.D) + kWarpsPerBlock - 1) / kWarpsPerBlock);
-    REGNN_DISPATCH_FINALIZE(fgrid);
+    if (dropout != nullptr) REGNN_DISPATCH_FINALIZE(fgrid, true);
+    else REGNN_DISPATCH_FINALIZE(fgrid, false);
   }
   return check_launch("regnn_gat_fwd");
 }
@@ -1391,14 +1455,17 @@ extern "C" int regnn_gat_bwd_stats(const float* out, const float* Gd, const floa
 extern "C" int regnn_gat_bwd_edges(const int32_t* indptr_t, const int32_t* indices_t, const int32_t* slot_t,
                                    const uint8_t* etype_t, const int32_t* eid, const float* theta, float alpha,
                                    int num_relations, const float* feat, const float* el, const float* stats,
-                                   float negative_slope, const float* keep, const float* Gd, int num_heads,
+                                   float negative_slope, const float* keep, const regnn_attn_dropout_t* dropout,
+                                   const float* Gd, int num_heads,
                                    int head_dim, int64_t row_begin, int64_t row_end, float* d_feat, float* d_el,
                                    float* dpre_csr, const float* attn_l, const regnn_rowsplit_t* split_t,
                                    float* split_workspace, const int32_t* row_order_t, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   REGNN_REQUIRE(indptr_t && feat && el && stats && Gd && d_feat && d_el, /* per-edge arrays may be NULL when E == 0 */
                 REGNN_ERR_INVALID_ARG, "gat_bwd_edges: null pointer");
-  REGNN_REQUIRE(keep == nullptr || eid != nullptr, REGNN_ERR_INVALID_ARG, "gat_bwd_edges: keep needs eid");
+  REGNN_REQUIRE(keep == nullptr || dropout == nullptr, REGNN_ERR_INVALID_ARG, "gat_bwd_edges: keep and dropout are exclusive");
+  REGNN_REQUIRE((keep == nullptr && dropout == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG,
+                "gat_bwd_edges: keep/dropout need eid");
   REGNN_REQUIRE(etype_t == nullptr || theta != nullptr, REGNN_ERR_INVALID_ARG, "gat_bwd_edges: etype without theta");
   int rc = check_shape("gat_bwd_edges", num_heads, head_dim, num_relations, etype_t != nullptr, true);
   if (rc != REGNN_OK) return rc;
@@ -1413,6 +1480,7 @@ extern "C" int regnn_gat_bwd_edges(const int32_t* indptr_t, const int32_t* indic
   a.a_csr_eid = eid; a.G = Gd; a.H = num_heads; a.D = head_dim; a.row_begin = row_begin; a.row_end = row_end;
   a.o0 = d_feat; a.o1 = d_el; a.o2 = dpre_csr; a.attn_l = attn_l;
   REGNN_REQUIRE(apply_split(a, split_t, split_workspace), REGNN_ERR_INVALID_ARG, "gat_bwd_edges: incomplete row split");
+  REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gat_bwd_edges: dropout heads / scale inconsistent");
   apply_order(a, row_order_t, split_t, rows);
   const size_t smem = sizeof(float) * ((size_t)a.R * num_heads) + 16;
   const unsigned grid = (unsigned)((rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock);
@@ -1421,7 +1489,8 @@ extern "C" int regnn_gat_bwd_edges(const int32_t* indptr_t, const int32_t* indic
     bool launched = false;
 #define REGNN_EDGES_CASE(G_, L_)                                                                   \
   if (G == G_ && lph == L_) {                                                                      \
-    if (keep != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true>), grid, smem);       \
+    if (dropout != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true, true>), grid, smem); \
+    else if (keep != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true>), grid, smem);  \
     else REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, false>), grid, smem);                      \
     launched = true;                                                                               \
   }
@@ -1565,13 +1634,16 @@ extern "C" int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, co
                                const uint8_t* etype_csr, const float* theta, float alpha,
                                int num_relations, const float* fs, const float* fd,
                                const float* attn, float negative_slope, const float* keep,
-                               int num_heads, int head_dim, int64_t row_begin, int64_t row_end,
+                               const regnn_attn_dropout_t* dropout, int num_heads, int head_dim, int64_t row_begin,
+                               int64_t row_end,
                                float* out, float* rowmax, float* rowsum, float* attn_out, float* logit_csr,
                                uint32_t* qmask, const regnn_rowsplit_t* split, float* split_workspace,
                                const int32_t* row_order, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   REGNN_REQUIRE(indptr && fs && fd && attn && out && rowmax && rowsum, REGNN_ERR_INVALID_ARG, "gatv2_fwd: null pointer");
-  REGNN_REQUIRE((keep == nullptr && attn_out == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG, "gatv2_fwd: keep/attn_out need eid");
+  REGNN_REQUIRE(keep == nullptr || dropout == nullptr, REGNN_ERR_INVALID_ARG, "gatv2_fwd: keep and dropout are exclusive");
+  REGNN_REQUIRE((keep == nullptr && dropout == nullptr && attn_out == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG,
+                "gatv2_fwd: keep/dropout/attn_out need eid");
   REGNN_REQUIRE(etype_csr == nullptr || theta != nullptr, REGNN_ERR_INVALID_ARG, "gatv2_fwd: etype without theta");
   int rc = check_shape("gatv2_fwd", num_heads, head_dim, num_relations, etype_csr != nullptr, true);
   if (rc != REGNN_OK) return rc;
@@ -1587,18 +1659,22 @@ extern "C" int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, co
   a.H = num_heads; a.D = head_dim; a.row_begin = row_begin; a.row_end = row_end;
   a.o0 = out; a.o1 = rowmax; a.o2 = rowsum; a.o3 = attn_out;
   REGNN_REQUIRE(apply_split(a, split, split_workspace), REGNN_ERR_INVALID_ARG, "gatv2_fwd: incomplete row split");
+  REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gatv2_fwd: dropout heads / scale inconsistent");
   apply_order(a, row_order, split, rows);
   const size_t smem = sizeof(float) * ((size_t)a.R * num_heads) + 16;
   const unsigned grid = (unsigned)((rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock);
   {
     const int G = rg_lanes(a.H * a.D), lph = min(G, head_dim / 4);
+    const bool hash = dropout != nullptr;
     const bool extra = keep != nullptr || attn_out != nullptr;
     bool launched = false;
 #define REGNN_V2F_CASE(G_, L_)                                                                   \
   if (G == G_ && lph == L_) {                                                                    \
-    rc = set_smem(extra ? gatv2_fwd_rg_kernel<G_, L_, true> : gatv2_fwd_rg_kernel<G_, L_, false>, smem);             \
+    rc = set_smem(hash ? gatv2_fwd_rg_kernel<G_, L_, true, true>                                                     \
+                       : (extra ? gatv2_fwd_rg_kernel<G_, L_, true> : gatv2_fwd_rg_kernel<G_, L_, false>), smem);    \
     if (rc != REGNN_OK) return rc;                                                                                   \
-    if (extra) gatv2_fwd_rg_kernel<G_, L_, true><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask);  \
+    if (hash) gatv2_fwd_rg_kernel<G_, L_, true, true><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask); \
+    else if (extra) gatv2_fwd_rg_kernel<G_, L_, true><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask); \
     else gatv2_fwd_rg_kernel<G_, L_, false><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask);       \
     launched = true;                                                                                                 \
   }
@@ -1612,7 +1688,8 @@ extern "C" int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, co
   }
   if (a.nfrag > 0) {
     const unsigned fgrid = (unsigned)(((int64_t)split->num_long * head_groups(a.H, a.D) + kWarpsPerBlock - 1) / kWarpsPerBlock);
-    REGNN_DISPATCH_FINALIZE(fgrid);
+    if (dropout != nullptr) REGNN_DISPATCH_FINALIZE(fgrid, true);
+    else REGNN_DISPATCH_FINALIZE(fgrid, false);
   }
   return check_launch("regnn_gatv2_fwd");
 }
@@ -1629,14 +1706,17 @@ extern "C" int64_t regnn_gatv2_bwd_edges_blocks(int64_t num_rows, int num_frags,
 extern "C" int regnn_gatv2_bwd_edges(const int32_t* indptr_t, const int32_t* indices_t, const int32_t* slot_t,
                                      const int32_t* eid, const float* fs, const float* stats, const float* logit_csr,
                                      const uint32_t* qmask, const float* attn, float negative_slope, const float* keep,
-                                     const float* Gd, int num_heads, int head_dim, int64_t row_begin, int64_t row_end,
+                                     const regnn_attn_dropout_t* dropout, const float* Gd, int num_heads, int head_dim,
+                                     int64_t row_begin, int64_t row_end,
                                      float* d_fs, float* dl_csr, float* d_attn_src, float* block_partials,
                                      double* partials, const regnn_rowsplit_t* split_t, float* split_workspace,
                                      const int32_t* row_order_t, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   REGNN_REQUIRE(indptr_t && fs && stats && attn && Gd && d_fs && d_attn_src && block_partials && partials,
                 REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: null pointer");  /* per-edge arrays may be NULL when E == 0 */
-  REGNN_REQUIRE(keep == nullptr || eid != nullptr, REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: keep needs eid");
+  REGNN_REQUIRE(keep == nullptr || dropout == nullptr, REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: keep and dropout are exclusive");
+  REGNN_REQUIRE((keep == nullptr && dropout == nullptr) || eid != nullptr, REGNN_ERR_INVALID_ARG,
+                "gatv2_bwd_edges: keep/dropout need eid");
   int rc = check_shape("gatv2_bwd_edges", num_heads, head_dim, 0, false, true);
   if (rc != REGNN_OK) return rc;
   REGNN_REQUIRE(aligned16(fs) && aligned16(stats) && aligned16(attn) && aligned16(Gd) && aligned16(d_fs) && aligned16(qmask),
@@ -1653,6 +1733,7 @@ extern "C" int regnn_gatv2_bwd_edges(const int32_t* indptr_t, const int32_t* ind
   a.a_csr = logit_csr; a.el = attn; a.slope = negative_slope; a.keep = keep; a.G = Gd; a.H = num_heads; a.D = head_dim;
   a.row_begin = row_begin; a.row_end = row_end; a.o0 = d_fs; a.o2 = dl_csr;
   REGNN_REQUIRE(apply_split(a, split_t, split_workspace), REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: incomplete row split");
+  REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: dropout heads / scale inconsistent");
   apply_order(a, row_order_t, split_t, rows);
   const int64_t nb = (rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock;
   {
@@ -1660,7 +1741,10 @@ extern "C" int regnn_gatv2_bwd_edges(const int32_t* indptr_t, const int32_t* ind
     bool launched = false;
 #define REGNN_V2E_CASE(G_, L_)                                                                                          \
   if (G == G_ && lph == L_) {                                                                                           \
-    if (keep != nullptr)                                                                                                \
+    if (dropout != nullptr)                                                                                             \
+      gatv2_bwd_edges_kernel<G_, L_, true, true><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask,            \
+                                                                                                  block_partials);     \
+    else if (keep != nullptr)                                                                                           \
       gatv2_bwd_edges_kernel<G_, L_, true><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask, block_partials); \
     else                                                                                                                \
       gatv2_bwd_edges_kernel<G_, L_, false><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask, block_partials);\

@@ -10,13 +10,6 @@
 
 namespace regnn {
 
-__host__ __device__ __forceinline__ uint32_t mix32(uint32_t z) {
-  z ^= z >> 16; z *= 0x7feb352du;
-  z ^= z >> 15; z *= 0x846ca68bu;
-  z ^= z >> 16;
-  return z;
-}
-
 __host__ __device__ __forceinline__ uint32_t feistel_perm(uint32_t x, uint32_t deg, uint32_t key) {
   int b = 2;
   while ((1u << b) < deg) b += 2;          // even number of bits, 2^b >= deg

@@ -7,6 +7,14 @@ all reductions are executed by the deterministic kernels in ``re_gnn_b200/csrc``
 import torch
 
 from . import ops
+from .dropout import HashedDropout, attn_dropout_key  # noqa: F401  (public: the dropout= argument of the attention cores)
+
+
+def _check_dropout(keep, dropout, name):
+    if keep is not None and dropout is not None:
+        raise ValueError('%s: pass either keep (an explicit [E, H] mask) or dropout (HashedDropout), not both' % name)
+    if dropout is not None and not isinstance(dropout, HashedDropout):
+        raise TypeError('%s: dropout must be a HashedDropout, got %s' % (name, type(dropout).__name__))
 
 
 class _WDegNorm(torch.autograd.Function):
@@ -121,14 +129,14 @@ class _GatAggregate(torch.autograd.Function):
     the scores come from different node sets)."""
 
     @staticmethod
-    def forward(ctx, graph, etv, feat, el, er, theta, alpha, slope, keep, want_attn, softmax_eps):
+    def forward(ctx, graph, etv, feat, el, er, theta, alpha, slope, keep, want_attn, softmax_eps, dropout):
         csr = graph.csr()
         et = etv[0] if etv is not None else None
         out, rowmax, rowsum, attn = ops.gat_fwd(csr, et, theta if et is not None else None, alpha, feat, el, er,
-                                                slope, keep, want_attn)
+                                                slope, keep, want_attn, **ops.dropout_kw(dropout))
         if softmax_eps:
             rowsum = _global_max_eps(csr, out, rowmax, rowsum, attn, softmax_eps)
-        ctx.graph, ctx.et, ctx.alpha, ctx.slope = graph, et, alpha, slope
+        ctx.graph, ctx.et, ctx.alpha, ctx.slope, ctx.dropout = graph, et, alpha, slope, dropout
         ctx.et_t = etv[1] if etv is not None else None
         ctx.save_for_backward(feat, el, er, theta if et is not None else None, keep, out, rowmax, rowsum)
         if want_attn:
@@ -141,14 +149,19 @@ class _GatAggregate(torch.autograd.Function):
         feat, el, er, theta, keep, out, rowmax, rowsum = ctx.saved_tensors
         csr = ctx.graph.csr()
         d_feat, d_el, d_er, d_theta, _, _ = ops.gat_bwd(csr, ctx.et, ctx.et_t, theta, ctx.alpha, feat, el, er, ctx.slope,
-                                                        keep, out, rowmax, rowsum, g.contiguous())
+                                                        keep, out, rowmax, rowsum, g.contiguous(),
+                                                        **ops.dropout_kw(ctx.dropout))
         return (None, None, d_feat, d_el, d_er, d_theta.view_as(theta) if d_theta is not None else None,
-                None, None, None, None, None)
+                None, None, None, None, None, None)
 
 
-def gat_aggregate(graph, etv, feat, el, er, theta, alpha, slope, keep=None, want_attn=False, softmax_eps=0.0):
-    """``softmax_eps`` > 0: the MAG stack's global-max softmax with ``+ eps`` in the denominator (``_global_max_eps``)."""
-    return _GatAggregate.apply(graph, etv, feat, el, er, theta, alpha, slope, keep, want_attn, softmax_eps)
+def gat_aggregate(graph, etv, feat, el, er, theta, alpha, slope, keep=None, want_attn=False, softmax_eps=0.0,
+                  dropout=None):
+    """``softmax_eps`` > 0: the MAG stack's global-max softmax with ``+ eps`` in the denominator (``_global_max_eps``).
+    Attention dropout: ``keep`` (an [E, H] mask in edge-id order) or ``dropout`` (a ``HashedDropout``: the kernels
+    compute the mask from the edge ids, nothing is drawn or stored)."""
+    _check_dropout(keep, dropout, 'gat_aggregate')
+    return _GatAggregate.apply(graph, etv, feat, el, er, theta, alpha, slope, keep, want_attn, softmax_eps, dropout)
 
 
 class _GatLayer(torch.autograd.Function):
@@ -157,14 +170,14 @@ class _GatLayer(torch.autograd.Function):
     backward with the gradients through el / er folded into its kernels (no [N,H,D] temporaries from autograd)."""
 
     @staticmethod
-    def forward(ctx, graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep, want_attn):
+    def forward(ctx, graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep, want_attn, dropout):
         csr = graph.csr()
         et = etv[0] if etv is not None else None
         feat = feat.contiguous()
         el, er = ops.attn_scores_fwd(feat, attn_l, attn_r)
         out, rowmax, rowsum, attn = ops.gat_fwd(csr, et, theta if et is not None else None, alpha, feat, el, er,
-                                                slope, keep, want_attn)
-        ctx.graph, ctx.et, ctx.alpha, ctx.slope = graph, et, alpha, slope
+                                                slope, keep, want_attn, **ops.dropout_kw(dropout))
+        ctx.graph, ctx.et, ctx.alpha, ctx.slope, ctx.dropout = graph, et, alpha, slope, dropout
         ctx.et_t = etv[1] if etv is not None else None
         ctx.save_for_backward(feat, el, er, attn_l, attn_r, theta if et is not None else None, keep, out, rowmax, rowsum)
         if want_attn:
@@ -178,27 +191,29 @@ class _GatLayer(torch.autograd.Function):
         csr = ctx.graph.csr()
         d_feat, _, _, d_theta, d_al, d_ar = ops.gat_bwd(csr, ctx.et, ctx.et_t, theta, ctx.alpha, feat, el, er, ctx.slope,
                                                         keep, out, rowmax, rowsum, g.contiguous(), attn_l=attn_l,
-                                                        attn_r=attn_r)
+                                                        attn_r=attn_r, **ops.dropout_kw(ctx.dropout))
         return (None, None, d_feat, d_al.view_as(attn_l), d_ar.view_as(attn_r),
-                d_theta.view_as(theta) if d_theta is not None else None, None, None, None, None)
+                d_theta.view_as(theta) if d_theta is not None else None, None, None, None, None, None)
 
 
-def gat_layer(graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep=None, want_attn=False):
-    """feat [N,H,D] (source and destination side are the same nodes) -> (out [N,H,D], attention | None)."""
-    return _GatLayer.apply(graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep, want_attn)
+def gat_layer(graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep=None, want_attn=False, dropout=None):
+    """feat [N,H,D] (source and destination side are the same nodes) -> (out [N,H,D], attention | None).
+    Attention dropout: ``keep`` or ``dropout`` (a ``HashedDropout``), as ``gat_aggregate``."""
+    _check_dropout(keep, dropout, 'gat_layer')
+    return _GatLayer.apply(graph, etv, feat, attn_l, attn_r, theta, alpha, slope, keep, want_attn, dropout)
 
 
 class _GatV2Aggregate(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, graph, etv, fs, fd, attn, theta, alpha, slope, keep, want_attn, softmax_eps):
+    def forward(ctx, graph, etv, fs, fd, attn, theta, alpha, slope, keep, want_attn, softmax_eps, dropout):
         csr = graph.csr()
         et = etv[0] if etv is not None else None
         train = any(ctx.needs_input_grad)
         out, rowmax, rowsum, a, saved = ops.gatv2_fwd(csr, et, theta if et is not None else None, alpha, fs, fd, attn,
-                                                      slope, keep, want_attn, save=train)
+                                                      slope, keep, want_attn, save=train, **ops.dropout_kw(dropout))
         if softmax_eps:
             rowsum = _global_max_eps(csr, out, rowmax, rowsum, a, softmax_eps)
-        ctx.graph, ctx.et, ctx.alpha, ctx.slope = graph, et, alpha, slope
+        ctx.graph, ctx.et, ctx.alpha, ctx.slope, ctx.dropout = graph, et, alpha, slope, dropout
         ctx.save_for_backward(fs, fd, attn, theta if et is not None else None, keep, out, rowmax, rowsum,
                               *(saved if train else ()))
         if want_attn:
@@ -211,13 +226,17 @@ class _GatV2Aggregate(torch.autograd.Function):
         fs, fd, attn, theta, keep, out, rowmax, rowsum, logit_csr, qmask = ctx.saved_tensors
         csr = ctx.graph.csr()
         d_fs, d_fd, d_attn, d_theta = ops.gatv2_bwd(csr, ctx.et, theta, ctx.alpha, fs, fd, attn, ctx.slope, keep, out,
-                                                    rowmax, rowsum, (logit_csr, qmask), g.contiguous())
+                                                    rowmax, rowsum, (logit_csr, qmask), g.contiguous(),
+                                                    **ops.dropout_kw(ctx.dropout))
         return (None, None, d_fs, d_fd, d_attn.view_as(attn),
-                d_theta.view_as(theta) if d_theta is not None else None, None, None, None, None, None)
+                d_theta.view_as(theta) if d_theta is not None else None, None, None, None, None, None, None)
 
 
-def gatv2_aggregate(graph, etv, fs, fd, attn, theta, alpha, slope, keep=None, want_attn=False, softmax_eps=0.0):
-    return _GatV2Aggregate.apply(graph, etv, fs, fd, attn, theta, alpha, slope, keep, want_attn, softmax_eps)
+def gatv2_aggregate(graph, etv, fs, fd, attn, theta, alpha, slope, keep=None, want_attn=False, softmax_eps=0.0,
+                    dropout=None):
+    """Attention dropout: ``keep`` or ``dropout`` (a ``HashedDropout``), as ``gat_aggregate``."""
+    _check_dropout(keep, dropout, 'gatv2_aggregate')
+    return _GatV2Aggregate.apply(graph, etv, fs, fd, attn, theta, alpha, slope, keep, want_attn, softmax_eps, dropout)
 
 
 class _GroupedLinear(torch.autograd.Function):

@@ -322,10 +322,25 @@ def _full(rb, re, n):
     return (rb, re) == (0, n)
 
 
-def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn=False, rows=None):
+def _drop(dropout, heads):
+    """byref(regnn_attn_dropout_t) of a ``dropout.HashedDropout`` for a call over ``heads`` heads, or None."""
+    return ctypes.byref(dropout.struct(heads)) if dropout is not None else None
+
+
+def dropout_kw(dropout):
+    """``{'dropout': dropout}``, or no keyword at all without dropout: callers that compose the stage wrappers pass it
+    this way, so that stand-ins of the stages written before the keyword existed keep working."""
+    return {} if dropout is None else {'dropout': dropout}
+
+
+def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn=False, rows=None, dropout=None,
+            eid=None):
     """-> (out, rowmax, rowsum, attention | None) for the rows of ``csr``.  ``feat`` / ``el`` are indexed by the column
-    ids of ``csr`` and may have more rows than the CSR (a halo of remote sources after the own rows)."""
+    ids of ``csr`` and may have more rows than the CSR (a halo of remote sources after the own rows).
+    ``dropout``: a ``HashedDropout`` (counter-based attention dropout, exclusive with ``keep``); ``eid``: the global edge
+    id of every slot when it is not ``csr['eid']`` (the in-view of a halo partition)."""
     feat, el, er, keep = _f32(feat), _f32(el), _f32(er), _f32(keep)
+    eid = csr.get('eid') if eid is None else eid
     _, h, d = feat.shape
     n = csr['indptr'].numel() - 1
     rb, re = _rows(rows, n)
@@ -341,24 +356,26 @@ def gat_fwd(csr, et_csr, theta, alpha, feat, el, er, slope, keep=None, want_attn
     sp, ws = _attn_split(csr.get('split'), h, d, dev)
     order = row_order(csr) if _full(rb, re, n) else None
     with torch.cuda.device(dev):
-        _lib.call('regnn_gat_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr.get('eid')), _ptr(et_csr),
-                  _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el), _ptr(er), float(slope), _ptr(keep), h, d,
+        _lib.call('regnn_gat_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(eid), _ptr(et_csr),
+                  _ptr(theta), float(alpha), r, _ptr(feat), _ptr(el), _ptr(er), float(slope), _ptr(keep),
+                  _drop(dropout, h), h, d,
                   rb, re, _ptr(out), _ptr(rowmax), _ptr(rowsum), _ptr(attn), sp, _ptr(ws), _ptr(order), _stream())
         _lib.count_launches(1 + (sp is not None))
     return out, rowmax, rowsum, attn
 
 
 def gat_bwd(csr, et_csr, et_t, theta, alpha, feat, el, er, slope, keep, out, rowmax, rowsum, g, attn_l=None,
-            attn_r=None):
+            attn_r=None, dropout=None):
     """Backward of ``gat_fwd`` as one gather pass (``gat_bwd_stats`` -> ``gat_bwd_edges`` -> ``gat_bwd_reduce``)
     -> (d_feat, d_el, d_er, d_theta | None, d_attn_l | None, d_attn_r | None).
     With ``attn_l`` / ``attn_r`` ([H*D], the projection-score vectors of layer/REGATConv.py:68-69, el = <feat, attn_l>,
     er = <feat, attn_r>) the gradients through the scores are folded in: ``d_feat`` is the total feature gradient and
-    the two parameter gradients are returned (``attn_scores_bwd``)."""
+    the two parameter gradients are returned (``attn_scores_bwd``).  ``dropout``: the ``HashedDropout`` of the forward."""
     stats = gat_bwd_stats(out, g, er, rowmax, rowsum)
     e = csr['indices'].numel()
     dpre = torch.empty((max(e, 1), stats.shape[1]), dtype=torch.float32, device=stats.device)[:e]   # never a NULL pointer
-    d_feat, d_el = gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=attn_l, keep=keep)
+    d_feat, d_el = gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=attn_l, keep=keep,
+                                 **dropout_kw(dropout))
     d_er, d_theta = gat_bwd_reduce(csr, et_csr, theta, alpha, dpre)
     d_al = d_ar = None
     if attn_l is not None:
@@ -382,13 +399,16 @@ def gat_bwd_stats(out, g, er, rowmax, rowsum):
     return stats
 
 
-def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=None, keep=None):
+def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn_l=None, keep=None, dropout=None,
+                  eid=None):
     """Source-major pass over the rows of the transposed view ``csr['indptr_t']`` -> (d_feat, d_el) of those rows; the
     logit gradient of every entry j is written to ``dpre[csr['slot_t'][j]]`` ([slots, H]).  ``feat`` / ``el``: the rows'
     own values; ``g`` / ``stats``: indexed by the column ids of the view.  ``attn_l`` folds the gradient through el into
-    d_feat; ``keep``: the attention-dropout mask of ``gat_fwd``, in edge-id order through ``csr['eid']``
-    (regnn_gat_bwd_edges)."""
+    d_feat; ``keep``: the attention-dropout mask of ``gat_fwd``, in edge-id order through ``csr['eid']``;
+    ``dropout``: the ``HashedDropout`` of ``gat_fwd`` instead; ``eid``: the edge id of every slot ``csr['slot_t']``
+    points at when that is not ``csr['eid']`` (the extended slots of a halo partition) (regnn_gat_bwd_edges)."""
     feat, el, g, keep = _f32(feat), _f32(el), _f32(g), _f32(keep)
+    eid = (csr['eid'] if eid is None else eid) if (keep is not None or dropout is not None) else None
     theta, et_t, r = _rel(theta, et_t)
     n = csr['indptr_t'].numel() - 1
     _, h, d = feat.shape
@@ -399,8 +419,9 @@ def gat_bwd_edges(csr, et_t, theta, alpha, feat, el, stats, slope, g, dpre, attn
     sp_t, ws_t = _attn_split(csr.get('split_t'), h, d, dev)
     with torch.cuda.device(dev):
         _lib.call('regnn_gat_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
-                  _ptr(et_t) if r else None, _ptr(csr['eid']) if keep is not None else None, _ptr(theta), float(alpha),
-                  r, _ptr(feat), _ptr(el), _ptr(stats), float(slope), _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_feat),
+                  _ptr(et_t) if r else None, _ptr(eid), _ptr(theta), float(alpha),
+                  r, _ptr(feat), _ptr(el), _ptr(stats), float(slope), _ptr(keep), _drop(dropout, h), _ptr(g), h, d, 0,
+                  n, _ptr(d_feat),
                   _ptr(d_el), _ptr(dpre), _ptr(attn_l), sp_t, _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
         _lib.count_launches(1 + (3 if sp_t is not None else 0))
     return d_feat, d_el
@@ -455,15 +476,16 @@ def attn_scores_fwd(feat, attn_l, attn_r):
 
 
 def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_attn=False, rows=None, save=False,
-              saved=None):
+              saved=None, dropout=None, eid=None):
     """-> (out, rowmax, rowsum, attention | None, saved | None).  ``save``: also store what the backward needs, the raw
     logit of every (CSR slot, head) and the 128-bit sign mask of fs[src]+fd[dst] per (slot, 128-float slice):
     ``saved = (logit_csr [E,H], qmask [E, ceil(H*D/128), 4] int32)``.  ``saved`` given (implies ``save``): the caller's
     buffers of that layout with at least E rows, written in place (partition.halo_gatv2 passes the head of its
     per-slot exchange buffers).  ``fs`` is indexed by the column ids of ``csr`` and may have more rows than the CSR (a
     halo of remote sources after the own rows); ``fd`` has one row per CSR row.  ``csr['eid']`` is only needed with
-    ``keep`` or ``want_attn``."""
+    ``keep``, ``dropout`` or ``want_attn``.  ``dropout`` / ``eid``: as ``gat_fwd``."""
     fs, fd, keep = _f32(fs), _f32(fd), _f32(keep)
+    eid = csr.get('eid') if eid is None else eid
     attn = _f32(attn).view(-1)
     n, h, d = fd.shape
     rb, re = _rows(rows, n)
@@ -489,8 +511,9 @@ def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_at
     sp, ws = _attn_split(csr.get('split'), h, d, dev)
     order = row_order(csr) if _full(rb, re, n) else None
     with torch.cuda.device(dev):
-        _lib.call('regnn_gatv2_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr.get('eid')), _ptr(et_csr),
-                  _ptr(theta), float(alpha), r, _ptr(fs), _ptr(fd), _ptr(attn), float(slope), _ptr(keep), h, d,
+        _lib.call('regnn_gatv2_fwd', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(eid), _ptr(et_csr),
+                  _ptr(theta), float(alpha), r, _ptr(fs), _ptr(fd), _ptr(attn), float(slope), _ptr(keep),
+                  _drop(dropout, h), h, d,
                   rb, re, _ptr(out), _ptr(rowmax), _ptr(rowsum), _ptr(att), _ptr(saved[0]) if save else None,
                   _ptr(saved[1]) if save else None, sp, _ptr(ws), _ptr(order), _stream())
         _lib.count_launches(1 + (sp is not None))
@@ -500,14 +523,16 @@ def gatv2_fwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep=None, want_at
 V2_STAGE_CHUNKS = 592   # REGNN_V2_STAGE_CHUNKS (csrc/gat.cu)
 
 
-def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax, rowsum, saved, g):
+def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax, rowsum, saved, g, dropout=None):
     """Backward of ``gatv2_fwd(..., save=True)``: ``gat_bwd_stats`` -> ``gatv2_bwd_edges`` (the one gather pass) ->
-    ``gatv2_bwd_dst`` (streaming) -> (d_fs, d_fd, d_attn [H*D], d_theta | None)."""
+    ``gatv2_bwd_dst`` (streaming) -> (d_fs, d_fd, d_attn [H*D], d_theta | None).  ``dropout``: the ``HashedDropout`` of
+    the forward."""
     logit_csr, qmask = saved
     stats = gat_bwd_stats(out, g, None, rowmax, rowsum)
     e = csr['indices'].numel()
     dl_csr = stats.new_empty((max(e, 1), stats.shape[1]))   # never a NULL pointer
-    d_fs, d_attn_src = gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl_csr, keep=keep)
+    d_fs, d_attn_src = gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl_csr, keep=keep,
+                                       **dropout_kw(dropout))
     d_fd, d_attn_dst, d_theta = gatv2_bwd_dst(csr, et_csr, theta, alpha, fd, dl_csr, qmask, attn, slope)
     return d_fs, d_fd, d_attn_src + d_attn_dst, d_theta
 
@@ -516,14 +541,15 @@ def gatv2_bwd(csr, et_csr, theta, alpha, fs, fd, attn, slope, keep, out, rowmax,
 # of cut edges to the source's owner before the edge pass and to return the per-slot dl between the two passes.  Full
 # row ranges.
 
-def gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl, keep=None):
+def gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl, keep=None, dropout=None, eid=None):
     """Source-major pass over the rows of the transposed view ``csr['indptr_t']`` -> (d_fs of those rows, their share
     d_attn_src [H*D] of d_attn); the logit and the sign mask of every entry j are read from, and its dl is written to,
     slot ``csr['slot_t'][j]`` of ``logit_csr`` / ``qmask`` / ``dl`` ([slots, H], [slots, C, 4], [slots, H]).  ``fs``: the
     rows' own values; ``g`` / ``stats`` (``gat_bwd_stats`` with er=None): indexed by the column ids of the view.
-    ``keep``: the attention-dropout mask of ``gatv2_fwd``, in edge-id order through ``csr['eid']``
-    (regnn_gatv2_bwd_edges)."""
+    ``keep``: the attention-dropout mask of ``gatv2_fwd``, in edge-id order through ``csr['eid']``; ``dropout`` /
+    ``eid``: as ``gat_bwd_edges`` (regnn_gatv2_bwd_edges)."""
     fs, keep, g = _f32(fs), _f32(keep), _f32(g)
+    eid = (csr['eid'] if eid is None else eid) if (keep is not None or dropout is not None) else None
     attn = _f32(attn).view(-1)
     n = csr['indptr_t'].numel() - 1
     _, h, d = fs.shape
@@ -538,8 +564,9 @@ def gatv2_bwd_edges(csr, fs, stats, logit_csr, qmask, attn, slope, g, dl, keep=N
     partials = torch.empty(V2_STAGE_CHUNKS * h * d, dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
         _lib.call('regnn_gatv2_bwd_edges', _ptr(csr['indptr_t']), _ptr(csr['indices_t']), _ptr(csr['slot_t']),
-                  _ptr(csr['eid']) if keep is not None else None, _ptr(fs), _ptr(stats), _ptr(logit_csr), _ptr(qmask),
-                  _ptr(attn), float(slope), _ptr(keep), _ptr(g), h, d, 0, n, _ptr(d_fs), _ptr(dl), _ptr(d_attn_src),
+                  _ptr(eid), _ptr(fs), _ptr(stats), _ptr(logit_csr), _ptr(qmask),
+                  _ptr(attn), float(slope), _ptr(keep), _drop(dropout, h), _ptr(g), h, d, 0, n, _ptr(d_fs), _ptr(dl),
+                  _ptr(d_attn_src),
                   _ptr(block_partials), _ptr(partials), sp_t, _ptr(ws_t), _ptr(row_order(csr, True)), _stream())
         _lib.count_launches(3 + (sp_t is not None))
     return d_fs, d_attn_src

@@ -382,19 +382,23 @@ class _HeadSlicedGat(torch.autograd.Function):
     and zeros elsewhere: the caller sums them across ranks (``allreduce_relation_grads``)."""
 
     @staticmethod
-    def forward(ctx, graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, xch):
+    def forward(ctx, graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, xch, dropout):
         csr = graph.csr()
         n = graph.number_of_nodes()
         rows_own, heads, dim = f_own.shape
         hs = heads // (len(bounds) - 1)
         sl = slice(rank * hs, (rank + 1) * hs)
+        # this rank's heads of the full-H mask: the counter hash takes the global head
+        dropout = dropout.for_heads(rank * hs, heads) if dropout is not None else None
         f_cols = _rows_to_head_slab(f_own, n, bounds, rank, group, xch).view(n, hs, dim)
         al, ar = attn_l[:, sl].contiguous(), attn_r[:, sl].contiguous()
         th = theta[:, sl].contiguous() if etv is not None else None
         el, er = ops.attn_scores_fwd(f_cols, al, ar)
-        out, rowmax, rowsum, _ = ops.gat_fwd(csr, etv[0] if etv is not None else None, th, alpha, f_cols, el, er, slope)
+        out, rowmax, rowsum, _ = ops.gat_fwd(csr, etv[0] if etv is not None else None, th, alpha, f_cols, el, er, slope,
+                                             **ops.dropout_kw(dropout))
         ctx.graph, ctx.etv, ctx.alpha, ctx.slope, ctx.bounds, ctx.rank, ctx.group, ctx.xch = \
             graph, etv, alpha, slope, bounds, rank, group, xch
+        ctx.dropout = dropout
         ctx.sl = sl
         ctx.save_for_backward(f_cols, el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta)
         return _head_slab_to_rows(out, rows_own, bounds, group, xch).view(rows_own, heads, dim)
@@ -407,21 +411,27 @@ class _HeadSlicedGat(torch.autograd.Function):
         g_cols = _rows_to_head_slab(g_own, n, ctx.bounds, ctx.rank, ctx.group, ctx.xch, grad=True).view(n, hs, dim)
         et, et_t = (ctx.etv[0], ctx.etv[1]) if ctx.etv is not None else (None, None)
         d_f, _, _, d_th, d_al, d_ar = ops.gat_bwd(ctx.graph.csr(), et, et_t, th, ctx.alpha, f_cols, el, er, ctx.slope,
-                                                   None, out, rowmax, rowsum, g_cols, attn_l=al, attn_r=ar)
+                                                   None, out, rowmax, rowsum, g_cols, attn_l=al, attn_r=ar,
+                                                   **ops.dropout_kw(ctx.dropout))
         d_f_own = _head_slab_to_rows(d_f, rows_own, ctx.bounds, ctx.group, ctx.xch, grad=True).view(rows_own, heads, dim)
         return (None, None, d_f_own, _head_slice_grad(attn_l, d_al, ctx.sl), _head_slice_grad(attn_r, d_ar, ctx.sl),
-                _head_slice_grad(theta, d_th, ctx.sl), None, None, None, None, None, None)
+                _head_slice_grad(theta, d_th, ctx.sl), None, None, None, None, None, None, None)
 
 
-def head_sliced_gat(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group=None, exchange=None):
+def head_sliced_gat(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group=None, exchange=None,
+                    dropout=None):
     """f_own [rows_own, H, D] -> out rows [rows_own, H, D]; see ``_HeadSlicedGat``.  ``exchange`` (a ``SlabExchange`` of
-    width H*D): the re-partitions run over peer memory inside our own kernels instead of NCCL / gloo all-to-alls."""
+    width H*D): the re-partitions run over peer memory inside our own kernels instead of NCCL / gloo all-to-alls.
+    ``dropout`` (a ``functional.HashedDropout`` over all H heads): attention dropout; rank q computes the mask of its
+    heads from the global head index, so the result is that of ``functional.gat_layer`` with the same ``dropout``."""
     _, heads, dim = f_own.shape
+    _check_hashed_dropout(dropout, 'head_sliced_gat')
     if not _uniform_rows(bounds) or heads % (len(bounds) - 1):
         raise ValueError('head-sliced attention needs equal row blocks and num_heads divisible by the number of ranks')
     if exchange is not None and exchange.feat != heads * dim:
         raise ValueError('head-sliced attention over peer memory needs a SlabExchange of width num_heads * head_dim')
-    return _HeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, exchange)
+    return _HeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, exchange,
+                                dropout)
 
 
 def allreduce_relation_grads(params, group=None, exchange=None):
@@ -485,8 +495,9 @@ class HaloPartition:
     ``attention=True`` (``halo_gat``) also keeps what the REGAT backward needs to send the logit gradient of an edge back
     to the owner of its destination (the slot belongs to the destination's in-view row):
 
-    * ``eid_in``: global edge ids of the in-view slots (the kernels read them only for attention dropout, which the
-      halo path does not take, so they stay out of ``csr``);
+    * ``eid_in``: global edge ids of the in-view slots (the kernels read them only for attention dropout, so they stay
+      out of ``csr``); ``eid_ext``: the same for the extended slots [e_in + tail] that ``csr['slot_t']`` points at --
+      ``eid_in``, then the global edge ids of the tail entries in tail order (the backward's dropout factors);
     * ``csr['slot_t']``: for every out-view entry (own source u -> destination v), its position in the **extended dpre
       buffer** [E_in_own + cut_out, H]: v's local in-view slot when v is own, else ``E_in_own + k`` with k its position
       in the **tail** -- grouped by owner, and within an owner by that owner's local slot (global slot order is both);
@@ -593,6 +604,7 @@ class HaloPartition:
         self.csr['slot_t'] = slot_t.to(torch.int32).contiguous()
         tail_owner = _owner(dst_of_t[remote][perm], bounds_t)
         self.tail_dst = (tail_glob - slot_bounds[tail_owner]).to(torch.int32).contiguous()
+        self.eid_ext = torch.cat([self.eid_in, csr['eid'][tail_glob]]).contiguous()
         self.tail_counts = torch.bincount(tail_owner, minlength=parts).tolist()
         self.tail_ptr = [0]
         for c in self.tail_counts:
@@ -847,7 +859,17 @@ def _return_dpre(part, dpre, group, xch):
         dpre.index_copy_(0, part.dpre_recv, recv)
 
 
-def _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope):
+def _dropout_in(part, dropout):
+    """Keywords of the forward kernel call over the in-view: the hashed dropout and the global edge ids of its slots."""
+    return {} if dropout is None else {'dropout': dropout, 'eid': part.eid_in}
+
+
+def _dropout_ext(part, dropout):
+    """Keywords of the source-major edge pass: the hashed dropout and the global edge ids of the extended slots."""
+    return {} if dropout is None else {'dropout': dropout, 'eid': part.eid_ext}
+
+
+def _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope, dropout=None):
     """-> (out, el, er, rowmax, rowsum) of the own rows from the filled [n_own + in-halo, H, D] feature buffer: el / er
     of own AND halo rows computed here (row-wise, so a halo row carries its owner's bits and el is never exchanged),
     then the fused kernel over the in-view."""
@@ -857,7 +879,7 @@ def _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope):
         return f_ext.new_zeros((0, heads, dim)), z, z, z, z
     el, er = ops.attn_scores_fwd(f_ext, attn_l, attn_r)
     out, rowmax, rowsum, _ = ops.gat_fwd(part.csr, part.et_in if theta is not None else None, theta, alpha, f_ext, el,
-                                         er, slope)
+                                         er, slope, **_dropout_in(part, dropout))
     return out, el[:n_own], er[:n_own], rowmax, rowsum
 
 
@@ -869,14 +891,15 @@ def _gat_stats(out, g_own, er, rowmax, rowsum):
     return ops.gat_bwd_stats(out, g_own, er, rowmax, rowsum).view(n_own, 4 * heads)
 
 
-def _gat_backward_edges(part, f_own, el, attn_l, theta, alpha, slope, g_ext, s_ext, dpre):
+def _gat_backward_edges(part, f_own, el, attn_l, theta, alpha, slope, g_ext, s_ext, dpre, dropout=None):
     """-> (d_feat without the destination-side score term, d_el) of the own rows; writes the logit gradient of every
     out-view entry into the extended ``dpre`` buffer [e_in + tail, H] through ``csr['slot_t']``."""
     n_own, heads, dim = f_own.shape
     if not n_own:
         return torch.zeros_like(f_own), f_own.new_zeros((0, heads))
     return ops.gat_bwd_edges(part.csr, part.et_out if theta is not None else None, theta, alpha, f_own, el,
-                             s_ext.view(-1, heads, 4), slope, g_ext.view(-1, heads, dim), dpre, attn_l=attn_l)
+                             s_ext.view(-1, heads, 4), slope, g_ext.view(-1, heads, dim), dpre, attn_l=attn_l,
+                             **_dropout_ext(part, dropout))
 
 
 def _gat_backward_reduce(part, f_own, d_feat, d_el, attn_r, theta, alpha, dpre):
@@ -902,12 +925,12 @@ class _HaloGat(torch.autograd.Function):
     own rows."""
 
     @staticmethod
-    def forward(ctx, part, f_own, attn_l, attn_r, theta, alpha, slope, group, xch):
+    def forward(ctx, part, f_own, attn_l, attn_r, theta, alpha, slope, group, xch, dropout):
         n_own, heads, dim = f_own.shape
         f_own = f_own.contiguous()
         f_ext = _fill_halo(part, f_own.view(n_own, heads * dim), 'in', group, xch).view(-1, heads, dim)
-        out, el, er, rowmax, rowsum = _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope)
-        ctx.part, ctx.alpha, ctx.slope, ctx.group, ctx.xch = part, alpha, slope, group, xch
+        out, el, er, rowmax, rowsum = _gat_forward(part, f_ext, attn_l, attn_r, theta, alpha, slope, dropout)
+        ctx.part, ctx.alpha, ctx.slope, ctx.group, ctx.xch, ctx.dropout = part, alpha, slope, group, xch, dropout
         ctx.save_for_backward(f_own, el, er, attn_l, attn_r, theta, out, rowmax, rowsum)
         return out
 
@@ -921,24 +944,35 @@ class _HaloGat(torch.autograd.Function):
         g_ext, s_ext = _fill_out_halo_gat(part, g_own.view(n_own, heads * dim), stats, ctx.group, xch)
         rows = part.e_in + part.tail_ptr[-1]
         dpre = xch.dpre[:rows] if xch is not None else f_own.new_empty((rows, heads))
-        d_feat, d_el = _gat_backward_edges(part, f_own, el, attn_l, theta, ctx.alpha, ctx.slope, g_ext, s_ext, dpre)
+        d_feat, d_el = _gat_backward_edges(part, f_own, el, attn_l, theta, ctx.alpha, ctx.slope, g_ext, s_ext, dpre,
+                                           ctx.dropout)
         _return_dpre(part, dpre, ctx.group, xch)
         d_feat, d_al, d_ar, d_th = _gat_backward_reduce(part, f_own, d_feat, d_el, attn_r, theta, ctx.alpha, dpre)
         return (None, d_feat, d_al.view_as(attn_l), d_ar.view_as(attn_r),
-                d_th.view_as(theta) if d_th is not None else None, None, None, None, None)
+                d_th.view_as(theta) if d_th is not None else None, None, None, None, None, None)
 
 
-def halo_gat(part, f_own, attn_l, attn_r, theta, alpha, slope, group=None, exchange=None, keep=None):
+def _check_hashed_dropout(dropout, name):
+    from .dropout import HashedDropout
+    if dropout is not None and not isinstance(dropout, HashedDropout):
+        raise TypeError('%s: dropout must be a functional.HashedDropout, got %s' % (name, type(dropout).__name__))
+
+
+def halo_gat(part, f_own, attn_l, attn_r, theta, alpha, slope, group=None, exchange=None, keep=None, dropout=None):
     """f_own [n_own, H, D] -> out [n_own, H, D] (``part``: this rank's ``HaloPartition`` built with ``attention=True``):
     the REGAT core of ``functional.gat_layer`` on destination-row blocks, exchanging only halo rows.  ``exchange`` (a
     ``HaloExchange`` with ``heads=H`` and width H*D): the features, dL/dY and the statistics are pushed over peer memory
     (regnn_halo_push) and the logit gradients of cut edges are scattered to their owners (regnn_halo_scatter); None:
     uneven all-to-alls (NCCL / gloo).  ``theta=None`` drops the relation term.  out and d_feat are bit-identical to
     ``functional.gat_layer``; ``attn_l.grad``, ``attn_r.grad`` and ``theta.grad`` hold this rank's shares
-    (``allreduce_relation_grads``)."""
+    (``allreduce_relation_grads``).  Attention dropout: ``dropout`` (a ``functional.HashedDropout``), whose mask every
+    rank computes from the global edge ids (``part.eid_in`` / ``part.eid_ext``) -- the result is that of
+    ``functional.gat_layer`` with the same ``dropout``; an explicit ``keep`` mask is refused."""
     _, heads, dim = f_own.shape
     if keep is not None:
-        raise ValueError('halo_gat: attention dropout is not supported (its mask is in edge-id order over all edges)')
+        raise ValueError('halo_gat: an explicit attention dropout mask is not supported (it is in edge-id order over all '
+                         'edges); pass dropout=functional.HashedDropout(p, key)')
+    _check_hashed_dropout(dropout, 'halo_gat')
     if not getattr(part, 'attention', False):
         raise ValueError('halo_gat needs a HaloPartition built with attention=True')
     _check_gat_shape(heads, dim, part.num_relations, theta is not None)
@@ -946,10 +980,10 @@ def halo_gat(part, f_own, attn_l, attn_r, theta, alpha, slope, group=None, excha
         raise ValueError('halo_gat: theta must be [R=%d, H=%d], got %s' % (part.num_relations, heads, tuple(theta.shape)))
     if exchange is not None and (exchange.heads != heads or exchange.feat != heads * dim):
         raise ValueError('halo_gat: the HaloExchange must be built with heads=%d and width %d' % (heads, heads * dim))
-    return _HaloGat.apply(part, f_own, attn_l, attn_r, theta, alpha, slope, group, exchange)
+    return _HaloGat.apply(part, f_own, attn_l, attn_r, theta, alpha, slope, group, exchange, dropout)
 
 
-def _virtual_halo_gat(parts, f, gout, attn_l, attn_r, theta, alpha, slope, scatter=False):
+def _virtual_halo_gat(parts, f, gout, attn_l, attn_r, theta, alpha, slope, scatter=False, dropout=None):
     """Every rank of ``HaloPartition.virtual_ranks(..., attention=True)`` one after another in one process (no process
     group), each on its local views: halos filled by indexing the global [N, H, D] arrays, the dpre tails returned with
     ``index_copy_`` at the owners' receive lists or -- ``scatter=True`` -- by regnn_halo_scatter into the P local buffers.
@@ -959,11 +993,11 @@ def _virtual_halo_gat(parts, f, gout, attn_l, attn_r, theta, alpha, slope, scatt
     g2 = gout.reshape(n, heads * dim)
     bounds = parts[0].bounds
     own = [slice(bounds[p], bounds[p + 1]) for p in range(len(parts))]
-    fw = [_gat_forward(part, f[part.rows_in], attn_l, attn_r, theta, alpha, slope) for part in parts]
+    fw = [_gat_forward(part, f[part.rows_in], attn_l, attn_r, theta, alpha, slope, dropout) for part in parts]
     stats = torch.cat([_gat_stats(o, gout[s].contiguous(), er, mx, sm) for (o, _, er, mx, sm), s in zip(fw, own)])
     dpres = [f.new_empty((part.e_in + part.tail_ptr[-1], heads)) for part in parts]
     edges = [_gat_backward_edges(part, f[s].contiguous(), fw[p][1], attn_l, theta, alpha, slope, g2[part.rows_out],
-                                 stats[part.rows_out], dpres[p]) for p, (part, s) in enumerate(zip(parts, own))]
+                                 stats[part.rows_out], dpres[p], dropout) for p, (part, s) in enumerate(zip(parts, own))]
     if scatter:
         ptrs = torch.tensor([d.data_ptr() for d in dpres], dtype=torch.int64, device=f.device)
         for p, part in enumerate(parts):
@@ -1015,7 +1049,7 @@ def _push_slot_records(part, slots, group, xch):
                                        group=group)
 
 
-def _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots):
+def _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots, dropout=None):
     """-> (out, rowmax, rowsum) of the own rows from the filled [n_own + in-halo, H, D] source features and the own
     rows' destination features; the logit and the sign mask of every in-view slot go to the head of ``slots``."""
     n_own, heads, dim = fd_own.shape
@@ -1023,18 +1057,18 @@ def _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots):
         z = fd_own.new_zeros((0, heads))
         return fd_own.new_zeros((0, heads, dim)), z, z
     out, rowmax, rowsum, _, _ = ops.gatv2_fwd(part.csr, part.et_in if theta is not None else None, theta, alpha, fs_ext,
-                                              fd_own, attn, slope, saved=slots)
+                                              fd_own, attn, slope, saved=slots, **_dropout_in(part, dropout))
     return out, rowmax, rowsum
 
 
-def _gatv2_backward_edges(part, fs_own, attn, slope, g_ext, s_ext, slots, dl):
+def _gatv2_backward_edges(part, fs_own, attn, slope, g_ext, s_ext, slots, dl, dropout=None):
     """-> (d_fs, this rank's d_attn_src [H*D]) of the own rows once the tails of ``slots`` are filled; writes the dl of
     every out-view entry into the extended ``dl`` buffer [e_in + tail, H] through ``csr['slot_t']``."""
     n_own, heads, dim = fs_own.shape
     if not n_own:
         return torch.zeros_like(fs_own), fs_own.new_zeros(heads * dim)
     return ops.gatv2_bwd_edges(part.csr, fs_own, s_ext.view(-1, heads, 4), slots[0], slots[1], attn, slope,
-                               g_ext.view(-1, heads, dim), dl)
+                               g_ext.view(-1, heads, dim), dl, **_dropout_ext(part, dropout))
 
 
 def _gatv2_backward_dst(part, fd_own, attn, theta, alpha, slope, dl, mask):
@@ -1061,13 +1095,14 @@ class _HaloGatV2(torch.autograd.Function):
     before the next forward, as for every ``HaloExchange``."""
 
     @staticmethod
-    def forward(ctx, part, fs_own, fd_own, attn, theta, alpha, slope, group, xch):
+    def forward(ctx, part, fs_own, fd_own, attn, theta, alpha, slope, group, xch, dropout):
         n_own, heads, dim = fs_own.shape
         fs_own, fd_own = fs_own.contiguous(), fd_own.contiguous()
         fs_ext = _fill_halo(part, fs_own.view(n_own, heads * dim), 'in', group, xch).view(-1, heads, dim)
         slots = _slot_buffers(part, heads, (heads * dim + 127) // 128, fs_own, xch)
-        out, rowmax, rowsum = _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots)
+        out, rowmax, rowsum = _gatv2_forward(part, fs_ext, fd_own, attn, theta, alpha, slope, slots, dropout)
         ctx.part, ctx.alpha, ctx.slope, ctx.group, ctx.xch, ctx.slots = part, alpha, slope, group, xch, slots
+        ctx.dropout = dropout
         ctx.save_for_backward(fs_own, fd_own, attn, theta, out, rowmax, rowsum)
         return out
 
@@ -1081,14 +1116,14 @@ class _HaloGatV2(torch.autograd.Function):
         g_ext, s_ext = _fill_out_halo_gat(part, g_own.view(n_own, heads * dim), stats, ctx.group, xch, slots=slots)
         rows = part.e_in + part.tail_ptr[-1]
         dl = xch.dpre[:rows] if xch is not None else fs_own.new_empty((max(rows, 1), heads))[:rows]
-        d_fs, d_attn_src = _gatv2_backward_edges(part, fs_own, attn, ctx.slope, g_ext, s_ext, slots, dl)
+        d_fs, d_attn_src = _gatv2_backward_edges(part, fs_own, attn, ctx.slope, g_ext, s_ext, slots, dl, ctx.dropout)
         _return_dpre(part, dl, ctx.group, xch)
         d_fd, d_attn_dst, d_th = _gatv2_backward_dst(part, fd_own, attn, theta, ctx.alpha, ctx.slope, dl, slots[1])
         return (None, d_fs, d_fd, (d_attn_src + d_attn_dst).view_as(attn),
-                d_th.view_as(theta) if d_th is not None else None, None, None, None, None)
+                d_th.view_as(theta) if d_th is not None else None, None, None, None, None, None)
 
 
-def halo_gatv2(part, fs_own, fd_own, attn, theta, alpha, slope, group=None, exchange=None, keep=None):
+def halo_gatv2(part, fs_own, fd_own, attn, theta, alpha, slope, group=None, exchange=None, keep=None, dropout=None):
     """fs_own, fd_own [n_own, H, D] -> out [n_own, H, D] (``part``: this rank's ``HaloPartition`` built with
     ``attention=True``): the REGATv2 core of ``functional.gatv2_aggregate`` on destination-row blocks, exchanging only
     halo rows and the per-slot records of cut edges.  With shared weights pass the same tensor as ``fs_own`` and
@@ -1098,10 +1133,13 @@ def halo_gatv2(part, fs_own, fd_own, attn, theta, alpha, slope, group=None, exch
     (regnn_halo_scatter); None: uneven all-to-alls (NCCL / gloo).  ``theta=None`` drops the relation term.  out, d_fs
     and d_fd are bit-identical to ``functional.gatv2_aggregate``; ``attn.grad`` and ``theta.grad`` hold this rank's
     shares (``allreduce_relation_grads``).  The MAG stack's ``softmax_eps`` (a global maximum over all logits) is not
-    taken."""
+    taken.  Attention dropout: ``dropout`` (a ``functional.HashedDropout``), as ``halo_gat``; an explicit ``keep`` mask
+    is refused."""
     _, heads, dim = fs_own.shape
     if keep is not None:
-        raise ValueError('halo_gatv2: attention dropout is not supported (its mask is in edge-id order over all edges)')
+        raise ValueError('halo_gatv2: an explicit attention dropout mask is not supported (it is in edge-id order over '
+                         'all edges); pass dropout=functional.HashedDropout(p, key)')
+    _check_hashed_dropout(dropout, 'halo_gatv2')
     if not getattr(part, 'attention', False):
         raise ValueError('halo_gatv2 needs a HaloPartition built with attention=True')
     _check_gat_shape(heads, dim, part.num_relations, theta is not None, 'halo_gatv2')
@@ -1114,10 +1152,10 @@ def halo_gatv2(part, fs_own, fd_own, attn, theta, alpha, slope, group=None, exch
     if exchange is not None and (exchange.heads != heads or exchange.feat != heads * dim or not exchange.gatv2):
         raise ValueError('halo_gatv2: the HaloExchange must be built with heads=%d, width %d and gatv2=True'
                          % (heads, heads * dim))
-    return _HaloGatV2.apply(part, fs_own, fd_own, attn, theta, alpha, slope, group, exchange)
+    return _HaloGatV2.apply(part, fs_own, fd_own, attn, theta, alpha, slope, group, exchange, dropout)
 
 
-def _virtual_halo_gatv2(parts, fs, fd, gout, attn, theta, alpha, slope, push=False):
+def _virtual_halo_gatv2(parts, fs, fd, gout, attn, theta, alpha, slope, push=False, dropout=None):
     """Every rank of ``HaloPartition.virtual_ranks(..., attention=True)`` one after another in one process (no process
     group), each on its local views: halos filled by indexing the global [N, H, D] arrays; the slot records of cut
     edges moved to the sources' owners by indexing and the dl tails returned with ``index_copy_`` at the owners'
@@ -1128,7 +1166,7 @@ def _virtual_halo_gatv2(parts, fs, fd, gout, attn, theta, alpha, slope, push=Fal
     bounds = parts[0].bounds
     own = [slice(bounds[p], bounds[p + 1]) for p in range(len(parts))]
     slots = [_slot_buffers(part, heads, (heads * dim + 127) // 128, fs, None) for part in parts]
-    fw = [_gatv2_forward(part, fs[part.rows_in], fd[s].contiguous(), attn, theta, alpha, slope, sl)
+    fw = [_gatv2_forward(part, fs[part.rows_in], fd[s].contiguous(), attn, theta, alpha, slope, sl, dropout)
           for part, s, sl in zip(parts, own, slots)]
     stats = torch.cat([_gat_stats(o, gout[s].contiguous(), None, mx, sm) for (o, mx, sm), s in zip(fw, own)])
     if push:
@@ -1146,7 +1184,7 @@ def _virtual_halo_gatv2(parts, fs, fd, gout, attn, theta, alpha, slope, push=Fal
                     dst[seg] = src.index_select(0, idx)
     dls = [fs.new_empty((max(part.e_in + part.tail_ptr[-1], 1), heads))[:part.e_in + part.tail_ptr[-1]] for part in parts]
     edges = [_gatv2_backward_edges(part, fs[s].contiguous(), attn, slope, g2[part.rows_out], stats[part.rows_out],
-                                   slots[p], dls[p]) for p, (part, s) in enumerate(zip(parts, own))]
+                                   slots[p], dls[p], dropout) for p, (part, s) in enumerate(zip(parts, own))]
     if push:
         ptrs = torch.tensor([d.data_ptr() for d in dls], dtype=torch.int64, device=fs.device)
         for p, part in enumerate(parts):
