@@ -310,6 +310,8 @@ int regnn_rowdot_norm_bwd(const float* norm, int norm_sides, const float* X, int
  *   keep tensor holding the hashed factors gives the same bits.
  * attn_out: optional [E,H] output of a*keep in EDGE-ID order (`get_attention`), NULL = skip.
  * Saves rowmax/rowsum [N,H] for the backward pass.  theta: [R,H].
+ * Shapes of every REGAT / REGATv2 entry point below: 1 <= num_heads <= REGNN_MAX_HEADS, head_dim a power of two in
+ * [4, 512], num_heads * head_dim <= 1024; anything else is REGNN_ERR_UNSUPPORTED_SHAPE.
  */
 int regnn_gat_fwd(const int32_t* indptr, const int32_t* indices, const int32_t* eid,
                   const uint8_t* etype_csr, const float* theta, float alpha, int num_relations,

@@ -7,8 +7,11 @@
 //
 // Mapping (all hot kernels): a row of H*D floats is cut into slices of min(H*D, 128) floats; G = 4 / 8 / 16 / 32 lanes
 // own one (row, slice) item with a 128-bit chunk each, so a warp works on 32/G rows and every gathered row is read with
-// coalesced LDG.128; heads never straddle a slice, per-head dot products are compile-time butterflies over the D/4 lanes
-// of a head.  Rows come from the degree-sorted row list, long rows are cut into fragments (merged by finalize kernels).
+// coalesced LDG.128; heads of D <= 128 never straddle a slice, per-head dot products are compile-time butterflies over
+// the D/4 lanes of a head.  A wide head (D = 256 / 512) is one warp item whose lanes hold CPL = D/128 chunks each, the
+// dot product being the lane's CPL partial dots + the 32-lane butterfly (kernels that reduce over a head take CPL; the
+// others work per slice and take wide heads as they are).  Rows come from the degree-sorted row list, long rows are cut
+// into fragments (merged by finalize kernels).
 #include <type_traits>
 
 #include "common.cuh"
@@ -144,16 +147,17 @@ struct RowItem {
   bool frag;
 };
 
-template <int G>
+// CPL > 1 (wide heads, G = 32): an item is a (row, head) pair and it.hg is the head; see kernels taking CPL below
+template <int G, int CPL = 1>
 __device__ __forceinline__ RowItem rg_item(const AttnArgs& a, int64_t wi, int grp) {
   constexpr int GPW = 32 / G;
   RowItem it{-1, 0, 0, 0, 0, false};
   const int64_t nrows = a.order != nullptr ? a.n_order : (a.row_end - a.row_begin);
-  const int64_t nitems = (a.nfrag + nrows) * a.hg_count;
+  const int64_t nitems = (a.nfrag + nrows) * (a.hg_count / CPL);
   const int64_t vi = wi * GPW + grp;
   if (vi >= nitems) return it;
   int64_t ri = vi;
-  if (a.hg_count > 1) split_item(vi, a.hg_count, &ri, &it.hg);
+  if (a.hg_count / CPL > 1) split_item(vi, a.hg_count / CPL, &ri, &it.hg);
   if (ri < a.nfrag) {
     it.frag = true;
     it.fi = ri;
@@ -175,10 +179,10 @@ __device__ __forceinline__ RowItem rg_item(const AttnArgs& a, int64_t wi, int gr
   }
   return it;
 }
-__device__ __forceinline__ int64_t rg_num_work(const AttnArgs& a, int G) {
+__device__ __forceinline__ int64_t rg_num_work(const AttnArgs& a, int G, int CPL = 1) {
   const int64_t nrows = a.order != nullptr ? a.n_order : (a.row_end - a.row_begin);
   const int GPW = 32 / G;
-  return ((a.nfrag + nrows) * a.hg_count + GPW - 1) / GPW;
+  return ((a.nfrag + nrows) * (a.hg_count / CPL) + GPW - 1) / GPW;
 }
 
 #ifndef REGNN_FWD_PF
@@ -308,7 +312,7 @@ gat_fwd_rg_kernel(AttnArgs a) {
   if (EXTRA && a.o3 != nullptr) {  // get_attention: stored logits -> a*keep, edge-id order; the lanes of a head share its slots
     __syncwarp();
     const int lph = min(G, a.D >> 2);
-    if (act)
+    if (act && ((it.hg << 7) & (a.D - 1)) == 0)   // D > 128: only the warp of a head's first slice, which stored its logits
       for (int t = lg & (lph - 1); t < len; t += lph) {
         const size_t o = (size_t)eidp[t] * H + h;
         float av = __expf(a.o3[o] - mm) * inv;
@@ -330,7 +334,9 @@ gat_fwd_rg_kernel(AttnArgs a) {
 //   gat_bwd_edges_kernel    d_feat[u], d_el[u], dpre[slot,h]  (source-major, row groups)      the gather pass
 //   gat_bwd_der_kernel      d_er[v,h] = sum_{slots of v} dpre[slot,h]                         streaming over [E,H]
 //   gat_bwd_bins_kernel     relation bins of dpre (lane-local, per-block double partials)     streaming over [E,H]
-template <int G>
+// CPL > 1 (D = 128 * CPL, G = 32): an item is a (node, head) pair, lane l reading columns h*D + 128*c + 4*l, c < CPL;
+// HG is then the number of heads
+template <int G, int CPL = 1>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 gat_bwd_stats_kernel(const float* __restrict__ out, const float* __restrict__ Gd, const float* __restrict__ er,
                      const float* __restrict__ rowmax, const float* __restrict__ rowsum, int64_t n, int H, int D,
@@ -344,10 +350,15 @@ gat_bwd_stats_kernel(const float* __restrict__ out, const float* __restrict__ Gd
        wi += (int64_t)gridDim.x * kWarpsPerBlock * GPW) {
     const int64_t vi = wi + grp;
     const int64_t v = vi / HG;
-    const int col = (int)(vi % HG) * 128 + lg * 4;
+    const int col = (int)(vi % HG) * (128 * CPL) + lg * 4;
     const bool act = vi < items && col < HD;
     float p = 0.f;
-    if (act) p = dot4(ldg4(out + (size_t)v * HD + col), ldg4(Gd + (size_t)v * HD + col));
+#pragma unroll
+    for (int c = 0; c < CPL; ++c)
+      if (act) {
+        const float q = dot4(ldg4(out + (size_t)v * HD + col + 128 * c), ldg4(Gd + (size_t)v * HD + col + 128 * c));
+        p = c == 0 ? q : p + q;
+      }
     p = group_sum_rt(p, lph);
     if (act && (col & (D - 1)) == 0) {
       const size_t vh = (size_t)v * H + (col >> d_shift);
@@ -377,9 +388,13 @@ gat_bwd_stats_kernel(const float* __restrict__ out, const float* __restrict__ Gd
 #define REGNN_GATB_U 2
 #endif
 // LPH = min(G, D/4): lanes per head (compile-time butterfly); KEEP: attention dropout, its factor from a.keep or -- HASH --
-// from hashed_keep
-template <int G, int LPH, bool KEEP, bool HASH = false>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_GATB_BLOCKS)
+// from hashed_keep.  CPL: 128-bit chunks per lane -- 1: the item is a (row | fragment, 128-float slice) pair; 2 / 4 (wide
+// heads, D = 128 * CPL, G = LPH = 32): the item is a (row | fragment, head) pair, lane l holding the columns
+// h*D + 128*c + 4*l, c < CPL (CPL coalesced 512-byte requests per gathered row), and a head's dot product is the sum of
+// the lane's CPL partial dots followed by the 32-lane butterfly.
+#define REGNN_WIDE_BLOCKS(CPL_, NARROW_) ((CPL_) == 1 ? (NARROW_) : ((CPL_) == 2 ? 4 : 2))
+template <int G, int LPH, bool KEEP, bool HASH = false, int CPL = 1>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_WIDE_BLOCKS(CPL, REGNN_GATB_BLOCKS))
 gat_bwd_edges_kernel(AttnArgs a) {
   static_assert(KEEP || !HASH, "HASH is a dropout mode");
   constexpr int U = REGNN_GATB_U;  // rows of G (and statistics vectors) in flight per lane
@@ -391,9 +406,9 @@ gat_bwd_edges_kernel(AttnArgs a) {
   const int lg = lane % G, grp = lane / G, gbase = lane & ~(G - 1);
   const int H = a.H, HD = H * a.D;
   const int64_t wi = (int64_t)blockIdx.x * kWarpsPerBlock + warp;
-  if (wi >= rg_num_work(a, G)) return;
-  const RowItem it = rg_item<G>(a, wi, grp);
-  const int col = it.hg * 128 + lg * 4;
+  if (wi >= rg_num_work(a, G, CPL)) return;
+  const RowItem it = rg_item<G, CPL>(a, wi, grp);
+  const int col = it.hg * (128 * CPL) + lg * 4;
   const bool col_ok = col < HD;
   const int h = col_ok ? (col >> a.d_shift) : 0;
   const bool act = it.v >= 0 && col_ok;
@@ -401,10 +416,13 @@ gat_bwd_edges_kernel(AttnArgs a) {
   const int len = it.v >= 0 ? it.len : 0;
   const int maxlen = __reduce_max_sync(0xffffffffu, len);
   const bool has_rel = a.etype != nullptr;
-  float4 fu = zero4();
+  float4 fu[CPL];
   float el_u = 0.f;
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) fu[c] = zero4();
   if (act) {
-    fu = ldg4(a.feat + (size_t)it.v * HD + col);
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) fu[c] = ldg4(a.feat + (size_t)it.v * HD + col + 128 * c);
     el_u = __ldg(a.el + (size_t)it.v * H + h);
   }
   // one IMAD.WIDE.U32 per gathered address: 32-bit index x 32-bit pitch (bytes) added to a 64-bit base
@@ -416,13 +434,15 @@ gat_bwd_edges_kernel(AttnArgs a) {
   const int32_t* ip = a.indices + it.begin;
   const int32_t* sp = a.eid + it.begin;
   const uint8_t* ep = a.etype + it.begin;
-  float4 acc = zero4();
+  float4 acc[CPL];
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) acc[c] = zero4();
   float del = 0.f;
 #if REGNN_GATB_PF
   // the G row slice and the statistics this lane's own slot will need, into L2 while the first rounds run
-  const char* pf_g = reinterpret_cast<const char*>(a.G + it.hg * 128);
-  const int pf_lines = (min(128, HD - it.hg * 128) * 4 + REGNN_PF_BYTES - 1) / REGNN_PF_BYTES;
-  const char* pf_s = reinterpret_cast<const char*>(a.fd) + (size_t)((it.hg * 128) >> a.d_shift) * 16;
+  const char* pf_g = reinterpret_cast<const char*>(a.G + it.hg * 128 * CPL);
+  const int pf_lines = (min(128 * CPL, HD - it.hg * 128 * CPL) * 4 + REGNN_PF_BYTES - 1) / REGNN_PF_BYTES;
+  const char* pf_s = reinterpret_cast<const char*>(a.fd) + (size_t)((it.hg * 128 * CPL) >> a.d_shift) * 16;
 #endif
 
   for (int t0 = 0; t0 < maxlen; t0 += G) {
@@ -442,20 +462,27 @@ gat_bwd_edges_kernel(AttnArgs a) {
     }
     const int cnt = min(G, maxlen - t0);
     for (int j = 0; j < cnt; j += U) {
-      float4 x[U], st[U];
+      float4 x[U][CPL], st[U];
       int sd[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         sd[u] = __shfl_sync(0xffffffffu, bi, gbase + j + u);
         const bool ok = sd[u] >= 0 && col_ok;
-        x[u] = ok ? ldg4(reinterpret_cast<const float*>(gbytes + (uint64_t)(uint32_t)sd[u] * gpitch)) : zero4();
+#pragma unroll
+        for (int c = 0; c < CPL; ++c)
+          x[u][c] = ok ? ldg4(reinterpret_cast<const float*>(gbytes + (uint64_t)(uint32_t)sd[u] * gpitch + 512 * c)) : zero4();
         // missing slot: rowmax = +inf makes exp(. - rowmax) = 0, so a = dpre = 0 without per-edge masks
         st[u] = ok ? __ldg(reinterpret_cast<const float4*>(sbytes + (uint64_t)(uint32_t)sd[u] * spitch))
                    : make_float4(0.f, INFINITY, 0.f, 0.f);
       }
       float da[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u) da[u] = group_sum<LPH>(dot4(fu, x[u]));
+      for (int u = 0; u < U; ++u) {
+        float p = dot4(fu[0], x[u][0]);
+#pragma unroll
+        for (int c = 1; c < CPL; ++c) p += dot4(fu[c], x[u][c]);
+        da[u] = group_sum<LPH>(p);
+      }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int ss = __shfl_sync(0xffffffffu, bs, gbase + j + u);
@@ -471,7 +498,8 @@ gat_bwd_edges_kernel(AttnArgs a) {
           }
         }
         const float dp = (at * da[u] - aa * st[u].w) * leaky_grad(pre, a.slope);
-        fma4(acc, at, x[u]);
+#pragma unroll
+        for (int c = 0; c < CPL; ++c) fma4(acc[c], at, x[u][c]);
         del += dp;
         if (leader && sd[u] >= 0) dpre_h[(uint64_t)(uint32_t)ss * (uint32_t)H] = dp;   // dpre per CSR slot
       }
@@ -479,12 +507,16 @@ gat_bwd_edges_kernel(AttnArgs a) {
   }
   if (!act) return;
   if (it.frag) {
-    st4(a.p0 + (size_t)it.fi * HD + col, acc);
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) st4(a.p0 + (size_t)it.fi * HD + col + 128 * c, acc[c]);
     if (leader) a.p1[(size_t)it.fi * H + h] = del;
     return;
   }
-  if (a.attn_l != nullptr) fma4(acc, del, ldg4(a.attn_l + col));   // gradient through el = <feat, attn_l>
-  st4(a.o0 + (size_t)it.v * HD + col, acc);
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) {
+    if (a.attn_l != nullptr) fma4(acc[c], del, ldg4(a.attn_l + col + 128 * c));   // gradient through el = <feat, attn_l>
+    st4(a.o0 + (size_t)it.v * HD + col + 128 * c, acc[c]);
+  }
   if (leader) a.o1[(size_t)it.v * H + h] = del;
 }
 
@@ -640,8 +672,9 @@ gat_bwd_bins_kernel(const uint8_t* __restrict__ etype, const float* __restrict__
 }
 
 // Projection scores of REGAT (layer/REGATConv.py:68-69): el[n,h] = <feat[n,h,:], attn_l[h,:]>, er likewise -- one
-// streaming pass over feat instead of two eager mul + sum pairs.  Same lane-group mapping as above.
-template <int G>
+// streaming pass over feat instead of two eager mul + sum pairs.  Same lane-group mapping as above (CPL as
+// gat_bwd_stats_kernel).
+template <int G, int CPL = 1>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 attn_scores_fwd_kernel(const float* __restrict__ feat, const float* __restrict__ attn_l, const float* __restrict__ attn_r,
                        int64_t n, int H, int D, int d_shift, int HG, float* __restrict__ el, float* __restrict__ er) {
@@ -654,13 +687,17 @@ attn_scores_fwd_kernel(const float* __restrict__ feat, const float* __restrict__
        wi += (int64_t)gridDim.x * kWarpsPerBlock * GPW) {
     const int64_t vi = wi + grp;
     const int64_t v = vi / HG;
-    const int col = (int)(vi % HG) * 128 + lg * 4;
+    const int col = (int)(vi % HG) * (128 * CPL) + lg * 4;
     const bool act = vi < items && col < HD;
     float pl = 0.f, pr = 0.f;
     if (act) {
-      const float4 f = ldg4(feat + (size_t)v * HD + col);
-      pl = dot4(f, ldg4(attn_l + col));
-      pr = dot4(f, ldg4(attn_r + col));
+#pragma unroll
+      for (int c = 0; c < CPL; ++c) {
+        const float4 f = ldg4(feat + (size_t)v * HD + col + 128 * c);
+        const float ql = dot4(f, ldg4(attn_l + col + 128 * c)), qr = dot4(f, ldg4(attn_r + col + 128 * c));
+        pl = c == 0 ? ql : pl + ql;
+        pr = c == 0 ? qr : pr + qr;
+      }
     }
     pl = group_sum_rt(pl, lph);
     pr = group_sum_rt(pr, lph);
@@ -744,11 +781,12 @@ attn_scores_bwd_kernel(const float* __restrict__ feat, const float* __restrict__
 #ifndef REGNN_V2F_BLOCKS
 #define REGNN_V2F_BLOCKS 4
 #endif
-template <int G, int LPH, bool EXTRA, bool HASH = false>   // EXTRA / HASH as gat_fwd_rg_kernel
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_V2F_BLOCKS)
+// CPL as gat_bwd_edges_kernel; a wide head still stores one 128-bit mask per (slot, 128-float slice), one per chunk
+template <int G, int LPH, bool EXTRA, bool HASH = false, int CPL = 1>   // EXTRA / HASH as gat_fwd_rg_kernel
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_WIDE_BLOCKS(CPL, REGNN_V2F_BLOCKS))
 gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__ qmask) {
   static_assert(EXTRA || !HASH, "the hashed dropout factor needs the edge ids");
-  constexpr int U = kUG;
+  constexpr int U = CPL == 1 ? kUG : 2;   // a wide head holds U * CPL gathered float4 per lane
   static_assert(G % U == 0, "a batch must not straddle a cooperative slot load");
   extern __shared__ __align__(16) float smem[];
   float* w_s = smem;
@@ -757,9 +795,9 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
   const int lg = lane % G, grp = lane / G, gbase = lane & ~(G - 1);
   const int H = a.H, HD = H * a.D;
   const int64_t wi = (int64_t)blockIdx.x * kWarpsPerBlock + warp;
-  if (wi >= rg_num_work(a, G)) return;  // warp-uniform
-  const RowItem it = rg_item<G>(a, wi, grp);
-  const int col = it.hg * 128 + lg * 4;
+  if (wi >= rg_num_work(a, G, CPL)) return;  // warp-uniform
+  const RowItem it = rg_item<G, CPL>(a, wi, grp);
+  const int col = it.hg * (128 * CPL) + lg * 4;
   const bool col_ok = col < HD;
   const int h = col_ok ? (col >> a.d_shift) : 0;
   const bool act = it.v >= 0 && col_ok;
@@ -767,9 +805,14 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
   const int len = it.v >= 0 ? it.len : 0;
   const int maxlen = __reduce_max_sync(0xffffffffu, len);
   const bool has_rel = a.etype != nullptr;
-  float4 fdv = zero4(), at = zero4();
-  if (act) fdv = ldg4(a.fd + (size_t)it.v * HD + col);
-  if (col_ok) at = ldg4(a.el + col);
+  float4 fdv[CPL], at[CPL];
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) {
+    fdv[c] = zero4();
+    at[c] = zero4();
+    if (act) fdv[c] = ldg4(a.fd + (size_t)it.v * HD + col + 128 * c);
+    if (col_ok) at[c] = ldg4(a.el + col + 128 * c);
+  }
   const char* fbytes = reinterpret_cast<const char*>(a.feat + (col_ok ? col : 0));
   const uint32_t fpitch = (uint32_t)HD * 4u;
   const float* w_h = w_s + h;
@@ -777,9 +820,11 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
   const uint8_t* ep = a.etype + it.begin;
   const int32_t* eidp = a.eid + it.begin;
   // saved outputs: 32-bit element offsets from the kernel-parameter bases (E * max(H, HG) < 2^32, checked by the caller)
-  const uint32_t moff = (uint32_t)it.begin * (uint32_t)a.hg_count + (uint32_t)it.hg;
+  const uint32_t moff = (uint32_t)it.begin * (uint32_t)a.hg_count + (uint32_t)(it.hg * CPL);
   const uint32_t loff = (uint32_t)it.begin * (uint32_t)H + (uint32_t)h;
-  float4 acc = zero4();
+  float4 acc[CPL];
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) acc[c] = zero4();
   float m = -INFINITY, s = 0.f;
 
   for (int t0 = 0; t0 < maxlen; t0 += G) {
@@ -792,8 +837,8 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
         if (EXTRA) beid = __ldg(eidp + t);
 #if REGNN_FWD_PF
         {
-          const char* fr = reinterpret_cast<const char*>(a.feat + it.hg * 128) + (uint64_t)(uint32_t)bi * fpitch;
-          const int nl = (min(128, HD - it.hg * 128) * 4 + REGNN_PF_BYTES - 1) / REGNN_PF_BYTES;
+          const char* fr = reinterpret_cast<const char*>(a.feat + it.hg * 128 * CPL) + (uint64_t)(uint32_t)bi * fpitch;
+          const int nl = (min(128 * CPL, HD - it.hg * 128 * CPL) * 4 + REGNN_PF_BYTES - 1) / REGNN_PF_BYTES;
           for (int k = 0; k < nl; ++k) prefetch_l2(fr + k * REGNN_PF_BYTES);
         }
 #endif
@@ -801,35 +846,47 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
     }
     const int cnt = min(G, maxlen - t0);
     for (int j = 0; j < cnt; j += U) {
-      float4 x[U];
+      float4 x[U][CPL];
       float l[U];
       int si[U], seid[EXTRA ? U : 1];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         si[u] = __shfl_sync(0xffffffffu, bi, gbase + j + u);
-        x[u] = (si[u] >= 0 && col_ok) ? ldg4(reinterpret_cast<const float*>(fbytes + (uint64_t)(uint32_t)si[u] * fpitch))
-                                      : zero4();
+#pragma unroll
+        for (int c = 0; c < CPL; ++c)
+          x[u][c] = (si[u] >= 0 && col_ok)
+                        ? ldg4(reinterpret_cast<const float*>(fbytes + (uint64_t)(uint32_t)si[u] * fpitch + 512 * c))
+                        : zero4();
       }
       float bm = -INFINITY;
 #pragma unroll
       for (int u = 0; u < U; ++u) {   // U independent head reductions
-        const float4 q = add4(x[u], fdv);
-        float lu = group_sum<LPH>(dot4(at, leaky4(q, a.slope)));
+        float4 q[CPL];
+#pragma unroll
+        for (int c = 0; c < CPL; ++c) q[c] = add4(x[u][c], fdv[c]);
+        float lu = dot4(at[0], leaky4(q[0], a.slope));
+#pragma unroll
+        for (int c = 1; c < CPL; ++c) lu += dot4(at[c], leaky4(q[c], a.slope));
+        lu = group_sum<LPH>(lu);
         if (has_rel) lu += w_h[__shfl_sync(0xffffffffu, be, gbase + j + u) * H];
         if (EXTRA) seid[u] = __shfl_sync(0xffffffffu, beid, gbase + j + u);
         l[u] = si[u] >= 0 ? lu : -INFINITY;
         bm = fmaxf(bm, l[u]);
         if (qmask != nullptr) {   // warp-uniform
-          uint4 b;
-          b.x = __ballot_sync(0xffffffffu, q.x > 0.f); b.y = __ballot_sync(0xffffffffu, q.y > 0.f);
-          b.z = __ballot_sync(0xffffffffu, q.z > 0.f); b.w = __ballot_sync(0xffffffffu, q.w > 0.f);
-          if (G < 32) {
-            constexpr uint32_t gm = G < 32 ? (1u << G) - 1u : 0xffffffffu;
-            b.x = (b.x >> gbase) & gm; b.y = (b.y >> gbase) & gm; b.z = (b.z >> gbase) & gm; b.w = (b.w >> gbase) & gm;
+#pragma unroll
+          for (int c = 0; c < CPL; ++c) {
+            uint4 b;
+            b.x = __ballot_sync(0xffffffffu, q[c].x > 0.f); b.y = __ballot_sync(0xffffffffu, q[c].y > 0.f);
+            b.z = __ballot_sync(0xffffffffu, q[c].z > 0.f); b.w = __ballot_sync(0xffffffffu, q[c].w > 0.f);
+            if (G < 32) {
+              constexpr uint32_t gm = G < 32 ? (1u << G) - 1u : 0xffffffffu;
+              b.x = (b.x >> gbase) & gm; b.y = (b.y >> gbase) & gm; b.z = (b.z >> gbase) & gm; b.w = (b.w >> gbase) & gm;
+            }
+            const uint32_t t = (uint32_t)(t0 + j + u);
+            if (si[u] >= 0 && lg == 0)   // 16 bytes per (slot, slice)
+              reinterpret_cast<uint4*>(qmask)[moff + t * (uint32_t)a.hg_count + c] = b;
+            if (c == CPL - 1 && si[u] >= 0 && leader) lcsr[loff + t * (uint32_t)H] = lu;
           }
-          const uint32_t t = (uint32_t)(t0 + j + u);
-          if (si[u] >= 0 && lg == 0) reinterpret_cast<uint4*>(qmask)[moff + t * (uint32_t)a.hg_count] = b;   // 16 bytes per (slot, slice)
-          if (si[u] >= 0 && leader) lcsr[loff + t * (uint32_t)H] = lu;
         }
       }
       if (bm > -INFINITY) {  // uniform within a lane group
@@ -837,7 +894,8 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
         const float sc = fast_exp(m - m_new);
         m = m_new;
         s *= sc;
-        scale4(acc, sc);
+#pragma unroll
+        for (int c = 0; c < CPL; ++c) scale4(acc[c], sc);
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           float p = fast_exp(l[u] - m_new);  // 0 for a missing slot
@@ -848,14 +906,17 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
             if (HASH) p *= hashed_keep(a, seid[u], h);
             else if (a.keep != nullptr) p *= __ldg(a.keep + o);
           }
-          fma4(acc, p, x[u]);
+#pragma unroll
+          for (int c = 0; c < CPL; ++c) fma4(acc[c], p, x[u][c]);
         }
       }
     }
   }
 
   if (it.frag) {
-    if (act) st4(a.p0 + (size_t)it.fi * HD + col, acc);
+#pragma unroll
+    for (int c = 0; c < CPL; ++c)
+      if (act) st4(a.p0 + (size_t)it.fi * HD + col + 128 * c, acc[c]);
     if (leader) {
       a.p1[(size_t)it.fi * H + h] = m;
       a.p2[(size_t)it.fi * H + h] = s;
@@ -865,8 +926,11 @@ gatv2_fwd_rg_kernel(AttnArgs a, float* __restrict__ lcsr, uint32_t* __restrict__
   const float inv = s > 0.f ? 1.f / s : 0.f;
   const float mm = len > 0 ? m : 0.f;
   if (act) {
-    scale4(acc, inv);
-    st4(a.o0 + (size_t)it.v * HD + col, acc);
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) {
+      scale4(acc[c], inv);
+      st4(a.o0 + (size_t)it.v * HD + col + 128 * c, acc[c]);
+    }
     if (leader) {
       a.o1[(size_t)it.v * H + h] = mm;
       a.o2[(size_t)it.v * H + h] = s;
@@ -932,37 +996,45 @@ __device__ __forceinline__ float4 mul4(float4 a, float4 b) { return make_float4(
 
 // AttnArgs: indptr/indices/eid = indptr_t/indices_t/slot_t, feat = fs, fd = stats (float4[N*H]), el = attn, a_csr = the
 // stored logits, a_csr_eid = slot -> edge id (keep / dropout only), o0 = d_fs, o2 = dl per slot.  dat_part: [gridDim.x][H*D].
-template <int G, int LPH, bool KEEP, bool HASH = false>   // KEEP / HASH as gat_bwd_edges_kernel
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_V2E_BLOCKS)
+// CPL as gat_bwd_edges_kernel: warp w of a block keeps the CPL slices of item group (block * warps + w) % (HG / CPL)
+template <int G, int LPH, bool KEEP, bool HASH = false, int CPL = 1>   // KEEP / HASH as gat_bwd_edges_kernel
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, REGNN_WIDE_BLOCKS(CPL, REGNN_V2E_BLOCKS))
 gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __restrict__ dat_part) {
   static_assert(KEEP || !HASH, "HASH is a dropout mode");
   constexpr int U = 2;
   static_assert(G % U == 0, "a round must not straddle a slot batch");
-  __shared__ __align__(16) float dat_s[kWarpsPerBlock * 128];
+  __shared__ __align__(16) float dat_s[kWarpsPerBlock * 128 * CPL];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int lg = lane % G, grp = lane / G, gbase = lane & ~(G - 1);
   const int H = a.H, HD = H * a.D, HG = a.hg_count;
   const int64_t wi = (int64_t)blockIdx.x * kWarpsPerBlock + warp;
   RowItem it{-1, 0, 0, 0, 0, false};
-  if (wi < rg_num_work(a, G)) it = rg_item<G>(a, wi, grp);
-  const int col = it.hg * 128 + lg * 4;
+  if (wi < rg_num_work(a, G, CPL)) it = rg_item<G, CPL>(a, wi, grp);
+  const int col = it.hg * (128 * CPL) + lg * 4;
   const bool col_ok = col < HD;
   const int h = col_ok ? (col >> a.d_shift) : 0;
   const bool act = it.v >= 0 && col_ok;
   const bool leader = act && (col & (a.D - 1)) == 0;
   const int len = it.v >= 0 ? it.len : 0;
   const int maxlen = __reduce_max_sync(0xffffffffu, len);
-  const float4 fu = act ? ldg4(a.feat + (size_t)it.v * HD + col) : zero4();
+  float4 fu[CPL];
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) fu[c] = act ? ldg4(a.feat + (size_t)it.v * HD + col + 128 * c) : zero4();
   const char* gbytes = reinterpret_cast<const char*>(a.G + (col_ok ? col : 0));
   const char* sbytes = reinterpret_cast<const char*>(a.fd) + (size_t)h * 16;
   const uint32_t gpitch = (uint32_t)HD * 4u, spitch = (uint32_t)H * 16u;
   const float* lh = a.a_csr + h;
   float* dlh = a.o2 + h;
-  const uint4* mk = reinterpret_cast<const uint4*>(qmask) + it.hg;
+  const uint4* mk = reinterpret_cast<const uint4*>(qmask) + it.hg * CPL;
   const int32_t* ip = a.indices + it.begin;
   const int32_t* sp = a.eid + it.begin;
-  float4 acc = zero4();
-  PhiAcc ta{zero4(), 0.f};
+  float4 acc[CPL];
+  PhiAcc ta[CPL];
+#pragma unroll
+  for (int c = 0; c < CPL; ++c) {
+    acc[c] = zero4();
+    ta[c] = PhiAcc{zero4(), 0.f};
+  }
   const uint32_t lanebit = 1u << lg;
 
   for (int t0 = 0; t0 < maxlen; t0 += G) {
@@ -976,9 +1048,9 @@ gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __
     }
     const int cnt = min(G, maxlen - t0);
     for (int j = 0; j < cnt; j += U) {
-      float4 x[U];
+      float4 x[U][CPL];
       float4 st[U];
-      uint4 mb[U];
+      uint4 mb[U][CPL];
       float lv[U];
       int sd[U], ss[U];
 #pragma unroll
@@ -986,16 +1058,25 @@ gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __
         sd[u] = __shfl_sync(0xffffffffu, bi, gbase + j + u);
         ss[u] = __shfl_sync(0xffffffffu, bs, gbase + j + u);
         const bool ok = sd[u] >= 0 && col_ok;
-        x[u] = ok ? ldg4(reinterpret_cast<const float*>(gbytes + (uint64_t)(uint32_t)sd[u] * gpitch)) : zero4();
+#pragma unroll
+        for (int c = 0; c < CPL; ++c)
+          x[u][c] = ok ? ldg4(reinterpret_cast<const float*>(gbytes + (uint64_t)(uint32_t)sd[u] * gpitch + 512 * c)) : zero4();
         // missing slot: rowmax = +inf makes exp(. - rowmax) = 0, so a = dl = 0 without per-edge masks
         st[u] = ok ? __ldg(reinterpret_cast<const float4*>(sbytes + (uint64_t)(uint32_t)sd[u] * spitch))
                    : make_float4(0.f, INFINITY, 0.f, 0.f);
         lv[u] = ok ? __ldg(lh + (uint64_t)(uint32_t)ss[u] * (uint32_t)H) : 0.f;
-        mb[u] = ok ? __ldg(mk + (uint64_t)(uint32_t)ss[u] * (uint32_t)HG) : make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+        for (int c = 0; c < CPL; ++c)
+          mb[u][c] = ok ? __ldg(mk + (uint64_t)(uint32_t)ss[u] * (uint32_t)HG + c) : make_uint4(0u, 0u, 0u, 0u);
       }
       float da[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u) da[u] = group_sum<LPH>(dot4(fu, x[u]));
+      for (int u = 0; u < U; ++u) {
+        float p = dot4(fu[0], x[u][0]);
+#pragma unroll
+        for (int c = 1; c < CPL; ++c) p += dot4(fu[c], x[u][c]);
+        da[u] = group_sum<LPH>(p);
+      }
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const float aa = __expf(lv[u] - st[u].y) * st[u].z;
@@ -1007,36 +1088,45 @@ gatv2_bwd_edges_kernel(AttnArgs a, const uint32_t* __restrict__ qmask, float* __
           }
         }
         const float dl = at * da[u] - aa * st[u].w;
-        fma4(acc, at, x[u]);
-        phi_add(ta, dl, mb[u], lanebit);
+#pragma unroll
+        for (int c = 0; c < CPL; ++c) {
+          fma4(acc[c], at, x[u][c]);
+          phi_add(ta[c], dl, mb[u][c], lanebit);
+        }
         if (leader && sd[u] >= 0) dlh[(uint64_t)(uint32_t)ss[u] * (uint32_t)H] = dl;
       }
     }
   }
-  float4 c = zero4();
-  const float4 T = phi_total(ta, a.slope);
-  if (act) {
-    const float4 at4 = ldg4(a.el + col);
-    acc.x = fmaf(at4.x, T.x, acc.x); acc.y = fmaf(at4.y, T.y, acc.y);
-    acc.z = fmaf(at4.z, T.z, acc.z); acc.w = fmaf(at4.w, T.w, acc.w);
-    st4((it.frag ? a.p0 + (size_t)it.fi * HD : a.o0 + (size_t)it.v * HD) + col, acc);
-    c = mul4(fu, T);
-  }
-  // d_attn share of this block: fold the lane groups of the warp (same columns, different rows), then the warps that
-  // own the same 128-float slice, in warp order
 #pragma unroll
-  for (int o = G; o < 32; o <<= 1) {
-    c.x += __shfl_xor_sync(0xffffffffu, c.x, o); c.y += __shfl_xor_sync(0xffffffffu, c.y, o);
-    c.z += __shfl_xor_sync(0xffffffffu, c.z, o); c.w += __shfl_xor_sync(0xffffffffu, c.w, o);
+  for (int k = 0; k < CPL; ++k) {
+    float4 c = zero4();
+    const float4 T = phi_total(ta[k], a.slope);
+    if (act) {
+      const float4 at4 = ldg4(a.el + col + 128 * k);
+      acc[k].x = fmaf(at4.x, T.x, acc[k].x); acc[k].y = fmaf(at4.y, T.y, acc[k].y);
+      acc[k].z = fmaf(at4.z, T.z, acc[k].z); acc[k].w = fmaf(at4.w, T.w, acc[k].w);
+      st4((it.frag ? a.p0 + (size_t)it.fi * HD : a.o0 + (size_t)it.v * HD) + col + 128 * k, acc[k]);
+      c = mul4(fu[k], T);
+    }
+    // d_attn share of this block: fold the lane groups of the warp (same columns, different rows), then the warps that
+    // own the same 128-float slice, in warp order
+#pragma unroll
+    for (int o = G; o < 32; o <<= 1) {
+      c.x += __shfl_xor_sync(0xffffffffu, c.x, o); c.y += __shfl_xor_sync(0xffffffffu, c.y, o);
+      c.z += __shfl_xor_sync(0xffffffffu, c.z, o); c.w += __shfl_xor_sync(0xffffffffu, c.w, o);
+    }
+    if (lane < G) st4(dat_s + (warp * CPL + k) * 128 + lg * 4, c);
   }
-  if (lane < G) st4(dat_s + warp * 128 + lg * 4, c);
   __syncthreads();
   float* outp = dat_part + (size_t)blockIdx.x * HD;
+  const int NI = HG / CPL;   // item groups: slices (CPL = 1) or heads
   for (int i = threadIdx.x; i < HD; i += blockDim.x) {
     float sum = 0.f;
+    const int sl = i / 128;
     if ((i & 127) < G * 4)
       for (int w = 0; w < kWarpsPerBlock; ++w)
-        if (HG == 1 || (int)(((int64_t)blockIdx.x * kWarpsPerBlock + w) % HG) == i / 128) sum += dat_s[w * 128 + (i & 127)];
+        if (NI == 1 || (int)(((int64_t)blockIdx.x * kWarpsPerBlock + w) % NI) == sl / CPL)
+          sum += dat_s[(w * CPL + sl % CPL) * 128 + (i & 127)];
     outp[i] = sum;
   }
 }
@@ -1226,7 +1316,7 @@ attn_frag_finalize_kernel(AttnArgs a, const int32_t* __restrict__ long_rows,
       a.o2[(size_t)v * H + hh] = S;
     }
   }
-  if (a.o3 != nullptr) {
+  if (a.o3 != nullptr && ((g.hg << 7) & (a.D - 1)) == 0) {   // D > 128: only the warp of a head's first slice
     __syncwarp();
     const int s0 = a.indptr[v], len = a.indptr[v + 1] - s0;
     for (int i = lane; i < len * g.nh; i += 32) {
@@ -1303,9 +1393,12 @@ static int check_shape(const char* who, int H, int D, int R, bool has_rel, bool 
   REGNN_REQUIRE(H >= 1 && H <= REGNN_MAX_HEADS, REGNN_ERR_UNSUPPORTED_SHAPE, "%s: num_heads=%d outside [1,%d]", who, H, REGNN_MAX_HEADS);
   REGNN_REQUIRE(D >= 4 && D % 4 == 0, REGNN_ERR_UNSUPPORTED_SHAPE, "%s: head_dim=%d must be a positive multiple of 4", who, D);
   REGNN_REQUIRE(pick_c(H * D) != 0, REGNN_ERR_UNSUPPORTED_SHAPE, "%s: H*D=%d exceeds 1024", who, H * D);
-  if (needs_dot)
-    REGNN_REQUIRE(D <= 128 && (D & (D - 1)) == 0, REGNN_ERR_UNSUPPORTED_SHAPE,
-                  "%s: head_dim=%d must be a power of two in [4,128]", who, D);
+  if (needs_dot) {
+    // a wide head (D > 128) keeps D/128 float4 accumulators per lane: D = 1024 would need 32 floats of each
+    REGNN_REQUIRE(D <= 512, REGNN_ERR_UNSUPPORTED_SHAPE, "%s: head_dim=%d exceeds 512 (the widest head of the attention kernels)",
+                  who, D);
+    REGNN_REQUIRE((D & (D - 1)) == 0, REGNN_ERR_UNSUPPORTED_SHAPE, "%s: head_dim=%d must be a power of two in [4,512]", who, D);
+  }
   if (has_rel)
     REGNN_REQUIRE(R >= 1 && R <= REGNN_MAX_RELATIONS && R * H <= 4096, REGNN_ERR_UNSUPPORTED_SHAPE,
                   "%s: num_relations=%d (x %d heads) unsupported", who, R, H);
@@ -1324,14 +1417,16 @@ static int check_shape(const char* who, int H, int D, int R, bool has_rel, bool 
                                                                              split->num_long)
 
 static int head_groups(int H, int D) { return (H * D + 127) / 128; }
+// 128-bit chunks per lane (CPL) of the kernels that reduce over a head: 1, or D/128 for a wide head (one warp per head)
+static int head_chunks(int D) { return D > 128 ? D / 128 : 1; }
 
 // lanes per row slice of the row-group REGAT kernels: min(H*D, 128) floats in 128-bit chunks, rounded up to 4/8/16/32
 static int rg_lanes(int HD) { return HD > 64 ? 32 : (HD > 32 ? 16 : (HD > 16 ? 8 : 4)); }
-// work items (warps) of a row-group kernel over `rows` rows
-static int64_t rg_work(const AttnArgs& a, int64_t rows) {
+// work items (warps) of a row-group kernel over `rows` rows, cpl chunks per lane (items per row: hg_count / cpl)
+static int64_t rg_work(const AttnArgs& a, int64_t rows, int cpl = 1) {
   const int gpw = 32 / rg_lanes(a.H * a.D);
   const int64_t nrows = a.order != nullptr ? a.n_order : rows;
-  return ((a.nfrag + nrows) * a.hg_count + gpw - 1) / gpw;
+  return ((a.nfrag + nrows) * (a.hg_count / cpl) + gpw - 1) / gpw;
 }
 // row_order lists the rows of the FULL range that are not long: only usable when the call covers [0, N)
 static void apply_order(AttnArgs& a, const int32_t* row_order, const regnn_rowsplit_t* split, int64_t rows) {
@@ -1434,19 +1529,21 @@ extern "C" int regnn_gat_bwd_stats(const float* out, const float* Gd, const floa
   AttnArgs a{};
   a.H = num_heads; a.D = head_dim;
   apply_split(a, nullptr, nullptr);
-  const int G = rg_lanes(num_heads * head_dim);
-  const int64_t work = (num_nodes * a.hg_count + 32 / G - 1) / (32 / G);
+  const int G = rg_lanes(num_heads * head_dim), cpl = head_chunks(head_dim), ni = a.hg_count / cpl;
+  const int64_t work = (num_nodes * ni + 32 / G - 1) / (32 / G);
   const int64_t want = (work + kWarpsPerBlock - 1) / kWarpsPerBlock;
   const unsigned grid = (unsigned)(want < 148 * 16 ? want : 148 * 16);
-#define REGNN_STATS(G_)                                                                                              \
-  gat_bwd_stats_kernel<G_><<<grid, kWarpsPerBlock * 32, 0, stream>>>(out, Gd, er, rowmax, rowsum, num_nodes, num_heads, \
-                                                                    head_dim, a.d_shift, a.hg_count,                \
-                                                                    reinterpret_cast<float4*>(stats))
-  switch (G) {
-    case 4: REGNN_STATS(4); break;
-    case 8: REGNN_STATS(8); break;
-    case 16: REGNN_STATS(16); break;
-    default: REGNN_STATS(32); break;
+#define REGNN_STATS(G_, C_)                                                                                              \
+  gat_bwd_stats_kernel<G_, C_><<<grid, kWarpsPerBlock * 32, 0, stream>>>(out, Gd, er, rowmax, rowsum, num_nodes,       \
+                                                                        num_heads, head_dim, a.d_shift, ni,           \
+                                                                        reinterpret_cast<float4*>(stats))
+  switch (G * cpl) {
+    case 4: REGNN_STATS(4, 1); break;
+    case 8: REGNN_STATS(8, 1); break;
+    case 16: REGNN_STATS(16, 1); break;
+    case 64: REGNN_STATS(32, 2); break;
+    case 128: REGNN_STATS(32, 4); break;
+    default: REGNN_STATS(32, 1); break;
   }
 #undef REGNN_STATS
   return check_launch("regnn_gat_bwd_stats");
@@ -1483,22 +1580,24 @@ extern "C" int regnn_gat_bwd_edges(const int32_t* indptr_t, const int32_t* indic
   REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gat_bwd_edges: dropout heads / scale inconsistent");
   apply_order(a, row_order_t, split_t, rows);
   const size_t smem = sizeof(float) * ((size_t)a.R * num_heads) + 16;
-  const unsigned grid = (unsigned)((rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock);
+  const int cpl = head_chunks(head_dim);
+  const unsigned grid = (unsigned)((rg_work(a, rows, cpl) + kWarpsPerBlock - 1) / kWarpsPerBlock);
   {
     const int G = rg_lanes(a.H * a.D), lph = min(G, head_dim / 4);
     bool launched = false;
-#define REGNN_EDGES_CASE(G_, L_)                                                                   \
-  if (G == G_ && lph == L_) {                                                                      \
-    if (dropout != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true, true>), grid, smem); \
-    else if (keep != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true>), grid, smem);  \
-    else REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, false>), grid, smem);                      \
-    launched = true;                                                                               \
+#define REGNN_EDGES_CASE(G_, L_, C_)                                                                             \
+  if (G == G_ && lph == L_ && cpl == C_) {                                                                       \
+    if (dropout != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true, true, C_>), grid, smem);        \
+    else if (keep != nullptr) REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, true, false, C_>), grid, smem);     \
+    else REGNN_DISPATCH_C((gat_bwd_edges_kernel<G_, L_, false, false, C_>), grid, smem);                         \
+    launched = true;                                                                                             \
   }
-    REGNN_EDGES_CASE(4, 1) REGNN_EDGES_CASE(4, 2) REGNN_EDGES_CASE(4, 4)
-    REGNN_EDGES_CASE(8, 1) REGNN_EDGES_CASE(8, 2) REGNN_EDGES_CASE(8, 4) REGNN_EDGES_CASE(8, 8)
-    REGNN_EDGES_CASE(16, 1) REGNN_EDGES_CASE(16, 2) REGNN_EDGES_CASE(16, 4) REGNN_EDGES_CASE(16, 8) REGNN_EDGES_CASE(16, 16)
-    REGNN_EDGES_CASE(32, 1) REGNN_EDGES_CASE(32, 2) REGNN_EDGES_CASE(32, 4) REGNN_EDGES_CASE(32, 8) REGNN_EDGES_CASE(32, 16)
-    REGNN_EDGES_CASE(32, 32)
+    REGNN_EDGES_CASE(4, 1, 1) REGNN_EDGES_CASE(4, 2, 1) REGNN_EDGES_CASE(4, 4, 1)
+    REGNN_EDGES_CASE(8, 1, 1) REGNN_EDGES_CASE(8, 2, 1) REGNN_EDGES_CASE(8, 4, 1) REGNN_EDGES_CASE(8, 8, 1)
+    REGNN_EDGES_CASE(16, 1, 1) REGNN_EDGES_CASE(16, 2, 1) REGNN_EDGES_CASE(16, 4, 1) REGNN_EDGES_CASE(16, 8, 1)
+    REGNN_EDGES_CASE(16, 16, 1)
+    REGNN_EDGES_CASE(32, 1, 1) REGNN_EDGES_CASE(32, 2, 1) REGNN_EDGES_CASE(32, 4, 1) REGNN_EDGES_CASE(32, 8, 1)
+    REGNN_EDGES_CASE(32, 16, 1) REGNN_EDGES_CASE(32, 32, 1) REGNN_EDGES_CASE(32, 32, 2) REGNN_EDGES_CASE(32, 32, 4)
 #undef REGNN_EDGES_CASE
     REGNN_REQUIRE(launched, REGNN_ERR_UNSUPPORTED_SHAPE, "gat_bwd_edges: no kernel for H=%d D=%d", num_heads, head_dim);
   }
@@ -1579,18 +1678,20 @@ extern "C" int regnn_attn_scores_fwd(const float* feat, const float* attn_l, con
   AttnArgs a{};
   a.H = num_heads; a.D = head_dim;
   apply_split(a, nullptr, nullptr);
-  const int G = rg_lanes(num_heads * head_dim);
-  const int64_t work = (num_nodes * a.hg_count + 32 / G - 1) / (32 / G);
+  const int G = rg_lanes(num_heads * head_dim), cpl = head_chunks(head_dim), ni = a.hg_count / cpl;
+  const int64_t work = (num_nodes * ni + 32 / G - 1) / (32 / G);
   const int64_t want = (work + kWarpsPerBlock - 1) / kWarpsPerBlock;
   const unsigned grid = (unsigned)(want < 148 * 16 ? want : 148 * 16);
-#define REGNN_SCORES_FWD(G_)                                                                                           \
-  attn_scores_fwd_kernel<G_><<<grid, kWarpsPerBlock * 32, 0, stream>>>(feat, attn_l, attn_r, num_nodes, num_heads, head_dim, \
-                                                                      a.d_shift, a.hg_count, el, er)
-  switch (G) {
-    case 4: REGNN_SCORES_FWD(4); break;
-    case 8: REGNN_SCORES_FWD(8); break;
-    case 16: REGNN_SCORES_FWD(16); break;
-    default: REGNN_SCORES_FWD(32); break;
+#define REGNN_SCORES_FWD(G_, C_)                                                                                      \
+  attn_scores_fwd_kernel<G_, C_><<<grid, kWarpsPerBlock * 32, 0, stream>>>(feat, attn_l, attn_r, num_nodes, num_heads, \
+                                                                          head_dim, a.d_shift, ni, el, er)
+  switch (G * cpl) {
+    case 4: REGNN_SCORES_FWD(4, 1); break;
+    case 8: REGNN_SCORES_FWD(8, 1); break;
+    case 16: REGNN_SCORES_FWD(16, 1); break;
+    case 64: REGNN_SCORES_FWD(32, 2); break;
+    case 128: REGNN_SCORES_FWD(32, 4); break;
+    default: REGNN_SCORES_FWD(32, 1); break;
   }
 #undef REGNN_SCORES_FWD
   return check_launch("regnn_attn_scores_fwd");
@@ -1662,27 +1763,33 @@ extern "C" int regnn_gatv2_fwd(const int32_t* indptr, const int32_t* indices, co
   REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gatv2_fwd: dropout heads / scale inconsistent");
   apply_order(a, row_order, split, rows);
   const size_t smem = sizeof(float) * ((size_t)a.R * num_heads) + 16;
-  const unsigned grid = (unsigned)((rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock);
+  const int cpl = head_chunks(head_dim);
+  const unsigned grid = (unsigned)((rg_work(a, rows, cpl) + kWarpsPerBlock - 1) / kWarpsPerBlock);
   {
     const int G = rg_lanes(a.H * a.D), lph = min(G, head_dim / 4);
     const bool hash = dropout != nullptr;
     const bool extra = keep != nullptr || attn_out != nullptr;
     bool launched = false;
-#define REGNN_V2F_CASE(G_, L_)                                                                   \
-  if (G == G_ && lph == L_) {                                                                    \
-    rc = set_smem(hash ? gatv2_fwd_rg_kernel<G_, L_, true, true>                                                     \
-                       : (extra ? gatv2_fwd_rg_kernel<G_, L_, true> : gatv2_fwd_rg_kernel<G_, L_, false>), smem);    \
-    if (rc != REGNN_OK) return rc;                                                                                   \
-    if (hash) gatv2_fwd_rg_kernel<G_, L_, true, true><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask); \
-    else if (extra) gatv2_fwd_rg_kernel<G_, L_, true><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask); \
-    else gatv2_fwd_rg_kernel<G_, L_, false><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask);       \
-    launched = true;                                                                                                 \
+#define REGNN_V2F_CASE(G_, L_, C_)                                                                                     \
+  if (G == G_ && lph == L_ && cpl == C_) {                                                                             \
+    rc = set_smem(hash ? gatv2_fwd_rg_kernel<G_, L_, true, true, C_>                                                   \
+                       : (extra ? gatv2_fwd_rg_kernel<G_, L_, true, false, C_>                                         \
+                                : gatv2_fwd_rg_kernel<G_, L_, false, false, C_>), smem);                               \
+    if (rc != REGNN_OK) return rc;                                                                                     \
+    if (hash)                                                                                                          \
+      gatv2_fwd_rg_kernel<G_, L_, true, true, C_><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask);   \
+    else if (extra)                                                                                                    \
+      gatv2_fwd_rg_kernel<G_, L_, true, false, C_><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask);  \
+    else                                                                                                               \
+      gatv2_fwd_rg_kernel<G_, L_, false, false, C_><<<grid, kWarpsPerBlock * 32, smem, stream>>>(a, logit_csr, qmask); \
+    launched = true;                                                                                                   \
   }
-    REGNN_V2F_CASE(4, 1) REGNN_V2F_CASE(4, 2) REGNN_V2F_CASE(4, 4)
-    REGNN_V2F_CASE(8, 1) REGNN_V2F_CASE(8, 2) REGNN_V2F_CASE(8, 4) REGNN_V2F_CASE(8, 8)
-    REGNN_V2F_CASE(16, 1) REGNN_V2F_CASE(16, 2) REGNN_V2F_CASE(16, 4) REGNN_V2F_CASE(16, 8) REGNN_V2F_CASE(16, 16)
-    REGNN_V2F_CASE(32, 1) REGNN_V2F_CASE(32, 2) REGNN_V2F_CASE(32, 4) REGNN_V2F_CASE(32, 8) REGNN_V2F_CASE(32, 16)
-    REGNN_V2F_CASE(32, 32)
+    REGNN_V2F_CASE(4, 1, 1) REGNN_V2F_CASE(4, 2, 1) REGNN_V2F_CASE(4, 4, 1)
+    REGNN_V2F_CASE(8, 1, 1) REGNN_V2F_CASE(8, 2, 1) REGNN_V2F_CASE(8, 4, 1) REGNN_V2F_CASE(8, 8, 1)
+    REGNN_V2F_CASE(16, 1, 1) REGNN_V2F_CASE(16, 2, 1) REGNN_V2F_CASE(16, 4, 1) REGNN_V2F_CASE(16, 8, 1)
+    REGNN_V2F_CASE(16, 16, 1)
+    REGNN_V2F_CASE(32, 1, 1) REGNN_V2F_CASE(32, 2, 1) REGNN_V2F_CASE(32, 4, 1) REGNN_V2F_CASE(32, 8, 1)
+    REGNN_V2F_CASE(32, 16, 1) REGNN_V2F_CASE(32, 32, 1) REGNN_V2F_CASE(32, 32, 2) REGNN_V2F_CASE(32, 32, 4)
 #undef REGNN_V2F_CASE
     REGNN_REQUIRE(launched, REGNN_ERR_UNSUPPORTED_SHAPE, "gatv2_fwd: no kernel for H=%d D=%d", num_heads, head_dim);
   }
@@ -1699,7 +1806,7 @@ extern "C" int64_t regnn_gatv2_bwd_edges_blocks(int64_t num_rows, int num_frags,
   if (num_rows < 0 || num_heads < 1 || head_dim < 4) return 0;
   const int HD = num_heads * head_dim, gpw = 32 / rg_lanes(HD);
   const int64_t nrows = ordered ? num_rows - num_long : num_rows;
-  const int64_t work = ((num_frags + nrows) * head_groups(num_heads, head_dim) + gpw - 1) / gpw;
+  const int64_t work = ((num_frags + nrows) * (head_groups(num_heads, head_dim) / head_chunks(head_dim)) + gpw - 1) / gpw;
   return (work + kWarpsPerBlock - 1) / kWarpsPerBlock;
 }
 
@@ -1735,26 +1842,30 @@ extern "C" int regnn_gatv2_bwd_edges(const int32_t* indptr_t, const int32_t* ind
   REGNN_REQUIRE(apply_split(a, split_t, split_workspace), REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: incomplete row split");
   REGNN_REQUIRE(apply_dropout(a, dropout), REGNN_ERR_INVALID_ARG, "gatv2_bwd_edges: dropout heads / scale inconsistent");
   apply_order(a, row_order_t, split_t, rows);
-  const int64_t nb = (rg_work(a, rows) + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  const int cpl = head_chunks(head_dim);
+  const int64_t nb = (rg_work(a, rows, cpl) + kWarpsPerBlock - 1) / kWarpsPerBlock;
   {
     const int G = rg_lanes(HD), lph = min(G, head_dim / 4);
     bool launched = false;
-#define REGNN_V2E_CASE(G_, L_)                                                                                          \
-  if (G == G_ && lph == L_) {                                                                                           \
-    if (dropout != nullptr)                                                                                             \
-      gatv2_bwd_edges_kernel<G_, L_, true, true><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask,            \
-                                                                                                  block_partials);     \
-    else if (keep != nullptr)                                                                                           \
-      gatv2_bwd_edges_kernel<G_, L_, true><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask, block_partials); \
-    else                                                                                                                \
-      gatv2_bwd_edges_kernel<G_, L_, false><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask, block_partials);\
-    launched = true;                                                                                                    \
+#define REGNN_V2E_CASE(G_, L_, C_)                                                                                     \
+  if (G == G_ && lph == L_ && cpl == C_) {                                                                             \
+    if (dropout != nullptr)                                                                                            \
+      gatv2_bwd_edges_kernel<G_, L_, true, true, C_><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask,       \
+                                                                                                      block_partials); \
+    else if (keep != nullptr)                                                                                          \
+      gatv2_bwd_edges_kernel<G_, L_, true, false, C_><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask,      \
+                                                                                                       block_partials);\
+    else                                                                                                               \
+      gatv2_bwd_edges_kernel<G_, L_, false, false, C_><<<(unsigned)nb, kWarpsPerBlock * 32, 0, stream>>>(a, qmask,     \
+                                                                                                        block_partials);\
+    launched = true;                                                                                                   \
   }
-    REGNN_V2E_CASE(4, 1) REGNN_V2E_CASE(4, 2) REGNN_V2E_CASE(4, 4)
-    REGNN_V2E_CASE(8, 1) REGNN_V2E_CASE(8, 2) REGNN_V2E_CASE(8, 4) REGNN_V2E_CASE(8, 8)
-    REGNN_V2E_CASE(16, 1) REGNN_V2E_CASE(16, 2) REGNN_V2E_CASE(16, 4) REGNN_V2E_CASE(16, 8) REGNN_V2E_CASE(16, 16)
-    REGNN_V2E_CASE(32, 1) REGNN_V2E_CASE(32, 2) REGNN_V2E_CASE(32, 4) REGNN_V2E_CASE(32, 8) REGNN_V2E_CASE(32, 16)
-    REGNN_V2E_CASE(32, 32)
+    REGNN_V2E_CASE(4, 1, 1) REGNN_V2E_CASE(4, 2, 1) REGNN_V2E_CASE(4, 4, 1)
+    REGNN_V2E_CASE(8, 1, 1) REGNN_V2E_CASE(8, 2, 1) REGNN_V2E_CASE(8, 4, 1) REGNN_V2E_CASE(8, 8, 1)
+    REGNN_V2E_CASE(16, 1, 1) REGNN_V2E_CASE(16, 2, 1) REGNN_V2E_CASE(16, 4, 1) REGNN_V2E_CASE(16, 8, 1)
+    REGNN_V2E_CASE(16, 16, 1)
+    REGNN_V2E_CASE(32, 1, 1) REGNN_V2E_CASE(32, 2, 1) REGNN_V2E_CASE(32, 4, 1) REGNN_V2E_CASE(32, 8, 1)
+    REGNN_V2E_CASE(32, 16, 1) REGNN_V2E_CASE(32, 32, 1) REGNN_V2E_CASE(32, 32, 2) REGNN_V2E_CASE(32, 32, 4)
 #undef REGNN_V2E_CASE
     REGNN_REQUIRE(launched, REGNN_ERR_UNSUPPORTED_SHAPE, "gatv2_bwd_edges: no kernel for H=%d D=%d", num_heads, head_dim);
   }

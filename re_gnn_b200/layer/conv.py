@@ -110,14 +110,15 @@ class REMixHopConv(_RelationEmbedded):
 
 
 def _kernel_head_dim(d):
-    """Head width the attention kernels run at: the next power of two >= max(4, d) (they reduce over the D/4
-    lanes of a head with butterfly shuffles).  Other widths -- e.g. ``out_feats = num_classes`` -- are zero-padded
-    by the layer: zero columns add nothing to any logit and their outputs / gradients are sliced away."""
+    """Head width the attention kernels run at: the next power of two >= max(4, d), at most 512 (they reduce over a
+    head with butterfly shuffles, a head wider than 128 floats held as D/128 chunks per lane).  Other widths -- e.g.
+    ``out_feats = num_classes`` -- are zero-padded by the layer: zero columns add nothing to any logit and their
+    outputs / gradients are sliced away."""
     p = 4
     while p < d:
         p *= 2
-    if p > 128:
-        raise ValueError('head width %d is not supported (at most 128 per head)' % d)
+    if p > 512:
+        raise ValueError('head width %d is not supported (at most 512 per head)' % d)
     return p
 
 
