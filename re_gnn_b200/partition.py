@@ -17,6 +17,8 @@ relation-degree norm for all rows; the caller sums the R-float relation gradient
      blocks into the peers' slabs, the ``regnn_spmm_*_scatter`` epilogues store finished rows into their owners'
      row blocks; torch symmetric memory supplies the mapped buffers and the device-side barrier.
    The norm gradient's row dots span all columns, but the row owner has complete rows: ``d_norm`` is a local pass.
+   The attention cores take the same scheme over their heads: ``head_sliced_gat`` (REGAT), ``head_sliced_gatv2``
+   (REGATv2).
 3. ``halo_propagate`` -- destination-row blocks that exchange only their **halo** (the remote rows their edges
    reference) and hold only local views (``HaloPartition``): every rank gathers E/P edges at the full row width.  The
    degree norm is computed inside from a local relation-count table (halo rows get their owner's bits); the exchange is
@@ -251,19 +253,28 @@ class SlabExchange(_PeerBuffers):
     (Y and dX, [per, F]) that the SpMM kernels of all ranks store finished rows into, and a [P, 256]-float table
     every rank writes its share of the relation gradient into (``allreduce_relation_grads``).  ``y_cols`` is a plain
     local slab: this rank's columns of Y, kept for the folded norm gradient of the backward kernel.  Create it once
-    per layer; a forward must be followed by its backward before the next forward (the buffers are reused)."""
+    per layer; a forward must be followed by its backward before the next forward (the buffers are reused).
 
-    def __init__(self, feat, bounds, rank, device, group=None):
+    ``gatv2=True`` (a ``head_sliced_gatv2`` call site): also a second column slab ``fd_cols`` for the destination
+    features and a second row block ``dfd_rows`` for their gradient."""
+
+    def __init__(self, feat, bounds, rank, device, group=None, gatv2=False):
         group = group if group is not None else dist.group.WORLD
         self.parts, self.per, self.rank, self.feat = len(bounds) - 1, _uniform_rows(bounds), rank, feat
         if not self.per or feat % (4 * self.parts):
             raise ValueError('SlabExchange needs equal row blocks and F divisible by 4 * ranks')
         self.fc = feat // self.parts
+        self.gatv2 = gatv2
         self._handles = []
         self.x_cols, self.x_ptrs = self._alloc(self.parts * self.per, self.fc, device, group)
         self.g_cols, self.g_ptrs = self._alloc(self.parts * self.per, self.fc, device, group)
         self.y_rows, self.y_ptrs = self._alloc(self.per, feat, device, group)
         self.dx_rows, self.dx_ptrs = self._alloc(self.per, feat, device, group)
+        if gatv2:
+            self.fd_cols, self.fd_ptrs = self._alloc(self.parts * self.per, self.fc, device, group)
+            self.dfd_rows, self.dfd_ptrs = self._alloc(self.per, feat, device, group)
+            self.fd_cols.zero_()
+            self.peer_dfd = _lib.PeerRows(self.dfd_ptrs.data_ptr(), self.parts, self.per, feat, rank * self.fc)
         self.grad_tab, self.grad_ptrs = self._alloc(self.parts, self.GRAD_SLOTS, device, group)
         self.y_cols = torch.zeros((self.parts * self.per, self.fc), dtype=torch.float32, device=device)
         self.x_cols.zero_()
@@ -336,30 +347,36 @@ def feature_sliced_propagate(graph, etv, x_own, theta, alpha, norm, bounds, rank
     return _ColumnSlabPropagate.apply(graph, etv, x_own, theta, alpha, norm, bounds, rank, group)
 
 
-def _rows_to_head_slab(own, n, bounds, rank, group, xch, grad=False):
-    """Row block [rows_own, H, D] -> this rank's head slab of all N rows [N, H*D/P]: one all-to-all, or (``xch``) pushed
-    into every rank's ``x_cols`` (``g_cols`` with ``grad``) over peer memory."""
-    own = own.flatten(1).contiguous()      # [0, H*D] for a rank that owns no rows
+def _rows_to_head_slabs(owns, n, bounds, rank, group, xch, slabs):
+    """Row blocks [rows_own, H, D] -> this rank's head slabs of all N rows [N, H*D/P], one per row block: one all-to-all
+    each, or (``xch``) pushed over peer memory into every rank's slab ``slabs[i]`` of the exchange ('x', 'g' or 'fd':
+    ``xch.x_cols`` / ``g_cols`` / ``fd_cols``), all pushes before one barrier."""
+    owns = [own.flatten(1).contiguous() for own in owns]      # [0, H*D] for a rank that owns no rows
     if xch is None:
-        return _rows_to_columns(own, _uniform_rows(bounds), len(bounds) - 1, group)[:n]
-    cols, ptrs = (xch.g_cols, xch.g_ptrs) if grad else (xch.x_cols, xch.x_ptrs)
-    ops.rows_to_slabs(own, xch.parts, rank * xch.per, ptrs)
-    xch.barrier()            # every rank's rows of my heads have landed in my slab
-    return cols[:n]
+        return [_rows_to_columns(own, _uniform_rows(bounds), len(bounds) - 1, group)[:n] for own in owns]
+    for own, s in zip(owns, slabs):
+        ops.rows_to_slabs(own, xch.parts, rank * xch.per, getattr(xch, s + '_ptrs'))
+    xch.barrier()            # every rank's rows of my heads have landed in my slabs
+    return [getattr(xch, s + '_cols')[:n] for s in slabs]
 
 
-def _head_slab_to_rows(slab, rows_own, bounds, group, xch, grad=False):
-    """Inverse of ``_rows_to_head_slab``: head slab [N, H/P, D] -> this rank's row block [rows_own, H*D], through
-    ``xch.y_rows`` (``dx_rows`` with ``grad``) over peer memory."""
-    n = slab.shape[0]
-    slab = slab.flatten(1)
+def _head_slabs_to_rows(slabs, rows_own, bounds, group, xch, blocks):
+    """Inverse of ``_rows_to_head_slabs``: head slabs [N, H/P, D] -> this rank's row blocks [rows_own, H*D], over peer
+    memory through the exchange's row block ``blocks[i]`` ('y', 'dx' or 'dfd': ``xch.y_rows`` / ``dx_rows`` /
+    ``dfd_rows``), all pushes before one barrier."""
+    slabs = [slab.flatten(1) for slab in slabs]
     if xch is None:
         parts, per = len(bounds) - 1, _uniform_rows(bounds)
-        pad = torch.cat([slab, slab.new_zeros((parts * per - n, slab.shape[1]))]) if parts * per > n else slab
-        return _columns_to_rows(pad.contiguous(), per, parts, rows_own, group)
-    ops.slabs_to_rows(slab, n, xch.peer_dx if grad else xch.peer_y)
-    xch.barrier()            # every rank's heads of my rows have landed in my row block
-    return (xch.dx_rows if grad else xch.y_rows)[:rows_own].clone()
+        rows = []
+        for slab in slabs:
+            n = slab.shape[0]
+            pad = torch.cat([slab, slab.new_zeros((parts * per - n, slab.shape[1]))]) if parts * per > n else slab
+            rows.append(_columns_to_rows(pad.contiguous(), per, parts, rows_own, group))
+        return rows
+    for slab, b in zip(slabs, blocks):
+        ops.slabs_to_rows(slab, slab.shape[0], getattr(xch, 'peer_' + b))
+    xch.barrier()            # every rank's heads of my rows have landed in my row blocks
+    return [getattr(xch, b + '_rows')[:rows_own].clone() for b in blocks]
 
 
 def _head_slice_grad(param, grad, sl):
@@ -375,7 +392,7 @@ class _HeadSlicedGat(torch.autograd.Function):
     """REGAT core (projection scores + fused logits / edge softmax / aggregation) sharded over the HEADS: attention
     heads are independent (el / er, the softmax statistics and the aggregation never mix heads), so rank q runs all
     rows for heads [q*H/P, (q+1)*H/P) -- the same column-slab scheme as the REGCN aggregation.  The four row <-> slab
-    re-partitions (``_rows_to_head_slab``, ``_head_slab_to_rows``) are one all-to-all each (NCCL; gloo in the CPU tests)
+    re-partitions (``_rows_to_head_slabs``, ``_head_slabs_to_rows``) are one all-to-all each (NCCL; gloo in the CPU tests)
     or, with a ``SlabExchange`` ``xch`` of width H*D, our own kernels over peer memory (regnn_rows_to_slabs,
     regnn_slabs_to_rows), where the head slab of the features stays in ``xch.x_cols`` for the backward.  Row block in,
     row block out; parameter gradients (attn_l, attn_r, relation embedding) come back with this rank's head slice filled
@@ -390,7 +407,7 @@ class _HeadSlicedGat(torch.autograd.Function):
         sl = slice(rank * hs, (rank + 1) * hs)
         # this rank's heads of the full-H mask: the counter hash takes the global head
         dropout = dropout.for_heads(rank * hs, heads) if dropout is not None else None
-        f_cols = _rows_to_head_slab(f_own, n, bounds, rank, group, xch).view(n, hs, dim)
+        f_cols = _rows_to_head_slabs((f_own,), n, bounds, rank, group, xch, ('x',))[0].view(n, hs, dim)
         al, ar = attn_l[:, sl].contiguous(), attn_r[:, sl].contiguous()
         th = theta[:, sl].contiguous() if etv is not None else None
         el, er = ops.attn_scores_fwd(f_cols, al, ar)
@@ -401,19 +418,20 @@ class _HeadSlicedGat(torch.autograd.Function):
         ctx.dropout = dropout
         ctx.sl = sl
         ctx.save_for_backward(f_cols, el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta)
-        return _head_slab_to_rows(out, rows_own, bounds, group, xch).view(rows_own, heads, dim)
+        return _head_slabs_to_rows((out,), rows_own, bounds, group, xch, ('y',))[0].view(rows_own, heads, dim)
 
     @staticmethod
     def backward(ctx, g_own):
         f_cols, el, er, al, ar, th, out, rowmax, rowsum, attn_l, attn_r, theta = ctx.saved_tensors
         n, hs, dim = f_cols.shape
         rows_own, heads, _ = g_own.shape
-        g_cols = _rows_to_head_slab(g_own, n, ctx.bounds, ctx.rank, ctx.group, ctx.xch, grad=True).view(n, hs, dim)
+        g_cols = _rows_to_head_slabs((g_own,), n, ctx.bounds, ctx.rank, ctx.group, ctx.xch, ('g',))[0].view(n, hs, dim)
         et, et_t = (ctx.etv[0], ctx.etv[1]) if ctx.etv is not None else (None, None)
         d_f, _, _, d_th, d_al, d_ar = ops.gat_bwd(ctx.graph.csr(), et, et_t, th, ctx.alpha, f_cols, el, er, ctx.slope,
                                                    None, out, rowmax, rowsum, g_cols, attn_l=al, attn_r=ar,
                                                    **ops.dropout_kw(ctx.dropout))
-        d_f_own = _head_slab_to_rows(d_f, rows_own, ctx.bounds, ctx.group, ctx.xch, grad=True).view(rows_own, heads, dim)
+        d_f_own = _head_slabs_to_rows((d_f,), rows_own, ctx.bounds, ctx.group, ctx.xch, ('dx',))[0]
+        d_f_own = d_f_own.view(rows_own, heads, dim)
         return (None, None, d_f_own, _head_slice_grad(attn_l, d_al, ctx.sl), _head_slice_grad(attn_r, d_ar, ctx.sl),
                 _head_slice_grad(theta, d_th, ctx.sl), None, None, None, None, None, None, None)
 
@@ -432,6 +450,115 @@ def head_sliced_gat(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, boun
         raise ValueError('head-sliced attention over peer memory needs a SlabExchange of width num_heads * head_dim')
     return _HeadSlicedGat.apply(graph, etv, f_own, attn_l, attn_r, theta, alpha, slope, bounds, rank, group, exchange,
                                 dropout)
+
+
+def _gatv2_slab_forward(graph, etv, fs_cols, fd_cols, attn, theta, alpha, slope, sl, heads, dropout):
+    """One rank's compute in the ``head_sliced_gatv2`` forward: the REGATv2 training forward over all N rows for the heads
+    ``sl`` of an H-head layer.  ``fs_cols`` / ``fd_cols`` [N, H/P, D] are the slabs; ``attn`` [1, H, D], ``theta`` [R, H]
+    and ``dropout`` (over all H heads) are narrowed to the slice here.  -> (out [N, H/P, D], the state
+    ``_gatv2_slab_backward`` needs: the sliced parameters, the row statistics and the per-slot logits and sign masks)."""
+    at = attn[:, sl].contiguous()
+    th = theta[:, sl].contiguous() if (etv is not None and theta is not None) else None
+    drop = dropout.for_heads(sl.start, heads) if dropout is not None else None
+    out, rowmax, rowsum, _, saved = ops.gatv2_fwd(graph.csr(), etv[0] if th is not None else None, th, alpha, fs_cols,
+                                                  fd_cols, at, slope, save=True, **ops.dropout_kw(drop))
+    return out, (at, th, drop, rowmax, rowsum, saved)
+
+
+def _gatv2_slab_backward(graph, etv, fs_cols, fd_cols, out, state, g_cols, alpha, slope):
+    """The backward of ``_gatv2_slab_forward`` -> (d_fs, d_fd [N, H/P, D], d_attn [H/P * D], d_theta [R, H/P] | None)."""
+    at, th, drop, rowmax, rowsum, saved = state
+    return ops.gatv2_bwd(graph.csr(), etv[0] if th is not None else None, th, alpha, fs_cols, fd_cols, at, slope, None,
+                         out, rowmax, rowsum, saved, g_cols, **ops.dropout_kw(drop))
+
+
+class _HeadSlicedGatV2(torch.autograd.Function):
+    """REGATv2 core (fused logits / edge softmax / aggregation of ``functional.gatv2_aggregate``) sharded over the HEADS:
+    the logit sum_d attn[h,d] * LeakyReLU(fs + fd), the softmax statistics, the stored logits and sign masks and the
+    aggregation never mix heads, so rank q runs all rows for heads [q*H/P, (q+1)*H/P) (``_gatv2_slab_forward`` /
+    ``_gatv2_slab_backward``).  Six row <-> slab re-partitions: fs, fd and out in the forward, dL/dY, d_fs and d_fd in
+    the backward (one each for fs and its gradient when ``shared``: fs is fd).  Each is an all-to-all (NCCL; gloo in the
+    CPU tests) or, with a ``SlabExchange`` ``xch`` built with ``gatv2=True``, a push over peer memory; both pushes of a
+    direction go before one barrier.  Parameter gradients come back with this rank's head slice filled and zeros
+    elsewhere (``allreduce_relation_grads``)."""
+
+    @staticmethod
+    def forward(ctx, graph, etv, fs_own, fd_own, attn, theta, alpha, slope, bounds, rank, group, xch, dropout, shared):
+        n = graph.number_of_nodes()
+        rows_own, heads, dim = fs_own.shape
+        hs = heads // (len(bounds) - 1)
+        sl = slice(rank * hs, (rank + 1) * hs)
+        owns, slabs = ((fs_own,), ('x',)) if shared else ((fs_own, fd_own), ('x', 'fd'))
+        cols = [c.view(n, hs, dim) for c in _rows_to_head_slabs(owns, n, bounds, rank, group, xch, slabs)]
+        fs_cols, fd_cols = cols[0], cols[-1]
+        out, state = _gatv2_slab_forward(graph, etv, fs_cols, fd_cols, attn, theta, alpha, slope, sl, heads, dropout)
+        ctx.graph, ctx.etv, ctx.alpha, ctx.slope, ctx.bounds, ctx.rank, ctx.group, ctx.xch = \
+            graph, etv, alpha, slope, bounds, rank, group, xch
+        ctx.sl, ctx.shared = sl, shared
+        ctx.slab = (fs_cols, fd_cols, out, state)
+        ctx.save_for_backward(attn, theta)
+        return _head_slabs_to_rows((out,), rows_own, bounds, group, xch, ('y',))[0].view(rows_own, heads, dim)
+
+    @staticmethod
+    def backward(ctx, g_own):
+        attn, theta = ctx.saved_tensors
+        fs_cols, fd_cols, out, state = ctx.slab
+        n, hs, dim = fs_cols.shape
+        rows_own, heads, _ = g_own.shape
+        g_cols = _rows_to_head_slabs((g_own,), n, ctx.bounds, ctx.rank, ctx.group, ctx.xch, ('g',))[0].view(n, hs, dim)
+        d_fs, d_fd, d_at, d_th = _gatv2_slab_backward(ctx.graph, ctx.etv, fs_cols, fd_cols, out, state, g_cols, ctx.alpha,
+                                                      ctx.slope)
+        # one tensor on both sides: its gradient is the sum (autograd would add the two row blocks the same way)
+        slabs, blocks = ((d_fs + d_fd,), ('dx',)) if ctx.shared else ((d_fs, d_fd), ('dx', 'dfd'))
+        rows = [r.view(rows_own, heads, dim) for r in _head_slabs_to_rows(slabs, rows_own, ctx.bounds, ctx.group, ctx.xch,
+                                                                          blocks)]
+        return (None, None, rows[0], None if ctx.shared else rows[1], _head_slice_grad(attn, d_at, ctx.sl),
+                _head_slice_grad(theta, d_th, ctx.sl), None, None, None, None, None, None, None, None)
+
+
+def head_sliced_gatv2(graph, etv, fs_own, fd_own, attn, theta, alpha, slope, bounds, rank, group=None, exchange=None,
+                      dropout=None, keep=None):
+    """fs_own, fd_own [rows_own, H, D] -> out rows [rows_own, H, D]: the REGATv2 core of ``functional.gatv2_aggregate``
+    with rank q computing heads [q*H/P, (q+1)*H/P) of all rows; see ``_HeadSlicedGatV2``.  Row blocks must be equal
+    (``row_blocks(..., balance='rows')``) and H divisible by P.  With shared weights (or one feature tensor for both
+    sides) pass the same tensor as ``fs_own`` and ``fd_own``: it is exchanged once.  ``exchange`` (a ``SlabExchange`` of
+    width H*D built with ``gatv2=True``): the re-partitions run over peer memory inside our own kernels instead of NCCL /
+    gloo all-to-alls.  ``etv=None`` or ``theta=None`` drops the relation term.  out, d_fs and d_fd are bit-identical to
+    ``gatv2_aggregate``; ``attn.grad`` and ``theta.grad`` hold this rank's head slice (``allreduce_relation_grads``).
+    ``dropout`` (a ``functional.HashedDropout`` over all H heads): attention dropout, as ``head_sliced_gat``; an explicit
+    ``keep`` mask is refused.  The MAG stack's ``softmax_eps`` (a global maximum over all logits) is not taken."""
+    _, heads, dim = fs_own.shape
+    if keep is not None:
+        raise ValueError('head_sliced_gatv2: an explicit attention dropout mask is not supported (it is in edge-id order '
+                         'over all edges); pass dropout=functional.HashedDropout(p, key)')
+    _check_hashed_dropout(dropout, 'head_sliced_gatv2')
+    if not _uniform_rows(bounds) or heads % (len(bounds) - 1):
+        raise ValueError('head-sliced attention needs equal row blocks and num_heads divisible by the number of ranks')
+    if tuple(fd_own.shape) != tuple(fs_own.shape):
+        raise ValueError('head_sliced_gatv2: fs_own and fd_own must both be [rows_own, H, D], got %s and %s'
+                         % (tuple(fs_own.shape), tuple(fd_own.shape)))
+    if exchange is not None and (exchange.feat != heads * dim or not exchange.gatv2):
+        raise ValueError('head_sliced_gatv2 over peer memory needs a SlabExchange of width num_heads * head_dim = %d '
+                         'built with gatv2=True' % (heads * dim))
+    return _HeadSlicedGatV2.apply(graph, etv, fs_own, fd_own, attn, theta, alpha, slope, bounds, rank, group, exchange,
+                                  dropout, fd_own is fs_own)
+
+
+def _virtual_head_sliced_gatv2(graph, etv, fs, fd, gout, attn, theta, alpha, slope, parts, dropout=None):
+    """The per-rank slab compute of ``head_sliced_gatv2`` for ranks q = 0..P-1 one after another in one process (no
+    process group, no exchange): rank q's slabs are its columns of the global [N, H, D] arrays.  -> (out, d_fs, d_fd,
+    d_attn [1, H, D], d_theta [R, H] | None), every result stitched along the heads."""
+    heads = fs.shape[1]
+    hs = heads // parts
+    res = []
+    for q in range(parts):
+        sl = slice(q * hs, (q + 1) * hs)
+        fs_q, fd_q, g_q = (t[:, sl].contiguous() for t in (fs, fd, gout))
+        out, state = _gatv2_slab_forward(graph, etv, fs_q, fd_q, attn, theta, alpha, slope, sl, heads, dropout)
+        d_fs, d_fd, d_at, d_th = _gatv2_slab_backward(graph, etv, fs_q, fd_q, out, state, g_q, alpha, slope)
+        res.append((out, d_fs, d_fd, d_at.view(1, hs, -1), d_th))
+    stitched = [torch.cat([r[i] for r in res], dim=1) for i in range(4)]
+    return tuple(stitched) + (torch.cat([r[4] for r in res], dim=1) if res[0][4] is not None else None,)
 
 
 def allreduce_relation_grads(params, group=None, exchange=None):

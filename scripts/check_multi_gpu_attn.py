@@ -1,9 +1,11 @@
 """Multi-rank GPU check + timing of the sharded attention / REMixHop paths (run under torchrun, one rank per GPU):
-``partition.head_sliced_gat`` (REGAT core, heads = column slabs, NCCL all-to-all on each side) and
-``partition.feature_sliced_propagate(theta=None)`` (REMixHop's un-weighted propagation over column slabs) against the
-single-device ``functional.gat_layer`` / ``functional.propagate`` on every rank: outputs and feature gradients on the
-rank's row block, parameter gradients after ``allreduce_relation_grads``.  Then the step is timed (CUDA events, max
-over ranks) next to the single-device step on the same graph.
+``partition.head_sliced_gat`` (REGAT core, heads = column slabs), ``partition.head_sliced_gatv2`` (REGATv2 core, the
+same over fs and fd) and ``partition.feature_sliced_propagate(theta=None)`` (REMixHop's un-weighted propagation over
+column slabs), each with the NCCL all-to-all and the peer-memory exchange, against the single-device
+``functional.gat_layer`` / ``functional.gatv2_aggregate`` / ``functional.propagate`` on every rank: outputs and feature
+gradients on the rank's row block, parameter gradients after ``allreduce_relation_grads``.  Then the step is timed (CUDA
+events, max over ranks) next to the single-device step on the same graph; at world size 1 the difference is the cost of
+the exchange path itself.
 
     torchrun ... scripts/check_multi_gpu_attn.py [graph_scale=1.0] [heads=8] [dim=16] [iters=10]"""
 import json
@@ -57,6 +59,7 @@ def main():
     ar0 = torch.randn(1, heads, dim, device=dev, generator=gen) * 0.3
     th0 = (torch.rand(r, heads, device=dev, generator=gen) + 0.5) / 100
     thn0 = (torch.rand(r, 1, device=dev, generator=gen) + 0.5) / 100
+    fd0 = torch.randn(n, heads, dim, device=dev, generator=gen) * 0.5
     bounds = partition.row_blocks(g.csr()['indptr'], world, balance='rows')
     rb, re = bounds[rank], bounds[rank + 1]
     res = {'n_gpus': world, 'num_nodes': int(n), 'num_edges': int(e), 'heads': heads, 'head_dim': dim}
@@ -97,6 +100,45 @@ def main():
         del out, grads
         tp = timed(lambda: gat_sharded(ex), iters, dev)
         res['regat'][name] = {'check': chk, 'sharded_ms': tp, 'speedup': t1 / tp, 'gteps_sharded': e / tp / 1e6}
+    del ref_out, ref_g
+
+    # ---- REGATv2 core, heads sharded
+    def gatv2_single():
+        leaves = [t.clone().requires_grad_(True) for t in (f, fd0, al0, th0)]
+        out, _ = RF.gatv2_aggregate(g, etv, *leaves, 100.0, 0.2)
+        out.backward(gout)
+        return out.detach(), [t.grad for t in leaves]
+
+    xch2 = partition.SlabExchange(heads * dim, bounds, rank, dev, gatv2=True)
+
+    def gatv2_sharded(exchange=None):
+        mine = [t[rb:re].clone().requires_grad_(True) for t in (f, fd0)] + [t.clone().requires_grad_(True)
+                                                                            for t in (al0, th0)]
+        out = partition.head_sliced_gatv2(g, etv, *mine, 100.0, 0.2, bounds, rank, exchange=exchange)
+        out.backward(gout[rb:re])
+        partition.allreduce_relation_grads(mine[2:])
+        return out.detach(), [t.grad for t in mine]
+    ref_out, ref_g = gatv2_single()
+    t1 = timed(lambda: gatv2_single(), iters, dev)
+    res['regatv2'] = {'single_gpu_ms': t1}
+    for name, ex in (('nccl_all_to_all', None), ('peer_memory', xch2)):
+        for rep in range(2):   # twice: the exchange buffers are reused
+            out, grads = gatv2_sharded(ex)
+        chk = {'out_equal': bool(torch.equal(out, ref_out[rb:re])),
+               'd_fs_equal': bool(torch.equal(grads[0], ref_g[0][rb:re])),
+               'd_fd_equal': bool(torch.equal(grads[1], ref_g[1][rb:re])),
+               'out_rel': rel(out, ref_out[rb:re]), 'd_fs_rel': rel(grads[0], ref_g[0][rb:re]),
+               'd_fd_rel': rel(grads[1], ref_g[1][rb:re]), 'd_attn_rel': rel(grads[2], ref_g[2]),
+               'd_theta_rel': rel(grads[3], ref_g[3])}
+        ok = (max(chk['out_rel'], chk['d_fs_rel'], chk['d_fd_rel']) < 1e-5 and
+              max(chk['d_attn_rel'], chk['d_theta_rel']) < 5e-5)
+        flag = torch.tensor([int(ok)], device=dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN)
+        ok_all = ok_all and bool(flag.item())
+        chk['all_ranks_ok'] = bool(flag.item())
+        del out, grads
+        tp = timed(lambda: gatv2_sharded(ex), iters, dev)
+        res['regatv2'][name] = {'check': chk, 'sharded_ms': tp, 'speedup': t1 / tp, 'gteps_sharded': e / tp / 1e6}
     del ref_out, ref_g
 
     # ---- REMixHop propagation: relation weights enter through the norm only, un-weighted column slabs
