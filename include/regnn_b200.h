@@ -437,6 +437,56 @@ int regnn_gatv2_bwd_dst(const int32_t* indptr, const uint8_t* etype_csr, const f
 int regnn_sample_neighbors(const int32_t* indptr, const int64_t* targets, int64_t num_targets, int fanout,
                            uint64_t key, int32_t* out_slot, void* stream);
 
+/* One layer of the sampler with device-resident sizes: samples `fanout` in-edges of every target (the slots of
+ * regnn_sample_neighbors), relabels the frontier and compacts the sampled edges, with no host synchronisation.
+ *   targets     [max_targets] global ids; the first *num_targets are used (num_targets NULL: all of them) -- the
+ *               info[REGNN_SAMPLE_INFO_SOURCES] word of the previous layer, so layers chain on the device
+ *   new_n_id    [max_sources >= max_targets + min(num_nodes, max_targets * fanout)]: the targets in their order, then
+ *               every sampled source that is not a target, once, in ascending global id (torch.unique's order)
+ *   src_local / dst_local / edge_id  [max_targets * fanout]: sampled edge e (targets in order, each target's slots in
+ *               sample order) is new_n_id[src_local[e]] -> target dst_local[e], global edge id edge_id[e]
+ *   row_off     [max_targets + 1]: exclusive scan of the per-target edge counts (the in-CSR offsets of the block)
+ *   src_hist    [max_sources]: sampled out-edges per local source
+ *   info        [REGNN_SAMPLE_INFO_WORDS] int32, zeroed and filled here (layout below)
+ *   pos_map     [num_nodes] int32, every entry 0x7fffffff on entry; flags [num_nodes] uint32, all 0 on entry; both are
+ *               restored before the last kernel ends, so one pair serves every layer and batch of a sampler
+ * split_threshold: the long-row threshold of regnn_rowsplit_t the split statistics in info are counted for.
+ * workspace: regnn_sample_layer_workspace_bytes(num_nodes, max_targets, fanout) bytes. */
+enum {
+  REGNN_SAMPLE_INFO_SOURCES = 0,          /* number of sources of the block (= targets of the next layer)        */
+  REGNN_SAMPLE_INFO_EDGES = 1,            /* number of sampled edges                                             */
+  REGNN_SAMPLE_INFO_EMPTY_ROWS = 2,       /* targets without a sampled in-edge                                   */
+  REGNN_SAMPLE_INFO_IN_SPLIT = 3,         /* (long rows, fragments) of the in-view                               */
+  REGNN_SAMPLE_INFO_IN_SPLIT_LOOPS = 5,   /*   ... with one self loop per target appended                        */
+  REGNN_SAMPLE_INFO_OUT_SPLIT = 7,        /* (long rows, fragments) of the transposed view                       */
+  REGNN_SAMPLE_INFO_OUT_SPLIT_LOOPS = 9,  /*   ... with one self loop per target appended                        */
+  REGNN_SAMPLE_INFO_WORDS = 16
+};
+size_t regnn_sample_layer_workspace_bytes(int64_t num_nodes, int64_t max_targets, int fanout);
+int regnn_sample_layer(const int32_t* indptr, const int32_t* indices, const int32_t* eid, int64_t num_nodes,
+                       const int64_t* targets, int64_t max_targets, const int32_t* num_targets, int fanout,
+                       uint64_t key, int split_threshold, int32_t* pos_map, uint32_t* flags, int64_t* new_n_id,
+                       int64_t max_sources, int64_t* src_local, int64_t* dst_local, int64_t* edge_id,
+                       uint32_t* row_off, int32_t* src_hist, int32_t* info, void* workspace, size_t workspace_bytes,
+                       void* stream);
+
+/* Both CSR views of one sampled block, bit-identical to regnn_csr_build + regnn_etype_permute +
+ * regnn_relation_counts on the block's edge list src_local -> dst_local (+ one self loop per target when
+ * self_loops, edge id num_sampled + v, typed num_edge_types + node_type[targets[v]]), without a host
+ * synchronisation.  Inputs are regnn_sample_layer's outputs (sizes read back by the caller) and the 0-based global
+ * edge_type / node_type.  Outputs: src / dst / etype1 [num_edges] in edge-id order (etype1 1-based), the CSR arrays
+ * of regnn_csr_build over num_src nodes, et_csr / et_t of regnn_etype_permute, and counts [num_src * num_relations]
+ * (NULL: not built).  An edge whose type lies outside [0, num_relations) stores 1 to *status (device int32, left
+ * untouched otherwise: the caller zeroes it and reads it at its next synchronisation) and is typed 0 in et_csr / et_t /
+ * counts.  workspace: regnn_csr_build_workspace_bytes(num_src, num_edges). */
+int regnn_block_csr_build(const int64_t* src_local, const int64_t* dst_local, const int64_t* edge_id,
+                          const uint32_t* row_off, const int64_t* targets, int64_t num_src, int64_t num_dst,
+                          int64_t num_sampled, const int64_t* edge_type, const int64_t* node_type, int num_edge_types,
+                          int self_loops, int num_relations, int64_t* src, int64_t* dst, int64_t* etype1,
+                          int32_t* indptr, int32_t* indices, int32_t* eid, int32_t* row, int32_t* indptr_t,
+                          int32_t* indices_t, int32_t* slot_t, uint8_t* et_csr, uint8_t* et_t, int32_t* counts,
+                          int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
+
 /* GraphSAINT random-walk roots (replaces torch_sparse `random_walk` behind
  * `GraphSAINTRandomWalkSampler(data, batch_size=20000, walk_length=2, ...)`, mag/regnn_saint.py:185-190):
  * root i starts at node hash(key, i) % N and takes `walk_length` steps along out-edges of the transposed view;

@@ -45,6 +45,11 @@ SIGNATURES = {
     'regnn_rowdot_norm_bwd': (_i32, [_p, _i32, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _i32, _p, _p]),
     'regnn_random_walk': (_i32, [_p, _p, _i64, _i64, _i32, ctypes.c_uint64, _p, _p]),
     'regnn_sample_neighbors': (_i32, [_p, _p, _i64, _i32, ctypes.c_uint64, _p, _p]),
+    'regnn_sample_layer_workspace_bytes': (_sz, [_i64, _i64, _i32]),
+    'regnn_sample_layer': (_i32, [_p, _p, _p, _i64, _p, _i64, _p, _i32, ctypes.c_uint64, _i32, _p, _p, _p, _i64, _p, _p,
+                                  _p, _p, _p, _p, _p, _sz, _p]),
+    'regnn_block_csr_build': (_i32, [_p, _p, _p, _p, _p, _i64, _i64, _i64, _p, _p, _i32, _i32, _i32, _p, _p, _p, _p, _p,
+                                     _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     'regnn_gat_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
                              _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gat_bwd_stats': (_i32, [_p, _p, _p, _p, _p, _i64, _i32, _i32, _p, _p]),

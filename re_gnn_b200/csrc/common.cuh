@@ -15,6 +15,13 @@ constexpr int kMaxPartialBlocks = 4736;  // 148 SMs x 32: cap on the grid of the
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);
 
+// csr_build.cu: device-wide exclusive scan (block_sums: ceil(n / 4096) + 1 entries; in == out is allowed) and the
+// source-sorted view of a destination-sorted CSR (workspace: regnn_csr_build_workspace_bytes(num_nodes, num_edges)).
+void exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uint32_t* block_sums, cudaStream_t stream);
+void build_transposed_view(const int32_t* indices, const int32_t* row, int64_t num_nodes, int64_t num_edges,
+                           int32_t* indptr_t, int32_t* indices_t, int32_t* slot_t, void* workspace,
+                           cudaStream_t stream);
+
 #define REGNN_REQUIRE(cond, code, ...)        \
   do {                                        \
     if (!(cond)) {                            \

@@ -91,8 +91,8 @@ __global__ void scan_apply_kernel(const uint32_t* __restrict__ in, int64_t n,
   }
 }
 
-static void exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uint32_t* block_sums,
-                               cudaStream_t stream) {
+void exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uint32_t* block_sums,
+                        cudaStream_t stream) {
   if (n <= 0) return;
   int64_t nb = (n + kScanTile - 1) / kScanTile;
   scan_reduce_kernel<<<(unsigned)nb, kScanThreads, 0, stream>>>(in, n, block_sums);
@@ -292,6 +292,20 @@ static SortBuffers carve(void* ws, int64_t n_edges) {
   return sb;
 }
 
+// Source-sorted view of a destination-sorted CSR: a stable sort of the CSR slots by their source id.
+void build_transposed_view(const int32_t* indices, const int32_t* row, int64_t num_nodes, int64_t num_edges,
+                           int32_t* indptr_t, int32_t* indices_t, int32_t* slot_t, void* workspace,
+                           cudaStream_t stream) {
+  SortBuffers sb = carve(workspace, num_edges);
+  const int T = 256;
+  const unsigned eb = (unsigned)((num_edges + T - 1) / T), ebp = (unsigned)((num_nodes + 1 + T - 1) / T);
+  uint32_t *keys, *vals;
+  if (num_edges > 0) init_keys32_kernel<<<eb, T, 0, stream>>>(indices, num_edges, sb.keys_a, sb.vals_a);
+  radix_sort_pairs(sb, num_edges, key_bits(num_nodes), &keys, &vals, stream);
+  boundary_fill_kernel<<<ebp, T, 0, stream>>>(keys, num_edges, num_nodes, indptr_t);
+  if (num_edges > 0) finish_csc_kernel<<<eb, T, 0, stream>>>(vals, row, num_edges, indices_t, slot_t);
+}
+
 }  // namespace regnn
 
 using namespace regnn;
@@ -328,14 +342,8 @@ extern "C" int regnn_csr_build(const int64_t* src, const int64_t* dst, int64_t n
     init_keys_kernel<<<eb, T, 0, stream>>>(dst, src, num_nodes, num_edges, sb.keys_a, sb.vals_a, sb.err);
   radix_sort_pairs(sb, num_edges, bits, &keys, &vals, stream);
   boundary_fill_kernel<<<ebp, T, 0, stream>>>(keys, num_edges, num_nodes, indptr);
-  if (num_edges > 0) {
-    finish_csr_kernel<<<eb, T, 0, stream>>>(keys, vals, src, num_edges, indices, eid, row);
-    // source-sorted view: stable sort of the CSR slots by their source id
-    init_keys32_kernel<<<eb, T, 0, stream>>>(indices, num_edges, sb.keys_a, sb.vals_a);
-  }
-  radix_sort_pairs(sb, num_edges, bits, &keys, &vals, stream);
-  boundary_fill_kernel<<<ebp, T, 0, stream>>>(keys, num_edges, num_nodes, indptr_t);
-  if (num_edges > 0) finish_csc_kernel<<<eb, T, 0, stream>>>(vals, row, num_edges, indices_t, slot_t);
+  if (num_edges > 0) finish_csr_kernel<<<eb, T, 0, stream>>>(keys, vals, src, num_edges, indices, eid, row);
+  build_transposed_view(indices, row, num_nodes, num_edges, indptr_t, indices_t, slot_t, workspace, stream);
 
   int rc = check_launch("regnn_csr_build");
   if (rc != REGNN_OK) return rc;

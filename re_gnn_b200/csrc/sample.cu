@@ -30,22 +30,23 @@ __host__ __device__ __forceinline__ uint32_t feistel_perm(uint32_t x, uint32_t d
   return y;
 }
 
+// The j-th sampled in-edge slot of node t, or -1 when j >= min(in-degree, fanout).
+__device__ __forceinline__ int32_t sampled_slot(const int32_t* __restrict__ indptr, int64_t t, uint32_t j, int fanout,
+                                                uint32_t key_lo, uint32_t key_hi) {
+  const int32_t s0 = indptr[t];
+  const uint32_t deg = (uint32_t)(indptr[t + 1] - s0);
+  if (j >= deg) return -1;
+  if (deg <= (uint32_t)fanout) return s0 + (int32_t)j;
+  return s0 + (int32_t)feistel_perm(j, deg, mix32(key_lo ^ mix32((uint32_t)t + key_hi)));
+}
+
 __global__ void sample_neighbors_kernel(const int32_t* __restrict__ indptr, const int64_t* __restrict__ targets,
                                         int64_t num_targets, int fanout, uint32_t key_lo, uint32_t key_hi,
                                         int32_t* __restrict__ out_slot) {
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (tid >= num_targets * fanout) return;
   const int64_t i = tid / fanout;
-  const uint32_t j = (uint32_t)(tid % fanout);
-  const int64_t t = targets[i];
-  const int32_t s0 = indptr[t];
-  const uint32_t deg = (uint32_t)(indptr[t + 1] - s0);
-  int32_t slot = -1;
-  if (j < deg) {
-    if (deg <= (uint32_t)fanout) slot = s0 + (int32_t)j;
-    else slot = s0 + (int32_t)feistel_perm(j, deg, mix32(key_lo ^ mix32((uint32_t)t + key_hi)));
-  }
-  out_slot[tid] = slot;
+  out_slot[tid] = sampled_slot(indptr, targets[i], (uint32_t)(tid % fanout), fanout, key_lo, key_hi);
 }
 
 }  // namespace regnn
@@ -95,4 +96,242 @@ extern "C" int regnn_random_walk(const int32_t* indptr_t, const int32_t* indices
   regnn::random_walk_kernel<<<(unsigned)((num_roots + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       indptr_t, indices_t, num_nodes, num_roots, walk_length, (uint32_t)(key & 0xffffffffu), (uint32_t)(key >> 32), walks);
   return regnn::check_launch("regnn_random_walk");
+}
+
+// ---- Device-built minibatch blocks -------------------------------------------------------------------------
+// One sampled layer without a host round trip (regnn_sample_layer), and the CSR views of one block straight from
+// it (regnn_block_csr_build).  Target i's valid slots are the first k_i = min(in-degree, fanout) of its fan-out row,
+// so the sampled edges, compacted in sample order, are the block's in-CSR already: row_off = exclusive scan of k_i.
+// Relabelling: targets store their position in a persistent [N] map, sampled sources that are not targets raise a
+// flag, and an exclusive scan of the flags in global-id order gives every new source its position -- new sources
+// in ascending global id, as torch.unique orders them.  Stores of equal values, integer counters and atomicMin
+// only: the result does not depend on the order in which threads run.
+namespace regnn {
+
+constexpr int32_t kUnmapped = 0x7fffffff;   // pos_map entry of a node that is not a target of the current layer
+
+__device__ __forceinline__ int64_t targets_of(const int32_t* num_targets, int64_t max_targets) {
+  return num_targets ? (int64_t)*num_targets : max_targets;
+}
+
+// Long-row statistics of the row split of a CSR view (graph.py: _row_split): rows with more than `threshold`
+// slots and the number of `threshold`-slot fragments they are cut into.
+__device__ __forceinline__ void count_long_row(int64_t deg, int threshold, int32_t* stats) {
+  if (deg > threshold) {
+    atomicAdd(stats, 1);
+    atomicAdd(stats + 1, (int32_t)((deg + threshold - 1) / threshold));
+  }
+}
+
+__global__ void frontier_rows_kernel(const int32_t* __restrict__ indptr, const int64_t* __restrict__ targets,
+                                     int64_t max_targets, const int32_t* __restrict__ num_targets, int fanout,
+                                     int threshold, int32_t* __restrict__ pos_map, int64_t* __restrict__ new_n_id,
+                                     uint32_t* __restrict__ row_off, int32_t* __restrict__ info) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i > max_targets) return;
+  const int64_t t = targets_of(num_targets, max_targets);
+  uint32_t k = 0;
+  if (i < t) {
+    const int64_t v = targets[i];
+    atomicMin(&pos_map[v], (int32_t)i);     // a repeated target keeps its first position
+    new_n_id[i] = v;
+    k = (uint32_t)min(indptr[v + 1] - indptr[v], fanout);
+    if (k == 0) atomicAdd(&info[REGNN_SAMPLE_INFO_EMPTY_ROWS], 1);
+    count_long_row(k, threshold, info + REGNN_SAMPLE_INFO_IN_SPLIT);
+    count_long_row(k + 1, threshold, info + REGNN_SAMPLE_INFO_IN_SPLIT_LOOPS);
+  }
+  row_off[i] = k;     // scanned in place afterwards; entry max_targets becomes the number of sampled edges
+}
+
+__global__ void frontier_slots_kernel(const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                                      const int32_t* __restrict__ eid, const int64_t* __restrict__ targets,
+                                      int64_t max_targets, const int32_t* __restrict__ num_targets, int fanout,
+                                      uint32_t key_lo, uint32_t key_hi, const uint32_t* __restrict__ row_off,
+                                      const int32_t* __restrict__ pos_map, uint32_t* __restrict__ flags,
+                                      int32_t* __restrict__ src_global, int64_t* __restrict__ dst_local,
+                                      int64_t* __restrict__ edge_id) {
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t i = tid / fanout;
+  if (i >= targets_of(num_targets, max_targets)) return;
+  const uint32_t j = (uint32_t)(tid % fanout), e0 = row_off[i];
+  if (j >= row_off[i + 1] - e0) return;
+  const int32_t slot = sampled_slot(indptr, targets[i], j, fanout, key_lo, key_hi);
+  const int64_t e = (int64_t)e0 + j;
+  const int32_t u = indices[slot];
+  src_global[e] = u;
+  dst_local[e] = i;
+  edge_id[e] = eid[slot];
+  if (pos_map[u] == kUnmapped) flags[u] = 1u;
+}
+
+__global__ void frontier_relabel_kernel(int64_t max_targets, const int32_t* __restrict__ num_targets,
+                                        const uint32_t* __restrict__ row_off, int64_t num_nodes,
+                                        const int32_t* __restrict__ src_global, const int32_t* __restrict__ pos_map,
+                                        const uint32_t* __restrict__ flags, const uint32_t* __restrict__ excl,
+                                        int64_t* __restrict__ new_n_id, int64_t* __restrict__ src_local,
+                                        int32_t* __restrict__ src_hist, int32_t* __restrict__ info) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t t = targets_of(num_targets, max_targets);
+  const int64_t num_edges = row_off[max_targets];
+  if (e == 0) {
+    info[REGNN_SAMPLE_INFO_SOURCES] = (int32_t)(t + excl[num_nodes - 1] + flags[num_nodes - 1]);
+    info[REGNN_SAMPLE_INFO_EDGES] = (int32_t)num_edges;
+  }
+  if (e >= num_edges) return;
+  const int32_t u = src_global[e];
+  int64_t p = pos_map[u];
+  if (p == kUnmapped) {
+    p = t + excl[u];
+    new_n_id[p] = u;
+  }
+  src_local[e] = p;
+  atomicAdd(&src_hist[p], 1);
+}
+
+// Restores pos_map / flags for the next layer and counts the long rows of the block's transposed view.
+__global__ void frontier_finish_kernel(int64_t max_sources, int64_t max_targets, const int32_t* __restrict__ num_targets,
+                                       const int64_t* __restrict__ new_n_id, const int32_t* __restrict__ src_hist,
+                                       int threshold, int32_t* __restrict__ pos_map, uint32_t* __restrict__ flags,
+                                       int32_t* __restrict__ info) {
+  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= max_sources || v >= info[REGNN_SAMPLE_INFO_SOURCES]) return;
+  const int64_t t = targets_of(num_targets, max_targets);
+  const int64_t u = new_n_id[v];
+  if (v < t) pos_map[u] = kUnmapped;
+  else flags[u] = 0u;
+  const int32_t d = src_hist[v];
+  count_long_row(d, threshold, info + REGNN_SAMPLE_INFO_OUT_SPLIT);
+  count_long_row(d + (v < t ? 1 : 0), threshold, info + REGNN_SAMPLE_INFO_OUT_SPLIT_LOOPS);
+}
+
+__global__ void block_csr_fill_kernel(const int64_t* __restrict__ src_local, const int64_t* __restrict__ dst_local,
+                                      const int64_t* __restrict__ edge_id, const uint32_t* __restrict__ row_off,
+                                      const int64_t* __restrict__ targets, int64_t num_src, int64_t num_dst,
+                                      int64_t num_sampled, const int64_t* __restrict__ edge_type,
+                                      const int64_t* __restrict__ node_type, int num_edge_types, int loops,
+                                      int64_t* __restrict__ src, int64_t* __restrict__ dst, int64_t* __restrict__ etype1,
+                                      int32_t* __restrict__ indptr, int32_t* __restrict__ indices,
+                                      int32_t* __restrict__ eid, int32_t* __restrict__ row,
+                                      uint8_t* __restrict__ et_csr, int num_relations, int32_t* __restrict__ status) {
+  const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (x <= num_src) indptr[x] = (int32_t)(x <= num_dst ? row_off[x] + loops * x : num_sampled + loops * num_dst);
+  if (x >= num_sampled + loops * num_dst) return;
+  int64_t u, v, s, ty;
+  if (x < num_sampled) {           // sampled edge x of row v: slot x + v when every earlier row ends in its loop
+    u = src_local[x];
+    v = dst_local[x];
+    s = x + loops * v;
+    ty = edge_type[edge_id[x]];
+  } else {                         // typed self loop of target v (edge id num_sampled + v): the last slot of row v
+    v = x - num_sampled;
+    u = v;
+    s = (int64_t)row_off[v + 1] + v;
+    ty = node_type[targets[v]] + num_edge_types;
+  }
+  src[x] = u;
+  dst[x] = v;
+  etype1[x] = ty + 1;
+  if (ty < 0 || ty >= num_relations) {   // reported through *status; slot typed 0 so no table is indexed out of range
+    *status = 1;
+    ty = 0;
+  }
+  indices[s] = (int32_t)u;
+  eid[s] = (int32_t)x;
+  row[s] = (int32_t)v;
+  et_csr[s] = (uint8_t)ty;
+}
+
+__global__ void etype_transpose_kernel(const uint8_t* __restrict__ et_csr, const int32_t* __restrict__ slot_t,
+                                       int64_t n, uint8_t* __restrict__ et_t) {
+  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n) et_t[j] = et_csr[slot_t[j]];
+}
+
+static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+static int64_t scan_blocks(int64_t n) { return (n + 4095) / 4096 + 1; }
+static unsigned grid_of(int64_t n) { return (unsigned)((n > 0 ? n + 255 : 256) / 256); }
+
+}  // namespace regnn
+
+extern "C" size_t regnn_sample_layer_workspace_bytes(int64_t num_nodes, int64_t max_targets, int fanout) {
+  const int64_t slots = max_targets * fanout, nb = scan_blocks(num_nodes > max_targets ? num_nodes : max_targets + 1);
+  return align256((size_t)(slots > 0 ? slots : 1) * 4) + align256((size_t)(num_nodes > 0 ? num_nodes : 1) * 4) +
+         align256((size_t)nb * 4);
+}
+
+extern "C" int regnn_sample_layer(const int32_t* indptr, const int32_t* indices, const int32_t* eid, int64_t num_nodes,
+                                  const int64_t* targets, int64_t max_targets, const int32_t* num_targets, int fanout,
+                                  uint64_t key, int split_threshold, int32_t* pos_map, uint32_t* flags,
+                                  int64_t* new_n_id, int64_t max_sources, int64_t* src_local, int64_t* dst_local,
+                                  int64_t* edge_id, uint32_t* row_off, int32_t* src_hist, int32_t* info,
+                                  void* workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  REGNN_REQUIRE(indptr && indices && eid && pos_map && flags && new_n_id && src_local && dst_local && edge_id &&
+                row_off && src_hist && info && workspace && (max_targets == 0 || targets),
+                REGNN_ERR_INVALID_ARG, "sample_layer: null pointer");
+  REGNN_REQUIRE(num_nodes >= 1 && num_nodes < ((int64_t)1 << 31) - 1 && max_targets >= 0 && fanout >= 1 &&
+                split_threshold >= 1, REGNN_ERR_INVALID_ARG, "sample_layer: bad sizes");
+  const int64_t slots = max_targets * fanout;
+  REGNN_REQUIRE(slots < ((int64_t)1 << 31) - 1, REGNN_ERR_UNSUPPORTED_SHAPE, "sample_layer: %lld slots exceed int32",
+                (long long)slots);
+  REGNN_REQUIRE(max_sources >= max_targets + (slots < num_nodes ? slots : num_nodes), REGNN_ERR_INVALID_ARG,
+                "sample_layer: max_sources=%lld below max_targets + min(num_nodes, max_targets * fanout)",
+                (long long)max_sources);
+  REGNN_REQUIRE(workspace_bytes >= regnn_sample_layer_workspace_bytes(num_nodes, max_targets, fanout),
+                REGNN_ERR_WORKSPACE_TOO_SMALL, "sample_layer workspace too small");
+  char* p = (char*)workspace;
+  int32_t* src_global = (int32_t*)p;
+  p += align256((size_t)(slots > 0 ? slots : 1) * 4);
+  uint32_t* excl = (uint32_t*)p;
+  p += align256((size_t)num_nodes * 4);
+  uint32_t* block_sums = (uint32_t*)p;
+  const uint32_t key_lo = (uint32_t)(key & 0xffffffffu), key_hi = (uint32_t)(key >> 32);
+
+  cudaMemsetAsync(info, 0, REGNN_SAMPLE_INFO_WORDS * sizeof(int32_t), stream);
+  cudaMemsetAsync(src_hist, 0, (size_t)(max_sources > 0 ? max_sources : 1) * sizeof(int32_t), stream);
+  frontier_rows_kernel<<<grid_of(max_targets + 1), 256, 0, stream>>>(indptr, targets, max_targets, num_targets, fanout,
+                                                                     split_threshold, pos_map, new_n_id, row_off, info);
+  exclusive_scan_u32(row_off, row_off, max_targets + 1, block_sums, stream);
+  frontier_slots_kernel<<<grid_of(slots), 256, 0, stream>>>(indptr, indices, eid, targets, max_targets, num_targets,
+                                                            fanout, key_lo, key_hi, row_off, pos_map, flags, src_global,
+                                                            dst_local, edge_id);
+  exclusive_scan_u32(flags, excl, num_nodes, block_sums, stream);
+  frontier_relabel_kernel<<<grid_of(slots), 256, 0, stream>>>(max_targets, num_targets, row_off, num_nodes, src_global,
+                                                              pos_map, flags, excl, new_n_id, src_local, src_hist, info);
+  frontier_finish_kernel<<<grid_of(max_sources), 256, 0, stream>>>(max_sources, max_targets, num_targets, new_n_id,
+                                                                   src_hist, split_threshold, pos_map, flags, info);
+  return check_launch("regnn_sample_layer");
+}
+
+extern "C" int regnn_block_csr_build(const int64_t* src_local, const int64_t* dst_local, const int64_t* edge_id,
+                                     const uint32_t* row_off, const int64_t* targets, int64_t num_src, int64_t num_dst,
+                                     int64_t num_sampled, const int64_t* edge_type, const int64_t* node_type,
+                                     int num_edge_types, int self_loops, int num_relations, int64_t* src, int64_t* dst,
+                                     int64_t* etype1, int32_t* indptr, int32_t* indices, int32_t* eid, int32_t* row,
+                                     int32_t* indptr_t, int32_t* indices_t, int32_t* slot_t, uint8_t* et_csr,
+                                     uint8_t* et_t, int32_t* counts, int32_t* status, void* workspace,
+                                     size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const int loops = self_loops ? 1 : 0;
+  const int64_t num_edges = num_sampled + loops * num_dst;
+  REGNN_REQUIRE(num_dst >= 0 && num_src >= num_dst && num_sampled >= 0, REGNN_ERR_INVALID_ARG,
+                "block_csr_build: bad sizes");
+  REGNN_REQUIRE(num_src < ((int64_t)1 << 31) - 1 && num_edges < ((int64_t)1 << 31) - 1, REGNN_ERR_UNSUPPORTED_SHAPE,
+                "block_csr_build: block exceeds int32 indexing");
+  REGNN_REQUIRE(num_relations >= 1 && num_relations <= REGNN_MAX_RELATIONS, REGNN_ERR_UNSUPPORTED_SHAPE,
+                "num_relations=%d outside [1, %d]", num_relations, REGNN_MAX_RELATIONS);
+  REGNN_REQUIRE(row_off && indptr && indptr_t && workspace && (num_sampled == 0 || (src_local && dst_local && edge_id &&
+                edge_type)) && status && (num_edges == 0 || (src && dst && etype1 && indices && eid && row && indices_t &&
+                slot_t && et_csr && et_t)) && (!loops || num_dst == 0 || (targets && node_type)),
+                REGNN_ERR_INVALID_ARG, "block_csr_build: null pointer");
+  REGNN_REQUIRE(workspace_bytes >= regnn_csr_build_workspace_bytes(num_src, num_edges), REGNN_ERR_WORKSPACE_TOO_SMALL,
+                "block_csr_build workspace too small");
+  block_csr_fill_kernel<<<grid_of((num_edges > num_src ? num_edges : num_src + 1)), 256, 0, stream>>>(
+      src_local, dst_local, edge_id, row_off, targets, num_src, num_dst, num_sampled, edge_type, node_type,
+      num_edge_types, loops, src, dst, etype1, indptr, indices, eid, row, et_csr, num_relations, status);
+  build_transposed_view(indices, row, num_src, num_edges, indptr_t, indices_t, slot_t, workspace, stream);
+  if (num_edges > 0) etype_transpose_kernel<<<grid_of(num_edges), 256, 0, stream>>>(et_csr, slot_t, num_edges, et_t);
+  int rc = check_launch("regnn_block_csr_build");
+  if (rc != REGNN_OK || counts == nullptr) return rc;
+  return regnn_relation_counts(row, et_csr, num_edges, num_src, num_relations, counts, stream);
 }

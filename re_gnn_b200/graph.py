@@ -38,19 +38,25 @@ SPLIT_THRESHOLD = 256   # rows with more slots are cut into fragments of this ma
 COUNTS_MAX_BYTES = 4 << 30   # build the [N,R] relation-count table only while it stays below this size
 
 
-def _row_split(indptr, threshold):
+def _row_split(indptr, threshold, sizes=None):
     """Long-row decomposition of one CSR view (``regnn_rowsplit_t``): index bookkeeping with torch ops on the
-    device, once per graph.  Returns None when no row exceeds the threshold."""
+    device, once per graph.  Returns None when no row exceeds the threshold.  ``sizes``: (long rows, fragments)
+    when the caller already knows them, which keeps the host from waiting for the device."""
     deg = (indptr[1:] - indptr[:-1]).to(torch.int64)
-    long_rows = torch.nonzero(deg > threshold).view(-1)
-    if long_rows.numel() == 0:
-        return None
+    if sizes is not None:
+        if sizes[0] == 0:
+            return None
+        long_rows = torch.nonzero_static(deg > threshold, size=int(sizes[0])).view(-1)
+    else:
+        long_rows = torch.nonzero(deg > threshold).view(-1)
+        if long_rows.numel() == 0:
+            return None
     nfr = (deg[long_rows] + threshold - 1) // threshold
     frag_ptr = torch.zeros(long_rows.numel() + 1, dtype=torch.int64, device=indptr.device)
     frag_ptr[1:] = torch.cumsum(nfr, 0)
-    total = int(frag_ptr[-1].item())
-    frag_row = torch.repeat_interleave(long_rows, nfr)
-    within = torch.arange(total, device=indptr.device) - torch.repeat_interleave(frag_ptr[:-1], nfr)
+    total = int(frag_ptr[-1].item()) if sizes is None else int(sizes[1])
+    frag_row = torch.repeat_interleave(long_rows, nfr, output_size=total)
+    within = torch.arange(total, device=indptr.device) - torch.repeat_interleave(frag_ptr[:-1], nfr, output_size=total)
     frag_begin = indptr.to(torch.int64)[frag_row] + within * threshold
     t = dict(long_rows=long_rows.to(torch.int32), frag_ptr=frag_ptr.to(torch.int32),
              frag_row=frag_row.to(torch.int32), frag_begin=frag_begin.to(torch.int32))
@@ -79,6 +85,20 @@ class Graph:
         self._csr = None
         self._etype_cache = {}
         self._zero_in_degree = None
+
+    @classmethod
+    def from_csr(cls, src, dst, num_nodes, csr, etype_views=None, has_zero_in_degree=None):
+        """A graph whose device structures are already built (``NeighborSampler`` blocks): ``src`` / ``dst`` in
+        edge-id order, ``csr`` the dict ``csr()`` returns (``split`` / ``split_t`` included), ``etype_views`` an
+        optional ``(e_feat, num_relations, et_csr, et_t, counts)`` entry of the ``etype_views`` cache and
+        ``has_zero_in_degree`` the answer when it is known on the host."""
+        g = cls(src, dst, num_nodes)
+        g._csr = csr
+        g._zero_in_degree = has_zero_in_degree
+        if etype_views is not None:
+            e_feat, num_relations, et_csr, et_t, counts = etype_views
+            g._etype_cache[g._etype_key(e_feat, num_relations)] = (et_csr, et_t, counts, e_feat)
+        return g
 
     # ---- DGLGraph surface ---------------------------------------------------------------------
     @classmethod
@@ -162,11 +182,15 @@ class Graph:
         self._csr = out
         return out
 
+    @staticmethod
+    def _etype_key(e_feat, num_relations):
+        return (e_feat.data_ptr(), e_feat._version, int(e_feat.numel()), int(num_relations))
+
     def etype_views(self, e_feat, num_relations):
         """uint8 0-based edge types in CSR-slot order and transposed-entry order for the reference's
         1-based int64 ``e_feat`` (edge-id order).  Cached per tensor (data_ptr, version); a cached entry holds a
         reference to the tensor, so the key cannot be recycled by the allocator while the entry lives."""
-        key = (e_feat.data_ptr(), e_feat._version, int(e_feat.numel()), int(num_relations))
+        key = self._etype_key(e_feat, num_relations)
         hit = self._etype_cache.get(key)
         if hit is not None:
             return hit[:3]

@@ -261,12 +261,24 @@ class REGNN(nn.Module):
             node_type, local_node_idx = node_type[n_id], local_node_idx[n_id]
         return _grouped_input(self.lins, x_dict, node_type, local_node_idx)
 
-    def forward(self, n_id, x_dict, adjs, edge_type, node_type, local_node_idx):
+    def prebuilt_blocks(self, blocks, edge_type, node_type):
+        """The ``(Graph, etype1)`` of every device-sampled block (``sampling.Block.prebuilt``) for these convolutions,
+        for ``forward(..., blocks=...)``."""
+        conv = self.convs[0]
+        return [b.prebuilt(edge_type, node_type, self.num_edge_types, conv.self_loop_type, conv.relation_weight.shape[0])
+                for b in blocks]
+
+    def forward(self, n_id, x_dict, adjs, edge_type, node_type, local_node_idx, blocks=None):
+        """``blocks``: optional ``prebuilt_blocks`` of the batch, passed to the convolutions instead of building each
+        block's graph from ``adjs``."""
         x = self.group_input(x_dict, node_type, local_node_idx, n_id)
         node_type = node_type[n_id]
         for i, (edge_index, e_id, size) in enumerate(adjs):
             x_target, node_type = x[:size[1]], node_type[:size[1]]
-            x = self.convs[i]((x, x_target), edge_index, edge_type[e_id], node_type)
+            if blocks is None:
+                x = self.convs[i]((x, x_target), edge_index, edge_type[e_id], node_type)
+            else:
+                x = self.convs[i]((x, x_target), edge_index, None, node_type, block=blocks[i])
             x = F.dropout(F.relu(x), p=self.dropout, training=self.training)
         return self.out_lin(x).log_softmax(dim=-1)
 
@@ -303,12 +315,14 @@ def allreduce_gradients(params, world_size, group=None):
 
 def train_step(model, optimizer, sampler, seeds, labels, x_dict, edge_type, node_type, local_node_idx, epoch, batch,
                world_size=1):
-    """One sampled-minibatch training step (mag/regnn_ns.py:399-407 + gradient all-reduce).
+    """One sampled-minibatch training step (mag/regnn_ns.py:399-407 + gradient all-reduce).  A batch sampled on a
+    CUDA device reaches the convolutions with its graphs prebuilt from the sample.
     Returns (loss tensor, number of sampled edges)."""
     n_id, blocks = sampler.sample(seeds, epoch=epoch, batch=batch)
     adjs = [(b.edge_index, b.eid, b.size) for b in blocks]
+    prebuilt = model.prebuilt_blocks(blocks, edge_type, node_type) if n_id.is_cuda else None
     optimizer.zero_grad(set_to_none=True)
-    out = model(n_id, x_dict, adjs, edge_type, node_type, local_node_idx)
+    out = model(n_id, x_dict, adjs, edge_type, node_type, local_node_idx, blocks=prebuilt)
     loss = F.nll_loss(out, labels)
     loss.backward()
     allreduce_gradients(list(model.parameters()), world_size)
