@@ -1295,7 +1295,7 @@ static bool pick_shape(int F, bool vec_ok, Shape* s) {
   }
 #define REGNN_DISPATCH_SHAPES(CALL)                                                            \
   REGNN_DISPATCH_GC(4, 1, 4, CALL) REGNN_DISPATCH_GC(8, 1, 4, CALL) REGNN_DISPATCH_GC(16, 1, 4, CALL) \
-  REGNN_DISPATCH_GC(16, 2, 4, CALL) REGNN_DISPATCH_GC(16, 3, 4, CALL)                          \
+  REGNN_DISPATCH_GC(16, 3, 4, CALL)                                                            \
   REGNN_DISPATCH_GC(32, 1, 4, CALL) REGNN_DISPATCH_GC(32, 2, 4, CALL) REGNN_DISPATCH_GC(32, 3, 4, CALL) \
   REGNN_DISPATCH_GC(32, 4, 4, CALL) REGNN_DISPATCH_GC(32, 8, 4, CALL)                          \
   REGNN_DISPATCH_GC(4, 1, 1, CALL) REGNN_DISPATCH_GC(8, 1, 1, CALL) REGNN_DISPATCH_GC(16, 1, 1, CALL) \
@@ -1496,7 +1496,8 @@ static int spmm_fwd_impl(const int32_t* indptr, const int32_t* indices, const ui
   if (rows == 0) return REGNN_OK;
   StreamShape sh;
   REGNN_REQUIRE(pick_stream_shape(feat, common_align({X, Y, split_workspace}, {ldx, ldy, (int64_t)feat}), &sh),
-                REGNN_ERR_UNSUPPORTED_SHAPE, "spmm_fwd: feature width %d too wide (max 1024 aligned / 256 unaligned)", feat);
+                REGNN_ERR_UNSUPPORTED_SHAPE, "spmm_fwd: feature width %d too wide (max 1024 with 16-byte, 512 with 8-byte, 256 with 4-byte "
+                "aligned operands)", feat);
   StreamArgs sa{};
   sa.s = SpmmArgs{indptr, indices, etype, theta, alpha, num_relations, norm_src, norm_dst, X, ldx, Y, ldy,
                   row_begin, row_end, feat, nullptr, nullptr, 0, 0, 0x7fffffff, nullptr};

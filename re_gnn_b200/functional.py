@@ -71,7 +71,7 @@ class _Propagate(torch.autograd.Function):
         dx = d_theta = d_norm = xdx = None
         if need_theta and ops.fused_bwd_fits(x.shape[1], theta.numel()):
             # one gather pass over the transposed view: dX, the relation gradient and the norm gradient together
-            fold = need_norm and ops.fused_dnorm_fits(x.shape[1]) and x.data_ptr() % 16 == 0 and y.data_ptr() % 16 == 0
+            fold = need_norm and ops.fused_dnorm_fits(x.shape[1], x, g, y)
             dx, d_theta, extra = ops.spmm_bwd_fused(csr, ctx.etv[1], theta, ctx.alpha, norm, x, g, sides=ctx.sides,
                                                     want_xdx=need_norm and not fold and bool(ctx.sides & 1),
                                                     y=y if fold else None, want_dnorm=fold)

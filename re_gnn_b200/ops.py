@@ -170,9 +170,13 @@ def spmm_bwd_fused(csr, et_t, theta, alpha, norm, x, g, rows=None, sides=3, out=
     return out, d_theta, (d_norm if want_dnorm else xdx)
 
 
-def fused_dnorm_fits(feat, rows_full=True):
-    """True when regnn_spmm_bwd_fused can also produce d_norm (lane-group kernel: F <= NARROW_FEAT, F % 4 == 0)."""
-    return rows_full and feat <= NARROW_FEAT and feat % 4 == 0
+def fused_dnorm_fits(feat, *operands, rows_full=True):
+    """True when regnn_spmm_bwd_fused can also produce d_norm (lane-group kernel: F <= NARROW_FEAT, F % 4 == 0, and
+    16-byte aligned rows in every operand).  ``operands``: the tensors the call will get -- X, G, Y and the dX output
+    when the caller supplies one (None entries are skipped).  One misaligned operand rules the lane-group kernel out,
+    and the library then refuses d_norm; autograd does hand out such gradients (a narrow view of a ``cat`` gradient)."""
+    return rows_full and feat <= NARROW_FEAT and feat % 4 == 0 and all(
+        t is None or (t.data_ptr() % 16 == 0 and t.stride(0) % 4 == 0) for t in operands)
 
 
 SMEM_BUDGET = 227 * 1024   # dynamic shared memory one block can opt in to on sm_100a

@@ -889,7 +889,7 @@ def _halo_backward(part, x_own, y_own, g_ext, theta, alpha, weighted, deg, norm)
     norm_own = norm[:n_own]
     d_theta = None
     if weighted:
-        fold = ops.fused_dnorm_fits(f)
+        fold = ops.fused_dnorm_fits(f, x_own, g_ext, y_own)
         dx_own, d_theta, extra = ops.spmm_bwd_fused(csr, part.et_out, theta, alpha, norm_out, x_own, g_ext,
                                                     want_xdx=not fold, y=y_own if fold else None, want_dnorm=fold)
         d_norm = extra if fold else ops.rowdot_norm_bwd(norm_own, x_own, y_own, g_own, dx_own, xdx=extra)

@@ -132,3 +132,33 @@ def test_halo_propagate_world1_nccl(weighted):
             assert _rel(th.grad, rdth) < 1e-6
     finally:
         dist.destroy_process_group()
+
+
+def test_halo_propagate_misaligned_rows_world1():
+    """x_own 4 bytes past 16-byte alignment (a contiguous view the caller owns): the folded norm gradient cannot run,
+    the backward takes the xdx + row-dot path; Y and dX equal functional.propagate bit for bit."""
+    import torch.distributed as dist
+    if not dist.is_initialized():
+        os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
+        os.environ.setdefault('MASTER_PORT', str(29400 + os.getpid() % 400))
+        dist.init_process_group('nccl', rank=0, world_size=1, device_id=torch.device(DEV))
+    try:
+        d = synth.hetero_graph_local('acm', 1, 0.9, seed=4, scale=0.2)
+        g, etv = _setup(d)
+        n, f = d['num_nodes'], 64
+        gen = torch.Generator(device=DEV).manual_seed(9)
+        x = torch.randn(n, f, device=DEV, generator=gen)
+        gout = torch.randn(n, f, device=DEV, generator=gen)
+        theta = (torch.rand(d['num_relations'], 1, device=DEV, generator=gen) + 0.5) / 100
+        ry, rdx, rdth = _single(g, etv, x, gout, theta, True)
+        part = partition.HaloPartition(g, etv, d['community_bounds'], 0)
+        buf = torch.empty(n * f + 1, device=DEV)
+        xs = buf[1:].view(n, f).copy_(x).requires_grad_(True)
+        assert xs.is_contiguous() and xs.data_ptr() % 16 == 4
+        th = theta.clone().requires_grad_(True)
+        out = partition.halo_propagate(part, xs, th, 100.0)
+        out.backward(gout)
+        assert torch.equal(out.detach(), ry) and torch.equal(xs.grad, rdx)
+        assert _rel(th.grad, rdth) < 1e-6
+    finally:
+        dist.destroy_process_group()
