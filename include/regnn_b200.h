@@ -494,6 +494,42 @@ int regnn_block_csr_build(const int64_t* src_local, const int64_t* dst_local, co
 int regnn_random_walk(const int32_t* indptr_t, const int32_t* indices_t, int64_t num_nodes, int64_t num_roots,
                       int walk_length, uint64_t key, int64_t* walks, void* stream);
 
+/* GraphSAINT subgraph induced by the walk nodes (replaces the relabelling and edge selection of
+ * `GraphSAINTRandomWalkSampler`, mag/regnn_saint.py:185-190), in two calls with one small host read between them: the
+ * host learns the induced edge count from info to size the edge arrays.  No host synchronisation inside either call;
+ * the result does not depend on the order in which threads run.
+ *   indptr / indices / eid  the graph's destination-sorted CSR over num_nodes nodes and num_edges slots
+ *   nodes       [num_listed] int64 node ids, repeats allowed (the flattened walks of regnn_random_walk); ids outside
+ *               [0, num_nodes) are ignored.  max_rows = min(num_nodes, num_listed)
+ *   flags       [num_nodes] uint32, all 0 on entry to count; count sets the listed nodes' flags and fill clears them
+ *               again, so one map serves every batch of a sampler
+ * regnn_induced_subgraph_count:
+ *   n_id        [max_rows]: the distinct listed nodes in ascending global id (torch.unique's order); the first
+ *               info[REGNN_SAMPLE_INFO_SOURCES] = n_sub entries are written
+ *   row_off     [max_rows + 1] uint32: in-CSR offsets of the subgraph (entries past n_sub hold the edge count), the
+ *               row_off regnn_block_csr_build reads
+ *   src_hist    [max_rows] int32: induced out-edges per subgraph node
+ *   info        [REGNN_SAMPLE_INFO_WORDS] int32, zeroed and filled here: SOURCES = n_sub, EDGES = induced edges E_sub,
+ *               EMPTY_ROWS, IN_SPLIT from the row lengths, OUT_SPLIT from src_hist; the *_LOOPS words stay 0 (the
+ *               subgraph has no self loops of its own)
+ * regnn_induced_subgraph_fill (num_rows = n_sub and num_sub_edges = E_sub, read back from info):
+ *   src_local / dst_local / edge_id  [num_sub_edges] int64: induced edge e is n_id[src_local[e]] -> n_id[dst_local[e]]
+ *               with global edge id edge_id[e], in (destination row, CSR slot) order -- its slot in the subgraph's
+ *               in-CSR is e
+ * Both calls take the same graph, num_listed and workspace, and the workspace (the flag scan and the table of 256-slot
+ * row fragments, max_rows + ceil(num_edges / 256) entries) must be left untouched between them:
+ * regnn_induced_subgraph_workspace_bytes(num_nodes, num_edges, num_listed) bytes.  Node ids and num_edges (hence E_sub)
+ * must stay below 2^31 - 1. */
+size_t regnn_induced_subgraph_workspace_bytes(int64_t num_nodes, int64_t num_edges, int64_t num_listed);
+int regnn_induced_subgraph_count(const int32_t* indptr, const int32_t* indices, int64_t num_nodes, int64_t num_edges,
+                                 const int64_t* nodes, int64_t num_listed, int split_threshold, uint32_t* flags,
+                                 int64_t* n_id, uint32_t* row_off, int32_t* src_hist, int32_t* info, void* workspace,
+                                 size_t workspace_bytes, void* stream);
+int regnn_induced_subgraph_fill(const int32_t* indptr, const int32_t* indices, const int32_t* eid, int64_t num_nodes,
+                                int64_t num_edges, int64_t num_listed, uint32_t* flags, const int64_t* n_id,
+                                int64_t num_rows, int64_t num_sub_edges, int64_t* src_local, int64_t* dst_local,
+                                int64_t* edge_id, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Grouped per-node-type input projection (model/REGCN.py:36-39, model/REGAT.py:56-58, model/REMixHop.py:89-92:
  * `fc_list[t](features_list[t])` per type + torch.cat; mag/regnn_ns.py:300-326 `group_input`: per type a boolean mask,

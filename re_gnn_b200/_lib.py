@@ -50,6 +50,9 @@ SIGNATURES = {
                                   _p, _p, _p, _p, _p, _sz, _p]),
     'regnn_block_csr_build': (_i32, [_p, _p, _p, _p, _p, _i64, _i64, _i64, _p, _p, _i32, _i32, _i32, _p, _p, _p, _p, _p,
                                      _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    'regnn_induced_subgraph_workspace_bytes': (_sz, [_i64, _i64, _i64]),
+    'regnn_induced_subgraph_count': (_i32, [_p, _p, _i64, _i64, _p, _i64, _i32, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    'regnn_induced_subgraph_fill': (_i32, [_p, _p, _p, _i64, _i64, _i64, _p, _p, _i64, _i64, _p, _p, _p, _p, _sz, _p]),
     'regnn_gat_fwd': (_i32, [_p, _p, _p, _p, _p, _f32, _i32, _p, _p, _p, _f32, _p, _p, _i32, _i32, _i64, _i64,
                              _p, _p, _p, _p, _p, _p, _p, _p]),
     'regnn_gat_bwd_stats': (_i32, [_p, _p, _p, _p, _p, _i64, _i32, _i32, _p, _p]),

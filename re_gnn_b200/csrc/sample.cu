@@ -335,3 +335,241 @@ extern "C" int regnn_block_csr_build(const int64_t* src_local, const int64_t* ds
   if (rc != REGNN_OK || counts == nullptr) return rc;
   return regnn_relation_counts(row, et_csr, num_edges, num_src, num_relations, counts, stream);
 }
+
+// ---- GraphSAINT induced subgraph (mag/regnn_saint.py:185-190: GraphSAINTRandomWalkSampler) ----------------------
+// The subgraph of the walk nodes: its nodes are the distinct listed nodes in ascending global id (torch.unique's
+// order), its edges every in-edge of those rows whose source is listed too, in (row, CSR slot) order -- which is the
+// subgraph's in-CSR already.  Listed nodes raise a flag in a persistent [N] map; an exclusive scan of the flags over
+// all N gives node v its row excl[v].  Each row's slot range is cut into fragments of at most kInducedFragSlots slots
+// (MAG hub rows have 10^4-10^5 in-edges, and walks reach a row in proportion to its in-degree), one warp per
+// fragment: warp ballots count the kept slots, a scan of the fragment counts gives every fragment its output offset,
+// and the fill replays the ballots to write each kept slot at that offset plus its rank.  Stores of equal values,
+// integer counters and scans only: the result does not depend on the order in which threads run.
+namespace regnn {
+
+constexpr int kInducedFragSlots = 256;
+
+static int64_t induced_frag_capacity(int64_t num_edges, int64_t max_rows) {
+  return max_rows + (num_edges + kInducedFragSlots - 1) / kInducedFragSlots;   // sum of max(1, ceil(deg / 256))
+}
+
+struct InducedWorkspace {
+  uint32_t* excl;         // [num_nodes] exclusive scan of the flags: the row of a listed node
+  uint32_t* frag_first;   // [max_rows + 1] first fragment of each row (scan of the per-row fragment counts)
+  uint32_t* frag_row;     // [frag_cap] row of each fragment
+  uint32_t* frag_off;     // [frag_cap + 1] output offset of each fragment (scan of the kept-slot counts)
+  uint32_t* block_sums;   // scan spine
+};
+
+static size_t induced_workspace_layout(int64_t num_nodes, int64_t num_edges, int64_t max_rows, char* base,
+                                       InducedWorkspace* ws) {
+  const int64_t cap = induced_frag_capacity(num_edges, max_rows);
+  int64_t longest = num_nodes > cap + 1 ? num_nodes : cap + 1;
+  if (max_rows + 1 > longest) longest = max_rows + 1;
+  const size_t sizes[5] = {align256((size_t)(num_nodes > 0 ? num_nodes : 1) * 4), align256((size_t)(max_rows + 1) * 4),
+                           align256((size_t)(cap > 0 ? cap : 1) * 4), align256((size_t)(cap + 1) * 4),
+                           align256((size_t)scan_blocks(longest) * 4)};
+  uint32_t** parts[5] = {&ws->excl, &ws->frag_first, &ws->frag_row, &ws->frag_off, &ws->block_sums};
+  size_t off = 0;
+  for (int i = 0; i < 5; ++i) {
+    if (base) *parts[i] = (uint32_t*)(base + off);
+    off += sizes[i];
+  }
+  return off;
+}
+
+__global__ void induced_flag_kernel(const int64_t* __restrict__ nodes, int64_t num_listed, int64_t num_nodes,
+                                    uint32_t* __restrict__ flags) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= num_listed) return;
+  const int64_t v = nodes[i];
+  if (v >= 0 && v < num_nodes) flags[v] = 1u;
+}
+
+// One thread per node: a listed node v stores itself at row excl[v] and the number of fragments of its slot range
+// (at least one, so that every row owns a fragment and row_off[r] is the offset of its first one).
+__global__ void induced_rows_kernel(const int32_t* __restrict__ indptr, int64_t num_nodes,
+                                    const uint32_t* __restrict__ flags, const uint32_t* __restrict__ excl,
+                                    int64_t* __restrict__ n_id, uint32_t* __restrict__ frag_count,
+                                    int32_t* __restrict__ info) {
+  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (v == 0) info[REGNN_SAMPLE_INFO_SOURCES] = (int32_t)(excl[num_nodes - 1] + flags[num_nodes - 1]);
+  if (v >= num_nodes || !flags[v]) return;
+  const uint32_t r = excl[v];
+  const int64_t deg = indptr[v + 1] - indptr[v];
+  n_id[r] = v;
+  frag_count[r] = deg > kInducedFragSlots ? (uint32_t)((deg + kInducedFragSlots - 1) / kInducedFragSlots) : 1u;
+}
+
+// One warp per fragment (frag_cap + 1 warps; those past the last fragment store a zero count for the scan).
+__global__ void induced_frag_count_kernel(const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                                          const uint32_t* __restrict__ flags, const uint32_t* __restrict__ excl,
+                                          const int64_t* __restrict__ n_id, const uint32_t* __restrict__ frag_first,
+                                          int64_t frag_cap, const int32_t* __restrict__ info,
+                                          uint32_t* __restrict__ frag_row, uint32_t* __restrict__ frag_count,
+                                          int32_t* __restrict__ src_hist) {
+  const int64_t f = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (f > frag_cap) return;
+  const int64_t n_sub = info[REGNN_SAMPLE_INFO_SOURCES];
+  if (f >= (int64_t)frag_first[n_sub]) {
+    if (lane == 0) frag_count[f] = 0u;
+    return;
+  }
+  int64_t lo = 0, hi = n_sub;                // the row r with frag_first[r] <= f < frag_first[r + 1]
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if ((int64_t)frag_first[mid] <= f) lo = mid;
+    else hi = mid;
+  }
+  const int64_t v = n_id[lo];
+  const int64_t s0 = indptr[v] + (f - (int64_t)frag_first[lo]) * kInducedFragSlots;
+  const int64_t s1 = min(s0 + kInducedFragSlots, (int64_t)indptr[v + 1]);
+  uint32_t kept = 0;
+  for (int64_t base = s0; base < s1; base += 32) {
+    const int64_t s = base + lane;
+    bool keep = false;
+    if (s < s1) {
+      const int32_t u = indices[s];
+      keep = flags[u] != 0u;
+      if (keep) atomicAdd(&src_hist[excl[u]], 1);
+    }
+    kept += __popc(__ballot_sync(0xffffffffu, keep));
+  }
+  if (lane == 0) {
+    frag_row[f] = (uint32_t)lo;
+    frag_count[f] = kept;
+  }
+}
+
+// One thread per row slot 0..max_rows: row_off from the fragment offsets, and the statistics of both views.
+__global__ void induced_rows_finish_kernel(int64_t max_rows, const uint32_t* __restrict__ frag_first,
+                                           const uint32_t* __restrict__ frag_off, const int32_t* __restrict__ src_hist,
+                                           int threshold, uint32_t* __restrict__ row_off, int32_t* __restrict__ info) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r > max_rows) return;
+  const int64_t n_sub = info[REGNN_SAMPLE_INFO_SOURCES];
+  const uint32_t e0 = frag_off[frag_first[r < n_sub ? r : n_sub]];
+  row_off[r] = e0;
+  if (r == n_sub) info[REGNN_SAMPLE_INFO_EDGES] = (int32_t)e0;
+  if (r >= n_sub) return;
+  const int64_t deg = (int64_t)frag_off[frag_first[r + 1]] - e0;
+  if (deg == 0) atomicAdd(&info[REGNN_SAMPLE_INFO_EMPTY_ROWS], 1);
+  count_long_row(deg, threshold, info + REGNN_SAMPLE_INFO_IN_SPLIT);
+  count_long_row(src_hist[r], threshold, info + REGNN_SAMPLE_INFO_OUT_SPLIT);
+}
+
+// The count kernel's ballots again, each kept slot written at its fragment's offset plus its rank in the fragment.
+__global__ void induced_fill_kernel(const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                                    const int32_t* __restrict__ eid, const uint32_t* __restrict__ flags,
+                                    const uint32_t* __restrict__ excl, const int64_t* __restrict__ n_id,
+                                    int64_t num_rows, int64_t num_sub_edges, const uint32_t* __restrict__ frag_first,
+                                    const uint32_t* __restrict__ frag_row, const uint32_t* __restrict__ frag_off,
+                                    int64_t* __restrict__ src_local, int64_t* __restrict__ dst_local,
+                                    int64_t* __restrict__ edge_id) {
+  const int64_t f = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (f >= (int64_t)frag_first[num_rows]) return;
+  const uint32_t r = frag_row[f];
+  const int64_t v = n_id[r];
+  const int64_t s0 = indptr[v] + (f - (int64_t)frag_first[r]) * kInducedFragSlots;
+  const int64_t s1 = min(s0 + kInducedFragSlots, (int64_t)indptr[v + 1]);
+  int64_t out = frag_off[f];
+  for (int64_t base = s0; base < s1; base += 32) {
+    const int64_t s = base + lane;
+    int32_t u = 0;
+    bool keep = false;
+    if (s < s1) {
+      u = indices[s];
+      keep = flags[u] != 0u;
+    }
+    const uint32_t ballot = __ballot_sync(0xffffffffu, keep);
+    const int64_t e = out + __popc(ballot & ((1u << lane) - 1u));
+    if (keep && e < num_sub_edges) {
+      src_local[e] = excl[u];
+      dst_local[e] = r;
+      edge_id[e] = eid[s];
+    }
+    out += __popc(ballot);
+  }
+}
+
+__global__ void induced_clear_flags_kernel(const int64_t* __restrict__ n_id, int64_t num_rows,
+                                           uint32_t* __restrict__ flags) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < num_rows) flags[n_id[r]] = 0u;
+}
+
+static unsigned warp_grid_of(int64_t warps) { return grid_of(warps * 32); }
+
+}  // namespace regnn
+
+extern "C" size_t regnn_induced_subgraph_workspace_bytes(int64_t num_nodes, int64_t num_edges, int64_t num_listed) {
+  InducedWorkspace ws;
+  const int64_t max_rows = num_listed < num_nodes ? num_listed : num_nodes;
+  return induced_workspace_layout(num_nodes, num_edges, max_rows < 0 ? 0 : max_rows, nullptr, &ws);
+}
+
+extern "C" int regnn_induced_subgraph_count(const int32_t* indptr, const int32_t* indices, int64_t num_nodes,
+                                            int64_t num_edges, const int64_t* nodes, int64_t num_listed,
+                                            int split_threshold, uint32_t* flags, int64_t* n_id, uint32_t* row_off,
+                                            int32_t* src_hist, int32_t* info, void* workspace, size_t workspace_bytes,
+                                            void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  REGNN_REQUIRE(indptr && flags && n_id && row_off && src_hist && info && workspace && (num_listed == 0 || nodes) &&
+                (num_edges == 0 || indices), REGNN_ERR_INVALID_ARG, "induced_subgraph_count: null pointer");
+  REGNN_REQUIRE(num_nodes >= 1 && num_listed >= 0 && num_edges >= 0 && split_threshold >= 1, REGNN_ERR_INVALID_ARG,
+                "induced_subgraph_count: bad sizes");
+  REGNN_REQUIRE(num_nodes < ((int64_t)1 << 31) - 1 && num_edges < ((int64_t)1 << 31) - 1, REGNN_ERR_UNSUPPORTED_SHAPE,
+                "induced_subgraph_count: %lld nodes / %lld edges exceed int32 indexing", (long long)num_nodes,
+                (long long)num_edges);
+  REGNN_REQUIRE(workspace_bytes >= regnn_induced_subgraph_workspace_bytes(num_nodes, num_edges, num_listed),
+                REGNN_ERR_WORKSPACE_TOO_SMALL, "induced_subgraph workspace too small");
+  const int64_t max_rows = num_listed < num_nodes ? num_listed : num_nodes;
+  const int64_t cap = induced_frag_capacity(num_edges, max_rows);
+  InducedWorkspace ws;
+  induced_workspace_layout(num_nodes, num_edges, max_rows, (char*)workspace, &ws);
+
+  cudaMemsetAsync(info, 0, REGNN_SAMPLE_INFO_WORDS * sizeof(int32_t), stream);
+  cudaMemsetAsync(src_hist, 0, (size_t)(max_rows > 0 ? max_rows : 1) * sizeof(int32_t), stream);
+  cudaMemsetAsync(ws.frag_first, 0, (size_t)(max_rows + 1) * sizeof(uint32_t), stream);
+  induced_flag_kernel<<<grid_of(num_listed), 256, 0, stream>>>(nodes, num_listed, num_nodes, flags);
+  exclusive_scan_u32(flags, ws.excl, num_nodes, ws.block_sums, stream);
+  induced_rows_kernel<<<grid_of(num_nodes), 256, 0, stream>>>(indptr, num_nodes, flags, ws.excl, n_id, ws.frag_first,
+                                                              info);
+  exclusive_scan_u32(ws.frag_first, ws.frag_first, max_rows + 1, ws.block_sums, stream);
+  induced_frag_count_kernel<<<warp_grid_of(cap + 1), 256, 0, stream>>>(indptr, indices, flags, ws.excl, n_id,
+                                                                       ws.frag_first, cap, info, ws.frag_row,
+                                                                       ws.frag_off, src_hist);
+  exclusive_scan_u32(ws.frag_off, ws.frag_off, cap + 1, ws.block_sums, stream);
+  induced_rows_finish_kernel<<<grid_of(max_rows + 1), 256, 0, stream>>>(max_rows, ws.frag_first, ws.frag_off, src_hist,
+                                                                        split_threshold, row_off, info);
+  return check_launch("regnn_induced_subgraph_count");
+}
+
+extern "C" int regnn_induced_subgraph_fill(const int32_t* indptr, const int32_t* indices, const int32_t* eid,
+                                           int64_t num_nodes, int64_t num_edges, int64_t num_listed, uint32_t* flags,
+                                           const int64_t* n_id, int64_t num_rows, int64_t num_sub_edges,
+                                           int64_t* src_local, int64_t* dst_local, int64_t* edge_id, void* workspace,
+                                           size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const int64_t max_rows = num_listed < num_nodes ? num_listed : num_nodes;
+  REGNN_REQUIRE(indptr && flags && n_id && workspace && (num_edges == 0 || (indices && eid)) &&
+                (num_sub_edges == 0 || (src_local && dst_local && edge_id)), REGNN_ERR_INVALID_ARG,
+                "induced_subgraph_fill: null pointer");
+  REGNN_REQUIRE(num_nodes >= 1 && num_edges >= 0 && num_listed >= 0 && num_rows >= 0 && num_rows <= max_rows &&
+                num_sub_edges >= 0 && num_sub_edges <= num_edges, REGNN_ERR_INVALID_ARG,
+                "induced_subgraph_fill: bad sizes");
+  REGNN_REQUIRE(num_nodes < ((int64_t)1 << 31) - 1 && num_edges < ((int64_t)1 << 31) - 1, REGNN_ERR_UNSUPPORTED_SHAPE,
+                "induced_subgraph_fill: %lld nodes / %lld edges exceed int32 indexing", (long long)num_nodes,
+                (long long)num_edges);
+  REGNN_REQUIRE(workspace_bytes >= regnn_induced_subgraph_workspace_bytes(num_nodes, num_edges, num_listed),
+                REGNN_ERR_WORKSPACE_TOO_SMALL, "induced_subgraph workspace too small");
+  InducedWorkspace ws;
+  induced_workspace_layout(num_nodes, num_edges, max_rows, (char*)workspace, &ws);
+  induced_fill_kernel<<<warp_grid_of(induced_frag_capacity(num_edges, max_rows)), 256, 0, stream>>>(
+      indptr, indices, eid, flags, ws.excl, n_id, num_rows, num_sub_edges, ws.frag_first, ws.frag_row, ws.frag_off,
+      src_local, dst_local, edge_id);
+  induced_clear_flags_kernel<<<grid_of(num_rows), 256, 0, stream>>>(n_id, num_rows, flags);
+  return check_launch("regnn_induced_subgraph_fill");
+}

@@ -358,14 +358,19 @@ class SaintREGCNConv(nn.Module):
         nn.init.zeros_(self.bias)
         nn.init.constant_(self.relation_weight, 1.0 / self.scaling_factor)
 
-    def forward(self, x, edge_index, edge_type, return_weights=False, graph=None, edge_keep=None):
-        """``edge_keep`` (optional bool [E]): the dropout mask to use instead of drawing one (tests)."""
+    def forward(self, x, edge_index, edge_type, return_weights=False, graph=None, edge_keep=None, block=None):
+        """``edge_keep`` (optional bool [E]): the dropout mask to use instead of drawing one (tests).  ``block``: the
+        subgraph's ``(Graph, etype1)`` from ``Block.prebuilt`` (``edge_index`` is then not read); its edge-type views are
+        already cached for ``etype1``.  ``edge_type`` stays the 0-based type of every edge."""
         x_src, x_target = x if isinstance(x, tuple) else (x, x)
         n_src, n_dst = x_src.shape[0], x_target.shape[0]
+        etype1 = None
+        if block is not None:
+            graph, etype1 = block
         if graph is None:
             graph = Graph(edge_index[0], edge_index[1], n_src)
         r = self.num_edge_types
-        etv = graph.etype_views(edge_type + 1, r)
+        etv = graph.etype_views(edge_type + 1 if etype1 is None else etype1, r)
         theta, alpha = self.relation_weight.view(-1, 1), self.scaling_factor
         if self.use_softmax:
             w = F.leaky_relu(theta * alpha)                                   # [R,1]: differentiable, R floats
@@ -422,12 +427,16 @@ class SaintREGCN(nn.Module):
             node_type, local_node_idx = node_type[n_id], local_node_idx[n_id]
         return _grouped_input(self.lins, x_dict, node_type, local_node_idx)
 
-    def forward(self, x_dict, edge_index, edge_type, node_type, local_node_idx):
+    def forward(self, x_dict, edge_index, edge_type, node_type, local_node_idx, block=None):
+        """``block``: the subgraph's prebuilt ``(Graph, etype1)`` (``Block.prebuilt``), shared by every layer; without it
+        the layers share one ``Graph`` built from ``edge_index``."""
         x = self.group_input(x_dict, node_type, local_node_idx)
-        graph = Graph(edge_index[0], edge_index[1], x.shape[0])     # one CSR for all layers of this subgraph
+        graph = None
+        if block is None:
+            graph = Graph(edge_index[0], edge_index[1], x.shape[0])     # one CSR for all layers of this subgraph
         for layer, conv in enumerate(self.convs):
             x_pre = x
-            x = conv(x, edge_index, edge_type, graph=graph)
+            x = conv(x, edge_index, edge_type, graph=graph, block=block)
             if layer != self.num_layers - 1:
                 if self.residual:
                     x = x + x_pre
@@ -440,13 +449,20 @@ class SaintREGCN(nn.Module):
 def saint_train_step(model, optimizer, sampler, labels, train_mask, x_dict, edge_type, node_type, local_node_idx,
                      epoch, batch, world_size=1):
     """One GraphSAINT training step (mag/regnn_saint.py:427-443 + gradient all-reduce): loss on the training nodes
-    of the sampled subgraph.  Returns (loss, number of subgraph edges)."""
-    n_id, edge_index, eid = sampler.sample(epoch=epoch, batch=batch)
+    of the sampled subgraph.  On a CUDA device the subgraph reaches the layers with its graph prebuilt from the sample
+    (``sample_block`` + ``Block.prebuilt``, no self loops).  Returns (loss, number of subgraph edges)."""
+    if sampler.graph.device.type == 'cuda':
+        n_id, block = sampler.sample_block(epoch=epoch, batch=batch)
+        prebuilt = block.prebuilt(edge_type, node_type, model.num_edge_types, 1, model.num_edge_types)
+        edge_index, eid, num_edges = None, block.eid, block.src.numel()
+    else:
+        n_id, edge_index, eid = sampler.sample(epoch=epoch, batch=batch)
+        prebuilt, num_edges = None, edge_index.shape[1]
     optimizer.zero_grad(set_to_none=True)
-    out = model(x_dict, edge_index, edge_type[eid], node_type[n_id], local_node_idx[n_id])
+    out = model(x_dict, edge_index, edge_type[eid], node_type[n_id], local_node_idx[n_id], block=prebuilt)
     mask = train_mask[n_id]
     loss = F.nll_loss(out[mask], labels[n_id][mask])
     loss.backward()
     allreduce_gradients(list(model.parameters()), world_size)
     optimizer.step()
-    return loss.detach(), int(edge_index.shape[1])
+    return loss.detach(), int(num_edges)

@@ -10,7 +10,8 @@ of (seed, epoch, rank, batch index), so data-parallel ranks draw independent bat
 Sampling, relabelling and edge compaction of every layer run on the device (``regnn_sample_layer``) with the
 frontier sizes kept there; the host reads them all in ONE small copy per batch.  Each block can then build its
 CSR views on the device without another synchronisation (``Block.prebuilt``), so a training step does not
-rebuild them from the edge list.
+rebuild them from the edge list.  The GraphSAINT sampler hands its induced subgraph over the same way
+(``regnn_induced_subgraph_count`` / ``_fill``, one host read per batch).
 """
 import ctypes
 
@@ -44,7 +45,7 @@ class Block:
 
     def __init__(self, src_local, dst_local, eid, n_src, n_dst):
         self.src, self.dst, self.eid, self.n_src, self.n_dst = src_local, dst_local, eid, int(n_src), int(n_dst)
-        self._sample = None     # (targets, row_off, info) of regnn_sample_layer for blocks sampled on the device
+        self._sample = None     # (targets, row_off, info, status) of blocks sampled on the device
 
     @property
     def edge_index(self):
@@ -60,7 +61,7 @@ class Block:
         every structure the convolutions read already in place: both CSR views, both row splits and the edge-type
         views for ``num_relations`` relations.  No host synchronisation.  ``edge_type`` / ``node_type``: 0-based
         types of the full graph's edges and nodes.  A type outside [0, num_relations) cannot be reported without a
-        synchronisation: the block's edge is typed 0 and the sampler's next ``sample`` raises."""
+        synchronisation: the block's edge is typed 0 and the sampler's next batch raises."""
         if self._sample is None:
             raise RuntimeError('Block.prebuilt needs a block sampled on a CUDA device')
         targets, row_off, info, status = self._sample
@@ -101,6 +102,8 @@ _INFO_SOURCES, _INFO_EDGES, _INFO_EMPTY_ROWS = 0, 1, 2
 _INFO_IN_SPLIT, _INFO_IN_SPLIT_LOOPS, _INFO_OUT_SPLIT, _INFO_OUT_SPLIT_LOOPS = 3, 5, 7, 9
 _INFO_WORDS = 16
 _SAMPLE_LAYER_LAUNCHES = 12     # 2 memsets, 4 kernels, 2 three-kernel scans
+_INDUCED_COUNT_LAUNCHES = 16    # 3 memsets, 4 kernels, 3 three-kernel scans
+_INDUCED_FILL_LAUNCHES = 2      # fill, flag reset
 
 
 def _block_build_launches(n, e, counts):
@@ -225,11 +228,17 @@ class SaintRandomWalkSampler:
     """GraphSAINT random-walk sampler (``GraphSAINTRandomWalkSampler(data, batch_size=roots, walk_length=...)``,
     mag/regnn_saint.py:185-190; ``sample_coverage=0`` so no normalisation statistics): ``roots`` random start
     nodes, ``walk_length`` steps along out-edges (``regnn_random_walk``), then the subgraph INDUCED by the visited
-    nodes.  Returns ``(n_id, edge_index_local [2,E'], eid)`` with ``n_id`` sorted ascending."""
+    nodes.  On a CUDA device the subgraph is extracted, relabelled and handed over as a ``Block`` whose CSR views
+    ``Block.prebuilt`` builds without rebuilding them from the edge list (``regnn_induced_subgraph_count`` / ``_fill``),
+    with one host synchronisation per batch."""
 
     def __init__(self, graph: Graph, roots, walk_length, seed=0, rank=0):
         self.graph, self.roots, self.walk_length = graph, int(roots), int(walk_length)
         self.seed, self.rank = int(seed), int(rank)
+        # (flags, status, workspace) on the device: the [N] flag map of regnn_induced_subgraph_count, which the fill
+        # leaves as it found it, the type-check word of Block.prebuilt, and the workspace the two calls of a batch share.
+        # Shared by all batches, so one sampler samples on one stream at a time.
+        self._maps = None
 
     def walks(self, key):
         csr = self.graph.csr()
@@ -243,11 +252,78 @@ class SaintRandomWalkSampler:
             _lib.count_launches(1)
         return out
 
+    def _key(self, epoch, batch):
+        return layer_key(self.seed, epoch, self.rank, batch, 0x5A1)
+
     def sample(self, epoch=0, batch=0):
+        """-> (n_id sorted ascending, edge_index_local [2, E'], eid): the edges are every in-edge of a subgraph node
+        whose source is in the subgraph too, ordered by (destination, CSR slot).  Built from ``sample_block`` on a CUDA
+        device."""
+        if not self.graph.csr()['indptr'].is_cuda:
+            return self.reference_sample(epoch, batch)
+        n_id, block = self.sample_block(epoch, batch)
+        return n_id, block.edge_index, block.eid
+
+    def sample_block(self, epoch=0, batch=0):
+        """-> (n_id, Block) of the batch: ``Block(src_local, dst_local, eid, n_sub, n_sub)`` over the ``sample`` edges.
+        The host waits for the device once, for the subgraph's sizes; an out-of-range type given to ``Block.prebuilt``
+        of an earlier batch is raised here."""
+        return self.induced_block(self.walks(self._key(epoch, batch)).view(-1))
+
+    def induced_block(self, nodes):
+        """(n_id, Block) of the subgraph induced by ``nodes`` (int64 CUDA tensor of node ids, repeats allowed).  If a
+        call fails part-way, the flag map is dropped and rebuilt by the next call."""
+        csr = self.graph.csr()
+        n, e = self.graph.number_of_nodes(), self.graph.number_of_edges()
+        nodes = nodes.to(torch.int64).contiguous()
+        dev, listed = nodes.device, nodes.numel()
+        rows = min(n, listed)
+        ws_bytes = _lib.load().regnn_induced_subgraph_workspace_bytes(n, e, listed)
+        i32, i64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.int64, device=dev)
+        with torch.cuda.device(dev):
+            if self._maps is None:
+                self._maps = (torch.zeros(n, **i32), torch.zeros(1, **i32), torch.empty(0, dtype=torch.uint8, device=dev))
+            flags, status, ws = self._maps
+            if ws.numel() < ws_bytes:
+                ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+                self._maps = (flags, status, ws)
+            n_id, hist = torch.empty(max(rows, 1), **i64), torch.empty(max(rows, 1), **i32)
+            row_off = torch.empty(rows + 1, **i32)
+            info = torch.empty((2, _INFO_WORDS), **i32)
+            try:
+                _lib.call('regnn_induced_subgraph_count', _ptr(csr['indptr']), _ptr(csr['indices']), n, e, _ptr(nodes),
+                          listed, SPLIT_THRESHOLD, _ptr(flags), _ptr(n_id), _ptr(row_off), _ptr(hist), _ptr(info[0]),
+                          _ptr(ws), ws_bytes, _stream())
+                _lib.count_launches(_INDUCED_COUNT_LAUNCHES)
+                info[1, :1].copy_(status)
+                sizes, checked = info.cpu().tolist()     # the one host synchronisation of the batch
+                n_sub, e_sub = sizes[_INFO_SOURCES], sizes[_INFO_EDGES]
+                src_local, dst_local, eid = (torch.empty(max(e_sub, 1), **i64)[:e_sub] for _ in range(3))
+                _lib.call('regnn_induced_subgraph_fill', _ptr(csr['indptr']), _ptr(csr['indices']), _ptr(csr['eid']), n,
+                          e, listed, _ptr(flags), _ptr(n_id), n_sub, e_sub, _ptr(src_local), _ptr(dst_local), _ptr(eid),
+                          _ptr(ws), ws_bytes, _stream())
+                _lib.count_launches(_INDUCED_FILL_LAUNCHES)
+            except BaseException:
+                self._maps = None       # the count may have left flags set
+                raise
+        if checked[0]:
+            status.zero_()
+            raise RuntimeError('Block.prebuilt of an earlier batch of this sampler was given an edge type outside '
+                               '[0, num_relations): its block typed those edges 0')
+        b = Block(src_local, dst_local, eid, n_sub, n_sub)
+        b._sample = (n_id[:n_sub], row_off[:n_sub + 1], sizes, status)
+        return n_id[:n_sub], b
+
+    def reference_sample(self, epoch=0, batch=0):
+        """The same batch with torch ops (``torch.unique`` over the walk nodes, a ``.item()`` for the candidate slot
+        count and a boolean mask over the candidate edges, each waiting for the device): ``sample``'s path for CPU
+        tensors, which only the CPU emulation of the operators produces (the library has no CPU path), and the
+        reference the device path is checked and timed against (tests/test_saint_subgraph_gpu.py,
+        scripts/check_saint_step.py)."""
         csr = self.graph.csr()
         n = self.graph.number_of_nodes()
         dev = csr['indptr'].device
-        n_id = torch.unique(self.walks(layer_key(self.seed, epoch, self.rank, batch, 0x5A1)).view(-1))
+        n_id = torch.unique(self.walks(self._key(epoch, batch)).view(-1))
         relabel = torch.full((n,), -1, dtype=torch.int64, device=dev)
         relabel[n_id] = torch.arange(n_id.numel(), device=dev)
         indptr = csr['indptr'].to(torch.int64)
